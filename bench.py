@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 metric   Mrays/s (primary + shadow + reflection rays, also reported by kind) and ms/frame
 workload configs[2]: dragon-class scene (procedural 868 352-triangle stand-in for the missing dragon.ply,
@@ -15,6 +15,8 @@ N > 1    one process per GPU (torchrun), scene replicated; all GPUs render the s
          into GPU 0's framebuffer (peer stores); strong scaling of the same frame
 --impl reference   the reference's own boss/worker CPU renderer (oracle/_ref/ct_ref, compiled from the unmodified
          sources) on this box's host cores, same scene files, same metric.
+--dump-outputs DIR the frame the last timed step rendered, as DIR/frame.npy (see dump_frame), so that two builds can be
+         compared pixel for pixel on the same inputs.
 """
 from __future__ import annotations
 
@@ -180,6 +182,22 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": float(np.median(self.mhz)), "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.mhz)}
 
 
+DUMP_SAMPLE_PX = 1 << 22        # frames larger than 64 MB as float32 (dragon8k) are dumped as this many sampled pixels
+
+
+def dump_frame(out_dir: str, frame: np.ndarray) -> None:
+    """frame.npy: the read-back bitmap as float32 (its 0x00RRGGBB words are below 2^24, so the conversion is exact).
+    Above 64 MB, a fixed sample of DUMP_SAMPLE_PX pixels (seed 0, in raster order) and their flat indices in
+    frame_index.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    vals = frame.astype(np.float32)
+    if vals.nbytes > 64 << 20:
+        idx = np.sort(np.random.default_rng(0).choice(frame.size, DUMP_SAMPLE_PX, replace=False))
+        np.save(os.path.join(out_dir, "frame_index.npy"), idx.astype(np.float64))
+        vals = vals.reshape(-1)[idx]
+    np.save(os.path.join(out_dir, "frame.npy"), vals)
+
+
 def physical_gpu_index(local_rank: int) -> int:
     vis = os.environ.get("CUDA_VISIBLE_DEVICES")
     if vis:
@@ -334,7 +352,10 @@ def main():
     ap.add_argument("--workload", default="dragon4k", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--tile-rows", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR/frame.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
     # stdout carries exactly one line, the JSON (NCCL / torchrun banners go to stderr with everything else)
@@ -478,6 +499,8 @@ def main():
     if N > 1:
         dist.barrier()
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:
+        dump_frame(args.dump_outputs, gpu.readback())          # GPU 0's framebuffer as the last timed step left it
     # end-to-end: host camera in, host bitmap out, wall clock -- one frame at a time (latency) ...
     for _ in range(2):
         frame(True)

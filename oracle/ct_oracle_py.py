@@ -14,6 +14,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "_build", "libct_oracle.so")
 REF_DIR = os.path.join(HERE, "_ref")
+# The reference's own sources (a checkout of jeng/CobbleTrace), which this repository does not carry: oracle/Makefile
+# compiles them into REF_DIR when CT_REFERENCE_SRC names them.
+REF_SRC = os.environ.get("CT_REFERENCE_SRC", "")
 
 
 class _Scene(C.Structure):

@@ -13,7 +13,7 @@ from oracle import ct_oracle_py as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/ct_ref not built (needs /root/reference once)")
+@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/ct_ref not built (needs the reference's sources once: CT_REFERENCE_SRC)")
 def test_reference_arm_prints_one_json_line():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "cube640", "--steps", "2", "--warmup", "1"],
                        capture_output=True, text=True, timeout=600, cwd=ROOT)

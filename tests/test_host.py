@@ -12,7 +12,7 @@ from oracle import ct_oracle_py as O
 
 SCENES = ["scene_file_cube", "scene_import", "pc_big", "scene_import_bunny"]
 REF_SCENES = os.path.join(O.REF_DIR, "scenes")
-need_ref = pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
+need_ref = pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built (needs the reference's sources: CT_REFERENCE_SRC)")
 
 
 @pytest.mark.parametrize("name", SCENES)

@@ -1,5 +1,5 @@
 """Live cross-check: the plain-C restatement against the compiled, unmodified reference (oracle/_ref).
-Skipped where /root/reference was not available at build time; the committed goldens cover that case."""
+Skipped where the reference's sources (CT_REFERENCE_SRC) were not available at build time; the committed goldens cover that case."""
 import os
 
 import numpy as np
@@ -8,7 +8,7 @@ import pytest
 import cobbletrace_b200 as ct
 from oracle import ct_oracle_py as O
 
-pytestmark = pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built (needs the reference's sources: CT_REFERENCE_SRC)")
 SCENES = os.path.join(O.REF_DIR, "scenes")
 
 
