@@ -24,7 +24,7 @@ REFERENCE_MAX_DEPTH = 10   # raythread.cpp:508
 ABI_SYMBOLS = [
     "ct_gpu_abi_version", "ct_gpu_device_count", "ct_gpu_last_error", "ct_gpu_upload_scene", "ct_gpu_set_camera",
     "ct_gpu_set_stream", "ct_gpu_render_tile", "ct_gpu_readback", "ct_gpu_readback_async", "ct_gpu_readback_wait", "ct_gpu_readback_hits", "ct_gpu_get_counters",
-    "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest",
+    "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
 ]
 
@@ -109,6 +109,7 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_framebuffer.argtypes = [C.c_int, C.POINTER(vp), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     L.ct_gpu_gather_rows.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int]
     L.ct_gpu_debug_closest.argtypes = [C.c_int, C.c_uint32, vp, vp, vp, vp, vp, vp]
+    L.ct_gpu_debug_early.argtypes = [C.c_int, C.c_int, C.c_uint32, vp, vp, vp, vp, vp]
     L.ct_gpu_debug_primitives.argtypes = [C.c_int, C.c_uint32, vp, vp, vp, vp, vp, vp, vp, vp]
     L.ct_gpu_debug_filter.argtypes = [C.c_int, C.c_uint32, vp, vp, vp, vp, vp, vp, C.c_double, vp]
     L.ct_gpu_filter_stats.argtypes = [C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
@@ -306,6 +307,15 @@ class GpuRenderer:
         found = np.zeros(n, np.uint32); index = np.zeros(n, np.uint32); t = np.zeros(n, np.float32)
         _check(self.L, self.L.ct_gpu_debug_closest(self.device, n, _ptr(o), _ptr(d), _ptr(t0), _ptr(found), _ptr(index), _ptr(t)))
         return found, index, t
+
+    def debug_early(self, origins, directions, mode):
+        """ct_gpu_debug_early: mode 0 = shadow rays (found = occluded), 1 = reflection rays (index = first pass in DFS order).
+        Returns (found, index, path) with path 0 own walk, 1 k_overflow, 2 k_overflow_huge, 3 finished in place."""
+        o = np.ascontiguousarray(origins, np.float64).reshape(-1, 3); d = np.ascontiguousarray(directions, np.float64).reshape(-1, 3)
+        n = o.shape[0]
+        found = np.zeros(n, np.uint32); index = np.zeros(n, np.uint32); path = np.zeros(n, np.uint32)
+        _check(self.L, self.L.ct_gpu_debug_early(self.device, int(mode), n, _ptr(o), _ptr(d), _ptr(found), _ptr(index), _ptr(path)))
+        return found, index, path
 
     def debug_primitives(self, origins, directions, ray_t, tri, bmin, bmax):
         o = np.ascontiguousarray(origins, np.float64).reshape(-1, 3); d = np.ascontiguousarray(directions, np.float64).reshape(-1, 3)

@@ -83,6 +83,10 @@ struct DeviceState {
     const char *stage_name[kMaxLaunches] = {};
     int stage_depth[kMaxLaunches] = {};
     bool can_overflow = false;       // some traversal could exceed the visit budget: k_overflow launches are needed
+    // leaf positions increase along the reference's DFS (bvh_depth).  The parked first-line passes (k_overflow<kFirstLine>,
+    // k_overflow_huge) and k_primary_split's replay take the lowest position for the DFS-first one; on a tree without this
+    // property reflection rays are never parked and parked primary rays go to k_primary_long (first_line_budget, render_impl)
+    bool leaf_dfs_order = true;
     // per-depth path state (render_impl hands each launch a Params view of its depth, so that the shadow / shade
     // chain of one depth can run on its own stream next to the bounce chain of the next)
     float *hitb_t_all = nullptr; uint32_t *hitb_pos_all = nullptr;      // [depth][cap]
@@ -200,15 +204,19 @@ int dev_alloc(DeviceState &s, T **out, size_t count, bool zero = false) {
 
 
 // depth of the reference's DFS (stack entries needed) -- iterative to survive degenerate trees.  Also marks the nodes the
-// DFS reaches (array slots nobody points at may hold anything) and rejects leaves whose triangle ranges overlap.
-int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *ok, std::vector<uint8_t> &reachable) {
+// DFS reaches (array slots nobody points at may hold anything) and rejects leaves whose triangle ranges overlap.  The walk visits
+// the nodes in the reference's order (left child, then left + 1) and reports in *dfs_order whether the leaves' triangle ranges
+// come in increasing position along it -- true of every tree BuildBVH makes (bvh.cpp:70-97), not of every tree a caller may pass.
+int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *ok, bool *dfs_order, std::vector<uint8_t> &reachable) {
     std::vector<std::pair<uint32_t, int>> st;
     std::vector<uint8_t> covered(n_tri, 0);
     reachable.assign(n_nodes, 0);
     st.push_back({0u, 1});
     int best = 0;
     size_t visited = 0;
+    uint64_t next_first = 0;                    // leaf ranges seen so far end below this position
     *ok = true;
+    *dfs_order = true;
     while (!st.empty()) {
         auto [i, d] = st.back();
         st.pop_back();
@@ -218,10 +226,12 @@ int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *
         const ct_bvh_node &nd = nodes[i];
         if (nd.triangle_count == 0) {
             if ((uint64_t)nd.left_node + 1u >= n_nodes || nd.left_node == 0u) { *ok = false; return 0; }
-            st.push_back({nd.left_node, d + 1});
             st.push_back({nd.left_node + 1, d + 1});
+            st.push_back({nd.left_node, d + 1});                                  // popped first: the reference's order
         } else {
             if ((uint64_t)nd.first_triangle_index + nd.triangle_count > n_tri) { *ok = false; return 0; }
+            if (nd.first_triangle_index < next_first) *dfs_order = false;
+            next_first = (uint64_t)nd.first_triangle_index + nd.triangle_count;
             for (uint32_t k = 0; k < nd.triangle_count; k++) {
                 uint8_t &c = covered[nd.first_triangle_index + k];
                 if (c) { *ok = false; return 0; }                                  // two leaves hold the same position
@@ -233,6 +243,11 @@ int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *
 }
 
 int launch_grid(const DeviceState &s, int blocks_per_sm) { return s.n_sm * blocks_per_sm; }
+
+// The walk budget of the first-line (reflection) rays: unlimited -- never parked, the walk in the ray's own thread keeps the
+// reference's DFS order on any tree -- when leaf positions do not increase along the DFS (DeviceState::leaf_dfs_order).  The cost
+// on such a tree: a reflection ray cast from a shading point 2^32 ray lengths away walks the whole tree in one thread.
+uint32_t first_line_budget(const DeviceState &s) { return s.leaf_dfs_order ? s.p.budget : 0xffffffffu; }
 
 // L2 residency of the walk's hot set.  The fp32 child pairs and fp32 triangles (76 MB for the dragon-class scene) are
 // read by every walk step, at random; everything else a frame touches (ray queues, hit records, occlusion masks, colour
@@ -302,9 +317,9 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     if (d->max_depth < 0 || d->max_depth > 15) return fail(CT_ERR_LIMIT, "max_depth %d outside 0..15", d->max_depth);
     if ((d->flags & CT_FLAG_SUPERSAMPLING) && (d->flags & CT_FLAG_KEEP_HITS))
         return fail(CT_ERR_INVALID, "CT_FLAG_SUPERSAMPLING cannot be combined with CT_FLAG_KEEP_HITS (a pixel has 16 primary rays)");
-    bool ok = true;
+    bool ok = true, dfs_order = true;
     std::vector<uint8_t> reachable;
-    int depth = bvh_depth(d->nodes, d->n_nodes, d->n_triangles, &ok, reachable);
+    int depth = bvh_depth(d->nodes, d->n_nodes, d->n_triangles, &ok, &dfs_order, reachable);
     if (!ok) return fail(CT_ERR_INVALID, "BVH is malformed (child or triangle range out of bounds, overlapping leaves, a cycle or a shared child)");
     if (depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", depth, kStackMax);
     TRY(check_device(device));
@@ -329,6 +344,7 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     s.p.warp_budget = g_warp_budget_option > 0 ? (uint32_t)std::min<long long>(g_warp_budget_option, 1ll << 30) : kWarpBudget;
     s.p.primary_budget = g_primary_budget_option < 0 ? 0u : g_primary_budget_option > 0 ? (uint32_t)std::min<long long>(g_primary_budget_option, 1ll << 30) : kDefaultPrimaryBudget;
     s.flags = d->flags;
+    s.leaf_dfs_order = dfs_order;
 
     const bool timing = getenv("CT_GPU_TIMING") != nullptr;
     auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
@@ -705,7 +721,7 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
         }
         TRY(mark("primary", 0));
         if (park_primary) {
-            if (g_primary_split) {
+            if (g_primary_split && s.leaf_dfs_order) {          // (its replay takes leaf positions for the reference's test order)
                 if (count) k_primary_split<true><<<s.n_sm * 4, kOvfThreads, 0, st>>>(v0);
                 else k_primary_split<false><<<s.n_sm * 4, kOvfThreads, 0, st>>>(v0);
                 TRY(mark("primary_split", 0));
@@ -721,6 +737,7 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
         const int ovf_b = 2 * d, ovf_s = 2 * d + 1;
         if (d > 0) {
             Params vb = v;
+            vb.budget = first_line_budget(s);
             if (s.can_overflow) { vb.ovf = s.ovf_all + (size_t)pk.ovf_cap * ovf_b; vb.ovf_huge = s.ovf_huge_all + (size_t)pk.ovf_cap * ovf_b; }
             if (count) k_bounce<true><<<grid, kBlockThreads, 0, st>>>(vb, d, work++, ovf_b);
             else k_bounce<false><<<grid, kBlockThreads, 0, st>>>(vb, d, work++, ovf_b);
@@ -1196,6 +1213,59 @@ int ct_gpu_debug_closest(int device, uint32_t n, const double *origins, const do
     if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
     if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
     if (tclosest) CUX(cudaMemcpy(tclosest, d_tc, 4ull * n, cudaMemcpyDeviceToHost));
+    cleanup();
+    return CT_OK;
+}
+
+int ct_gpu_debug_early(int device, int mode, uint32_t n, const double *origins, const double *directions,
+                       uint32_t *found, uint32_t *index, uint32_t *path) {
+    if (!origins || !directions) return fail(CT_ERR_INVALID, "NULL ray arrays");
+    if (mode != 0 && mode != 1) return fail(CT_ERR_INVALID, "mode must be 0 (shadow ray) or 1 (reflection ray)");
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    if (n == 0) return CT_OK;
+    double *d_o = nullptr, *d_d = nullptr; uint32_t *d_f = nullptr, *d_i = nullptr, *d_p = nullptr, *d_occ = nullptr, *d_hpos = nullptr, *d_huge = nullptr;
+    float *d_ht = nullptr; OvfRay *d_ovf = nullptr; DevSched *d_sched = nullptr; DevTotals *d_tot = nullptr;
+    int rc = CT_OK;
+    auto cleanup = [&]() { cudaFree(d_o); cudaFree(d_d); cudaFree(d_f); cudaFree(d_i); cudaFree(d_p); cudaFree(d_occ); cudaFree(d_hpos); cudaFree(d_huge);
+                           cudaFree(d_ht); cudaFree(d_ovf); cudaFree(d_sched); cudaFree(d_tot); };
+    CUX(cudaMalloc(&d_o, 24ull * n)); CUX(cudaMalloc(&d_d, 24ull * n));
+    CUX(cudaMalloc(&d_f, 4ull * n)); CUX(cudaMalloc(&d_i, 4ull * n)); CUX(cudaMalloc(&d_p, 4ull * n));
+    CUX(cudaMalloc(&d_occ, 4ull * n)); CUX(cudaMalloc(&d_hpos, 4ull * n)); CUX(cudaMalloc(&d_ht, 4ull * n));
+    CUX(cudaMalloc(&d_sched, sizeof(DevSched))); CUX(cudaMalloc(&d_tot, sizeof(DevTotals)));
+    CUX(cudaMemcpy(d_o, origins, 24ull * n, cudaMemcpyHostToDevice));
+    CUX(cudaMemcpy(d_d, directions, 24ull * n, cudaMemcpyHostToDevice));
+    CUX(cudaMemset(d_occ, 0, 4ull * n)); CUX(cudaMemset(d_f, 0, 4ull * n)); CUX(cudaMemset(d_i, 0, 4ull * n));
+    CUX(cudaMemset(d_sched, 0, sizeof(DevSched))); CUX(cudaMemset(d_tot, 0, sizeof(DevTotals)));
+    // the scene's Params with this call's parking buffers, as a frame's launches see theirs: one occlusion word per ray (bit 0), one
+    // hit record per ray; without k_overflow launches (can_overflow false) a ray over its budget is finished in place
+    Params v = s.p;
+    v.sched = d_sched; v.tot = d_tot; v.occ = d_occ; v.occ_words = 1; v.hitb_t = d_ht; v.hitb_pos = d_hpos;
+    if (mode == 1) v.budget = first_line_budget(s);
+    v.ovf = nullptr; v.ovf_huge = nullptr; v.ovf_cap = 0;
+    if (s.can_overflow) {
+        v.ovf_cap = std::min<uint32_t>(n, s.p.ovf_cap);
+        CUX(cudaMalloc(&d_ovf, sizeof(OvfRay) * (size_t)v.ovf_cap)); CUX(cudaMalloc(&d_huge, 4ull * v.ovf_cap));
+        v.ovf = d_ovf; v.ovf_huge = d_huge;
+    }
+    CUX(cudaStreamSynchronize(s.stream));
+    const uint32_t blocks = (n + kBlockThreads - 1) / kBlockThreads;
+    if (mode == 0) k_debug_early<kAnyHit><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_f, d_i, d_p);
+    else k_debug_early<kFirstLine><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_f, d_i, d_p);
+    CUX(cudaGetLastError());
+    if (s.can_overflow) {                                     // the grids render_impl launches them with
+        if (mode == 0) { k_overflow<kAnyHit, false><<<s.n_sm * 2, kOvfThreads, 0, s.stream>>>(v, 0); k_overflow_huge<kAnyHit, false><<<s.n_sm * 4, 256, 0, s.stream>>>(v, 0); }
+        else { k_overflow<kFirstLine, false><<<s.n_sm * 2, kOvfThreads, 0, s.stream>>>(v, 0); k_overflow_huge<kFirstLine, false><<<s.n_sm * 4, 256, 0, s.stream>>>(v, 0); }
+        CUX(cudaGetLastError());
+        k_debug_early_parked<<<(n + 255) / 256, 256, 0, s.stream>>>(v, mode, n, d_f, d_i, d_p);
+        CUX(cudaGetLastError());
+    }
+    CUX(cudaStreamSynchronize(s.stream));
+    if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
+    if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
+    if (path) CUX(cudaMemcpy(path, d_p, 4ull * n, cudaMemcpyDeviceToHost));
     cleanup();
     return CT_OK;
 }

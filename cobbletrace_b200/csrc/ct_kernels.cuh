@@ -168,6 +168,40 @@ CT_DEV bool park_ray(const Params &P, int ovf_idx, const double *r64, uint32_t t
     return true;
 }
 
+// The per-ray loop of the early-exit kernels (k_shadow, k_bounce, k_debug_early): the walk with the budget; a walk given up at the
+// budget is parked for k_overflow (target / bit: where k_overflow stores the answer), or -- parking buffer full -- walked again
+// right here without a budget.  A shadow ray whose origin lies so far outside the scene that every box passes (a shading point 2^32
+// ray lengths away, SURVEY 0.4) is parked at its first visit: no point in walking up to the budget first, k_overflow hands it
+// straight to k_overflow_huge.  WARP-LEVEL: every lane calls it.  Returns, for an active lane, how the ray was finished (kWalked,
+// kParked, kInPlace); finish(res, tc, pos) receives the answer of a walk that was not given up, over(parked) hears of one that was.
+enum { kWalked = 0, kParked = 1, kInPlace = 3 };
+template <TraverseMode MODE, bool COUNT, class Finish, class Over>
+CT_DEV int walk_or_park(const Params &P, const TRay &r, const double *r64, bool active, uint32_t budget, int ovf_idx, uint32_t target,
+                        uint32_t bit, uint32_t &n_parked, LocalCount &lc, uint32_t *sm, const DevWide *top, uint32_t n_top, Finish &&finish,
+                        Over &&over) {
+    if (MODE == kAnyHit && active && (double)r.om > 0x1p20 * fmax(fmax(P.bound[0], P.bound[1]), P.bound[2])) budget = 0u;
+    int how = kWalked;
+    while (true) {                                                      // warp-uniform: traverse_early is warp-synchronous
+        float tc; uint32_t pos;
+        const int res = traverse_early_any<MODE, COUNT>(P, r, active, budget, tc, pos, lc, sm, top, n_top);
+        bool again = false;
+        if (active) {
+            if (res == kTravOverBudget) {
+                n_parked++;
+                again = !park_ray(P, ovf_idx, r64, target, bit);        // parking buffer full: finish in place, no budget
+                budget = 0xffffffffu;
+                how = again ? kInPlace : kParked;
+                over(!again);
+            } else {
+                finish(res, tc, pos);
+            }
+        }
+        active = again;
+        if (!__any_sync(kFullMask, again)) break;
+    }
+    return how;
+}
+
 // Primary rays.  Persistent warps take chunks of 32 or 64 slots from the tile's cursor -- one counter for the whole
 // tile, which in a multi-GPU frame lives on the root GPU and is shared by all devices over NVLink (dynamic
 // stealing at chunk granularity, SURVEY 8e) -- and remember which chunks they took: the later stages of this
@@ -389,7 +423,8 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary_long(cons
 // four children conservatively against best + 2 sigma, tests accepted leaves on the spot (a barycentric pass within best + sigma
 // becomes a candidate once the exact test of its leaf's own box confirms that the reference can reach it) and hands accepted interior
 // children back; the warp-wide minimum of t is exchanged once per round.  Afterwards the lanes' candidates within sigma of the
-// minimum are gathered and lane 0 replays the reference's update rules over them in leaf order -- the argument is
+// minimum are gathered and lane 0 replays the reference's update rules over them in leaf order (= the reference's test order
+// where leaf positions increase along the DFS; render_impl sends the parked rays of other trees to k_primary_long) -- the argument is
 // traverse_wide_nearest's, the CPU prototype tests/test_free_closest_prototype.py::test_frontier_walk_equals_reference_walk.
 // A walk of ~300 DEPENDENT pair visits (the floor under k_primary, DESIGN.md 6) becomes ~12 rounds: a round descends two levels of
 // the reference's tree whatever the number of boxes the ray grazes.  Undecided rays (more than 32 candidates, a candidate whose leaf
@@ -608,26 +643,8 @@ __global__ void __launch_bounds__(kBlockThreads, CT_SHADOW_BLOCKS) k_shadow(cons
             n_shadow++;
             word = q * P.occ_words + (L.index >> 5); bit = L.index & 31u;
         }
-        uint32_t budget = P.budget;
-        // an origin this far outside the scene (a shading point 2^32 ray lengths away, SURVEY 0.4) makes every box pass: no point
-        // in walking up to the budget first -- park the ray at its first visit, k_overflow hands it straight to k_overflow_huge
-        if (active && (double)tr.om > 0x1p20 * fmax(fmax(P.bound[0], P.bound[1]), P.bound[2])) budget = 0u;
-        while (true) {                                                  // warp-uniform: traverse_early is warp-synchronous
-            float stc; uint32_t spos;
-            int res = traverse_early_any<kAnyHit, COUNT>(P, tr, active, budget, stc, spos, lc, sm, top_nodes, n_top);
-            bool again = false;
-            if (active) {
-                if (res == kTravOverBudget) {
-                    n_parked++;
-                    again = !park_ray(P, ovf_idx, r64, word, bit);      // parking buffer full: finish in place, no budget
-                    budget = 0xffffffffu;
-                } else if (res == kTravHit) {
-                    atomicOr(&P.occ[word], 1u << bit);
-                }
-            }
-            active = again;
-            if (!__any_sync(0xffffffffu, again)) break;
-        }
+        walk_or_park<kAnyHit, COUNT>(P, tr, r64, active, P.budget, ovf_idx, word, bit, n_parked, lc, sm, top_nodes, n_top,
+                                     [&](int res, float, uint32_t) { if (res == kTravHit) atomicOr(&P.occ[word], 1u << bit); }, [](bool) {});
     }
     warp_add(&P.tot->rays_shadow, n_shadow);
     warp_add(&P.tot->rays_shadow_reused, n_reused);
@@ -792,27 +809,16 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_bounce(const __gr
             tray_setup(r, ray, P.bound, r64);
             clear_occ(P, q);
         }
-        uint32_t budget = P.budget;
-        while (true) {                                                  // warp-uniform: traverse is warp-synchronous
-            float tc; uint32_t pos;
-            int res = traverse_early_any<kFirstLine, COUNT>(P, r, active, budget, tc, pos, lc, sm, top_nodes, n_top);
-            bool again = false;
-            if (active) {
-                if (res == kTravOverBudget) {
-                    n_parked++;
-                    again = !park_ray(P, ovf_idx, r64, q, 0u);          // parking buffer full: finish in place, no budget
-                    budget = 0xffffffffu;
-                    far = true;                                         // k_overflow answers later: let k_shadow look at the path
-                    parked = !again;
-                } else {                                                // found is always true: 0 != 1e30f (:227)
-                    P.hitb_t[q] = tc;
-                    P.hitb_pos[q] = (pos == kNoPos) ? P.pos_of_tri0 : pos;
-                    far = tc != 0.0f || (P.parent_q[cur][q] & kNoReuse);
-                }
-            }
-            active = again;
-            if (!__any_sync(kFullMask, again)) break;
-        }
+        walk_or_park<kFirstLine, COUNT>(P, r, r64, active, P.budget, ovf_idx, q, 0u, n_parked, lc, sm, top_nodes, n_top,
+            [&](int, float tc, uint32_t pos) {                          // found is always true: 0 != 1e30f (:227)
+                P.hitb_t[q] = tc;
+                P.hitb_pos[q] = (pos == kNoPos) ? P.pos_of_tri0 : pos;
+                far = tc != 0.0f || (P.parent_q[cur][q] & kNoReuse);
+            },
+            [&](bool p) {
+                far = true;                                             // k_overflow answers later: let k_shadow look at the path
+                parked = p;
+            });
         if (kFusedEmit) {             // the recursion step of the paths whose hit is final (parked ones: k_emit after k_overflow)
             const bool fin = q < n && !parked;
             uint32_t pslot = 0, ppos = kNoPos; float ptc = 0.0f;
@@ -840,8 +846,9 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_bounce(const __gr
 // order, because ray.t never changes before the exit, so the set of boxes that pass is fixed:
 //   kAnyHit     occluded  <=>  SOME triangle reachable through passing boxes has a bary pass with 1e-4 < t < 1e30;
 //   kFirstLine  closestIndex = the bary-passing reachable triangle that the DFS meets first = the one with the
-//               smallest leaf position (BuildBVH hands the left child the lower part of the parent's index range,
-//               bvh.cpp:70-97, so leaf positions increase along the DFS).
+//               smallest leaf position where leaf positions increase along the DFS (BuildBVH hands the left child the
+//               lower part of the parent's index range, bvh.cpp:70-97).  A caller's tree need not: upload checks it
+//               (bvh_depth), and on a tree without it first-line rays are never parked (first_line_budget).
 // Tests the triangles of an accepted leaf for a parked ray.  kAnyHit: 1 if one of them occludes, else 0;
 // kFirstLine: the first (lowest) leaf position with a barycentric pass, else kNoPos.
 template <TraverseMode MODE, bool COUNT>
@@ -1091,6 +1098,50 @@ __global__ void k_debug_closest(const __grid_constant__ Params P, uint32_t n, co
     if (found) found[i] = f ? 1u : 0u;
     if (index) index[i] = (pos == kNoPos) ? 0u : P.tris[pos].orig;
     if (tclosest) tclosest[i] = tc;
+}
+
+// ct_gpu_debug_early: ray i is a shadow ray (kAnyHit, ray.t = 1e30f) or a reflection ray (kFirstLine, ray.t = 0) run through
+// walk_or_park as k_shadow / k_bounce run theirs; a parked ray's answer is delivered by the real k_overflow / k_overflow_huge into
+// P.occ[i] bit 0 / P.hitb_pos[i] (the caller hands them buffers of its own).  path[i]: 0 own walk, 1 parked, 3 finished in place.
+template <TraverseMode MODE>
+__global__ void __launch_bounds__(kBlockThreads) k_debug_early(const __grid_constant__ Params P, uint32_t n, const double *org, const double *dir,
+                                                               uint32_t *found, uint32_t *index, uint32_t *path) {
+    __shared__ uint32_t walk_sm[kWalkWords * kBlockThreads];          // launched with kBlockThreads threads per block, like k_shadow
+    uint32_t *const sm = MODE == kAnyHit ? walk_sm + threadIdx.x : nullptr;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = i < n;                                         // walk_or_park is warp-level: every lane calls it
+    LocalCount lc;
+    double r64[kRay64];
+    TRay tr;
+    if (active) {
+        Ray r;
+        r.o = ld3(org + 3ull * i); r.d = ld3(dir + 3ull * i); r.t = MODE == kAnyHit ? kRayTInit : 0.0f;
+        tray_setup(tr, r, P.bound, r64);
+    }
+    uint32_t n_parked = 0;
+    const int how = walk_or_park<MODE, false>(P, tr, r64, active, P.budget, 0, i, 0u, n_parked, lc, sm, nullptr, 0u,
+        [&](int res, float, uint32_t pos) {
+            found[i] = res == kTravHit ? 1u : 0u;
+            index[i] = (MODE == kAnyHit || pos == kNoPos) ? 0u : P.tris[pos].orig;
+        }, [](bool) {});
+    if (active) path[i] = (uint32_t)how;
+}
+
+// ... the parked rays' answers, after k_overflow / k_overflow_huge; path 2 for the rays k_overflow handed on
+__global__ void k_debug_early_parked(const __grid_constant__ Params P, int first_line, uint32_t n, uint32_t *found, uint32_t *index, uint32_t *path) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < P.sched->huge_count[0]) path[P.ovf[P.ovf_huge[i]].target] = 2u;
+    if (i >= n) return;
+    const uint32_t how = path[i];                                      // (another thread may have made it 2 already)
+    if (how != (uint32_t)kParked && how != 2u) return;
+    if (first_line) {
+        const uint32_t pos = P.hitb_pos[i];
+        found[i] = 1u;                                                 // 0 != 1e30f (raythread.cpp:227)
+        index[i] = pos == kNoPos ? 0u : P.tris[pos].orig;
+    } else {
+        found[i] = P.occ[i] & 1u;
+        index[i] = 0u;
+    }
 }
 
 __global__ void k_debug_primitives(uint32_t n, const double *org, const double *dir, float *ray_t, const double *tri,

@@ -502,8 +502,10 @@ CT_DEV void traverse_closest_refill(const Params &P, Job &job, LocalCount &lc) {
 //   kAnyHit    shadow rays (ray.t = 1e30f): only `found` is used (raythread.cpp:306), i.e. whether SOME triangle
 //              reachable through accepted boxes has a barycentric pass with 1e-4 < t < 1e30 (SURVEY A7);
 //   kFirstLine reflection rays (ray.t = 0, raythread.cpp:373): the first barycentric pass in DFS order becomes
-//              closestIndex with tclosest = 0 (SURVEY 0.4) = the passing reachable triangle with the LOWEST leaf
-//              position (leaf positions increase along the DFS).
+//              closestIndex with tclosest = 0 (SURVEY 0.4).  The walks here keep the DFS order, so they find it on any
+//              tree; the parked passes (overflow_merge, k_overflow_huge) take the LOWEST leaf position instead, which is
+//              the same pass only where leaf positions increase along the DFS -- upload checks that (bvh_depth) and
+//              never parks a first-line ray on a tree without it (first_line_budget).
 // ray.t never changes before the exit, so the set of accepted boxes is fixed and the moment a leaf is tested
 // cannot change the answer.  The loop therefore walks interior nodes only and DEFERS accepted leaves to a short
 // list, in DFS order; the warp alternates between a walk phase and a leaf phase in which its lanes test their
@@ -597,7 +599,7 @@ CT_DEV int traverse_early(const Params &P, const TRay &r, bool active, const uin
 // levels down with box_maybe and skips the boxes in between -- a child's verdict implies its ancestors' -- so a ray
 // descends the tree in 1 / kWideLevels of the dependent fetches and pays the loop's bookkeeping once per kWide boxes.
 // Accepted children are pushed in reverse order and popped: the visit order is the reference's DFS order, deferred
-// leaves reach the list in DFS order, and kFirstLine's "first pass of a leaf phase" is the lowest leaf position as in
+// leaves reach the list in DFS order, and kFirstLine's "first pass of a leaf phase" is the DFS-first pass as in
 // traverse_early (kAnyHit appends accepted leaves to the list at once; its answer does not depend on the order).
 // A triangle that passes the exact test counts only if the reference's walk reaches its leaf (candidate_reached).
 // WARP-SYNCHRONOUS, same contract as traverse_early; a stack that would overflow ends the walk as kTravOverBudget (the

@@ -286,6 +286,14 @@ int ct_gpu_mark_rows(int device, int row_start, int row_end);
 int ct_gpu_debug_closest(int device, uint32_t n, const double *origins, const double *directions, const float *t0,
                          uint32_t *found, uint32_t *index, float *tclosest);
 
+/* Known-answer-test entry for the early-exit walks: mode 0 = shadow ray (ray.t = 1e30f, found = occluded, raythread.cpp:304-306),
+ * mode 1 = reflection ray (ray.t = 0: index = first barycentric pass in DFS order, 0 when none, raythread.cpp:373).
+ * The rays take the path a frame's rays take, with the options in effect at upload (traversal_budget, overflow_warp_budget,
+ * any_leaves): the walk, parking, k_overflow, k_overflow_huge.  path[i] (may be NULL): 0 finished by its own walk, 1 by k_overflow,
+ * 2 by k_overflow_huge, 3 finished in place (parking buffer full). */
+int ct_gpu_debug_early(int device, int mode, uint32_t n, const double *origins, const double *directions,
+                       uint32_t *found, uint32_t *index, uint32_t *path);
+
 /* Known-answer-test entry for the two primitives (bvh.cpp:147 IntersectTriangle, :165 IntersectAABB):
  * n independent (ray, triangle, box) cases.  tri: n x 9, bmin/bmax: n x 3.  ray_t is in/out. */
 int ct_gpu_debug_primitives(int device, uint32_t n, const double *origins, const double *directions, float *ray_t,

@@ -457,6 +457,12 @@ int ct_oracle_closest(const ct_oracle_scene *s, const double org[3], const doubl
     return r.t != RAY_T_INIT;
 }
 
+void ct_oracle_closest_many(const ct_oracle_scene *s, uint64_t n, const double *org, const double *dir, const float *ray_t0,
+                            uint32_t *found, uint32_t *index, float *tclosest) {
+    for (uint64_t i = 0; i < n; i++)
+        found[i] = (uint32_t)ct_oracle_closest(s, org + 3 * i, dir + 3 * i, ray_t0[i], index + i, tclosest + i);
+}
+
 /* ---- bvh.cpp:16-120 build: midpoint split on the longest axis, leaves <= 2 or unsplittable -------- */
 typedef struct {
     uint32_t n_tri, used;

@@ -80,6 +80,9 @@ int ct_oracle_intersect_aabb(const double org[3], const double dir[3], float ray
 /* ClosestIntersection (raythread.cpp:197-227) for an arbitrary ray; returns found, fills index/t. */
 int ct_oracle_closest(const ct_oracle_scene *s, const double org[3], const double dir[3], float ray_t0,
                       uint32_t *index, float *tclosest);
+/* ct_oracle_closest for n rays (org / dir: n x 3, ray_t0[n]); found, index, tclosest: n each. */
+void ct_oracle_closest_many(const ct_oracle_scene *s, uint64_t n, const double *org, const double *dir, const float *ray_t0,
+                            uint32_t *found, uint32_t *index, float *tclosest);
 uint32_t ct_oracle_shade_color(uint32_t material_color, float intensity); /* ColorToHsv + HsvToColor, color.h:114-126 */
 uint32_t ct_oracle_blend(uint32_t local_color, uint32_t reflected_color, float reflection); /* raythread.cpp:375-379 */
 

@@ -148,6 +148,18 @@ class OracleScene:
         found = lib().ct_oracle_closest(C.byref(self.c), _ptr(org), _ptr(direction), np.float32(t0), C.byref(idx), C.byref(t))
         return bool(found), int(idx.value), float(t.value)
 
+    def closest_many(self, org, direction, t0=1e30):
+        """closest() for n rays in one call: (found, index, t) arrays."""
+        org = np.ascontiguousarray(org, np.float64).reshape(-1, 3); direction = np.ascontiguousarray(direction, np.float64).reshape(-1, 3)
+        n = org.shape[0]
+        t0 = np.ascontiguousarray(np.broadcast_to(np.asarray(t0, np.float32), (n,)))
+        found = np.zeros(n, np.uint32); index = np.zeros(n, np.uint32); t = np.zeros(n, np.float32)
+        L = lib()
+        L.ct_oracle_closest_many.restype = None
+        L.ct_oracle_closest_many.argtypes = [C.POINTER(_Scene), C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.ct_oracle_closest_many(C.byref(self.c), n, _ptr(org), _ptr(direction), _ptr(t0), _ptr(found), _ptr(index), _ptr(t))
+        return found, index, t
+
 
 def prehit_check(scene: "OracleScene", org, direction):
     """Prototype check (ct_oracle.c): reference-order closest-hit walk vs "order-free pre-hit phase + rebuilt stack"
