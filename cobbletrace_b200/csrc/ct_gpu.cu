@@ -249,6 +249,21 @@ int launch_grid(const DeviceState &s, int blocks_per_sm) { return s.n_sm * block
 // on such a tree: a reflection ray cast from a shading point 2^32 ray lengths away walks the whole tree in one thread.
 uint32_t first_line_budget(const DeviceState &s) { return s.leaf_dfs_order ? s.p.budget : 0xffffffffu; }
 
+// The primary rays k_primary parked into v.ovf (slot 0 of the parking buffers) are finished by k_primary_split (option
+// "primary_split", one ray per warp) or by k_primary_long (32 to a warp).  k_primary_split's replay takes leaf positions for the
+// reference's test order, so a tree whose leaf positions do not increase along the DFS (DeviceState::leaf_dfs_order) always gets
+// k_primary_long.  Returns true when k_primary_split was launched.
+bool launch_parked_primary(const DeviceState &s, const Params &v, bool count, cudaStream_t st, int work_idx) {
+    if (g_primary_split && s.leaf_dfs_order) {
+        if (count) k_primary_split<true><<<s.n_sm * 4, kOvfThreads, 0, st>>>(v);
+        else k_primary_split<false><<<s.n_sm * 4, kOvfThreads, 0, st>>>(v);
+        return true;
+    }
+    if (count) k_primary_long<true><<<launch_grid(s, 8), kBlockThreads, 0, st>>>(v, work_idx);
+    else k_primary_long<false><<<launch_grid(s, 8), kBlockThreads, 0, st>>>(v, work_idx);
+    return false;
+}
+
 // L2 residency of the walk's hot set.  The fp32 child pairs and fp32 triangles (76 MB for the dragon-class scene) are
 // read by every walk step, at random; everything else a frame touches (ray queues, hit records, occlusion masks, colour
 // stacks, the fp64 records behind the filters) streams through once.  Left to the default policy the streams evict the
@@ -721,15 +736,9 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
         }
         TRY(mark("primary", 0));
         if (park_primary) {
-            if (g_primary_split && s.leaf_dfs_order) {          // (its replay takes leaf positions for the reference's test order)
-                if (count) k_primary_split<true><<<s.n_sm * 4, kOvfThreads, 0, st>>>(v0);
-                else k_primary_split<false><<<s.n_sm * 4, kOvfThreads, 0, st>>>(v0);
-                TRY(mark("primary_split", 0));
-            } else {
-                if (count) k_primary_long<true><<<grid, kBlockThreads, 0, st>>>(v0, work++);
-                else k_primary_long<false><<<grid, kBlockThreads, 0, st>>>(v0, work++);
-                TRY(mark("primary_long", 0));
-            }
+            const bool split = launch_parked_primary(s, v0, count, st, work);
+            if (!split) work++;
+            TRY(mark(split ? "primary_split" : "primary_long", 0));
         }
     }
     for (int d = 0; d <= depth_max; d++) {
@@ -1265,6 +1274,58 @@ int ct_gpu_debug_early(int device, int mode, uint32_t n, const double *origins, 
     CUX(cudaStreamSynchronize(s.stream));
     if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
     if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
+    if (path) CUX(cudaMemcpy(path, d_p, 4ull * n, cudaMemcpyDeviceToHost));
+    cleanup();
+    return CT_OK;
+}
+
+int ct_gpu_debug_primary(int device, uint32_t n, const double *origins, const double *directions, uint32_t park_cap,
+                         uint32_t *found, uint32_t *index, float *tclosest, uint32_t *path) {
+    if (!origins || !directions) return fail(CT_ERR_INVALID, "NULL ray arrays");
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    if (n == 0) return CT_OK;
+    double *d_o = nullptr, *d_d = nullptr; uint32_t *d_f = nullptr, *d_i = nullptr, *d_p = nullptr, *d_occ = nullptr, *d_hpos = nullptr;
+    float *d_ht = nullptr, *d_tc = nullptr; OvfRay *d_ovf = nullptr; DevSched *d_sched = nullptr; DevTotals *d_tot = nullptr;
+    int rc = CT_OK;
+    auto cleanup = [&]() { cudaFree(d_o); cudaFree(d_d); cudaFree(d_f); cudaFree(d_i); cudaFree(d_p); cudaFree(d_occ); cudaFree(d_hpos);
+                           cudaFree(d_ht); cudaFree(d_tc); cudaFree(d_ovf); cudaFree(d_sched); cudaFree(d_tot); };
+    CUX(cudaMalloc(&d_o, 24ull * n)); CUX(cudaMalloc(&d_d, 24ull * n));
+    CUX(cudaMalloc(&d_f, 4ull * n)); CUX(cudaMalloc(&d_i, 4ull * n)); CUX(cudaMalloc(&d_p, 4ull * n)); CUX(cudaMalloc(&d_tc, 4ull * n));
+    CUX(cudaMalloc(&d_occ, 4ull * n)); CUX(cudaMalloc(&d_hpos, 4ull * n)); CUX(cudaMalloc(&d_ht, 4ull * n));
+    CUX(cudaMalloc(&d_sched, sizeof(DevSched))); CUX(cudaMalloc(&d_tot, sizeof(DevTotals)));
+    CUX(cudaMemcpy(d_o, origins, 24ull * n, cudaMemcpyHostToDevice));
+    CUX(cudaMemcpy(d_d, directions, 24ull * n, cudaMemcpyHostToDevice));
+    CUX(cudaMemset(d_sched, 0, sizeof(DevSched))); CUX(cudaMemset(d_tot, 0, sizeof(DevTotals)));
+    // the scene's Params with this call's hit records, occlusion words and parking buffer, as k_primary's launch sees its own: path q
+    // = slot = ray i; max_depth 0, so that the hit kernels run no recursion step; no framebuffer-layout hit records
+    Params v = s.p;
+    v.sched = d_sched; v.tot = d_tot; v.occ = d_occ; v.occ_words = 1; v.hit0_t = d_ht; v.hit0_pos = d_hpos;
+    v.cap = n; v.max_depth = 0; v.dbg_found = nullptr; v.dbg_index = nullptr; v.dbg_t = nullptr;
+    v.ovf = nullptr; v.ovf_huge = nullptr; v.ovf_cap = 0; v.split_path = d_p;
+    const bool park = s.can_overflow && s.p.primary_budget > 0u;      // render_impl's rule
+    if (park) {
+        v.ovf_cap = std::min<uint32_t>(n, park_cap ? std::min(park_cap, s.p.ovf_cap) : s.p.ovf_cap);
+        CUX(cudaMalloc(&d_ovf, sizeof(OvfRay) * (size_t)v.ovf_cap));
+        v.ovf = d_ovf;
+    }
+    CUX(cudaStreamSynchronize(s.stream));
+    const uint32_t blocks = (n + kBlockThreads - 1) / kBlockThreads;
+    if (park) k_debug_primary<true><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_p);
+    else k_debug_primary<false><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_p);
+    CUX(cudaGetLastError());
+    if (park) {
+        launch_parked_primary(s, v, false, s.stream, 0);
+        CUX(cudaGetLastError());
+    }
+    k_debug_primary_hits<<<(n + 255) / 256, 256, 0, s.stream>>>(v, n, d_f, d_i, d_tc);
+    CUX(cudaGetLastError());
+    CUX(cudaStreamSynchronize(s.stream));
+    if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
+    if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
+    if (tclosest) CUX(cudaMemcpy(tclosest, d_tc, 4ull * n, cudaMemcpyDeviceToHost));
     if (path) CUX(cudaMemcpy(path, d_p, 4ull * n, cudaMemcpyDeviceToHost));
     cleanup();
     return CT_OK;

@@ -322,6 +322,31 @@ struct PrimaryJob {
     }
 };
 
+// The per-ray loop of the primary rays (k_primary, k_debug_primary): the closest-hit walk (ray.t = 1e30f), under PARK with a budget
+// of P.primary_budget pair visits when parking buffers exist.  A walk given up at the budget is parked for k_primary_long /
+// k_primary_split (target / bit: the path's q and slot), or -- parking buffer full -- walked again right here without a budget,
+// from ray.t = 1e30f: the walk given up has already lowered r.t.  WARP-LEVEL: every lane calls it.  Returns, for a lane with a ray,
+// how it was finished (kWalked, kParked, kInPlace); res / tc / pos are the answer of a ray that was not parked.
+template <bool COUNT, bool PARK>
+CT_DEV int primary_walk_or_park(const Params &P, TRay &r, const double *r64, bool got, uint32_t target, uint32_t bit, uint32_t &n_parked,
+                                LocalCount &lc, uint32_t *sm, int &res, float &tc, uint32_t &pos) {
+    const uint32_t budget = (PARK && P.primary_budget > 0u && P.ovf != nullptr) ? P.primary_budget : 0xffffffffu;
+    res = traverse_closest_any<COUNT, PARK>(P, r, got, tc, pos, lc, sm, budget);   // warp-synchronous
+    int how = kWalked;
+    const bool over = PARK && got && res == kTravOverBudget;
+    if (PARK && __any_sync(kFullMask, over)) {
+        bool redo = false;
+        if (over) { const bool parked = park_ray(P, 0, r64, target, bit); redo = !parked; how = parked ? kParked : kInPlace; n_parked++; }
+        if (__any_sync(kFullMask, redo)) {
+            if (redo) r.t = kRayTInit;
+            float tc2; uint32_t pos2;
+            const int res2 = traverse_closest_any<COUNT>(P, r, redo, tc2, pos2, lc, sm);
+            if (redo) { res = res2; tc = tc2; pos = pos2; }
+        }
+    }
+    return how;
+}
+
 // Primary rays.  Persistent warps take chunks of 32 (or 64) slots from the tile's cursor (next_chunk) and remember which
 // chunks they took: the later stages of this device work on exactly those.  By default a warp walks the 32 rays of a
 // chunk together (one 8x4 pixel block: neighbouring rays visit the same nodes); -DCT_REFILL_T=n (n = 1..32) selects
@@ -342,29 +367,14 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary(const __g
 #if CT_REFILL_T > 0
     traverse_closest_refill<COUNT>(P, job, lc);
 #else
-    const uint32_t all = kFullMask;
-    const uint32_t budget = (PARK && P.primary_budget > 0u && P.ovf != nullptr) ? P.primary_budget : 0xffffffffu;
     while (true) {
         bool got = false;
         double r64[kRay64];
         TRay r;
-        if (!job.refill(P, all, got, r, r64)) break;          // a whole chunk's worth of slots: one per lane
-        float tc; uint32_t pos;
-        int res = traverse_closest_any<COUNT, PARK>(P, r, got, tc, pos, lc, sm, budget);   // warp-synchronous
-        // a walk given up at the budget: the ray is parked and walked again by k_primary_long, among long walks only
-        bool parked = false;
-        const bool over = PARK && got && res == kTravOverBudget;
-        if (PARK && __any_sync(all, over)) {
-            bool redo = false;
-            if (over) { parked = park_ray(P, 0, r64, job.q, job.slot); redo = !parked; n_parked++; }
-            if (__any_sync(all, redo)) {                          // parking buffer full: walk again right here, without a budget
-                if (redo) r.t = kRayTInit;
-                float tc2; uint32_t pos2;
-                const int res2 = traverse_closest_any<COUNT>(P, r, redo, tc2, pos2, lc, sm);
-                if (redo) { res = res2; tc = tc2; pos = pos2; }
-            }
-        }
-        const bool done = got && !parked, found = res == kTravHit;
+        if (!job.refill(P, kFullMask, got, r, r64)) break;    // a whole chunk's worth of slots: one per lane
+        int res; float tc; uint32_t pos;
+        const int how = primary_walk_or_park<COUNT, PARK>(P, r, r64, got, job.q, job.slot, n_parked, lc, sm, res, tc, pos);
+        const bool done = got && how != kParked, found = res == kTravHit;
         if (done) job.finish(P, found, tc, pos);
         if (P.max_depth > 0)          // the recursion step at once, while ray and hit are at hand (no k_emit pass over the tile)
             emit_paths(P, 0, done, job.q, job.slot, {r64[0], r64[1], r64[2]}, {r64[3], r64[4], r64[5]}, tc,
@@ -429,8 +439,10 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary_long(cons
 // A walk of ~300 DEPENDENT pair visits (the floor under k_primary, DESIGN.md 6) becomes ~12 rounds: a round descends two levels of
 // the reference's tree whatever the number of boxes the ray grazes.  Undecided rays (more than 32 candidates, a candidate whose leaf
 // starts beyond the minimum + sigma, t >= FINF, a full stack, rays outside the slop analysis) are walked by lane 0 in the
-// reference's order.
+// reference's order.  P.split_path (ct_gpu_debug_primary only) receives 2 | outcome << 8 by q, outcome one of kSplit*.
 constexpr int kSplitStack = 512;         // pending wide nodes per warp: (node, lower end of its near bracket)
+enum { kSplitDecided = 0, kSplitNoSigma = 1, kSplitNotNested = 2, kSplitFinf = 3, kSplitCandFull = 4, kSplitStackFull = 5,
+       kSplitLate = 6, kSplitMany = 7 };
 template <bool COUNT>
 __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_constant__ Params P) {
     const uint32_t n = min(P.sched->ovf_count[0], P.ovf_cap);
@@ -458,13 +470,14 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
         bool found = false;
         float tc = kFinf;                                 // raythread.cpp:204
         uint32_t pos = kNoPos;
+        uint32_t why = kSplitDecided;                     // why an ordered walk decides the ray (kSplit*), for P.split_path
         if (!ordered) {
             if (COUNT && lane == 0) lc.box++;
             if (root_accept(P, r)) {
                 float cand_t[kNearCand], cand_tmin[kNearCand];
                 uint32_t cand_pos[kNearCand], cand_code[kNearCand];
                 int ncand = 0;
-                bool undecided = false;
+                uint32_t undecided = 0;                                            // bit 0: a t >= FINF, bit 1: a full candidate list
                 float best = kRayTInit, band = kRayTInit, thr = kRayTInit;          // this lane's view; made warp-wide once per round
                 if (lane == 0) { stk[0] = 0u; stk_near[0] = -kRayTInit; }
                 __syncwarp();
@@ -494,7 +507,7 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
                                 if (COUNT) lc.tri++;
                                 const TriHit th = leaf_triangle<false, COUNT>(P, r, tp, lc);
                                 if (!(th.hit & (th.t > kEps) & (th.t < kRayTInit))) continue;      // would not lower a ray.t of 1e30f (bvh.cpp:161)
-                                if (!(th.t < kFinf)) { undecided = true; continue; }
+                                if (!(th.t < kFinf)) { undecided |= 1u; continue; }
                                 if (!(th.t <= band)) continue;
                                 const uint32_t code = __ldg(P.tri_parent + tp);        // the triangle's leaf: 2 * pair + side
                                 if (COUNT) lc.box_exact++;
@@ -507,7 +520,7 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
                                         if (cand_t[j] <= band) { cand_t[m] = cand_t[j]; cand_tmin[m] = cand_tmin[j]; cand_pos[m] = cand_pos[j]; cand_code[m] = cand_code[j]; m++; }
                                     ncand = m;
                                 }
-                                if (ncand == kNearCand) undecided = true;
+                                if (ncand == kNearCand) undecided |= 2u;
                                 else { cand_t[ncand] = th.t; cand_tmin[ncand] = bt.tmin; cand_pos[ncand] = tp; cand_code[ncand] = code; ncand++; }
                             }
                         }
@@ -522,7 +535,12 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
 #pragma unroll
                     for (int d = 1; d < 32; d <<= 1) { const uint32_t v = __shfl_up_sync(kFullMask, incl, d); if ((int)lane >= d) incl += v; }
                     const uint32_t total = __shfl_sync(kFullMask, incl, 31);
-                    if (__any_sync(kFullMask, undecided) || sp + total > (uint32_t)kSplitStack) { ordered = true; break; }
+                    if (__any_sync(kFullMask, undecided) || sp + total > (uint32_t)kSplitStack) {
+                        const uint32_t u = __reduce_or_sync(kFullMask, undecided);
+                        why = (u & 1u) ? kSplitFinf : (u & 2u) ? kSplitCandFull : kSplitStackFull;
+                        ordered = true;
+                        break;
+                    }
                     const uint32_t at = sp + incl - n_out;
                     for (uint32_t k = 0; k < n_out; k++) { stk[at + k] = out_ref[k]; stk_near[at + k] = out_near[k]; }
                     sp += total;
@@ -541,7 +559,7 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
 #pragma unroll
                     for (int d = 1; d < 32; d <<= 1) { const uint32_t v = __shfl_up_sync(kFullMask, incl, d); if ((int)lane >= d) incl += v; }
                     const uint32_t total = __shfl_sync(kFullMask, incl, 31);
-                    if (__any_sync(kFullMask, late) || total > 32u) ordered = true;
+                    if (__any_sync(kFullMask, late) || total > 32u) { why = __any_sync(kFullMask, late) ? kSplitLate : kSplitMany; ordered = true; }
                     else {
                         uint32_t *const g_pos = stk, *const g_code = stk + 32;
                         float *const g_t = stk_near, *const g_tmin = stk_near + 32;
@@ -582,6 +600,10 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
             if (!slot_pixel(P, slot, x, y, fbi)) fbi = -1;
             n_rays++;
             store_primary_hit(P, slot, q, fbi, found, tc, pos);
+            if (P.split_path) {
+                if (ordered && why == kSplitDecided) why = !(r.sg > 0.0f) ? kSplitNoSigma : kSplitNotNested;     // ordered from the start
+                P.split_path[q] = 2u | (why << 8);
+            }
         }
         if (P.max_depth > 0)
             emit_paths(P, 0, lane == 0, q, slot, {r64[0], r64[1], r64[2]}, {r64[3], r64[4], r64[5]}, tc,
@@ -1144,7 +1166,44 @@ __global__ void k_debug_early_parked(const __grid_constant__ Params P, int first
     }
 }
 
-__global__ void k_debug_primitives(uint32_t n, const double *org, const double *dir, float *ray_t, const double *tri,
+// ct_gpu_debug_primary: ray i is a primary ray (ray.t = 1e30f) of path q = slot = i run through primary_walk_or_park as k_primary runs
+// its rays; the hit record goes to P.hit0_t[i] / P.hit0_pos[i] (buffers of the caller's), that of a parked ray from the real
+// k_primary_long / k_primary_split.  path[i]: 0 own walk, 1 parked, 3 finished in place (k_primary_split rewrites its rays' codes).
+template <bool PARK>
+__global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(const __grid_constant__ Params P, uint32_t n, const double *org,
+                                                                             const double *dir, uint32_t *path) {
+    __shared__ uint32_t closest_sm[kClosestWords * kBlockThreads];     // launched with kBlockThreads threads per block, like k_primary
+    uint32_t *const sm = kSmClosest > 0 ? closest_sm + threadIdx.x : nullptr;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = i < n;                                         // primary_walk_or_park is warp-level: every lane calls it
+    LocalCount lc;
+    double r64[kRay64];
+    TRay r;
+    if (active) {
+        Ray ray;
+        ray.o = ld3(org + 3ull * i); ray.d = ld3(dir + 3ull * i); ray.t = kRayTInit;
+        tray_setup(r, ray, P.bound, r64);
+        tray_nearest_setup(r, P.bound);
+    }
+    uint32_t n_parked = 0;
+    int res; float tc; uint32_t pos;
+    const int how = primary_walk_or_park<false, PARK>(P, r, r64, active, i, i, n_parked, lc, sm, res, tc, pos);
+    if (!active) return;
+    path[i] = (uint32_t)how;
+    if (how != kParked) store_primary_hit(P, i, i, -1, res == kTravHit, tc, pos);
+}
+
+// ... every ray's answer from its hit record (found, ClosestIntersection's closestIndex and tclosest)
+__global__ void k_debug_primary_hits(const __grid_constant__ Params P, uint32_t n, uint32_t *found, uint32_t *index, float *tclosest) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t pos = P.hit0_pos[i];                                // pos_of_tri0 for a hit without a closestIndex: index 0
+    found[i] = pos != kNoPos ? 1u : 0u;
+    index[i] = pos == kNoPos ? 0u : P.tris[pos].orig;
+    tclosest[i] = P.hit0_t[i];
+}
+
+__global__ void k_debug_primitives(uint32_t n,const double *org, const double *dir, float *ray_t, const double *tri,
                                    const double *bmin, const double *bmax, uint32_t *tri_hit, uint32_t *box_hit,
                                    uint32_t *filter_out, double bound_scale, bool tri_filter) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;

@@ -161,6 +161,7 @@ struct Params {
     // parked rays
     OvfRay *ovf; uint32_t ovf_cap;
     uint32_t *ovf_huge;                          // indices (into ovf) of the rays k_overflow left to k_overflow_huge
+    uint32_t *split_path;                        // optional (ct_gpu_debug_primary; NULL in frames): by q, how k_primary_split decided the ray
     const uint32_t *pair_parent;                 // pair -> 2 * parent pair + side of its own box (kNoPos for the root's children pair)
     const uint32_t *tri_parent;                  // leaf position -> 2 * pair + side of the box of the leaf that holds it (kNoPos: root leaf)
     DevSched *sched;

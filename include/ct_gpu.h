@@ -294,6 +294,19 @@ int ct_gpu_debug_closest(int device, uint32_t n, const double *origins, const do
 int ct_gpu_debug_early(int device, int mode, uint32_t n, const double *origins, const double *directions,
                        uint32_t *found, uint32_t *index, uint32_t *path);
 
+/* Known-answer-test entry for the primary rays: ClosestIntersection with ray.t = 1e30f (raythread.cpp:197-227) for n arbitrary
+ * rays, taking the path a frame's primary rays take under the options in effect at upload (primary_budget) and at the call
+ * (primary_split): the walk of k_primary, parking, the real k_primary_long or k_primary_split, or the walk again in place when the
+ * parking buffer is full.  park_cap: capacity of the parking buffer, 0 = a frame's (a small value forces the in-place path).
+ * found / index / tclosest as ct_gpu_debug_closest returns them.  path[i] (all outputs may be NULL): low byte 0 finished by its own
+ * walk, 1 by k_primary_long, 2 by k_primary_split, 3 in place; for 2 the next byte says how k_primary_split decided it: 0 by its
+ * frontier and replay, or walked in the reference's order because 1 the ray is outside the rounding analysis (sigma = 0), 2 the tree
+ * is not nested, 3 a candidate has t >= FINF, 4 a lane's candidate list is full, 5 the warp's node stack is full, 6 a candidate's
+ * leaf box starts beyond the minimum + sigma, 7 more than 32 candidates lie within sigma of the minimum.  Works on buffers of its
+ * own: frames rendered afterwards are unchanged. */
+int ct_gpu_debug_primary(int device, uint32_t n, const double *origins, const double *directions, uint32_t park_cap,
+                         uint32_t *found, uint32_t *index, float *tclosest, uint32_t *path);
+
 /* Known-answer-test entry for the two primitives (bvh.cpp:147 IntersectTriangle, :165 IntersectAABB):
  * n independent (ray, triangle, box) cases.  tri: n x 9, bmin/bmax: n x 3.  ray_t is in/out. */
 int ct_gpu_debug_primitives(int device, uint32_t n, const double *origins, const double *directions, float *ray_t,
