@@ -17,6 +17,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 GPU_LIB = os.path.join(PKG, "libct_gpu.so")
 
 CT_FLAG_WIDE, CT_FLAG_KEEP_HITS, CT_FLAG_COUNT_TESTS, CT_FLAG_STAGE_TIMING, CT_FLAG_SUBSAMPLING, CT_FLAG_SUPERSAMPLING = 1, 2, 4, 8, 16, 32
+CT_FLAG_BUILD_BVH = 64
 BACKGROUND = 0x333333      # raythread.cpp:59
 REFERENCE_MAX_DEPTH = 10   # raythread.cpp:508
 
@@ -26,6 +27,7 @@ ABI_SYMBOLS = [
     "ct_gpu_set_stream", "ct_gpu_render_tile", "ct_gpu_readback", "ct_gpu_readback_async", "ct_gpu_readback_wait", "ct_gpu_readback_hits", "ct_gpu_get_counters",
     "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early", "ct_gpu_debug_primary",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
+    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array",
 ]
 
 
@@ -76,6 +78,11 @@ MAT_DT = np.dtype([("color", "<u4"), ("specular", "<i4"), ("reflection", "<f4")]
 LIGHT_DT = np.dtype([("type", "<i4"), ("intensity", "<f4"), ("pos", "<f8", 3), ("dir", "<f8", 3)])
 assert NODE_DT.itemsize == C.sizeof(BvhNode) == 64 and MAT_DT.itemsize == C.sizeof(Material) == 12
 assert LIGHT_DT.itemsize == C.sizeof(Light) == 56
+# == ct_scene_summary (ct_gpu_debug_scene_array "summary")
+SUMMARY_DT = np.dtype([("n_pairs", "<u4"), ("n_wide", "<u4"), ("root_ref", "<u4"), ("root_cnt", "<u4"), ("pos_of_tri0", "<u4"), ("nested", "<u4"),
+                       ("leaf_dfs_order", "<u4"), ("can_overflow", "<u4"), ("bound", "<f8", 3), ("depth", "<i4"), ("pad", "<u4")])
+assert SUMMARY_DT.itemsize == 64
+SCENE_ARRAYS = ("wide", "pairs32", "pairs64", "tris32", "tris", "materials", "pair_parent", "tri_parent", "summary")
 
 _lib = None
 
@@ -124,6 +131,8 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_shutdown.argtypes = [C.c_int]
     L.ct_gpu_set_option.argtypes = [C.c_char_p, C.c_longlong]
     L.ct_gpu_overflow_stats.argtypes = [C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+    L.ct_gpu_build_bvh.argtypes = [C.c_int, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, vp]
+    L.ct_gpu_debug_scene_array.argtypes = [C.c_int, C.c_char_p, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     if path == GPU_LIB:
         _lib = L
     return L
@@ -157,10 +166,13 @@ class GpuRenderer:
 
     # -- ct_gpu_upload_scene ------------------------------------------------------------------------
     def upload(self, fs: FlatScene, width: int, height: int, max_depth: int = REFERENCE_MAX_DEPTH, flags: int = 0,
-               background: int = BACKGROUND, viewport=(1.0, 1.0, 1.0), triangle_stride: int = 72):
+               background: int = BACKGROUND, viewport=(1.0, 1.0, 1.0), triangle_stride: int = 72, build_bvh: bool = False):
         """`triangle_stride` = 96 lays the vertices out like the reference's triangle_t (scenefile.h:36-41: p1, p2, p3 and
-        a centroid the tracer never reads -- filled with NaNs here so that a wrong stride cannot go unnoticed)."""
-        if not fs.has_bvh():
+        a centroid the tracer never reads -- filled with NaNs here so that a wrong stride cannot go unnoticed).
+        `build_bvh`: the device builds the reference's tree from the triangles (CT_FLAG_BUILD_BVH); a tree `fs` carries is ignored."""
+        if build_bvh:
+            flags |= CT_FLAG_BUILD_BVH
+        elif not fs.has_bvh():
             raise ValueError("FlatScene has no BVH: build it on the host first (cobbletrace_b200.host.build_bvh)")
         tri = np.ascontiguousarray(fs.tri, np.float64)
         if triangle_stride != 72:
@@ -173,14 +185,14 @@ class GpuRenderer:
         if fs.n_lights:
             lights["type"][:fs.n_lights], lights["intensity"][:fs.n_lights] = fs.light_type, fs.light_intensity
             lights["pos"][:fs.n_lights], lights["dir"][:fs.n_lights] = fs.light_pos, fs.light_dir
-        nodes = pack_nodes(fs)
-        idx = np.ascontiguousarray(fs.tri_index, np.uint32)
+        nodes = None if build_bvh else pack_nodes(fs)
+        idx = None if build_bvh else np.ascontiguousarray(fs.tri_index, np.uint32)
         d = SceneDesc()
         d.struct_size = C.sizeof(SceneDesc)
         d.flags = flags
         d.n_triangles, d.triangle_stride = fs.n_tri, triangle_stride
         d.triangles, d.materials = _ptr(tri), _ptr(mats)
-        d.n_nodes, d.n_lights = fs.n_nodes, fs.n_lights
+        d.n_nodes, d.n_lights = (0 if build_bvh else fs.n_nodes), fs.n_lights
         d.nodes, d.tri_indexes, d.lights = _ptr(nodes), _ptr(idx), _ptr(lights)
         d.camera_position = (C.c_double * 3)(*np.asarray(fs.cam_pos, np.float64).tolist())
         d.camera_rotation = (C.c_double * 9)(*np.asarray(fs.cam_rot, np.float64).tolist())
@@ -348,6 +360,14 @@ class GpuRenderer:
         _check(self.L, self.L.ct_gpu_debug_filter(self.device, n, _ptr(o), _ptr(d), _ptr(rt), _ptr(tr), _ptr(mn), _ptr(mx), float(bound_scale), _ptr(out)))
         return out
 
+    def debug_scene_array(self, name: str) -> np.ndarray:
+        """ct_gpu_debug_scene_array: the bytes of one array the upload built (api.SCENE_ARRAYS); "summary" as a SUMMARY_DT record."""
+        n = C.c_size_t()
+        _check(self.L, self.L.ct_gpu_debug_scene_array(self.device, name.encode(), None, 0, C.byref(n)))
+        out = np.zeros(n.value, np.uint8)
+        _check(self.L, self.L.ct_gpu_debug_scene_array(self.device, name.encode(), _ptr(out), out.size, C.byref(n)))
+        return out.view(SUMMARY_DT)[0] if name == "summary" else out
+
     def filter_stats(self):
         """(box tests, triangle tests) the fp32 filters left to the fp64 arithmetic (needs CT_FLAG_COUNT_TESTS)."""
         a = C.c_uint64(); b = C.c_uint64()
@@ -374,6 +394,25 @@ def set_option(name: str, value: int) -> None:
     """ct_gpu_set_option: library-wide knob applied by the next upload (e.g. "traversal_budget")."""
     L = load_library()
     _check(L, L.ct_gpu_set_option(name.encode(), int(value)))
+
+
+def build_bvh(fs: FlatScene, device: int = 0, triangle_stride: int = 72) -> FlatScene:
+    """`fs` with the node arrays and tri_index of the reference's BuildBVH, built on `device` by ct_gpu_build_bvh.
+    `triangle_stride` lays the triangles out as GpuRenderer.upload does."""
+    import dataclasses
+    L = load_library()
+    n = fs.n_tri
+    tri = np.ascontiguousarray(fs.tri, np.float64).reshape(n, 9)
+    if triangle_stride != 72:
+        wide = np.full((n, triangle_stride // 8), np.nan)
+        wide[:, :9] = tri
+        tri = wide
+    nodes = np.zeros(max(2 * n - 1, 1), NODE_DT)
+    idx = np.zeros(max(n, 1), np.uint32)
+    used = _check(L, L.ct_gpu_build_bvh(int(device), n, _ptr(tri), triangle_stride, _ptr(nodes), nodes.shape[0], _ptr(idx)))
+    nodes = nodes[:used]
+    return dataclasses.replace(fs, node_min=nodes["min"].copy(), node_max=nodes["max"].copy(), node_left=nodes["left"].copy(),
+                               node_first=nodes["first"].copy(), node_count=nodes["count"].copy(), tri_index=idx[:n].copy())
 
 
 def device_count() -> int:

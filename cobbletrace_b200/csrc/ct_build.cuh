@@ -3,6 +3,7 @@
 #pragma once
 
 #include "ct_layout.cuh"
+#include "ct_bvh_build.cuh"   // bb_scan
 
 namespace {
 
@@ -101,6 +102,94 @@ __global__ void __launch_bounds__(256) k_build_tris(const unsigned char *__restr
         if (materials[k].reflection > 0.0f) refl = true;
     }
     if (__any_sync(0xffffffffu, refl) && (threadIdx.x & 31u) == 0) atomicOr(&rep->any_reflective, 1u);
+}
+
+// ---- the early-exit walks' wide tree (DevWide), built from the binary tree on the device --------------------------------
+// kWideLevels levels of the reference's tree per wide node, children in DFS order.  Wide nodes are numbered breadth-first: a
+// queue, each node's interior children taken in entry order.  One wide level at a time: k_wide_count counts every node's interior
+// entries, an exclusive scan over the level's nodes in id order gives their children's ids, k_wide_fill writes the records.  The
+// walk starts at the root and follows child links only, so array slots a caller's tree does not reach are never read.
+__device__ int wide_entries(const ct_bvh_node *__restrict__ nodes, uint32_t root, uint32_t cur[kWide]) {
+    int n_cur = 2;
+    cur[0] = nodes[root].left_node; cur[1] = cur[0] + 1u;
+    for (int lvl = 1; lvl < kWideLevels; lvl++) {
+        uint32_t nxt[kWide];
+        int n_nxt = 0;
+        for (int i = 0; i < n_cur; i++) {
+            const ct_bvh_node &c = nodes[cur[i]];
+            if (c.triangle_count != 0) nxt[n_nxt++] = cur[i];
+            else { nxt[n_nxt++] = c.left_node; nxt[n_nxt++] = c.left_node + 1u; }
+        }
+        n_cur = n_nxt;
+        for (int i = 0; i < n_cur; i++) cur[i] = nxt[i];
+    }
+    return n_cur;
+}
+
+__global__ void __launch_bounds__(kBbThreads) k_wide_count(const ct_bvh_node *__restrict__ nodes, const uint32_t *__restrict__ root_of,
+                                                           uint32_t b, uint32_t e, uint32_t *__restrict__ cnt) {
+    for (uint32_t w = b + bb_tid(); w < e; w += bb_stride()) {
+        uint32_t cur[kWide];
+        const int n_cur = wide_entries(nodes, root_of[w], cur);
+        uint32_t c = 0;
+        for (int i = 0; i < n_cur; i++) c += nodes[cur[i]].triangle_count == 0 ? 1u : 0u;
+        cnt[w - b] = c;
+    }
+    if (bb_tid() == 0) cnt[e - b] = 0u;
+}
+
+__global__ void __launch_bounds__(kBbThreads) k_wide_fill(const ct_bvh_node *__restrict__ nodes, uint32_t *__restrict__ root_of, uint32_t b, uint32_t e,
+                                                          const uint32_t *__restrict__ cnt, DevWide *__restrict__ wide) {
+    for (uint32_t w = b + bb_tid(); w < e; w += bb_stride()) {
+        uint32_t cur[kWide];
+        const int n_cur = wide_entries(nodes, root_of[w], cur);
+        uint32_t next = e + cnt[w - b];
+        DevWide rec;
+        for (int i = 0; i < kWide; i++) {
+            DevWideChild &x = rec.c[i];
+            if (i >= n_cur) {
+                for (int a = 0; a < 3; a++) { x.bmin[a] = 1e30f; x.bmax[a] = -1e30f; }
+                x.ref = kNoPos; x.cnt = 0u;
+                continue;
+            }
+            const ct_bvh_node &c = nodes[cur[i]];
+            for (int a = 0; a < 3; a++) { x.bmin[a] = __double2float_rn(c.aabb_min[a]); x.bmax[a] = __double2float_rn(c.aabb_max[a]); }
+            x.cnt = c.triangle_count;
+            if (c.triangle_count != 0) x.ref = c.first_triangle_index;
+            else { root_of[next] = cur[i]; x.ref = next++; }
+        }
+        wide[w] = rec;
+    }
+}
+
+// Collapses the tree below nodes[0] (interior) into wide[0 .. *n_wide); root_of, cnt: scratch of n_pairs + 1 entries, tile_sum of
+// (n_pairs + 1) / kBbScanTile + 1.  Synchronises once per wide level.
+cudaError_t build_wide(const ct_bvh_node *nodes, uint32_t *root_of, uint32_t *cnt, uint32_t *tile_sum, DevWide *wide, int n_sm,
+                       cudaStream_t st, uint32_t *n_wide) {
+    const int grid = n_sm * 8;
+    auto blocks_for = [&](uint32_t m) { return (int)std::max<uint32_t>(1u, std::min<uint32_t>((uint32_t)grid, (m + kBbThreads - 1u) / kBbThreads)); };
+    cudaError_t e = cudaMemsetAsync(root_of, 0, sizeof(uint32_t), st);
+    uint32_t b = 0, end = 1;
+    while (e == cudaSuccess && b < end) {
+        k_wide_count<<<blocks_for(end - b), kBbThreads, 0, st>>>(nodes, root_of, b, end, cnt);
+        if ((e = bb_scan(cnt, end - b, tile_sum, st)) != cudaSuccess) break;
+        k_wide_fill<<<blocks_for(end - b), kBbThreads, 0, st>>>(nodes, root_of, b, end, cnt, wide);
+        uint32_t more = 0;
+        if ((e = cudaMemcpyAsync(&more, cnt + (end - b), sizeof more, cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;
+        if ((e = cudaStreamSynchronize(st)) != cudaSuccess) break;
+        b = end; end += more;
+    }
+    *n_wide = end;
+    return e;
+}
+
+// The interior numbering of a tree built on the device (every node reachable): pid[i] = interior nodes before i, kLeafMark for a
+// leaf.  pid holds n_nodes + 1 entries.
+__global__ void __launch_bounds__(kBbThreads) k_pid_flags(const ct_bvh_node *__restrict__ nodes, uint32_t n_nodes, uint32_t *__restrict__ pid) {
+    for (uint32_t i = bb_tid(); i <= n_nodes; i += bb_stride()) pid[i] = i < n_nodes && nodes[i].triangle_count == 0 ? 1u : 0u;
+}
+__global__ void __launch_bounds__(kBbThreads) k_pid_leaves(const ct_bvh_node *__restrict__ nodes, uint32_t n_nodes, uint32_t *__restrict__ pid) {
+    for (uint32_t i = bb_tid(); i < n_nodes; i += bb_stride()) if (nodes[i].triangle_count != 0) pid[i] = kLeafMark;
 }
 
 }  // namespace

@@ -38,6 +38,7 @@
 #include <ctime>
 #include <cstdlib>
 #include <mutex>
+#include <string>
 #include <thread>
 #include <vector>
 
@@ -45,6 +46,7 @@
 #include "ct_layout.cuh"     // constants, device structs, Params
 #include "ct_traverse.cuh"   // the BVH walks
 #include "ct_kernels.cuh"    // the kernels of a tile
+#include "ct_bvh_build.cuh"  // the reference's BuildBVH on the device (ct_gpu_build_bvh, CT_FLAG_BUILD_BVH)
 #include "ct_build.cuh"      // upload-time scene build kernels
 
 namespace {
@@ -87,6 +89,7 @@ struct DeviceState {
     // k_overflow_huge) and k_primary_split's replay take the lowest position for the DFS-first one; on a tree without this
     // property reflection rays are never parked and parked primary rays go to k_primary_long (first_line_budget, render_impl)
     bool leaf_dfs_order = true;
+    int depth = 0;                   // the tree's depth (the reference's DFS stack entries)
     // per-depth path state (render_impl hands each launch a Params view of its depth, so that the shadow / shade
     // chain of one depth can run on its own stream next to the bounce chain of the next)
     float *hitb_t_all = nullptr; uint32_t *hitb_pos_all = nullptr;      // [depth][cap]
@@ -242,6 +245,22 @@ int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *
     return best;
 }
 
+// Device buffers and a stream that live for one ct_gpu_upload_scene call: the staged copies of the caller's arrays, the tree
+// built with CT_FLAG_BUILD_BVH (arena), the wide tree's scratch.  Freed when the call returns, whatever it returns.
+struct Staging {
+    std::vector<void *> ptrs;
+    BbArena arena;
+    cudaStream_t st = nullptr;
+    ~Staging() { if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } cudaFree(arena.base); for (void *q : ptrs) cudaFree(q); }
+    template <typename T> cudaError_t alloc(T **out, size_t count) {
+        void *q = nullptr;
+        const cudaError_t e = cudaMalloc(&q, std::max<size_t>(count, 1) * sizeof(T));
+        if (e == cudaSuccess) ptrs.push_back(q);
+        *out = static_cast<T *>(q);
+        return e;
+    }
+};
+
 int launch_grid(const DeviceState &s, int blocks_per_sm) { return s.n_sm * blocks_per_sm; }
 
 // The walk budget of the first-line (reflection) rays: unlimited -- never parked, the walk in the ray's own thread keeps the
@@ -326,25 +345,98 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     if (!d || d->struct_size != sizeof(ct_scene_desc)) return fail(CT_ERR_INVALID, "ct_scene_desc missing or struct_size != %zu", sizeof(ct_scene_desc));
     if (d->n_triangles == 0 || !d->triangles || !d->materials) return fail(CT_ERR_INVALID, "scene has no triangles");
     if (d->triangle_stride < 72 || d->triangle_stride % 8) return fail(CT_ERR_INVALID, "triangle_stride must be >= 72 and a multiple of 8");
-    if (d->n_nodes == 0 || !d->nodes || !d->tri_indexes) return fail(CT_ERR_INVALID, "scene has no BVH (build it with the reference's BuildBVH or ct_host_build_bvh)");
+    const bool build = (d->flags & CT_FLAG_BUILD_BVH) != 0;
+    if (build) {
+        if (d->n_nodes != 0 || d->nodes || d->tri_indexes) return fail(CT_ERR_INVALID, "CT_FLAG_BUILD_BVH builds the tree: n_nodes must be 0, nodes and tri_indexes NULL");
+        if (d->n_triangles >= (1u << 31)) return fail(CT_ERR_LIMIT, "%u triangles: the device build takes fewer than 2^31", d->n_triangles);
+    } else if (d->n_nodes == 0 || !d->nodes || !d->tri_indexes) {
+        return fail(CT_ERR_INVALID, "scene has no BVH (build it with the reference's BuildBVH or ct_host_build_bvh, or pass CT_FLAG_BUILD_BVH)");
+    }
     if (d->n_lights && !d->lights) return fail(CT_ERR_INVALID, "n_lights > 0 but lights == NULL");
     if (d->width <= 0 || d->height <= 0 || (int64_t)d->width * d->height > (1ll << 30)) return fail(CT_ERR_INVALID, "bad frame size %dx%d", d->width, d->height);
     if (d->max_depth < 0 || d->max_depth > 15) return fail(CT_ERR_LIMIT, "max_depth %d outside 0..15", d->max_depth);
     if ((d->flags & CT_FLAG_SUPERSAMPLING) && (d->flags & CT_FLAG_KEEP_HITS))
         return fail(CT_ERR_INVALID, "CT_FLAG_SUPERSAMPLING cannot be combined with CT_FLAG_KEEP_HITS (a pixel has 16 primary rays)");
-    bool ok = true, dfs_order = true;
+    bool ok = true, dfs_order = true;          // a tree BuildBVH makes has its leaves in DFS order (bvh.cpp:70-97)
     std::vector<uint8_t> reachable;
-    int depth = bvh_depth(d->nodes, d->n_nodes, d->n_triangles, &ok, &dfs_order, reachable);
-    if (!ok) return fail(CT_ERR_INVALID, "BVH is malformed (child or triangle range out of bounds, overlapping leaves, a cycle or a shared child)");
-    if (depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", depth, kStackMax);
+    int depth = 0;
+    if (!build) {
+        depth = bvh_depth(d->nodes, d->n_nodes, d->n_triangles, &ok, &dfs_order, reachable);
+        if (!ok) return fail(CT_ERR_INVALID, "BVH is malformed (child or triangle range out of bounds, overlapping leaves, a cycle or a shared child)");
+        if (depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", depth, kStackMax);
+    }
     TRY(check_device(device));
     DEVICE_GUARD(device);
     std::lock_guard<std::mutex> lock(g_mutex);
     DeviceState &s = g_dev[device];
+    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
+    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
+    const double t_begin = now_ms();
+    double t_mark = t_begin;
+    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_upload_scene: %-28s %7.1f ms\n", what, t - t_mark); t_mark = t; } };
+    int n_sm = 0;
+    CU(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
+
+    // The binary tree, the leaf permutation and the triangles on the device.  With CT_FLAG_BUILD_BVH the tree is built here, into
+    // buffers of the upload's own, BEFORE the previous scene is released: a refused tree leaves that scene loaded.
+    const size_t tri_bytes = (size_t)(d->n_triangles - 1) * d->triangle_stride + 72;      // the last triangle may end at its third vertex
+    Staging stg;
+    CU(cudaStreamCreateWithFlags(&stg.st, cudaStreamNonBlocking));
+    const ct_bvh_node *raw_nodes = nullptr; const uint32_t *raw_idx = nullptr; const unsigned char *raw_tris = nullptr;
+    uint32_t *raw_pid = nullptr;
+    uint32_t n_nodes = d->n_nodes, n_pairs = 0;
+    ct_bvh_node root{};
+    if (build) {
+        BbBuffers bf;
+        bb_carve(stg.arena, d->n_triangles, tri_bytes, bf);
+        CU(cudaMalloc(&stg.arena.base, stg.arena.used));
+        stg.arena.used = 0;
+        bb_carve(stg.arena, d->n_triangles, tri_bytes, bf);
+        CU(cudaMemcpyAsync(bf.raw, d->triangles, tri_bytes, cudaMemcpyHostToDevice, stg.st));
+        CU(bb_build(bf, d->triangle_stride, d->n_triangles, n_sm, stg.st, &n_nodes, &depth));
+        CU(cudaMemcpyAsync(&root, bf.out, sizeof root, cudaMemcpyDeviceToHost, stg.st));
+        CU(cudaStreamSynchronize(stg.st));
+        lap("BVH built on the device");
+        if (depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", depth, kStackMax);
+        n_pairs = (n_nodes - 1u) / 2u;                                      // every node is reachable: 1 + 2 * interior nodes
+        uint32_t *ptile = nullptr;                                          // interior numbering: a scan over the node order
+        CU(stg.alloc(&raw_pid, (size_t)n_nodes + 1)); CU(stg.alloc(&ptile, ((size_t)n_nodes + 1) / kBbScanTile + 1));
+        const int blocks = std::max(1, std::min(n_sm * 8, (int)((n_nodes + kBbThreads) / kBbThreads)));
+        k_pid_flags<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, n_nodes, raw_pid);
+        CU(bb_scan(raw_pid, n_nodes, ptile, stg.st));
+        k_pid_leaves<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, n_nodes, raw_pid);
+        CU(cudaGetLastError());
+        raw_nodes = bf.out; raw_idx = bf.tri_index; raw_tris = bf.raw;
+    } else {
+        root = d->nodes[0];
+        // nodes: reference layout -> per-interior-node child pairs, built on the device from the raw arrays (k_build_pairs); the host
+        // only numbers the interior nodes it validated
+        std::vector<uint32_t> pid_of(d->n_nodes, kNoPos);
+        for (uint32_t i = 0; i < d->n_nodes; i++)
+            if (reachable[i]) pid_of[i] = d->nodes[i].triangle_count == 0 ? n_pairs++ : kLeafMark;      // unreachable slots get no record and write nothing
+        ct_bvh_node *rn = nullptr; uint32_t *ri = nullptr; unsigned char *rt = nullptr;
+        CU(stg.alloc(&rn, d->n_nodes)); CU(stg.alloc(&raw_pid, d->n_nodes)); CU(stg.alloc(&ri, d->n_triangles)); CU(stg.alloc(&rt, tri_bytes));
+        CU(cudaMemcpyAsync(rn, d->nodes, (size_t)d->n_nodes * sizeof(ct_bvh_node), cudaMemcpyHostToDevice, stg.st));
+        CU(cudaMemcpyAsync(raw_pid, pid_of.data(), (size_t)d->n_nodes * 4, cudaMemcpyHostToDevice, stg.st));
+        CU(cudaMemcpyAsync(ri, d->tri_indexes, (size_t)d->n_triangles * 4, cudaMemcpyHostToDevice, stg.st));
+        CU(cudaMemcpyAsync(rt, d->triangles, tri_bytes, cudaMemcpyHostToDevice, stg.st));
+        raw_nodes = rn; raw_idx = ri; raw_tris = rt;
+        lap("interior-node numbering (host)");
+    }
+    // the early-exit walks' wide tree, into scratch first: its size decides the layout of the hot allocation below
+    DevWide *wide_tmp = nullptr;
+    uint32_t n_wide = 0;
+    if (root.triangle_count == 0) {
+        uint32_t *root_of = nullptr, *wcnt = nullptr, *wtile = nullptr;
+        CU(stg.alloc(&wide_tmp, n_pairs)); CU(stg.alloc(&root_of, (size_t)n_pairs + 1)); CU(stg.alloc(&wcnt, (size_t)n_pairs + 1));
+        CU(stg.alloc(&wtile, ((size_t)n_pairs + 1) / kBbScanTile + 1));
+        CU(build_wide(raw_nodes, root_of, wcnt, wtile, wide_tmp, n_sm, stg.st, &n_wide));
+    }
+    CU(cudaStreamSynchronize(stg.st));
+    lap("wide tree (device)");
+
     free_device(s);
-    cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, device));
-    s.n_sm = prop.multiProcessorCount;
+    s.n_sm = n_sm;
     CU(cudaStreamCreateWithFlags(&s.own_stream, cudaStreamNonBlocking));
     s.stream = s.own_stream;
     CU(cudaEventCreate(&s.ev0));
@@ -360,73 +452,15 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     s.p.primary_budget = g_primary_budget_option < 0 ? 0u : g_primary_budget_option > 0 ? (uint32_t)std::min<long long>(g_primary_budget_option, 1ll << 30) : kDefaultPrimaryBudget;
     s.flags = d->flags;
     s.leaf_dfs_order = dfs_order;
+    s.depth = depth;
 
-    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
-    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
-    const double t_begin = now_ms();
-    double t_mark = t_begin;
-    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_upload_scene: %-28s %7.1f ms\n", what, t - t_mark); t_mark = t; } };
     Params &p = s.p;
     p.n_tri = d->n_triangles; p.n_lights = d->n_lights;
-    // nodes: reference layout -> per-interior-node child pairs (fp32 for the filter, fp64 for the exact path), built on
-    // the device from the raw arrays (k_build_pairs / k_build_tris); the host only numbers the interior nodes
-    std::vector<uint32_t> pid_of(d->n_nodes, kNoPos);
-    uint32_t n_pairs = 0;
-    for (uint32_t i = 0; i < d->n_nodes; i++)
-        if (reachable[i]) pid_of[i] = d->nodes[i].triangle_count == 0 ? n_pairs++ : kLeafMark;      // unreachable slots get no record and write nothing
-    auto child_ref = [&](uint32_t c, uint32_t &ref, uint32_t &cnt) {
-        const ct_bvh_node &n = d->nodes[c];
-        cnt = n.triangle_count;
-        ref = cnt ? n.first_triangle_index : pid_of[c];
-    };
-    child_ref(0, p.root_ref, p.root_cnt);
+    p.root_cnt = root.triangle_count;
+    p.root_ref = root.triangle_count ? root.first_triangle_index : 0u;      // an interior root is pair 0
     p.n_pairs = n_pairs;
-    p.n_nodes = d->n_nodes;
-    s.can_overflow = (uint64_t)d->n_nodes + d->n_triangles > p.budget;      // parked rays: only when a DFS can run past the budget at all
-    lap("interior-node numbering (host)");
-    // the early-exit walks' wide tree: kWideLevels levels of the reference's tree per node, children in DFS order
-    std::vector<DevWide> wide;
-    if (d->nodes[0].triangle_count == 0) {
-        std::vector<uint32_t> root_of;                  // wide node -> the interior node whose descendants it holds
-        std::vector<uint32_t> wid_of(d->n_nodes, kNoPos);
-        root_of.reserve(n_pairs / 2 + 1);
-        root_of.push_back(0u); wid_of[0] = 0u;
-        wide.reserve(n_pairs / 2 + 1);
-        for (size_t w = 0; w < root_of.size(); w++) {
-            uint32_t cur[kWide], nxt[kWide];
-            int n_cur = 2;
-            cur[0] = d->nodes[root_of[w]].left_node; cur[1] = cur[0] + 1u;
-            for (int lvl = 1; lvl < kWideLevels; lvl++) {
-                int n_nxt = 0;
-                for (int i = 0; i < n_cur; i++) {
-                    const ct_bvh_node &c = d->nodes[cur[i]];
-                    if (c.triangle_count != 0) nxt[n_nxt++] = cur[i];
-                    else { nxt[n_nxt++] = c.left_node; nxt[n_nxt++] = c.left_node + 1u; }
-                }
-                n_cur = n_nxt;
-                memcpy(cur, nxt, sizeof cur);
-            }
-            DevWide rec;
-            for (int i = 0; i < kWide; i++) {
-                DevWideChild &e = rec.c[i];
-                if (i >= n_cur) {
-                    for (int a = 0; a < 3; a++) { e.bmin[a] = 1e30f; e.bmax[a] = -1e30f; }
-                    e.ref = kNoPos; e.cnt = 0u;
-                    continue;
-                }
-                const ct_bvh_node &c = d->nodes[cur[i]];
-                for (int a = 0; a < 3; a++) { e.bmin[a] = (float)c.aabb_min[a]; e.bmax[a] = (float)c.aabb_max[a]; }
-                e.cnt = c.triangle_count;
-                if (c.triangle_count != 0) e.ref = c.first_triangle_index;
-                else {
-                    if (wid_of[cur[i]] == kNoPos) { wid_of[cur[i]] = (uint32_t)root_of.size(); root_of.push_back(cur[i]); }
-                    e.ref = wid_of[cur[i]];
-                }
-            }
-            wide.push_back(rec);
-        }
-    }
-    lap("wide tree (host)");
+    p.n_nodes = n_nodes;
+    s.can_overflow = (uint64_t)n_nodes + d->n_triangles > p.budget;      // parked rays: only when a DFS can run past the budget at all
 
     DevPair32 *dp32 = nullptr; DevPair64 *dp64 = nullptr; DevTri *dt = nullptr; DevTri32 *dt32 = nullptr; ct_material *dm = nullptr;
     uint32_t *dpp = nullptr, *dtp = nullptr;
@@ -434,16 +468,15 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
         // the records every walk step reads -- fp32 child pairs and fp32 triangles -- share ONE allocation, so that a single
         // L2 access-policy window can cover them (apply_l2_policy)
         const size_t pair_bytes = ((size_t)std::max<uint32_t>(n_pairs, 1) * sizeof(DevPair32) + 255u) & ~(size_t)255u;
-        const size_t wide_bytes = (wide.size() * sizeof(DevWide) + 255u) & ~(size_t)255u;
+        const size_t wide_bytes = ((size_t)n_wide * sizeof(DevWide) + 255u) & ~(size_t)255u;
         unsigned char *hot = nullptr;
         s.hot_bytes = wide_bytes + pair_bytes + (size_t)d->n_triangles * sizeof(DevTri32);
         TRY(dev_alloc(s, &hot, s.hot_bytes));
         s.hot_base = hot;
-        if (!wide.empty()) {
-            CU(cudaMemcpyAsync(hot, wide.data(), wide.size() * sizeof(DevWide), cudaMemcpyHostToDevice, s.stream));
-            CU(cudaStreamSynchronize(s.stream));
+        if (n_wide) {
+            CU(cudaMemcpyAsync(hot, wide_tmp, (size_t)n_wide * sizeof(DevWide), cudaMemcpyDeviceToDevice, s.stream));
             p.wide = reinterpret_cast<const DevWide *>(hot);
-            p.n_wide = (uint32_t)wide.size();
+            p.n_wide = n_wide;
         }
         dp32 = reinterpret_cast<DevPair32 *>(hot + wide_bytes); dt32 = reinterpret_cast<DevTri32 *>(hot + wide_bytes + pair_bytes);
     }
@@ -453,37 +486,25 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     if (s.can_overflow) TRY(dev_alloc(s, &dpp, std::max<uint32_t>(n_pairs, 1)));
     BuildReport rep{};
     {
-        // staging copies of the caller's arrays, freed again below
-        ct_bvh_node *raw_nodes = nullptr; uint32_t *raw_pid = nullptr, *raw_idx = nullptr, *seen = nullptr; unsigned char *raw_tris = nullptr; BuildReport *drep = nullptr;
-        const size_t tri_bytes = (size_t)(d->n_triangles - 1) * d->triangle_stride + 72;      // the last triangle may end at its third vertex
-        auto release = [&] { cudaFree(raw_nodes); cudaFree(raw_pid); cudaFree(raw_idx); cudaFree(raw_tris); cudaFree(drep); cudaFree(seen); };
-        auto staged = [&](cudaError_t e) { if (e != cudaSuccess) { release(); free_device(s); } return e; };
-        CU(staged(cudaMalloc(&raw_nodes, (size_t)d->n_nodes * sizeof(ct_bvh_node))));
-        CU(staged(cudaMalloc(&raw_pid, (size_t)d->n_nodes * 4)));
-        CU(staged(cudaMalloc(&raw_idx, (size_t)d->n_triangles * 4)));
-        CU(staged(cudaMalloc(&raw_tris, tri_bytes)));
-        CU(staged(cudaMalloc(&drep, sizeof rep)));
+        uint32_t *seen = nullptr; BuildReport *drep = nullptr;
+        auto staged = [&](cudaError_t e) { if (e != cudaSuccess) free_device(s); return e; };
+        CU(staged(stg.alloc(&drep, 1)));
         const size_t seen_words = ((size_t)d->n_triangles + 31u) / 32u;
-        CU(staged(cudaMalloc(&seen, seen_words * 4)));
+        CU(staged(stg.alloc(&seen, seen_words)));
         CU(staged(cudaMemsetAsync(seen, 0, seen_words * 4, s.stream)));
         rep.bad_pos = kNoPos; rep.pos0 = kNoPos;
         CU(staged(cudaMemcpyAsync(drep, &rep, sizeof rep, cudaMemcpyHostToDevice, s.stream)));
-        CU(staged(cudaMemcpyAsync(raw_nodes, d->nodes, (size_t)d->n_nodes * sizeof(ct_bvh_node), cudaMemcpyHostToDevice, s.stream)));
-        CU(staged(cudaMemcpyAsync(raw_pid, pid_of.data(), (size_t)d->n_nodes * 4, cudaMemcpyHostToDevice, s.stream)));
         if (dpp) CU(staged(cudaMemsetAsync(dpp, 0xff, (size_t)std::max<uint32_t>(n_pairs, 1) * 4, s.stream)));
         CU(staged(cudaMemsetAsync(dtp, 0xff, (size_t)d->n_triangles * 4, s.stream)));
         const int build_blocks = s.n_sm * 8;
-        k_build_pairs<<<build_blocks, 256, 0, s.stream>>>(raw_nodes, raw_pid, d->n_nodes, dp32, dp64, dpp, dtp, d->n_triangles, drep);
-        CU(staged(cudaMemcpyAsync(raw_idx, d->tri_indexes, (size_t)d->n_triangles * 4, cudaMemcpyHostToDevice, s.stream)));
-        CU(staged(cudaMemcpyAsync(raw_tris, d->triangles, tri_bytes, cudaMemcpyHostToDevice, s.stream)));
+        k_build_pairs<<<build_blocks, 256, 0, s.stream>>>(raw_nodes, raw_pid, n_nodes, dp32, dp64, dpp, dtp, d->n_triangles, drep);
         CU(staged(cudaMemcpyAsync(dm, d->materials, (size_t)d->n_triangles * sizeof(ct_material), cudaMemcpyHostToDevice, s.stream)));
         k_build_tris<<<build_blocks, 256, 0, s.stream>>>(raw_tris, (uint32_t)d->triangle_stride, raw_idx, dm, d->n_triangles, dt, dt32, seen, drep);
         CU(staged(cudaGetLastError()));
         CU(staged(cudaMemcpyAsync(&rep, drep, sizeof rep, cudaMemcpyDeviceToHost, s.stream)));
         CU(staged(cudaStreamSynchronize(s.stream)));
-        release();
     }
-    if (rep.bad_pos != kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes[%u] = %u out of range", rep.bad_pos, d->tri_indexes[rep.bad_pos]); }
+    if (rep.bad_pos != kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes[%u] = %u out of range", rep.bad_pos, build ? 0u : d->tri_indexes[rep.bad_pos]); }
     if (rep.duplicate || rep.pos0 == kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes is not a permutation of 0..n_triangles-1 (an index occurs twice)"); }
     p.pos_of_tri0 = rep.pos0;
     p.nested = (!rep.not_nested && !rep.boxes_bad) ? 1u : 0u;
@@ -492,7 +513,7 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
         double bound;
         memcpy(&bound, &rep.bound_bits[a], sizeof bound);
         p.bound[a] = (!rep.boxes_bad && bound < 1e30) ? bound : INFINITY;
-        p.root_min[a] = d->nodes[0].aabb_min[a]; p.root_max[a] = d->nodes[0].aabb_max[a];
+        p.root_min[a] = root.aabb_min[a]; p.root_max[a] = root.aabb_max[a];
         p.root_min32[a] = (float)p.root_min[a]; p.root_max32[a] = (float)p.root_max[a];
     }
     p.pairs32 = dp32; p.pairs64 = dp64; p.tris = dt; p.tris32 = dt32; p.materials = dm;
@@ -589,6 +610,91 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     for (cudaStream_t a : s.aux) TRY(apply_l2_policy(s, device, a));
     if (timing) fprintf(stderr, "ct_gpu_upload_scene: L2 window %zu bytes, set-aside %zu bytes; total %.1f ms\n", s.l2_window, s.l2_set_aside, now_ms() - t_begin);
     s.loaded = true;
+    return CT_OK;
+}
+
+int ct_gpu_build_bvh(int device, uint32_t n_triangles, const void *triangles, uint32_t triangle_stride, ct_bvh_node *nodes,
+                     uint32_t nodes_capacity, uint32_t *tri_indexes) {
+    if (n_triangles == 0) return fail(CT_ERR_INVALID, "cannot build a BVH over zero triangles");
+    if (n_triangles >= (1u << 31)) return fail(CT_ERR_LIMIT, "%u triangles: the device build takes fewer than 2^31", n_triangles);
+    if (!triangles || !nodes || !tri_indexes) return fail(CT_ERR_INVALID, "triangles, nodes and tri_indexes must not be NULL");
+    if (triangle_stride < 72 || triangle_stride % 8) return fail(CT_ERR_INVALID, "triangle_stride must be >= 72 and a multiple of 8");
+    if (nodes_capacity < 2u * n_triangles - 1u) return fail(CT_ERR_INVALID, "nodes_capacity %u < 2 n - 1 = %u", nodes_capacity, 2u * n_triangles - 1u);
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    auto cu_fail = [](cudaError_t e, const char *what) {
+        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "ct_gpu_build_bvh: %s: %s", what, cudaGetErrorString(e));
+    };
+    int n_sm = 0;
+    cudaError_t e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
+    if (e != cudaSuccess) return cu_fail(e, "cudaDeviceGetAttribute");
+    // a stream and buffers of its own: a scene uploaded on this device is not touched
+    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
+    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
+    double t_mark = now_ms();
+    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_build_bvh: %-28s %7.2f ms\n", what, t - t_mark); t_mark = t; } };
+    cudaStream_t st = nullptr;
+    if ((e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking)) != cudaSuccess) return cu_fail(e, "cudaStreamCreate");
+    BbArena arena;
+    struct Release { cudaStream_t s; BbArena &a; ~Release() { cudaStreamSynchronize(s); cudaStreamDestroy(s); cudaFree(a.base); } } release{st, arena};
+    const size_t tri_bytes = (size_t)(n_triangles - 1) * triangle_stride + 72;      // the last triangle may end at its third vertex
+    BbBuffers bf;
+    bb_carve(arena, n_triangles, tri_bytes, bf);
+    if ((e = cudaMalloc(&arena.base, arena.used)) != cudaSuccess) { arena.base = nullptr; return cu_fail(e, "cudaMalloc"); }
+    arena.used = 0;
+    bb_carve(arena, n_triangles, tri_bytes, bf);
+    lap("allocation");
+    if ((e = cudaMemcpyAsync(bf.raw, triangles, tri_bytes, cudaMemcpyHostToDevice, st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
+    lap("triangles to the device");
+    uint32_t n_nodes = 0;
+    int depth = 0;
+    if ((e = bb_build(bf, triangle_stride, n_triangles, n_sm, st, &n_nodes, &depth)) != cudaSuccess) return cu_fail(e, "build");
+    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
+    if (timing) fprintf(stderr, "ct_gpu_build_bvh: %u nodes, %d levels\n", n_nodes, depth);
+    lap("tree built on the device");
+    if (n_nodes > (uint32_t)INT32_MAX) return fail(CT_ERR_LIMIT, "%u nodes do not fit the return value", n_nodes);
+    if ((e = cudaMemcpyAsync(nodes, bf.out, (size_t)n_nodes * sizeof(ct_bvh_node), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaMemcpyAsync(tri_indexes, bf.tri_index, (size_t)n_triangles * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
+    lap("tree to the host");
+    return (int)n_nodes;
+}
+
+int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t capacity, size_t *bytes) {
+    if (!name || !bytes) return fail(CT_ERR_INVALID, "name and bytes must not be NULL");
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    const Params &p = s.p;
+    ct_scene_summary sum{};
+    const void *src = nullptr;
+    size_t n = 0;
+    const std::string nm(name);
+    if (nm == "wide") { src = p.wide; n = (size_t)p.n_wide * sizeof(DevWide); }
+    else if (nm == "pairs32") { src = p.pairs32; n = (size_t)p.n_pairs * sizeof(DevPair32); }
+    else if (nm == "pairs64") { src = p.pairs64; n = (size_t)p.n_pairs * sizeof(DevPair64); }
+    else if (nm == "tris32") { src = p.tris32; n = (size_t)p.n_tri * sizeof(DevTri32); }
+    else if (nm == "tris") { src = p.tris; n = (size_t)p.n_tri * sizeof(DevTri); }
+    else if (nm == "materials") { src = p.materials; n = (size_t)p.n_tri * sizeof(ct_material); }
+    else if (nm == "pair_parent") { src = p.pair_parent; n = p.pair_parent ? (size_t)p.n_pairs * sizeof(uint32_t) : 0; }
+    else if (nm == "tri_parent") { src = p.tri_parent; n = (size_t)p.n_tri * sizeof(uint32_t); }
+    else if (nm == "summary") {
+        sum.n_pairs = p.n_pairs; sum.n_wide = p.n_wide; sum.root_ref = p.root_ref; sum.root_cnt = p.root_cnt; sum.pos_of_tri0 = p.pos_of_tri0;
+        sum.nested = p.nested; sum.leaf_dfs_order = s.leaf_dfs_order ? 1u : 0u; sum.can_overflow = s.can_overflow ? 1u : 0u;
+        for (int a = 0; a < 3; a++) sum.bound[a] = p.bound[a];
+        sum.depth = s.depth;
+        n = sizeof sum;
+    } else {
+        return fail(CT_ERR_INVALID, "unknown scene array \"%s\"", name);
+    }
+    *bytes = n;
+    if (!dst || n == 0) return CT_OK;
+    if (capacity < n) return fail(CT_ERR_INVALID, "%s needs %zu bytes, capacity is %zu", name, n, capacity);
+    if (nm == "summary") { memcpy(dst, &sum, n); return CT_OK; }
+    CU(cudaMemcpyAsync(dst, src, n, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaStreamSynchronize(s.stream));
     return CT_OK;
 }
 

@@ -77,6 +77,9 @@ enum {
                                  generator keyed on (x, y, call number) instead -- the same function the parity
                                  harness substitutes for rand() in the compiled reference (DESIGN.md, sampling modes).  16x the rays of a plain frame.
                                  Combines with CT_FLAG_SUBSAMPLING as in the reference (not with CT_FLAG_KEEP_HITS). */
+    CT_FLAG_BUILD_BVH = 64u,  /* ct_gpu_upload_scene builds the tree itself from the triangles (as ct_gpu_build_bvh does, on the device,
+                                 in place: nothing goes back to the host); n_nodes must be 0 and nodes, tri_indexes NULL.  A tree deeper
+                                 than the device traversal stack is refused with CT_ERR_LIMIT and the previous scene stays loaded */
     CT_FLAG_SUBSAMPLING = 16u /* settings.subsampling (raythread.cpp:512-531): of the rows of a tile (= one worker's
                                  partition) every other one and the last are traced, the rows between get the average
                                  of their neighbours.  Tiles must be rendered in the order the caller wants their
@@ -124,6 +127,37 @@ const char *ct_gpu_last_error(void);
  * the BVH built by the reference's BuildBVH (bvh.cpp:108) to `device` as SoA arrays and allocates the
  * device framebuffer (zero-filled, like cobbletrace.cpp:57).  Re-uploading replaces the previous scene. */
 int ct_gpu_upload_scene(int device, const ct_scene_desc *desc);
+
+/* The reference's InitializeBVHState + BuildBVH (bvh.cpp:16-120) on `device`: the same tree, node for node and index for
+ * index, every field included (_pad = 0), as the reference and ct_host_build_bvh make it.  Triangles are given as in
+ * ct_scene_desc: 9 doubles p1,p2,p3 at the start of each record, triangle_stride >= 72 and a multiple of 8.  Writes
+ * nodes[0 .. nodesUsed) and tri_indexes[0 .. n_triangles) and returns nodesUsed (= 1 + 2 * interior nodes).
+ * nodes_capacity must be at least 2 n - 1 (what InitializeBVHState allocates), else CT_ERR_INVALID; n = 0 is
+ * CT_ERR_INVALID, n >= 2^31 CT_ERR_LIMIT.  Trees of any depth are built (the depth limit applies to rendering only).
+ * Synchronous; works on a stream and buffers of its own, so a scene uploaded on `device` and its frames are not
+ * affected (its kernels may wait for the call: freeing the call's buffers synchronises the device).  A failed allocation
+ * returns CT_ERR_OOM and leaves nothing allocated. */
+int ct_gpu_build_bvh(int device, uint32_t n_triangles, const void *triangles, uint32_t triangle_stride, ct_bvh_node *nodes,
+                     uint32_t nodes_capacity, uint32_t *tri_indexes);
+
+/* What ct_gpu_upload_scene derived from the tree, for tests that compare two uploads (ct_gpu_debug_scene_array "summary"). */
+typedef struct ct_scene_summary {
+    uint32_t n_pairs;          /* interior nodes (child-pair records) */
+    uint32_t n_wide;           /* wide nodes of the early-exit walks (0 for a leaf root) */
+    uint32_t root_ref, root_cnt;   /* the root: its pair (interior) or first leaf position and triangle count (leaf) */
+    uint32_t pos_of_tri0;      /* leaf position of triangle 0 */
+    uint32_t nested;           /* every child box lies inside its parent's */
+    uint32_t leaf_dfs_order;   /* leaf positions increase along the reference's DFS */
+    uint32_t can_overflow;     /* a walk can exceed the visit budget (parking buffers allocated) */
+    double bound[3];           /* largest |coordinate| of any box per axis (INFINITY: some box not finite or unordered) */
+    int32_t depth;             /* the tree's depth (DFS stack entries) */
+    uint32_t _pad;
+} ct_scene_summary;
+
+/* Debug export: copies one of the arrays ct_gpu_upload_scene built into dst and sets *bytes to its size.  Names: "wide",
+ * "pairs32", "pairs64", "tris32", "tris", "materials", "pair_parent" (0 bytes when no walk can be parked), "tri_parent",
+ * "summary" (a ct_scene_summary).  dst == NULL only reports *bytes; capacity < *bytes is CT_ERR_INVALID.  Synchronises. */
+int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t capacity, size_t *bytes);
 
 /* Replaces the camera half of HandleUpdates (raythread.cpp:557-572) for an already uploaded scene. */
 int ct_gpu_set_camera(int device, const double position[3], const double rotation[9]);
