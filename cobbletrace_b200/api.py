@@ -27,8 +27,9 @@ ABI_SYMBOLS = [
     "ct_gpu_set_stream", "ct_gpu_render_tile", "ct_gpu_readback", "ct_gpu_readback_async", "ct_gpu_readback_wait", "ct_gpu_readback_hits", "ct_gpu_get_counters",
     "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early", "ct_gpu_debug_primary",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
-    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array",
+    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays",
 ]
+RAY_KINDS = {"primary": 0, "shadow": 1, "reflection": 2}     # CT_RAY_PRIMARY, CT_RAY_SHADOW, CT_RAY_REFLECTION
 
 
 class CtError(RuntimeError):
@@ -63,6 +64,12 @@ class SceneDesc(C.Structure):    # == ct_scene_desc
                 ("nodes", C.c_void_p), ("tri_indexes", C.c_void_p), ("lights", C.c_void_p),
                 ("camera_position", C.c_double * 3), ("camera_rotation", C.c_double * 9), ("viewport", C.c_float * 3),
                 ("width", C.c_int32), ("height", C.c_int32), ("max_depth", C.c_int32), ("background", C.c_uint32)]
+
+
+class RayQuery(C.Structure):     # == ct_ray_query
+    _fields_ = [("struct_size", C.c_uint32), ("kind", C.c_int32), ("n", C.c_uint32), ("_pad", C.c_uint32),
+                ("origins", C.c_void_p), ("directions", C.c_void_p), ("found", C.c_void_p), ("index", C.c_void_p),
+                ("tclosest", C.c_void_p), ("stream", C.c_void_p)]
 
 
 class RayCounters(C.Structure):  # == ct_ray_counters
@@ -133,6 +140,7 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_overflow_stats.argtypes = [C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.ct_gpu_build_bvh.argtypes = [C.c_int, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, vp]
     L.ct_gpu_debug_scene_array.argtypes = [C.c_int, C.c_char_p, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.ct_gpu_trace_rays.argtypes = [C.c_int, C.POINTER(RayQuery)]
     if path == GPU_LIB:
         _lib = L
     return L
@@ -311,6 +319,54 @@ class GpuRenderer:
 
     def gather_rows_to(self, dst_device: int, row_start: int, row_end: int):
         _check(self.L, self.L.ct_gpu_gather_rows(self.device, dst_device, row_start, row_end))
+
+    # -- ct_gpu_trace_rays ----------------------------------------------------------------------------
+    def trace_rays(self, origins, directions, kind: str = "primary"):
+        """ClosestIntersection for n rays of one kind the reference casts ("primary": ray.t = 1e30f, the closest hit; "shadow":
+        occlusion; "reflection": ray.t = 0, the first barycentric pass in DFS order), bit for bit; see ct_gpu_trace_rays.
+        Returns (found, index, tclosest), None for what the kind does not define (shadow rays: found only).
+
+        torch tensors: float64, shape (n, 3), contiguous, on cuda:<device>.  They are read in place, the work runs on
+        torch.cuda.current_stream(device), and the results are int32 / float32 tensors on the device that are valid in that
+        stream's order: the call does not synchronise.  numpy arrays: copied to the device, traced, synchronised, returned as
+        numpy (found / index uint32, tclosest float32)."""
+        import torch
+        if kind not in RAY_KINDS:
+            raise ValueError(f"kind must be one of {sorted(RAY_KINDS)}, not {kind!r}")
+        dev = torch.device("cuda", self.device)
+        if isinstance(origins, np.ndarray) and isinstance(directions, np.ndarray):
+            o = torch.from_numpy(np.ascontiguousarray(origins, np.float64).reshape(-1, 3)).to(dev)
+            d = torch.from_numpy(np.ascontiguousarray(directions, np.float64).reshape(-1, 3)).to(dev)
+            out = self.trace_rays(o, d, kind)
+            torch.cuda.current_stream(dev).synchronize()
+            found, index, t = (None if x is None else x.cpu().numpy() for x in out)
+            return (found.view(np.uint32), None if index is None else index.view(np.uint32), t)
+        for name, a in (("origins", origins), ("directions", directions)):
+            if not isinstance(a, torch.Tensor):
+                raise ValueError(f"{name}: a torch tensor or a numpy array, not {type(a).__name__}")
+            if a.device != dev:
+                raise ValueError(f"{name} is on {a.device}, this renderer traces on {dev}")
+            if a.dtype != torch.float64:
+                raise ValueError(f"{name} is {a.dtype}, rays are float64")
+            if a.dim() != 2 or a.shape[1] != 3:
+                raise ValueError(f"{name} has shape {tuple(a.shape)}, rays are (n, 3)")
+            if not a.is_contiguous():
+                raise ValueError(f"{name} is not contiguous")
+        if origins.shape != directions.shape:
+            raise ValueError(f"origins {tuple(origins.shape)} and directions {tuple(directions.shape)} differ in shape")
+        n = origins.shape[0]
+        found = torch.empty(n, dtype=torch.int32, device=dev)
+        index = None if kind == "shadow" else torch.empty(n, dtype=torch.int32, device=dev)
+        t = None if kind == "shadow" else torch.empty(n, dtype=torch.float32, device=dev)
+        q = RayQuery()
+        q.struct_size, q.kind, q.n = C.sizeof(RayQuery), RAY_KINDS[kind], n
+        q.origins, q.directions = origins.data_ptr() or None, directions.data_ptr() or None
+        q.found = found.data_ptr() or None
+        q.index = None if index is None else (index.data_ptr() or None)
+        q.tclosest = None if t is None else (t.data_ptr() or None)
+        q.stream = torch.cuda.current_stream(dev).cuda_stream or 1      # (handle 0, torch's default stream, is cudaStreamLegacy = 1)
+        _check(self.L, self.L.ct_gpu_trace_rays(self.device, C.byref(q)))
+        return found, index, t
 
     # -- KAT entry points -----------------------------------------------------------------------------
     def debug_closest(self, origins, directions, t0):

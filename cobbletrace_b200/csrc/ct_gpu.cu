@@ -325,6 +325,111 @@ int read_totals(DeviceState &s, ct_ray_counters *out) {   // synchronises the st
     return CT_OK;
 }
 
+// The one path of the ray queries (ct_gpu_trace_rays) and of the KAT entries ct_gpu_debug_early / ct_gpu_debug_primary: n rays in
+// device memory of one kind, the walk of the frame's kernel for that kind with this call's scratch as its hit records, occlusion
+// words and parking buffers, the real second-pass kernels for the parked rays, then k_ray_results.  Enqueued on `st`; the scratch
+// is one stream-ordered allocation, freed in stream order.  bin: walk the rays in the binning pass's order (k_ray_bin_*).
+// park_cap: the primary rays' parking buffer, 0 = a frame's.  path (may be NULL): how each ray was finished (ct_gpu_debug_*).
+int trace_impl(DeviceState &s, int kind, uint32_t n, const double *org, const double *dir, uint32_t *found, uint32_t *index,
+               float *tclosest, uint32_t *path, uint32_t park_cap, bool bin, cudaStream_t st) {
+    const bool primary = kind == CT_RAY_PRIMARY;
+    const bool park = primary ? s.can_overflow && s.p.primary_budget > 0u : s.can_overflow;      // render_impl's rules
+    uint32_t ovf_cap = 0;
+    if (park) ovf_cap = std::min<uint32_t>(n, primary && park_cap ? std::min(park_cap, s.p.ovf_cap) : s.p.ovf_cap);
+    const uint32_t n_tiles = (kRayCells + 1u + kBbScanTile - 1u) / kBbScanTile;
+    // the scratch: scheduler and totals records, one occlusion word and one hit record per ray, the parking buffer and huge list,
+    // the binning arrays -- carved from one allocation (first pass: sizes only)
+    char *base = nullptr;
+    size_t used = 0;
+    auto take = [&](size_t bytes) { char *q = base ? base + used : nullptr; used += (bytes + 255u) & ~(size_t)255u; return q; };
+    DevSched *sched = nullptr; DevTotals *tot = nullptr; uint32_t *occ = nullptr, *hpos = nullptr, *huge = nullptr; float *ht = nullptr;
+    OvfRay *ovf = nullptr; uint16_t *cell = nullptr; uint32_t *count = nullptr, *tiles = nullptr, *order = nullptr;
+    auto carve = [&]() {
+        used = 0;
+        sched = (DevSched *)take(sizeof(DevSched)); tot = (DevTotals *)take(sizeof(DevTotals));
+        occ = (uint32_t *)take(4ull * n); ht = (float *)take(4ull * n); hpos = (uint32_t *)take(4ull * n);
+        if (ovf_cap) { ovf = (OvfRay *)take(sizeof(OvfRay) * (size_t)ovf_cap); huge = (uint32_t *)take(4ull * ovf_cap); }
+        if (bin) {
+            cell = (uint16_t *)take(2ull * n); count = (uint32_t *)take(4ull * (kRayCells + 1u));
+            tiles = (uint32_t *)take(4ull * n_tiles); order = (uint32_t *)take(4ull * n);
+        }
+    };
+    carve();
+    cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&base), used, st);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "cudaMallocAsync(%zu bytes): %s", used, cudaGetErrorString(e));
+    }
+    carve();
+    Params v = s.p;
+    v.sched = sched; v.tot = tot; v.occ = occ; v.occ_words = 1;
+    v.hit0_t = v.hitb_t = ht; v.hit0_pos = v.hitb_pos = hpos;
+    v.cap = n; v.max_depth = 0; v.dbg_found = nullptr; v.dbg_index = nullptr; v.dbg_t = nullptr;
+    v.ovf = ovf; v.ovf_huge = huge; v.ovf_cap = ovf_cap; v.split_path = path;
+    if (kind == CT_RAY_REFLECTION) v.budget = first_line_budget(s);
+    // everything below is enqueued; a failure still frees the scratch in stream order
+    auto enqueue = [&]() -> cudaError_t {
+        cudaError_t r = cudaMemsetAsync(sched, 0, (size_t)((char *)occ - (char *)sched), st);       // DevSched and DevTotals
+        if (r != cudaSuccess) return r;
+        if (bin) {
+            if ((r = cudaMemsetAsync(count, 0, 4ull * (kRayCells + 1u), st)) != cudaSuccess) return r;
+            k_ray_bin_count<<<(n + kBinChunk - 1u) / kBinChunk, kBinThreads, 0, st>>>(v, n, org, dir, cell, count);
+            if ((r = bb_scan(count, kRayCells, tiles, st)) != cudaSuccess) return r;
+            k_ray_bin_scatter<<<std::min<uint32_t>((uint32_t)s.n_sm * 8u, (n + kBinThreads - 1u) / kBinThreads), kBinThreads, 0, st>>>(n, cell, count, order);
+        }
+        const uint32_t blocks = (n + kBlockThreads - 1) / kBlockThreads;
+        if (primary) {
+            if (park) k_debug_primary<true><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            else k_debug_primary<false><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            if (park) launch_parked_primary(s, v, false, st, 0);
+        } else if (kind == CT_RAY_SHADOW) {
+            k_debug_early<kAnyHit><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            if (park) { k_overflow<kAnyHit, false><<<s.n_sm * 2, kOvfThreads, 0, st>>>(v, 0); k_overflow_huge<kAnyHit, false><<<s.n_sm * 4, 256, 0, st>>>(v, 0); }
+        } else {
+            k_debug_early<kFirstLine><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            if (park) { k_overflow<kFirstLine, false><<<s.n_sm * 2, kOvfThreads, 0, st>>>(v, 0); k_overflow_huge<kFirstLine, false><<<s.n_sm * 4, 256, 0, st>>>(v, 0); }
+        }
+        const int mode = primary ? kClosest : kind == CT_RAY_SHADOW ? kAnyHit : kFirstLine;
+        k_ray_results<<<(n + 255) / 256, 256, 0, st>>>(v, mode, n, found, index, tclosest, path);
+        return cudaGetLastError();
+    };
+    const cudaError_t r = enqueue();
+    const cudaError_t f = cudaFreeAsync(base, st);
+    if (r != cudaSuccess) return fail(CT_ERR_CUDA, "ray query: %s", cudaGetErrorString(r));
+    if (f != cudaSuccess) return fail(CT_ERR_CUDA, "cudaFreeAsync: %s", cudaGetErrorString(f));
+    return CT_OK;
+}
+
+// ct_gpu_debug_early / ct_gpu_debug_primary: host arrays in and out around trace_impl on the render stream, rays in the caller's
+// order (each ray's path code is that of the ray-by-ray tested walk), synchronous.
+int debug_query(int device, int kind, uint32_t n, const double *origins, const double *directions, uint32_t park_cap,
+                uint32_t *found, uint32_t *index, float *tclosest, uint32_t *path) {
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    if (n == 0) return CT_OK;
+    double *d_o = nullptr, *d_d = nullptr; uint32_t *d_f = nullptr, *d_i = nullptr, *d_p = nullptr; float *d_tc = nullptr;
+    int rc = CT_OK;
+    auto cleanup = [&]() { cudaFree(d_o); cudaFree(d_d); cudaFree(d_f); cudaFree(d_i); cudaFree(d_p); cudaFree(d_tc); };
+#define CUX(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(CT_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); cleanup(); return rc; } } while (0)
+    CUX(cudaMalloc(&d_o, 24ull * n)); CUX(cudaMalloc(&d_d, 24ull * n));
+    CUX(cudaMalloc(&d_f, 4ull * n)); CUX(cudaMalloc(&d_i, 4ull * n)); CUX(cudaMalloc(&d_p, 4ull * n)); CUX(cudaMalloc(&d_tc, 4ull * n));
+    CUX(cudaMemcpy(d_o, origins, 24ull * n, cudaMemcpyHostToDevice));
+    CUX(cudaMemcpy(d_d, directions, 24ull * n, cudaMemcpyHostToDevice));
+    CUX(cudaStreamSynchronize(s.stream));
+    rc = trace_impl(s, kind, n, d_o, d_d, d_f, d_i, kind == CT_RAY_SHADOW ? nullptr : d_tc, d_p, park_cap, false, s.stream);
+    if (rc != CT_OK) { cudaStreamSynchronize(s.stream); cleanup(); return rc; }
+    CUX(cudaStreamSynchronize(s.stream));
+    if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
+    if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
+    if (tclosest) CUX(cudaMemcpy(tclosest, d_tc, 4ull * n, cudaMemcpyDeviceToHost));
+    if (path) CUX(cudaMemcpy(path, d_p, 4ull * n, cudaMemcpyDeviceToHost));
+    cleanup();
+#undef CUX
+    return CT_OK;
+}
+
 }  // namespace
 
 // ==== exported C ABI ==========================================================================================
@@ -1336,105 +1441,39 @@ int ct_gpu_debug_early(int device, int mode, uint32_t n, const double *origins, 
                        uint32_t *found, uint32_t *index, uint32_t *path) {
     if (!origins || !directions) return fail(CT_ERR_INVALID, "NULL ray arrays");
     if (mode != 0 && mode != 1) return fail(CT_ERR_INVALID, "mode must be 0 (shadow ray) or 1 (reflection ray)");
-    TRY(check_device(device));
-    DEVICE_GUARD(device);
-    DeviceState &s = g_dev[device];
-    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
-    if (n == 0) return CT_OK;
-    double *d_o = nullptr, *d_d = nullptr; uint32_t *d_f = nullptr, *d_i = nullptr, *d_p = nullptr, *d_occ = nullptr, *d_hpos = nullptr, *d_huge = nullptr;
-    float *d_ht = nullptr; OvfRay *d_ovf = nullptr; DevSched *d_sched = nullptr; DevTotals *d_tot = nullptr;
-    int rc = CT_OK;
-    auto cleanup = [&]() { cudaFree(d_o); cudaFree(d_d); cudaFree(d_f); cudaFree(d_i); cudaFree(d_p); cudaFree(d_occ); cudaFree(d_hpos); cudaFree(d_huge);
-                           cudaFree(d_ht); cudaFree(d_ovf); cudaFree(d_sched); cudaFree(d_tot); };
-    CUX(cudaMalloc(&d_o, 24ull * n)); CUX(cudaMalloc(&d_d, 24ull * n));
-    CUX(cudaMalloc(&d_f, 4ull * n)); CUX(cudaMalloc(&d_i, 4ull * n)); CUX(cudaMalloc(&d_p, 4ull * n));
-    CUX(cudaMalloc(&d_occ, 4ull * n)); CUX(cudaMalloc(&d_hpos, 4ull * n)); CUX(cudaMalloc(&d_ht, 4ull * n));
-    CUX(cudaMalloc(&d_sched, sizeof(DevSched))); CUX(cudaMalloc(&d_tot, sizeof(DevTotals)));
-    CUX(cudaMemcpy(d_o, origins, 24ull * n, cudaMemcpyHostToDevice));
-    CUX(cudaMemcpy(d_d, directions, 24ull * n, cudaMemcpyHostToDevice));
-    CUX(cudaMemset(d_occ, 0, 4ull * n)); CUX(cudaMemset(d_f, 0, 4ull * n)); CUX(cudaMemset(d_i, 0, 4ull * n));
-    CUX(cudaMemset(d_sched, 0, sizeof(DevSched))); CUX(cudaMemset(d_tot, 0, sizeof(DevTotals)));
-    // the scene's Params with this call's parking buffers, as a frame's launches see theirs: one occlusion word per ray (bit 0), one
-    // hit record per ray; without k_overflow launches (can_overflow false) a ray over its budget is finished in place
-    Params v = s.p;
-    v.sched = d_sched; v.tot = d_tot; v.occ = d_occ; v.occ_words = 1; v.hitb_t = d_ht; v.hitb_pos = d_hpos;
-    if (mode == 1) v.budget = first_line_budget(s);
-    v.ovf = nullptr; v.ovf_huge = nullptr; v.ovf_cap = 0;
-    if (s.can_overflow) {
-        v.ovf_cap = std::min<uint32_t>(n, s.p.ovf_cap);
-        CUX(cudaMalloc(&d_ovf, sizeof(OvfRay) * (size_t)v.ovf_cap)); CUX(cudaMalloc(&d_huge, 4ull * v.ovf_cap));
-        v.ovf = d_ovf; v.ovf_huge = d_huge;
-    }
-    CUX(cudaStreamSynchronize(s.stream));
-    const uint32_t blocks = (n + kBlockThreads - 1) / kBlockThreads;
-    if (mode == 0) k_debug_early<kAnyHit><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_f, d_i, d_p);
-    else k_debug_early<kFirstLine><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_f, d_i, d_p);
-    CUX(cudaGetLastError());
-    if (s.can_overflow) {                                     // the grids render_impl launches them with
-        if (mode == 0) { k_overflow<kAnyHit, false><<<s.n_sm * 2, kOvfThreads, 0, s.stream>>>(v, 0); k_overflow_huge<kAnyHit, false><<<s.n_sm * 4, 256, 0, s.stream>>>(v, 0); }
-        else { k_overflow<kFirstLine, false><<<s.n_sm * 2, kOvfThreads, 0, s.stream>>>(v, 0); k_overflow_huge<kFirstLine, false><<<s.n_sm * 4, 256, 0, s.stream>>>(v, 0); }
-        CUX(cudaGetLastError());
-        k_debug_early_parked<<<(n + 255) / 256, 256, 0, s.stream>>>(v, mode, n, d_f, d_i, d_p);
-        CUX(cudaGetLastError());
-    }
-    CUX(cudaStreamSynchronize(s.stream));
-    if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
-    if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
-    if (path) CUX(cudaMemcpy(path, d_p, 4ull * n, cudaMemcpyDeviceToHost));
-    cleanup();
-    return CT_OK;
+    return debug_query(device, mode == 0 ? CT_RAY_SHADOW : CT_RAY_REFLECTION, n, origins, directions, 0u, found, index, nullptr, path);
 }
 
 int ct_gpu_debug_primary(int device, uint32_t n, const double *origins, const double *directions, uint32_t park_cap,
                          uint32_t *found, uint32_t *index, float *tclosest, uint32_t *path) {
     if (!origins || !directions) return fail(CT_ERR_INVALID, "NULL ray arrays");
+    return debug_query(device, CT_RAY_PRIMARY, n, origins, directions, park_cap, found, index, tclosest, path);
+}
+
+int ct_gpu_trace_rays(int device, const ct_ray_query *q) {
+    if (!q || q->struct_size != sizeof(ct_ray_query)) return fail(CT_ERR_INVALID, "ct_ray_query missing or struct_size != %zu", sizeof(ct_ray_query));
+    if (q->kind != CT_RAY_PRIMARY && q->kind != CT_RAY_SHADOW && q->kind != CT_RAY_REFLECTION) return fail(CT_ERR_INVALID, "unknown ray kind %d", q->kind);
+    if (q->n >= (1u << 31)) return fail(CT_ERR_LIMIT, "%u rays: a query takes fewer than 2^31", q->n);
+    if (q->n > 0 && (!q->origins || !q->directions)) return fail(CT_ERR_INVALID, "NULL origins or directions with n = %u", q->n);
     TRY(check_device(device));
     DEVICE_GUARD(device);
     DeviceState &s = g_dev[device];
     if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
-    if (n == 0) return CT_OK;
-    double *d_o = nullptr, *d_d = nullptr; uint32_t *d_f = nullptr, *d_i = nullptr, *d_p = nullptr, *d_occ = nullptr, *d_hpos = nullptr;
-    float *d_ht = nullptr, *d_tc = nullptr; OvfRay *d_ovf = nullptr; DevSched *d_sched = nullptr; DevTotals *d_tot = nullptr;
-    int rc = CT_OK;
-    auto cleanup = [&]() { cudaFree(d_o); cudaFree(d_d); cudaFree(d_f); cudaFree(d_i); cudaFree(d_p); cudaFree(d_occ); cudaFree(d_hpos);
-                           cudaFree(d_ht); cudaFree(d_tc); cudaFree(d_ovf); cudaFree(d_sched); cudaFree(d_tot); };
-    CUX(cudaMalloc(&d_o, 24ull * n)); CUX(cudaMalloc(&d_d, 24ull * n));
-    CUX(cudaMalloc(&d_f, 4ull * n)); CUX(cudaMalloc(&d_i, 4ull * n)); CUX(cudaMalloc(&d_p, 4ull * n)); CUX(cudaMalloc(&d_tc, 4ull * n));
-    CUX(cudaMalloc(&d_occ, 4ull * n)); CUX(cudaMalloc(&d_hpos, 4ull * n)); CUX(cudaMalloc(&d_ht, 4ull * n));
-    CUX(cudaMalloc(&d_sched, sizeof(DevSched))); CUX(cudaMalloc(&d_tot, sizeof(DevTotals)));
-    CUX(cudaMemcpy(d_o, origins, 24ull * n, cudaMemcpyHostToDevice));
-    CUX(cudaMemcpy(d_d, directions, 24ull * n, cudaMemcpyHostToDevice));
-    CUX(cudaMemset(d_sched, 0, sizeof(DevSched))); CUX(cudaMemset(d_tot, 0, sizeof(DevTotals)));
-    // the scene's Params with this call's hit records, occlusion words and parking buffer, as k_primary's launch sees its own: path q
-    // = slot = ray i; max_depth 0, so that the hit kernels run no recursion step; no framebuffer-layout hit records
-    Params v = s.p;
-    v.sched = d_sched; v.tot = d_tot; v.occ = d_occ; v.occ_words = 1; v.hit0_t = d_ht; v.hit0_pos = d_hpos;
-    v.cap = n; v.max_depth = 0; v.dbg_found = nullptr; v.dbg_index = nullptr; v.dbg_t = nullptr;
-    v.ovf = nullptr; v.ovf_huge = nullptr; v.ovf_cap = 0; v.split_path = d_p;
-    const bool park = s.can_overflow && s.p.primary_budget > 0u;      // render_impl's rule
-    if (park) {
-        v.ovf_cap = std::min<uint32_t>(n, park_cap ? std::min(park_cap, s.p.ovf_cap) : s.p.ovf_cap);
-        CUX(cudaMalloc(&d_ovf, sizeof(OvfRay) * (size_t)v.ovf_cap));
-        v.ovf = d_ovf;
+    if (q->n == 0) return CT_OK;
+    const struct { const void *p; size_t align; const char *name; } arrays[] = {
+        {q->origins, 8, "origins"}, {q->directions, 8, "directions"}, {q->found, 4, "found"}, {q->index, 4, "index"}, {q->tclosest, 4, "tclosest"}};
+    for (const auto &a : arrays) {
+        if (!a.p) continue;
+        if ((uintptr_t)a.p % a.align) return fail(CT_ERR_INVALID, "%s is not %zu-byte aligned", a.name, a.align);
+        cudaPointerAttributes at{};
+        if (cudaPointerGetAttributes(&at, a.p) != cudaSuccess) { cudaGetLastError(); return fail(CT_ERR_INVALID, "%s: not a CUDA pointer", a.name); }
+        if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != device)
+            return fail(CT_ERR_INVALID, "%s is not device memory of device %d", a.name, device);
     }
-    CUX(cudaStreamSynchronize(s.stream));
-    const uint32_t blocks = (n + kBlockThreads - 1) / kBlockThreads;
-    if (park) k_debug_primary<true><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_p);
-    else k_debug_primary<false><<<blocks, kBlockThreads, 0, s.stream>>>(v, n, d_o, d_d, d_p);
-    CUX(cudaGetLastError());
-    if (park) {
-        launch_parked_primary(s, v, false, s.stream, 0);
-        CUX(cudaGetLastError());
-    }
-    k_debug_primary_hits<<<(n + 255) / 256, 256, 0, s.stream>>>(v, n, d_f, d_i, d_tc);
-    CUX(cudaGetLastError());
-    CUX(cudaStreamSynchronize(s.stream));
-    if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
-    if (index) CUX(cudaMemcpy(index, d_i, 4ull * n, cudaMemcpyDeviceToHost));
-    if (tclosest) CUX(cudaMemcpy(tclosest, d_tc, 4ull * n, cudaMemcpyDeviceToHost));
-    if (path) CUX(cudaMemcpy(path, d_p, 4ull * n, cudaMemcpyDeviceToHost));
-    cleanup();
-    return CT_OK;
+    const cudaStream_t st = q->stream ? static_cast<cudaStream_t>(q->stream) : s.stream;
+    const bool shadow = q->kind == CT_RAY_SHADOW;
+    return trace_impl(s, q->kind, q->n, q->origins, q->directions, q->found, shadow ? nullptr : q->index, shadow ? nullptr : q->tclosest,
+                      nullptr, 0u, CT_RAY_BINS != 0, st);
 }
 
 static int debug_primitives_impl(int device, uint32_t n, const double *origins, const double *directions, float *ray_t,

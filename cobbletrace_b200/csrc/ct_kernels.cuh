@@ -1122,16 +1122,96 @@ __global__ void k_debug_closest(const __grid_constant__ Params P, uint32_t n, co
     if (tclosest) tclosest[i] = tc;
 }
 
-// ct_gpu_debug_early: ray i is a shadow ray (kAnyHit, ray.t = 1e30f) or a reflection ray (kFirstLine, ray.t = 0) run through
-// walk_or_park as k_shadow / k_bounce run theirs; a parked ray's answer is delivered by the real k_overflow / k_overflow_huge into
-// P.occ[i] bit 0 / P.hitb_pos[i] (the caller hands them buffers of its own).  path[i]: 0 own walk, 1 parked, 3 finished in place.
+// ---- ray queries (ct_gpu_trace_rays; ct_gpu_debug_early / ct_gpu_debug_primary are host-memory wrappers of the same path) ----
+// Thread t walks ray order[t] (ray t when order is NULL): a ray's answer does not depend on which rays share its warp, so the
+// order the binning pass below gives the rays changes speed only.  Every answer -- the walk's own, and those of the parked rays
+// that the real k_overflow / k_overflow_huge, k_primary_long / k_primary_split deliver -- goes to the ray's hit record or
+// occlusion word at the CALLER's index i (the parking target), and k_ray_results turns these into the outputs at index i.
+
+// The ray's cell for the binning pass: the direction octant (3 bits), a Morton code of the origin clamped into the root box (3 x 3
+// bits) and the larger minor direction component relative to the major one (2 bits).  A ray with a non-finite component goes to
+// cell 0 (no float-to-int conversion of a NaN or an infinity).  The bit split lives here only.
+constexpr uint32_t kRayCellBits = 14, kRayCells = 1u << kRayCellBits;
+CT_DEV uint32_t ray_cell(const Params &P, const double *o, const double *d) {
+    bool finite = true;
+    for (int a = 0; a < 3; a++) finite &= isfinite(o[a]) & isfinite(d[a]);
+    if (!finite) return 0u;
+    uint32_t morton = 0;
+    for (int a = 0; a < 3; a++) {
+        const double ext = P.root_max[a] - P.root_min[a];
+        const double f = ext > 0.0 ? (o[a] - P.root_min[a]) / ext : 0.0;          // may be NaN (0 * inf) or +-inf: fmin / fmax clamp
+        const uint32_t c = min(7u, (uint32_t)(fmin(fmax(f, 0.0), 1.0) * 8.0));   // fmax(NaN, 0) = 0
+        for (int b = 0; b < 3; b++) morton |= ((c >> b) & 1u) << (3 * b + a);
+    }
+    const double ax = fabs(d[0]), ay = fabs(d[1]), az = fabs(d[2]);
+    const double major = fmax(fmax(ax, ay), az);
+    const double minor = ax == major ? fmax(ay, az) : ay == major ? fmax(ax, az) : fmax(ax, ay);
+    const uint32_t m2 = major > 0.0 ? min(3u, (uint32_t)(minor / major * 4.0)) : 0u;
+    const uint32_t oct = (d[0] < 0.0 ? 1u : 0u) | (d[1] < 0.0 ? 2u : 0u) | (d[2] < 0.0 ? 4u : 0u);
+    return (oct << 11) | (m2 << 9) | morton;
+}
+
+#ifndef CT_RAY_BINS
+#define CT_RAY_BINS 0                 // 1: queries walk their rays in the binning pass's order -- measured no faster on rays in a
+#endif                                //    random order or AO rays, slower on rays in pixel order (DESIGN.md 4, profiles/r04_trace_rays.txt)
+constexpr uint32_t kBinThreads = 512;
+constexpr uint32_t kBinChunk = 32768;   // rays per CTA of k_ray_bin_count: a 16-bit count of one cell cannot overflow
+
+// Binning, pass 1: every ray's cell, and the cells' counts -- per CTA in shared memory (two 16-bit counts to a word: kRayCells
+// of them in 32 KB), then added to count[0 .. kRayCells) (zeroed; count[kRayCells] == 0 for bb_scan).  CTA b takes rays
+// [b * kBinChunk, (b + 1) * kBinChunk).
+__global__ void __launch_bounds__(kBinThreads) k_ray_bin_count(const __grid_constant__ Params P, uint32_t n, const double *org, const double *dir,
+                                                               uint16_t *cell, uint32_t *count) {
+    __shared__ uint32_t hist[kRayCells / 2];
+    for (uint32_t c = threadIdx.x; c < kRayCells / 2; c += blockDim.x) hist[c] = 0u;
+    __syncthreads();
+    const uint32_t end = min(n, (blockIdx.x + 1u) * kBinChunk);
+    for (uint32_t i = blockIdx.x * kBinChunk + threadIdx.x; i < end; i += blockDim.x) {
+        const uint32_t c = ray_cell(P, org + 3ull * i, dir + 3ull * i);
+        cell[i] = (uint16_t)c;
+        atomicAdd(&hist[c >> 1], 1u << (16u * (c & 1u)));
+    }
+    __syncthreads();
+    for (uint32_t c = threadIdx.x; c < kRayCells; c += blockDim.x) {
+        const uint32_t k = (hist[c >> 1] >> (16u * (c & 1u))) & 0xffffu;
+        if (k) atomicAdd(&count[c], k);
+    }
+}
+
+// Binning, pass 2 (after bb_scan made count[] the cells' first positions): ray i goes to the next free position of its cell.  The
+// lanes of a warp that share a cell take their positions with one atomic.  The order within a cell is unspecified.
+__global__ void __launch_bounds__(kBinThreads) k_ray_bin_scatter(uint32_t n, const uint16_t *cell, uint32_t *start, uint32_t *order) {
+    for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
+        const uint32_t i = base + threadIdx.x;
+        const bool active = i < n;
+        const uint32_t c = active ? cell[i] : kRayCells;                 // (kRayCells: no cell, never stored)
+        const uint32_t lane = threadIdx.x & 31u, peers = __match_any_sync(kFullMask, c);
+        const uint32_t leader = __ffs(peers) - 1u, rank = __popc(peers & ((1u << lane) - 1u));
+        uint32_t at = 0;
+        if (active && lane == leader) at = atomicAdd(&start[c], (uint32_t)__popc(peers));
+        at = __shfl_sync(kFullMask, at, leader);
+        if (active) order[at + rank] = i;
+    }
+}
+
+// Which ray thread t walks (kNoPos: none).  An order entry that is not a ray index is skipped, never dereferenced.
+CT_DEV uint32_t query_ray(const uint32_t *order, uint32_t n, uint32_t t) {
+    if (t >= n) return kNoPos;
+    const uint32_t i = order ? order[t] : t;
+    return i < n ? i : kNoPos;
+}
+
+// Shadow rays (kAnyHit, ray.t = 1e30f: P.occ[i] = occluded) and reflection rays (kFirstLine, ray.t = 0: the hit record
+// P.hitb_t[i] / P.hitb_pos[i] as k_bounce writes it) through walk_or_park as k_shadow / k_bounce run theirs; the parked ones are
+// answered into the same words by k_overflow / k_overflow_huge.  path[i] (may be NULL): 0 own walk, 1 parked, 3 finished in place.
+// (__maxnreg__: left to itself ptxas gives the first-line walk 80 registers and spills; with up to 96 neither walk spills)
 template <TraverseMode MODE>
-__global__ void __launch_bounds__(kBlockThreads) k_debug_early(const __grid_constant__ Params P, uint32_t n, const double *org, const double *dir,
-                                                               uint32_t *found, uint32_t *index, uint32_t *path) {
+__global__ void __maxnreg__(96) k_debug_early(const __grid_constant__ Params P, uint32_t n, const uint32_t *order,
+                                                               const double *org, const double *dir, uint32_t *path) {
     __shared__ uint32_t walk_sm[kWalkWords * kBlockThreads];          // launched with kBlockThreads threads per block, like k_shadow
     uint32_t *const sm = MODE == kAnyHit ? walk_sm + threadIdx.x : nullptr;
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const bool active = i < n;                                         // walk_or_park is warp-level: every lane calls it
+    const uint32_t i = query_ray(order, n, blockIdx.x * blockDim.x + threadIdx.x);
+    const bool active = i != kNoPos;                                   // walk_or_park is warp-level: every lane calls it
     LocalCount lc;
     double r64[kRay64];
     TRay tr;
@@ -1142,40 +1222,23 @@ __global__ void __launch_bounds__(kBlockThreads) k_debug_early(const __grid_cons
     }
     uint32_t n_parked = 0;
     const int how = walk_or_park<MODE, false>(P, tr, r64, active, P.budget, 0, i, 0u, n_parked, lc, sm, nullptr, 0u,
-        [&](int res, float, uint32_t pos) {
-            found[i] = res == kTravHit ? 1u : 0u;
-            index[i] = (MODE == kAnyHit || pos == kNoPos) ? 0u : P.tris[pos].orig;
-        }, [](bool) {});
-    if (active) path[i] = (uint32_t)how;
+        [&](int res, float tc, uint32_t pos) {
+            if (MODE == kAnyHit) P.occ[i] = res == kTravHit ? 1u : 0u;
+            else { P.hitb_t[i] = tc; P.hitb_pos[i] = (pos == kNoPos) ? P.pos_of_tri0 : pos; }     // found is always true (:227)
+        }, [&](bool parked) { if (MODE == kAnyHit && parked) P.occ[i] = 0u; });      // k_overflow ORs the verdict in
+    if (active && path) path[i] = (uint32_t)how;
 }
 
-// ... the parked rays' answers, after k_overflow / k_overflow_huge; path 2 for the rays k_overflow handed on
-__global__ void k_debug_early_parked(const __grid_constant__ Params P, int first_line, uint32_t n, uint32_t *found, uint32_t *index, uint32_t *path) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < P.sched->huge_count[0]) path[P.ovf[P.ovf_huge[i]].target] = 2u;
-    if (i >= n) return;
-    const uint32_t how = path[i];                                      // (another thread may have made it 2 already)
-    if (how != (uint32_t)kParked && how != 2u) return;
-    if (first_line) {
-        const uint32_t pos = P.hitb_pos[i];
-        found[i] = 1u;                                                 // 0 != 1e30f (raythread.cpp:227)
-        index[i] = pos == kNoPos ? 0u : P.tris[pos].orig;
-    } else {
-        found[i] = P.occ[i] & 1u;
-        index[i] = 0u;
-    }
-}
-
-// ct_gpu_debug_primary: ray i is a primary ray (ray.t = 1e30f) of path q = slot = i run through primary_walk_or_park as k_primary runs
-// its rays; the hit record goes to P.hit0_t[i] / P.hit0_pos[i] (buffers of the caller's), that of a parked ray from the real
-// k_primary_long / k_primary_split.  path[i]: 0 own walk, 1 parked, 3 finished in place (k_primary_split rewrites its rays' codes).
+// Primary rays (ray.t = 1e30f) through primary_walk_or_park as k_primary runs its rays, path q = slot = i: the hit record goes to
+// P.hit0_t[i] / P.hit0_pos[i], that of a parked ray from the real k_primary_long / k_primary_split.  path[i] (may be NULL): 0 own
+// walk, 1 parked, 3 finished in place (k_primary_split rewrites its rays' codes through P.split_path).
 template <bool PARK>
-__global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(const __grid_constant__ Params P, uint32_t n, const double *org,
-                                                                             const double *dir, uint32_t *path) {
+__global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(const __grid_constant__ Params P, uint32_t n, const uint32_t *order,
+                                                                             const double *org, const double *dir, uint32_t *path) {
     __shared__ uint32_t closest_sm[kClosestWords * kBlockThreads];     // launched with kBlockThreads threads per block, like k_primary
     uint32_t *const sm = kSmClosest > 0 ? closest_sm + threadIdx.x : nullptr;
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const bool active = i < n;                                         // primary_walk_or_park is warp-level: every lane calls it
+    const uint32_t i = query_ray(order, n, blockIdx.x * blockDim.x + threadIdx.x);
+    const bool active = i != kNoPos;                                   // primary_walk_or_park is warp-level: every lane calls it
     LocalCount lc;
     double r64[kRay64];
     TRay r;
@@ -1189,18 +1252,29 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(con
     int res; float tc; uint32_t pos;
     const int how = primary_walk_or_park<false, PARK>(P, r, r64, active, i, i, n_parked, lc, sm, res, tc, pos);
     if (!active) return;
-    path[i] = (uint32_t)how;
+    if (path) path[i] = (uint32_t)how;
     if (how != kParked) store_primary_hit(P, i, i, -1, res == kTravHit, tc, pos);
 }
 
-// ... every ray's answer from its hit record (found, ClosestIntersection's closestIndex and tclosest)
-__global__ void k_debug_primary_hits(const __grid_constant__ Params P, uint32_t n, uint32_t *found, uint32_t *index, float *tclosest) {
+// Every ray's outputs from its hit record / occlusion word, after the parked rays' kernels (any output may be NULL):
+//   kClosest    found, ClosestIntersection's closestIndex and tclosest (P.hit0_*: pos_of_tri0 for a hit without a closestIndex);
+//   kFirstLine  found = 1 (0 != 1e30f, raythread.cpp:227), the first pass's index, tclosest 0 or FINF (P.hitb_*);
+//   kAnyHit     found = occluded, index 0 (P.occ bit 0).
+// path: 2 for the rays k_overflow handed to k_overflow_huge.
+__global__ void k_ray_results(const __grid_constant__ Params P, int mode, uint32_t n, uint32_t *found, uint32_t *index, float *tclosest,
+                              uint32_t *path) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (path && i < P.sched->huge_count[0]) path[P.ovf[P.ovf_huge[i]].target] = 2u;
     if (i >= n) return;
-    const uint32_t pos = P.hit0_pos[i];                                // pos_of_tri0 for a hit without a closestIndex: index 0
-    found[i] = pos != kNoPos ? 1u : 0u;
-    index[i] = pos == kNoPos ? 0u : P.tris[pos].orig;
-    tclosest[i] = P.hit0_t[i];
+    if (mode == kAnyHit) {
+        if (found) found[i] = P.occ[i] & 1u;
+        if (index) index[i] = 0u;
+        return;
+    }
+    const uint32_t pos = mode == kClosest ? P.hit0_pos[i] : P.hitb_pos[i];
+    if (found) found[i] = (mode == kFirstLine || pos != kNoPos) ? 1u : 0u;
+    if (index) index[i] = pos == kNoPos ? 0u : P.tris[pos].orig;
+    if (tclosest) tclosest[i] = mode == kClosest ? P.hit0_t[i] : P.hitb_t[i];
 }
 
 __global__ void k_debug_primitives(uint32_t n,const double *org, const double *dir, float *ray_t, const double *tri,

@@ -314,6 +314,46 @@ int ct_gpu_gather_rows(int src_device, int dst_device, int row_start, int row_en
  * -- those this device rendered, those gathered with ct_gpu_gather_rows, and those marked here. */
 int ct_gpu_mark_rows(int device, int row_start, int row_end);
 
+/* ---- ray queries on device memory -----------------------------------------------------------------------------
+ * ct_gpu_trace_rays traces n caller rays of one of the three kinds the reference casts through the uploaded scene.  Ray i's
+ * outputs equal, bit for bit, what the reference's ClosestIntersection (raythread.cpp:197-227) returns for it:
+ *   CT_RAY_PRIMARY     ray.t = 1e30f, the closest hit: found, index (closestIndex: the triangle's id in GetSceneTriangles order,
+ *                      0 when none) and tclosest;
+ *   CT_RAY_SHADOW      ray.t = 1e30f, occlusion (raythread.cpp:304-306): found = some reachable triangle passes with 1e-4 < t < 1e30;
+ *                      index and tclosest are not written;
+ *   CT_RAY_REFLECTION  ray.t = 0 (raythread.cpp:373): the first barycentric pass in DFS order; found is always 1, index that
+ *                      triangle's id (0 when none), tclosest 0 after a pass and FINF = 2^32 without one.
+ * The rays take the walks a frame's rays take, parking and the second-pass kernels included, under the options in effect at
+ * upload (traversal_budget, overflow_warp_budget, any_leaves, primary_budget) and at the call (primary_split).
+ *
+ * Every array lives in DEVICE (or managed) memory of `device` and holds n entries: origins and directions n x 3 doubles (8-byte
+ * aligned), found / index / tclosest n entries each (4-byte aligned; each may be NULL).  The call is asynchronous: it enqueues
+ * its work on `stream` (NULL = the device's render stream, see ct_gpu_set_stream) and returns; the outputs are valid once the
+ * stream reaches that point.  It does not synchronise: its scratch comes from the stream-ordered allocator and is freed in stream
+ * order, nothing is kept between calls, and the caller's stream is left as it is (no L2 access-policy window).  Queries read the
+ * scene's arrays only: frames, ct_gpu_get_counters, ct_gpu_overflow_stats and ct_gpu_reuse_stats are unchanged by them.  The
+ * scene must outlive the queries in flight; ct_gpu_upload_scene and ct_gpu_shutdown release the previous scene with cudaFree,
+ * which waits for all work on the device, queries included.
+ * Returns CT_OK; CT_ERR_INVALID for a NULL q, a wrong struct_size or kind, NULL rays with n > 0, an array that is not device
+ * memory of `device` (host memory, pageable or pinned, is refused) or is misaligned -- all checked before anything is enqueued;
+ * CT_ERR_LIMIT for n >= 2^31; CT_ERR_NO_SCENE; CT_ERR_OOM when the scratch cannot be allocated (nothing is enqueued then). */
+enum { CT_RAY_PRIMARY = 0, CT_RAY_SHADOW = 1, CT_RAY_REFLECTION = 2 };
+
+typedef struct ct_ray_query {
+    uint32_t struct_size;            /* = sizeof(ct_ray_query) */
+    int32_t kind;                    /* CT_RAY_* */
+    uint32_t n;                      /* rays; 0 is a no-op */
+    uint32_t _pad;
+    const double *origins;           /* n x 3 doubles, device memory of `device` */
+    const double *directions;        /* n x 3 doubles, device memory of `device` */
+    uint32_t *found;                 /* n, device memory; each output may be NULL */
+    uint32_t *index;                 /* n: closestIndex, 0 when none */
+    float *tclosest;                 /* n */
+    void *stream;                    /* cudaStream_t to run on; NULL = the device's render stream (ct_gpu_set_stream) */
+} ct_ray_query;
+
+int ct_gpu_trace_rays(int device, const ct_ray_query *q);
+
 /* Known-answer-test entry: ClosestIntersection (raythread.cpp:197-227) for n arbitrary rays through the
  * uploaded scene.  origins/directions: n x 3 doubles; t0: initial ray_t.t per ray (1e30f primary/shadow,
  * 0 for the reference's reflection rays, raythread.cpp:373).  Outputs may be NULL. */
