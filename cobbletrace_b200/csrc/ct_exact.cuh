@@ -65,7 +65,7 @@ struct TRay {
     float om;       // max|o_i|, rounded up
     bool filt;      // false: some axis cannot be bounded (d == 0, non-finite, absurd magnitudes) -> exact slab tests only
     bool tfilt;     // false: magnitudes outside the range the triangle filter's error analysis covers
-    float sg;       // tray_nearest_setup: the slop bound sigma of the order-free closest-hit walk, 0 = the ray may not take it
+    float sg;       // tray_nearest_setup: the slop bound sigma of the order-free closest-hit search (k_primary_split), 0 = the ray may not take it
     double *r64;
 };
 
@@ -117,7 +117,7 @@ CT_DEV void tray_setup(TRay &r, const Ray &ray, const double bound[3], double *r
     r.r64 = r64;
 }
 
-// Per-ray set-up of the ORDER-FREE closest-hit walk (traverse_wide_nearest, ct_traverse.cuh): sigma, a bound on
+// Per-ray set-up of the ORDER-FREE closest-hit search (k_primary_split, ct_kernels.cuh): sigma, a bound on
 //     tmin_ref(leaf box of Z) - t_ref(Z)
 // over every triangle Z of the scene that passes the reference's barycentric test for this ray -- how much EARLIER than
 // its own leaf's box a triangle can seem to be hit.  In real arithmetic that is <= 0 (a triangle lies inside the box of

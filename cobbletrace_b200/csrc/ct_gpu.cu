@@ -328,31 +328,26 @@ int read_totals(DeviceState &s, ct_ray_counters *out) {   // synchronises the st
 // The one path of the ray queries (ct_gpu_trace_rays) and of the KAT entries ct_gpu_debug_early / ct_gpu_debug_primary: n rays in
 // device memory of one kind, the walk of the frame's kernel for that kind with this call's scratch as its hit records, occlusion
 // words and parking buffers, the real second-pass kernels for the parked rays, then k_ray_results.  Enqueued on `st`; the scratch
-// is one stream-ordered allocation, freed in stream order.  bin: walk the rays in the binning pass's order (k_ray_bin_*).
+// is one stream-ordered allocation, freed in stream order.
 // park_cap: the primary rays' parking buffer, 0 = a frame's.  path (may be NULL): how each ray was finished (ct_gpu_debug_*).
 int trace_impl(DeviceState &s, int kind, uint32_t n, const double *org, const double *dir, uint32_t *found, uint32_t *index,
-               float *tclosest, uint32_t *path, uint32_t park_cap, bool bin, cudaStream_t st) {
+               float *tclosest, uint32_t *path, uint32_t park_cap, cudaStream_t st) {
     const bool primary = kind == CT_RAY_PRIMARY;
     const bool park = primary ? s.can_overflow && s.p.primary_budget > 0u : s.can_overflow;      // render_impl's rules
     uint32_t ovf_cap = 0;
     if (park) ovf_cap = std::min<uint32_t>(n, primary && park_cap ? std::min(park_cap, s.p.ovf_cap) : s.p.ovf_cap);
-    const uint32_t n_tiles = (kRayCells + 1u + kBbScanTile - 1u) / kBbScanTile;
-    // the scratch: scheduler and totals records, one occlusion word and one hit record per ray, the parking buffer and huge list,
-    // the binning arrays -- carved from one allocation (first pass: sizes only)
+    // the scratch: scheduler and totals records, one occlusion word and one hit record per ray, the parking buffer and huge list --
+    // carved from one allocation (first pass: sizes only)
     char *base = nullptr;
     size_t used = 0;
     auto take = [&](size_t bytes) { char *q = base ? base + used : nullptr; used += (bytes + 255u) & ~(size_t)255u; return q; };
     DevSched *sched = nullptr; DevTotals *tot = nullptr; uint32_t *occ = nullptr, *hpos = nullptr, *huge = nullptr; float *ht = nullptr;
-    OvfRay *ovf = nullptr; uint16_t *cell = nullptr; uint32_t *count = nullptr, *tiles = nullptr, *order = nullptr;
+    OvfRay *ovf = nullptr;
     auto carve = [&]() {
         used = 0;
         sched = (DevSched *)take(sizeof(DevSched)); tot = (DevTotals *)take(sizeof(DevTotals));
         occ = (uint32_t *)take(4ull * n); ht = (float *)take(4ull * n); hpos = (uint32_t *)take(4ull * n);
         if (ovf_cap) { ovf = (OvfRay *)take(sizeof(OvfRay) * (size_t)ovf_cap); huge = (uint32_t *)take(4ull * ovf_cap); }
-        if (bin) {
-            cell = (uint16_t *)take(2ull * n); count = (uint32_t *)take(4ull * (kRayCells + 1u));
-            tiles = (uint32_t *)take(4ull * n_tiles); order = (uint32_t *)take(4ull * n);
-        }
     };
     carve();
     cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&base), used, st);
@@ -371,22 +366,16 @@ int trace_impl(DeviceState &s, int kind, uint32_t n, const double *org, const do
     auto enqueue = [&]() -> cudaError_t {
         cudaError_t r = cudaMemsetAsync(sched, 0, (size_t)((char *)occ - (char *)sched), st);       // DevSched and DevTotals
         if (r != cudaSuccess) return r;
-        if (bin) {
-            if ((r = cudaMemsetAsync(count, 0, 4ull * (kRayCells + 1u), st)) != cudaSuccess) return r;
-            k_ray_bin_count<<<(n + kBinChunk - 1u) / kBinChunk, kBinThreads, 0, st>>>(v, n, org, dir, cell, count);
-            if ((r = bb_scan(count, kRayCells, tiles, st)) != cudaSuccess) return r;
-            k_ray_bin_scatter<<<std::min<uint32_t>((uint32_t)s.n_sm * 8u, (n + kBinThreads - 1u) / kBinThreads), kBinThreads, 0, st>>>(n, cell, count, order);
-        }
         const uint32_t blocks = (n + kBlockThreads - 1) / kBlockThreads;
         if (primary) {
-            if (park) k_debug_primary<true><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
-            else k_debug_primary<false><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            if (park) k_debug_primary<true><<<blocks, kBlockThreads, 0, st>>>(v, n, org, dir, path);
+            else k_debug_primary<false><<<blocks, kBlockThreads, 0, st>>>(v, n, org, dir, path);
             if (park) launch_parked_primary(s, v, false, st, 0);
         } else if (kind == CT_RAY_SHADOW) {
-            k_debug_early<kAnyHit><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            k_debug_early<kAnyHit><<<blocks, kBlockThreads, 0, st>>>(v, n, org, dir, path);
             if (park) { k_overflow<kAnyHit, false><<<s.n_sm * 2, kOvfThreads, 0, st>>>(v, 0); k_overflow_huge<kAnyHit, false><<<s.n_sm * 4, 256, 0, st>>>(v, 0); }
         } else {
-            k_debug_early<kFirstLine><<<blocks, kBlockThreads, 0, st>>>(v, n, order, org, dir, path);
+            k_debug_early<kFirstLine><<<blocks, kBlockThreads, 0, st>>>(v, n, org, dir, path);
             if (park) { k_overflow<kFirstLine, false><<<s.n_sm * 2, kOvfThreads, 0, st>>>(v, 0); k_overflow_huge<kFirstLine, false><<<s.n_sm * 4, 256, 0, st>>>(v, 0); }
         }
         const int mode = primary ? kClosest : kind == CT_RAY_SHADOW ? kAnyHit : kFirstLine;
@@ -418,7 +407,7 @@ int debug_query(int device, int kind, uint32_t n, const double *origins, const d
     CUX(cudaMemcpy(d_o, origins, 24ull * n, cudaMemcpyHostToDevice));
     CUX(cudaMemcpy(d_d, directions, 24ull * n, cudaMemcpyHostToDevice));
     CUX(cudaStreamSynchronize(s.stream));
-    rc = trace_impl(s, kind, n, d_o, d_d, d_f, d_i, kind == CT_RAY_SHADOW ? nullptr : d_tc, d_p, park_cap, false, s.stream);
+    rc = trace_impl(s, kind, n, d_o, d_d, d_f, d_i, kind == CT_RAY_SHADOW ? nullptr : d_tc, d_p, park_cap, s.stream);
     if (rc != CT_OK) { cudaStreamSynchronize(s.stream); cleanup(); return rc; }
     CUX(cudaStreamSynchronize(s.stream));
     if (found) CUX(cudaMemcpy(found, d_f, 4ull * n, cudaMemcpyDeviceToHost));
@@ -969,8 +958,7 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
         if (depth_max > 0) {
             // TraceRay's recursion step runs inside the hit kernels (emit_paths); what is left for a kernel of its own are the
             // reflection paths k_bounce had parked, whose hit k_overflow has just delivered
-            if (!kFusedEmit) { k_emit<<<grid, kBlockThreads, 0, st>>>(v, d, work++, nullptr, 0); TRY(mark("emit", d)); }
-            else if (d > 0 && s.can_overflow) {
+            if (d > 0 && s.can_overflow) {
                 k_emit<<<s.n_sm * 2, kBlockThreads, 0, st>>>(v, d, work++, s.ovf_all + (size_t)pk.ovf_cap * ovf_b, ovf_b);
                 TRY(mark("emit_late", d));
             }
@@ -1473,7 +1461,7 @@ int ct_gpu_trace_rays(int device, const ct_ray_query *q) {
     const cudaStream_t st = q->stream ? static_cast<cudaStream_t>(q->stream) : s.stream;
     const bool shadow = q->kind == CT_RAY_SHADOW;
     return trace_impl(s, q->kind, q->n, q->origins, q->directions, q->found, shadow ? nullptr : q->index, shadow ? nullptr : q->tclosest,
-                      nullptr, 0u, CT_RAY_BINS != 0, st);
+                      nullptr, 0u, st);
 }
 
 static int debug_primitives_impl(int device, uint32_t n, const double *origins, const double *directions, float *ray_t,

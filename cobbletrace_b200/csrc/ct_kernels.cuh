@@ -177,13 +177,12 @@ CT_DEV bool park_ray(const Params &P, int ovf_idx, const double *r64, uint32_t t
 enum { kWalked = 0, kParked = 1, kInPlace = 3 };
 template <TraverseMode MODE, bool COUNT, class Finish, class Over>
 CT_DEV int walk_or_park(const Params &P, const TRay &r, const double *r64, bool active, uint32_t budget, int ovf_idx, uint32_t target,
-                        uint32_t bit, uint32_t &n_parked, LocalCount &lc, uint32_t *sm, const DevWide *top, uint32_t n_top, Finish &&finish,
-                        Over &&over) {
+                        uint32_t bit, uint32_t &n_parked, LocalCount &lc, uint32_t *sm, Finish &&finish, Over &&over) {
     if (MODE == kAnyHit && active && (double)r.om > 0x1p20 * fmax(fmax(P.bound[0], P.bound[1]), P.bound[2])) budget = 0u;
     int how = kWalked;
     while (true) {                                                      // warp-uniform: traverse_early is warp-synchronous
         float tc; uint32_t pos;
-        const int res = traverse_early_any<MODE, COUNT>(P, r, active, budget, tc, pos, lc, sm, top, n_top);
+        const int res = traverse_early_any<MODE, COUNT>(P, r, active, budget, tc, pos, lc, sm);
         bool again = false;
         if (active) {
             if (res == kTravOverBudget) {
@@ -255,11 +254,7 @@ CT_DEV bool next_chunk(const Params &P, uint32_t n_chunks, bool &dealt_left, uin
     return false;
 }
 
-constexpr bool kFusedEmit = CT_REFILL_T == 0;      // the hit kernels run TraceRay's recursion step themselves (emit_paths)
 CT_DEV void emit_paths(const Params &P, int depth, bool active, uint32_t q, uint32_t slot, V3 o, V3 d, float tc, uint32_t pos, uint32_t &n_refl);
-
-// Lanes of `idle` in rank order: the r-th idle lane gets item r.
-CT_DEV uint32_t idle_rank(uint32_t idle) { return __popc(idle & ((1u << (threadIdx.x & 31u)) - 1u)); }
 
 // The closest-hit record of the depth-0 path (slot, q): ClosestIntersection's results as TraceRay sees them (raythread.cpp:227, :205).
 CT_DEV void store_primary_hit(const Params &P, uint32_t slot, uint32_t q, int fbi, bool found, float tc, uint32_t pos) {
@@ -274,8 +269,8 @@ CT_DEV void store_primary_hit(const Params &P, uint32_t slot, uint32_t q, int fb
     }
 }
 
-// k_primary's job (traverse_closest_refill): the warp takes chunks from the tile's cursor (next_chunk) and hands the slots
-// of its current chunk to lanes as they fall idle.
+// k_primary's rays: the warp takes chunks from the tile's cursor (next_chunk) and hands the slots of its current chunk to
+// its lanes, 32 at a time.
 struct PrimaryJob {
     uint32_t n_chunks, chunk;
     bool dealt_left;                                        // lane 0's view of this device's dealt share
@@ -283,7 +278,8 @@ struct PrimaryJob {
     uint32_t slot = 0, q = 0; int fbi = -1;                 // this lane's ray
     uint32_t n_rays = 0;
 
-    CT_DEV bool refill(const Params &P, uint32_t idle, bool &got, TRay &r, double *r64) {
+    // One slot per lane (got: the slot is a pixel to trace, r / r64 set up); false once the cursor is exhausted.
+    CT_DEV bool refill(const Params &P, bool &got, TRay &r, double *r64) {
         const uint32_t lane = threadIdx.x & 31u;
         if (pend_left == 0u) {
             unsigned long long base = ~0ull;
@@ -302,14 +298,15 @@ struct PrimaryJob {
             if (base == ~0ull) return false;
             pend_slot = (uint32_t)base; pend_q = mine << P.chunk_shift; pend_left = chunk;
         }
-        const uint32_t take = min((uint32_t)__popc(idle), pend_left), rank = idle_rank(idle);
-        if (((idle >> lane) & 1u) && rank < take) {
+        // rank == lane, written as the popcount of the lanes below it: with the plain `lane` k_primary compiles to other SASS
+        // (more spills), which measured slower together with traverse_closest's plain push (see there)
+        const uint32_t take = min(32u, pend_left), rank = __popc((1u << lane) - 1u);
+        if (rank < take) {
             slot = pend_slot + rank; q = pend_q + rank;     // q: this path's depth-0 number on this device
             int x, y;
             if (slot < P.n_slots && slot_pixel(P, slot, x, y, fbi)) {
                 const Ray ray = primary_ray(P, slot, x, y);
                 tray_setup(r, ray, P.bound, r64);
-                tray_nearest_setup(r, P.bound);
                 got = true;
             }
         }
@@ -329,9 +326,9 @@ struct PrimaryJob {
 // how it was finished (kWalked, kParked, kInPlace); res / tc / pos are the answer of a ray that was not parked.
 template <bool COUNT, bool PARK>
 CT_DEV int primary_walk_or_park(const Params &P, TRay &r, const double *r64, bool got, uint32_t target, uint32_t bit, uint32_t &n_parked,
-                                LocalCount &lc, uint32_t *sm, int &res, float &tc, uint32_t &pos) {
+                                LocalCount &lc, int &res, float &tc, uint32_t &pos) {
     const uint32_t budget = (PARK && P.primary_budget > 0u && P.ovf != nullptr) ? P.primary_budget : 0xffffffffu;
-    res = traverse_closest_any<COUNT, PARK>(P, r, got, tc, pos, lc, sm, budget);   // warp-synchronous
+    res = traverse_closest<COUNT, PARK>(P, r, got, tc, pos, lc, nullptr, budget);   // warp-synchronous
     int how = kWalked;
     const bool over = PARK && got && res == kTravOverBudget;
     if (PARK && __any_sync(kFullMask, over)) {
@@ -340,7 +337,7 @@ CT_DEV int primary_walk_or_park(const Params &P, TRay &r, const double *r64, boo
         if (__any_sync(kFullMask, redo)) {
             if (redo) r.t = kRayTInit;
             float tc2; uint32_t pos2;
-            const int res2 = traverse_closest_any<COUNT>(P, r, redo, tc2, pos2, lc, sm);
+            const int res2 = traverse_closest<COUNT>(P, r, redo, tc2, pos2, lc);
             if (redo) { res = res2; tc = tc2; pos = pos2; }
         }
     }
@@ -348,10 +345,9 @@ CT_DEV int primary_walk_or_park(const Params &P, TRay &r, const double *r64, boo
 }
 
 // Primary rays.  Persistent warps take chunks of 32 (or 64) slots from the tile's cursor (next_chunk) and remember which
-// chunks they took: the later stages of this device work on exactly those.  By default a warp walks the 32 rays of a
-// chunk together (one 8x4 pixel block: neighbouring rays visit the same nodes); -DCT_REFILL_T=n (n = 1..32) selects
-// traverse_closest_refill instead, which refills idle lanes from the next chunk -- measured SLOWER at every threshold
-// (DESIGN.md 5: 1.45 ms -> 1.86 / 2.12 / 2.29 ms for n = 16 / 8 / 4), the mixed warps lose the block's coherence.
+// chunks they took: the later stages of this device work on exactly those.  A warp walks 32 rays of a chunk together (one
+// 8x4 pixel block: neighbouring rays visit the same nodes; refilling idle lanes from the next chunk instead measured slower,
+// DESIGN.md 5).
 // PARK: walks longer than P.primary_budget pair visits are given up and parked for k_primary_long (option "primary_budget").
 template <bool COUNT, bool PARK>
 __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary(const __grid_constant__ Params P) {
@@ -361,26 +357,20 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary(const __g
     job.chunk = 1u << P.chunk_shift;
     job.n_chunks = (P.n_slots + job.chunk - 1u) >> P.chunk_shift;
     job.dealt_left = P.part_count > 1u && P.static_eighths > 0u;
-    __shared__ uint32_t closest_sm[kClosestWords * kBlockThreads];     // the top of the closest-hit walk's per-lane stack (traverse_closest)
-    uint32_t *const sm = kSmClosest > 0 ? closest_sm + threadIdx.x : nullptr;
     uint32_t n_parked = 0;
-#if CT_REFILL_T > 0
-    traverse_closest_refill<COUNT>(P, job, lc);
-#else
     while (true) {
         bool got = false;
         double r64[kRay64];
         TRay r;
-        if (!job.refill(P, kFullMask, got, r, r64)) break;    // a whole chunk's worth of slots: one per lane
+        if (!job.refill(P, got, r, r64)) break;
         int res; float tc; uint32_t pos;
-        const int how = primary_walk_or_park<COUNT, PARK>(P, r, r64, got, job.q, job.slot, n_parked, lc, sm, res, tc, pos);
+        const int how = primary_walk_or_park<COUNT, PARK>(P, r, r64, got, job.q, job.slot, n_parked, lc, res, tc, pos);
         const bool done = got && how != kParked, found = res == kTravHit;
         if (done) job.finish(P, found, tc, pos);
         if (P.max_depth > 0)          // the recursion step at once, while ray and hit are at hand (no k_emit pass over the tile)
             emit_paths(P, 0, done, job.q, job.slot, {r64[0], r64[1], r64[2]}, {r64[3], r64[4], r64[5]}, tc,
                        found ? (pos == kNoPos ? P.pos_of_tri0 : pos) : kNoPos, n_refl);
     }
-#endif
     warp_add(&P.tot->rays_reflection, n_refl);
     warp_add(&P.tot->rays_primary, job.n_rays);
     warp_add(&P.tot->rays_overflow, n_parked);
@@ -409,10 +399,9 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary_long(cons
             Ray ray; ray.o = ld3(o.o); ray.d = ld3(o.d); ray.t = kRayTInit;
             q = o.target; slot = o.bit;
             tray_setup(r, ray, P.bound, r64);
-            tray_nearest_setup(r, P.bound);
         }
         float tc; uint32_t pos;
-        const bool found = traverse_closest_any<COUNT>(P, r, active, tc, pos, lc) == kTravHit;
+        const bool found = traverse_closest<COUNT>(P, r, active, tc, pos, lc) == kTravHit;
         if (active) {
             int x, y, fbi = -1;
             if (!slot_pixel(P, slot, x, y, fbi)) fbi = -1;
@@ -428,18 +417,38 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary_long(cons
     if (COUNT) { warp_add(&P.tot->box_tests, lc.box); warp_add(&P.tot->tri_tests, lc.tri); warp_add(&P.tot->box_exact, lc.box_exact); warp_add(&P.tot->tri_exact, lc.tri_exact); }
 }
 
-// The parked primary rays, ONE RAY PER WARP (option "primary_split"): the order-free closest-hit search of traverse_wide_nearest
-// run as a frontier.  Per round every lane takes one pending node of the wide tree off a stack the warp shares, tests its
-// four children conservatively against best + 2 sigma, tests accepted leaves on the spot (a barycentric pass within best + sigma
-// becomes a candidate once the exact test of its leaf's own box confirms that the reference can reach it) and hands accepted interior
-// children back; the warp-wide minimum of t is exchanged once per round.  Afterwards the lanes' candidates within sigma of the
-// minimum are gathered and lane 0 replays the reference's update rules over them in leaf order (= the reference's test order
-// where leaf positions increase along the DFS; render_impl sends the parked rays of other trees to k_primary_long) -- the argument is
-// traverse_wide_nearest's, the CPU prototype tests/test_free_closest_prototype.py::test_frontier_walk_equals_reference_walk.
+// IntersectBVHClosest as an ORDER-FREE search (primary rays, ray.t = 1e30f).  On a nested tree the reference tests a triangle
+// iff its LEAF's own box passes IntersectAABB against the ray.t of that moment (DESIGN.md 2: ray.t only ever decreases, so
+// tmin(ancestor) <= tmin(leaf) < ray.t at the leaf's visit <= ray.t at the ancestor's visit).  Let G be the triangles with a
+// barycentric pass and 1e-4 < t < 1e30 whose leaf box passes the two conditions that do not involve ray.t, m = min t over G,
+// and sigma the ray's slop bound (tray_nearest_setup:  tmin(leaf of Z) <= t_Z + sigma  for every Z).  Then
+//   * ray.t never drops below m; the first triangle with t = m is tested unless ray.t <= tmin(its leaf) <= m + sigma by
+//     then -- either way the walk ends with ray.t <= m + sigma;
+//   * a triangle with t > tau changes the fate of one with t <= tau only by lowering ray.t to a value that blocks the
+//     latter's leaf, i.e. only if  tmin(that leaf) >= t > tau.
+// So with S = { Z in G : t_Z <= m + sigma }:  if every member of S has tmin(leaf) <= m + sigma, nothing outside S can block
+// a member of S, a tested member of S lowers ray.t below anything outside S, and replaying the reference's update rules
+// (bvh.cpp:161, 178, 212) over S alone, in leaf-position order (= the reference's test order), gives the reference's
+// ray.t, tclosest and closestIndex bit for bit.  Finding S needs no particular order: the search keeps best = min t so far
+// and prunes a box only when the LOWER end of its near bracket is >= best + 2 sigma: every triangle Z below it has
+// t_Z >= tmin(leaf of Z) - sigma >= tmin(box) - sigma >= best + sigma >= m + sigma (boxes are nested, best >= m; sigma
+// carries slack, so the inequality is strict) and is not in S.  Each barycentric pass within best + sigma becomes a
+// candidate once the exact fp64 test of its own leaf box confirms membership in G (that test also yields the reference's
+// tmin for the replay).  The argument is checked on the CPU by tests/test_free_closest_prototype.py.
+//
+// The parked primary rays, ONE RAY PER WARP (option "primary_split"): that search run as a frontier.  Per round every lane
+// takes one pending node of the wide tree off a stack the warp shares, tests its four children conservatively against
+// best + 2 sigma, tests accepted leaves on the spot (a barycentric pass within best + sigma becomes a candidate) and hands
+// accepted interior children back; the warp-wide minimum of t is exchanged once per round.  Afterwards the lanes' candidates
+// within sigma of the minimum (S) are gathered and lane 0 replays the reference's update rules over them in leaf order (= the
+// reference's test order where leaf positions increase along the DFS; render_impl sends the parked rays of other trees to
+// k_primary_long) -- the CPU prototype tests/test_free_closest_prototype.py::test_frontier_walk_equals_reference_walk.
 // A walk of ~300 DEPENDENT pair visits (the floor under k_primary, DESIGN.md 6) becomes ~12 rounds: a round descends two levels of
-// the reference's tree whatever the number of boxes the ray grazes.  Undecided rays (more than 32 candidates, a candidate whose leaf
-// starts beyond the minimum + sigma, t >= FINF, a full stack, rays outside the slop analysis) are walked by lane 0 in the
-// reference's order.  P.split_path (ct_gpu_debug_primary only) receives 2 | outcome << 8 by q, outcome one of kSplit*.
+// the reference's tree whatever the number of boxes the ray grazes.  Undecided rays (more than kNearCand candidates in a lane or 32
+// in the warp, a candidate whose leaf starts beyond the minimum + sigma, t >= FINF, a full stack, rays outside the slop analysis)
+// are walked by lane 0 in the reference's order.  P.split_path (ct_gpu_debug_primary only) receives 2 | outcome << 8 by q,
+// outcome one of kSplit*.
+constexpr int kNearCand = 4;             // candidates per lane
 constexpr int kSplitStack = 512;         // pending wide nodes per warp: (node, lower end of its near bracket)
 enum { kSplitDecided = 0, kSplitNoSigma = 1, kSplitNotNested = 2, kSplitFinf = 3, kSplitCandFull = 4, kSplitStackFull = 5,
        kSplitLate = 6, kSplitMany = 7 };
@@ -625,9 +634,6 @@ template <bool COUNT>
 __global__ void __launch_bounds__(kBlockThreads, CT_SHADOW_BLOCKS) k_shadow(const __grid_constant__ Params P, int depth, int work_idx, int ovf_idx) {
     LocalCount lc;
     uint32_t n_shadow = 0, n_parked = 0, n_reused = 0;
-    __shared__ __align__(128) DevWide top_nodes[kTopSmem > 0u ? kTopSmem : 1u];
-    __shared__ unsigned long long top_bar;
-    const uint32_t n_top = (kTopSmem > 0u && P.wide) ? stage_top_nodes(P, top_nodes, &top_bar, P.n_wide) : 0u;
     __shared__ uint32_t walk_sm[kWalkWords * kBlockThreads];          // the any-hit walk's per-lane stack and leaf list (traverse_wide)
     uint32_t *const sm = walk_sm + threadIdx.x;
     // depth >= 1 with shadow reuse: only the paths of the far list cast rays of their own; the others are counted here
@@ -665,7 +671,7 @@ __global__ void __launch_bounds__(kBlockThreads, CT_SHADOW_BLOCKS) k_shadow(cons
             n_shadow++;
             word = q * P.occ_words + (L.index >> 5); bit = L.index & 31u;
         }
-        walk_or_park<kAnyHit, COUNT>(P, tr, r64, active, P.budget, ovf_idx, word, bit, n_parked, lc, sm, top_nodes, n_top,
+        walk_or_park<kAnyHit, COUNT>(P, tr, r64, active, P.budget, ovf_idx, word, bit, n_parked, lc, sm,
                                      [&](int res, float, uint32_t) { if (res == kTravHit) atomicOr(&P.occ[word], 1u << bit); }, [](bool) {});
     }
     warp_add(&P.tot->rays_shadow, n_shadow);
@@ -726,18 +732,17 @@ CT_DEV void emit_paths(const Params &P, int depth, bool active, uint32_t q, uint
     }
 }
 
-// The same step as a kernel of its own, for the paths whose hit record a hit kernel could not finish itself: all paths of
-// `depth` (late_list == nullptr: builds in which the hit kernels do not emit, CT_REFILL_T), or the reflection paths k_bounce
-// had parked (their hit came from k_overflow).
+// The same step as a kernel of its own, for the paths whose hit record a hit kernel could not finish itself: the reflection
+// paths k_bounce had parked (late_list; their hit came from k_overflow).
 __global__ void __launch_bounds__(kBlockThreads) k_emit(const __grid_constant__ Params P, int depth, int work_idx, const OvfRay *late_list, int ovf_bounce) {
     uint32_t n_refl = 0;
-    const uint32_t n = late_list ? min(P.sched->ovf_count[ovf_bounce], P.ovf_cap) : (depth == 0 ? depth0_count(P) : P.sched->queue_count[depth]);
+    const uint32_t n = min(P.sched->ovf_count[ovf_bounce], P.ovf_cap);
     while (true) {
         unsigned long long base = warp_fetch(&P.sched->work[work_idx]);
         if (base >= n) break;
         uint32_t q = (uint32_t)base + (threadIdx.x & 31u);
         bool active = q < n;
-        if (active && late_list) q = late_list[q].target;
+        if (active) q = late_list[q].target;
         uint32_t slot = q, pos = kNoPos; int fbi = 0;
         Ray r; float tc = 0.0f;
         r.o = {0, 0, 0}; r.d = {0, 0, 0};
@@ -808,9 +813,6 @@ template <bool COUNT>
 __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_bounce(const __grid_constant__ Params P, int depth, int work_idx, int ovf_idx) {
     LocalCount lc;
     uint32_t n_parked = 0, n_refl = 0;
-    __shared__ __align__(128) DevWide top_nodes[kTopSmem > 0u ? kTopSmem : 1u];
-    __shared__ unsigned long long top_bar;
-    const uint32_t n_top = (kTopSmem > 0u && P.wide) ? stage_top_nodes(P, top_nodes, &top_bar, P.n_wide) : 0u;
     uint32_t *const sm = nullptr;                                     // (a first-line walk keeps its lists in local memory, traverse_wide)
     const uint32_t n = P.sched->queue_count[depth];
     const int cur = depth & 1;
@@ -831,7 +833,7 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_bounce(const __gr
             tray_setup(r, ray, P.bound, r64);
             clear_occ(P, q);
         }
-        walk_or_park<kFirstLine, COUNT>(P, r, r64, active, P.budget, ovf_idx, q, 0u, n_parked, lc, sm, top_nodes, n_top,
+        walk_or_park<kFirstLine, COUNT>(P, r, r64, active, P.budget, ovf_idx, q, 0u, n_parked, lc, sm,
             [&](int, float tc, uint32_t pos) {                          // found is always true: 0 != 1e30f (:227)
                 P.hitb_t[q] = tc;
                 P.hitb_pos[q] = (pos == kNoPos) ? P.pos_of_tri0 : pos;
@@ -841,12 +843,11 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_bounce(const __gr
                 far = true;                                             // k_overflow answers later: let k_shadow look at the path
                 parked = p;
             });
-        if (kFusedEmit) {             // the recursion step of the paths whose hit is final (parked ones: k_emit after k_overflow)
-            const bool fin = q < n && !parked;
-            uint32_t pslot = 0, ppos = kNoPos; float ptc = 0.0f;
-            if (fin) { pslot = P.path_slot[cur][q]; ptc = P.hitb_t[q]; ppos = P.hitb_pos[q]; }
-            emit_paths(P, depth, fin, q, pslot, {r64[0], r64[1], r64[2]}, {r64[3], r64[4], r64[5]}, ptc, ppos, n_refl);
-        }
+        // the recursion step of the paths whose hit is final (parked ones: k_emit after k_overflow)
+        const bool fin = q < n && !parked;
+        uint32_t pslot = 0, ppos = kNoPos; float ptc = 0.0f;
+        if (fin) { pslot = P.path_slot[cur][q]; ptc = P.hitb_t[q]; ppos = P.hitb_pos[q]; }
+        emit_paths(P, depth, fin, q, pslot, {r64[0], r64[1], r64[2]}, {r64[3], r64[4], r64[5]}, ptc, ppos, n_refl);
         // warp-aggregated append to the depth's far list (see shading_point_repeats: the others repeat their parent's shading point)
         if (P.reuse_shadow) {
             const uint32_t mask = __ballot_sync(kFullMask, far);
@@ -1108,13 +1109,11 @@ __global__ void k_debug_closest(const __grid_constant__ Params P, uint32_t n, co
     if (active) {
         r.o = ld3(org + 3ull * i); r.d = ld3(dir + 3ull * i); r.t = t0[i];
         tray_setup(tr, r, P.bound, r64);
-        tray_nearest_setup(tr, P.bound);
     }
     LocalCount lc; float tc, tc2; uint32_t pos, pos2;
     const bool first_line = r.t == 0.0f;
     bool f = traverse_early_any<kFirstLine, false>(P, tr, active && first_line, 0xffffffffu, tc, pos, lc, nullptr) == kTravHit;
-    __shared__ uint32_t closest_sm[kClosestWords * kBlockThreads];     // launched with kBlockThreads threads per block
-    bool f2 = traverse_closest_any<false>(P, tr, active && !first_line, tc2, pos2, lc, kSmClosest > 0 ? closest_sm + threadIdx.x : nullptr) == kTravHit;
+    bool f2 = traverse_closest<false>(P, tr, active && !first_line, tc2, pos2, lc) == kTravHit;
     if (!active) return;
     if (!first_line) { f = f2; tc = tc2; pos = pos2; }
     if (found) found[i] = f ? 1u : 0u;
@@ -1123,95 +1122,21 @@ __global__ void k_debug_closest(const __grid_constant__ Params P, uint32_t n, co
 }
 
 // ---- ray queries (ct_gpu_trace_rays; ct_gpu_debug_early / ct_gpu_debug_primary are host-memory wrappers of the same path) ----
-// Thread t walks ray order[t] (ray t when order is NULL): a ray's answer does not depend on which rays share its warp, so the
-// order the binning pass below gives the rays changes speed only.  Every answer -- the walk's own, and those of the parked rays
-// that the real k_overflow / k_overflow_huge, k_primary_long / k_primary_split deliver -- goes to the ray's hit record or
-// occlusion word at the CALLER's index i (the parking target), and k_ray_results turns these into the outputs at index i.
-
-// The ray's cell for the binning pass: the direction octant (3 bits), a Morton code of the origin clamped into the root box (3 x 3
-// bits) and the larger minor direction component relative to the major one (2 bits).  A ray with a non-finite component goes to
-// cell 0 (no float-to-int conversion of a NaN or an infinity).  The bit split lives here only.
-constexpr uint32_t kRayCellBits = 14, kRayCells = 1u << kRayCellBits;
-CT_DEV uint32_t ray_cell(const Params &P, const double *o, const double *d) {
-    bool finite = true;
-    for (int a = 0; a < 3; a++) finite &= isfinite(o[a]) & isfinite(d[a]);
-    if (!finite) return 0u;
-    uint32_t morton = 0;
-    for (int a = 0; a < 3; a++) {
-        const double ext = P.root_max[a] - P.root_min[a];
-        const double f = ext > 0.0 ? (o[a] - P.root_min[a]) / ext : 0.0;          // may be NaN (0 * inf) or +-inf: fmin / fmax clamp
-        const uint32_t c = min(7u, (uint32_t)(fmin(fmax(f, 0.0), 1.0) * 8.0));   // fmax(NaN, 0) = 0
-        for (int b = 0; b < 3; b++) morton |= ((c >> b) & 1u) << (3 * b + a);
-    }
-    const double ax = fabs(d[0]), ay = fabs(d[1]), az = fabs(d[2]);
-    const double major = fmax(fmax(ax, ay), az);
-    const double minor = ax == major ? fmax(ay, az) : ay == major ? fmax(ax, az) : fmax(ax, ay);
-    const uint32_t m2 = major > 0.0 ? min(3u, (uint32_t)(minor / major * 4.0)) : 0u;
-    const uint32_t oct = (d[0] < 0.0 ? 1u : 0u) | (d[1] < 0.0 ? 2u : 0u) | (d[2] < 0.0 ? 4u : 0u);
-    return (oct << 11) | (m2 << 9) | morton;
-}
-
-#ifndef CT_RAY_BINS
-#define CT_RAY_BINS 0                 // 1: queries walk their rays in the binning pass's order -- measured no faster on rays in a
-#endif                                //    random order or AO rays, slower on rays in pixel order (DESIGN.md 4, profiles/r04_trace_rays.txt)
-constexpr uint32_t kBinThreads = 512;
-constexpr uint32_t kBinChunk = 32768;   // rays per CTA of k_ray_bin_count: a 16-bit count of one cell cannot overflow
-
-// Binning, pass 1: every ray's cell, and the cells' counts -- per CTA in shared memory (two 16-bit counts to a word: kRayCells
-// of them in 32 KB), then added to count[0 .. kRayCells) (zeroed; count[kRayCells] == 0 for bb_scan).  CTA b takes rays
-// [b * kBinChunk, (b + 1) * kBinChunk).
-__global__ void __launch_bounds__(kBinThreads) k_ray_bin_count(const __grid_constant__ Params P, uint32_t n, const double *org, const double *dir,
-                                                               uint16_t *cell, uint32_t *count) {
-    __shared__ uint32_t hist[kRayCells / 2];
-    for (uint32_t c = threadIdx.x; c < kRayCells / 2; c += blockDim.x) hist[c] = 0u;
-    __syncthreads();
-    const uint32_t end = min(n, (blockIdx.x + 1u) * kBinChunk);
-    for (uint32_t i = blockIdx.x * kBinChunk + threadIdx.x; i < end; i += blockDim.x) {
-        const uint32_t c = ray_cell(P, org + 3ull * i, dir + 3ull * i);
-        cell[i] = (uint16_t)c;
-        atomicAdd(&hist[c >> 1], 1u << (16u * (c & 1u)));
-    }
-    __syncthreads();
-    for (uint32_t c = threadIdx.x; c < kRayCells; c += blockDim.x) {
-        const uint32_t k = (hist[c >> 1] >> (16u * (c & 1u))) & 0xffffu;
-        if (k) atomicAdd(&count[c], k);
-    }
-}
-
-// Binning, pass 2 (after bb_scan made count[] the cells' first positions): ray i goes to the next free position of its cell.  The
-// lanes of a warp that share a cell take their positions with one atomic.  The order within a cell is unspecified.
-__global__ void __launch_bounds__(kBinThreads) k_ray_bin_scatter(uint32_t n, const uint16_t *cell, uint32_t *start, uint32_t *order) {
-    for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
-        const uint32_t i = base + threadIdx.x;
-        const bool active = i < n;
-        const uint32_t c = active ? cell[i] : kRayCells;                 // (kRayCells: no cell, never stored)
-        const uint32_t lane = threadIdx.x & 31u, peers = __match_any_sync(kFullMask, c);
-        const uint32_t leader = __ffs(peers) - 1u, rank = __popc(peers & ((1u << lane) - 1u));
-        uint32_t at = 0;
-        if (active && lane == leader) at = atomicAdd(&start[c], (uint32_t)__popc(peers));
-        at = __shfl_sync(kFullMask, at, leader);
-        if (active) order[at + rank] = i;
-    }
-}
-
-// Which ray thread t walks (kNoPos: none).  An order entry that is not a ray index is skipped, never dereferenced.
-CT_DEV uint32_t query_ray(const uint32_t *order, uint32_t n, uint32_t t) {
-    if (t >= n) return kNoPos;
-    const uint32_t i = order ? order[t] : t;
-    return i < n ? i : kNoPos;
-}
+// Thread t walks ray t, in the caller's order.  Every answer -- the walk's own, and those of the parked rays that the real
+// k_overflow / k_overflow_huge, k_primary_long / k_primary_split deliver -- goes to the ray's hit record or occlusion word at the
+// CALLER's index i (the parking target), and k_ray_results turns these into the outputs at index i.
 
 // Shadow rays (kAnyHit, ray.t = 1e30f: P.occ[i] = occluded) and reflection rays (kFirstLine, ray.t = 0: the hit record
 // P.hitb_t[i] / P.hitb_pos[i] as k_bounce writes it) through walk_or_park as k_shadow / k_bounce run theirs; the parked ones are
 // answered into the same words by k_overflow / k_overflow_huge.  path[i] (may be NULL): 0 own walk, 1 parked, 3 finished in place.
 // (__maxnreg__: left to itself ptxas gives the first-line walk 80 registers and spills; with up to 96 neither walk spills)
 template <TraverseMode MODE>
-__global__ void __maxnreg__(96) k_debug_early(const __grid_constant__ Params P, uint32_t n, const uint32_t *order,
-                                                               const double *org, const double *dir, uint32_t *path) {
+__global__ void __maxnreg__(96) k_debug_early(const __grid_constant__ Params P, uint32_t n, const double *org, const double *dir,
+                                              uint32_t *path) {
     __shared__ uint32_t walk_sm[kWalkWords * kBlockThreads];          // launched with kBlockThreads threads per block, like k_shadow
     uint32_t *const sm = MODE == kAnyHit ? walk_sm + threadIdx.x : nullptr;
-    const uint32_t i = query_ray(order, n, blockIdx.x * blockDim.x + threadIdx.x);
-    const bool active = i != kNoPos;                                   // walk_or_park is warp-level: every lane calls it
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = i < n;                                         // walk_or_park is warp-level: every lane calls it
     LocalCount lc;
     double r64[kRay64];
     TRay tr;
@@ -1221,7 +1146,7 @@ __global__ void __maxnreg__(96) k_debug_early(const __grid_constant__ Params P, 
         tray_setup(tr, r, P.bound, r64);
     }
     uint32_t n_parked = 0;
-    const int how = walk_or_park<MODE, false>(P, tr, r64, active, P.budget, 0, i, 0u, n_parked, lc, sm, nullptr, 0u,
+    const int how = walk_or_park<MODE, false>(P, tr, r64, active, P.budget, 0, i, 0u, n_parked, lc, sm,
         [&](int res, float tc, uint32_t pos) {
             if (MODE == kAnyHit) P.occ[i] = res == kTravHit ? 1u : 0u;
             else { P.hitb_t[i] = tc; P.hitb_pos[i] = (pos == kNoPos) ? P.pos_of_tri0 : pos; }     // found is always true (:227)
@@ -1233,12 +1158,10 @@ __global__ void __maxnreg__(96) k_debug_early(const __grid_constant__ Params P, 
 // P.hit0_t[i] / P.hit0_pos[i], that of a parked ray from the real k_primary_long / k_primary_split.  path[i] (may be NULL): 0 own
 // walk, 1 parked, 3 finished in place (k_primary_split rewrites its rays' codes through P.split_path).
 template <bool PARK>
-__global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(const __grid_constant__ Params P, uint32_t n, const uint32_t *order,
-                                                                             const double *org, const double *dir, uint32_t *path) {
-    __shared__ uint32_t closest_sm[kClosestWords * kBlockThreads];     // launched with kBlockThreads threads per block, like k_primary
-    uint32_t *const sm = kSmClosest > 0 ? closest_sm + threadIdx.x : nullptr;
-    const uint32_t i = query_ray(order, n, blockIdx.x * blockDim.x + threadIdx.x);
-    const bool active = i != kNoPos;                                   // primary_walk_or_park is warp-level: every lane calls it
+__global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(const __grid_constant__ Params P, uint32_t n, const double *org,
+                                                                             const double *dir, uint32_t *path) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = i < n;                                         // primary_walk_or_park is warp-level: every lane calls it
     LocalCount lc;
     double r64[kRay64];
     TRay r;
@@ -1246,11 +1169,10 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_debug_primary(con
         Ray ray;
         ray.o = ld3(org + 3ull * i); ray.d = ld3(dir + 3ull * i); ray.t = kRayTInit;
         tray_setup(r, ray, P.bound, r64);
-        tray_nearest_setup(r, P.bound);
     }
     uint32_t n_parked = 0;
     int res; float tc; uint32_t pos;
-    const int how = primary_walk_or_park<false, PARK>(P, r, r64, active, i, i, n_parked, lc, sm, res, tc, pos);
+    const int how = primary_walk_or_park<false, PARK>(P, r, r64, active, i, i, n_parked, lc, res, tc, pos);
     if (!active) return;
     if (path) path[i] = (uint32_t)how;
     if (how != kParked) store_primary_hit(P, i, i, -1, res == kTravHit, tc, pos);

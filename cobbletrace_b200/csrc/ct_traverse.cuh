@@ -18,35 +18,15 @@ CT_DEV void load_tri(const DevTri *tris, uint32_t pos, V3 &p1, V3 &e1, V3 &e2) {
     e2 = {d.x, d.y, e};
 }
 
-// Optional (CT_PREFETCH=1): request the records of a pair's children as soon as the pair has arrived, so that their
-// latency overlaps this visit's slab tests.  Measured neutral-to-negative on full frames (the walks are issue
-// bound there), kept as a build-time experiment.
-CT_DEV void prefetch_children(const Params &P, const DevPair32 &pr) {
-#if defined(CT_PREFETCH) && CT_PREFETCH
-    const char *l = pr.l_cnt ? reinterpret_cast<const char *>(P.tris32 + pr.l_ref) : reinterpret_cast<const char *>(P.pairs32 + pr.l_ref);
-    const char *r = pr.r_cnt ? reinterpret_cast<const char *>(P.tris32 + pr.r_ref) : reinterpret_cast<const char *>(P.pairs32 + pr.r_ref);
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(l)); asm volatile("prefetch.global.L2 [%0];" ::"l"(l + 32));
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(r)); asm volatile("prefetch.global.L2 [%0];" ::"l"(r + 32));
-#endif
-}
-
 // 32 bytes per lane in ONE load instruction (ld.global.nc.v8 -> LDG.E.256, new with sm_100): a whole child of a wide
 // node, half a child pair.  The lanes of a walking warp read 32 different records, so every load instruction costs the
 // L1 one tag look-up per lane whatever its width -- the walks are bound by exactly that (l1tex throughput 79 % of peak in
-// k_shadow) -- and a 256-bit load halves the look-ups per record.  -DCT_LDG256=0: two 128-bit loads.  p: 32-byte aligned.
-#ifndef CT_LDG256
-#define CT_LDG256 1
-#endif
+// k_shadow) -- and a 256-bit load halves the look-ups per record.  p: 32-byte aligned.
 CT_DEV void ldg256(const void *p, float4 &a, uint4 &b) {
-#if CT_LDG256
     uint32_t x0, x1, x2, x3;
     asm("ld.global.nc.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
         : "=r"(x0), "=r"(x1), "=r"(x2), "=r"(x3), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w) : "l"(p));
     a = make_float4(__uint_as_float(x0), __uint_as_float(x1), __uint_as_float(x2), __uint_as_float(x3));
-#else
-    a = __ldg(reinterpret_cast<const float4 *>(p));
-    b = __ldg(reinterpret_cast<const uint4 *>(p) + 1);
-#endif
 }
 
 CT_DEV void load_pair32(const DevPair32 *pairs, uint32_t pid, DevPair32 &p) {
@@ -199,25 +179,18 @@ constexpr uint32_t kFullMask = 0xffffffffu;
 // lanes of a warp drift apart for the whole walk: measured 8 of 32 lanes active).
 // Returns kTravHit/kTravMiss = ray.t != 1e30f ("found"), or kTravOverBudget when the walk was given up after `budget` pair visits
 // (k_primary then parks the ray for k_primary_long: warps made of long walks only).
-#ifndef CT_SM_CLOSEST
-#define CT_SM_CLOSEST 0
-#endif
-constexpr int kSmClosest = CT_SM_CLOSEST;                         // stack entries of the closest-hit walk kept in shared memory
-constexpr int kClosestWords = kSmClosest > 0 ? 5 * kSmClosest : 1;   // k_primary declares closest_sm[kClosestWords * kBlockThreads]
-#ifndef CT_LEAF_HOLD
-#define CT_LEAF_HOLD 0
-#endif
-constexpr int kLeafHold = CT_LEAF_HOLD;
+// `spill` is never dereferenced: no push happens at sp < 0.  That branch is kept on purpose: until the compiler proves it dead,
+// its store through an unknown pointer stops LLVM from hoisting Params' fields out of the walk loop into registers, so ptxas
+// reads them from the constant bank at each use.  Without it k_primary / k_primary_long / k_primary_split compile to other
+// SASS, k_primary_long<false> with 16 more bytes of stack and more spills, and (with PrimaryJob::refill's plain `lane`) the
+// dragon 4K stages measured slower on a B200 at 1000 W: k_primary 1.546 -> 1.553 ms, k_primary_long 0.395 -> 0.414 ms.
 template <bool COUNT, bool BUDGETED = false>
-CT_DEV int traverse_closest(const Params &P, TRay &r, bool active, float &tclosest, uint32_t &closest_pos, LocalCount &lc, uint32_t *sm = nullptr,
-                            const uint32_t budget = 0xffffffffu) {
+CT_DEV int traverse_closest(const Params &P, TRay &r, bool active, float &tclosest, uint32_t &closest_pos, LocalCount &lc,
+                            uint32_t *spill = nullptr, const uint32_t budget = 0xffffffffu) {
     // stack entry = a pushed right child: (ref, cnt), the bracket of its tmin and its parent pair (to find its fp64
-    // bounds again when the bracket cannot decide).  The first kSmClosest entries live in shared memory (sm = this thread's
-    // column of the kernel's closest_sm array, five words per entry; see traverse_wide for the why), the rest in local memory.
-    constexpr int kSm = kSmClosest;
-    uint32_t stk_ref[kStackMax - kSm], stk_cnt[kStackMax - kSm], stk_src[kStackMax - kSm];
-    float stk_lo[kStackMax - kSm], stk_hi[kStackMax - kSm];
-    auto sm_at = [&](int i, int w) -> uint32_t & { return sm[(5 * i + w) * kBlockThreads]; };
+    // bounds again when the bracket cannot decide)
+    uint32_t stk_ref[kStackMax], stk_cnt[kStackMax], stk_src[kStackMax];
+    float stk_lo[kStackMax], stk_hi[kStackMax];
     int sp = 0;
     uint32_t visits = 0;       // pair visits so far
     bool over = false;
@@ -230,223 +203,6 @@ CT_DEV int traverse_closest(const Params &P, TRay &r, bool active, float &tclose
         live = root_accept(P, r);
     }
     while (__any_sync(kFullMask, live)) {
-        // -DCT_LEAF_HOLD=K (experiment): a lane that has reached a leaf waits until K lanes hold one (or nobody is left to
-        // walk), so that the triangle tests -- which otherwise run in most iterations for a handful of lanes -- are shared
-        bool hold = false;
-        if (kLeafHold > 0) {
-            const uint32_t at_leaf = __ballot_sync(kFullMask, live & (cur_cnt > 0)), walking = __ballot_sync(kFullMask, live & (cur_cnt == 0));
-            hold = walking != 0u && __popc(at_leaf) < kLeafHold;
-        }
-        if (live) {
-            bool need_pop = true;
-            if (cur_cnt > 0) {
-                if (hold) need_pop = false;
-                else for (uint32_t i = 0; i < cur_cnt; i++) {
-                    uint32_t pos = cur_ref + i;
-                    if (COUNT) lc.tri++;
-                    const TriHit th = leaf_triangle<false, COUNT>(P, r, pos, lc);
-                    if (th.hit) {
-                        if (th.t > kEps) r.t = macro_min(r.t, th.t);               // bvh.cpp:161
-                        if (r.t != kRayTInit && r.t < tclosest) {                  // bvh.cpp:212
-                            closest_pos = pos; tclosest = r.t;
-                        }
-                    }
-                }
-            } else {
-                CT_CHECK(cur_ref < P.n_pairs);
-                if (BUDGETED && ++visits > budget) { over = true; live = false; continue; }      // a long walk: the caller parks the ray (k_primary<COUNT, true>)
-                DevPair32 pr;
-                load_pair32(P.pairs32, cur_ref, pr);
-                prefetch_children(P, pr);
-                if (COUNT) lc.box += 2;
-                bool hit_l, hit_r; float r_lo, r_hi;
-                pair_accept<COUNT>(P, r, cur_ref, pr, hit_l, hit_r, r_lo, r_hi, lc);
-                if (hit_l & hit_r) {
-                    CT_CHECK(sp < kStackMax);
-                    if (sp < kSm) {
-                        sm_at(sp, 0) = pr.r_ref; sm_at(sp, 1) = pr.r_cnt; sm_at(sp, 2) = cur_ref;
-                        sm_at(sp, 3) = __float_as_uint(r_lo); sm_at(sp, 4) = __float_as_uint(r_hi);
-                    } else {
-                        const int k = sp - kSm;
-                        stk_ref[k] = pr.r_ref; stk_cnt[k] = pr.r_cnt; stk_lo[k] = r_lo; stk_hi[k] = r_hi; stk_src[k] = cur_ref;
-                    }
-                    sp++;
-                }
-                if (hit_l | hit_r) {
-                    cur_ref = hit_l ? pr.l_ref : pr.r_ref; cur_cnt = hit_l ? pr.l_cnt : pr.r_cnt;
-                    need_pop = false;
-                }
-            }
-            if (need_pop) {
-                live = false;
-                while (sp > 0) {
-                    --sp;
-                    const bool in_sm = sp < kSm;
-                    const int k = sp - kSm;
-                    const float lo = in_sm ? __uint_as_float(sm_at(sp, 3)) : stk_lo[k];
-                    if (lo >= r.t) continue;                                  // the deferred `tmin < ray.t` of bvh.cpp:178
-                    const float hi = in_sm ? __uint_as_float(sm_at(sp, 4)) : stk_hi[k];
-                    if (!(hi < r.t)) {
-                        if (COUNT) lc.box_exact++;
-                        BoxTimes e = exact_child(P.pairs64, in_sm ? sm_at(sp, 2) : stk_src[k], 1u, r.r64);
-                        if (!(e.tmin < r.t)) continue;
-                    }
-                    cur_ref = in_sm ? sm_at(sp, 0) : stk_ref[k]; cur_cnt = in_sm ? sm_at(sp, 1) : stk_cnt[k]; live = true;
-                    break;
-                }
-            }
-        }
-    }
-    if (!active) return kTravMiss;
-    if (BUDGETED && over) return kTravOverBudget;          // given up after `budget` pair visits: ray.t, tclosest, closest_pos are those of a walk half done
-    return r.t != kRayTInit ? kTravHit : kTravMiss;
-}
-
-// The same walk with CONSERVATIVE tests at the interior boxes (nested tree, r.filt: see box_maybe above).  The reference
-// reaches a leaf iff the leaf's OWN box passes IntersectAABB against the ray.t of that moment, whatever happened on the way
-// down -- so the boxes on the way only have to be accepted whenever the reference accepts them (box_maybe: the lower end of
-// the near bracket, the upper end of the far bracket: half the FMAs of pair_accept, no undecided case, no fp64 fallback),
-// and the exact verdict (certified bracket, fp64 when it cannot decide) is needed once per leaf the walk OPENS, against
-// the ray.t of that moment, from the leaf's own bounds in its parent's pair record.  The visit order stays the reference's
-// (left subtree first; a right child is pushed with the lower end of its near bracket and dropped when popped if ray.t
-// has fallen to it), so the leaves are scanned in DFS order with the reference's ray.t: same triangles tested in the same
-// order, same ray.t / tclosest / closestIndex.  Box-test COUNTS are this walk's own (a superset of the reference's boxes).
-// WARP-SYNCHRONOUS; lanes whose ray does not allow conservative tests pass active = false and take traverse_closest.
-template <bool T_FAR>
-CT_DEV bool box_maybe_lo(const TRay &r, const float bmin[3], const float bmax[3], float &near_lo) {
-    float nl[3], fh[3];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        const bool pos = r.rdf[k] > 0.0f;
-        nl[k] = __fmaf_rd(pos ? bmin[k] : bmax[k], r.rdf[k], r.cl[k]);
-        fh[k] = __fmaf_ru(pos ? bmax[k] : bmin[k], r.rdf[k], r.cu[k]);
-    }
-    near_lo = fmaxf(fmaxf(nl[0], nl[1]), nl[2]);
-    const float far_hi = fminf(fminf(fh[0], fh[1]), fh[2]);
-    const bool no = T_FAR ? ((far_hi < near_lo) | (far_hi <= 0.0f)) : ((far_hi < near_lo) | (far_hi <= 0.0f) | (near_lo >= r.t));
-    return !no;
-}
-
-template <bool COUNT>
-CT_DEV int traverse_closest_cons(const Params &P, TRay &r, bool active, float &tclosest, uint32_t &closest_pos, LocalCount &lc) {
-    uint32_t stk_ref[kStackMax], stk_cnt[kStackMax], stk_src[kStackMax];      // a pushed right child: (ref, cnt), its parent pair
-    float stk_lo[kStackMax];                                                  // ... and the lower end of its near bracket
-    int sp = 0;
-    tclosest = kFinf;          // raythread.cpp:204
-    closest_pos = kNoPos;
-    uint32_t cur_ref = P.root_ref, cur_cnt = P.root_cnt, cur_code = kNoPos;   // code = 2 * pair + side of the node's own box (kNoPos: the root)
-    bool live = false;
-    if (active) {
-        if (COUNT) lc.box++;
-        live = root_accept(P, r);
-    }
-    while (__any_sync(kFullMask, live)) {
-        if (live) {
-            bool need_pop = true;
-            if (cur_cnt > 0) {
-                bool acc = true;                                              // (the root itself: accepted above)
-                if (cur_code != kNoPos) {                                     // IntersectAABB for the leaf's own box, now
-                    const uint32_t pid = cur_code >> 1, side = cur_code & 1u;
-                    const float4 *q = reinterpret_cast<const float4 *>(P.pairs32 + pid);
-                    const float4 x = __ldg(q + side), y = __ldg(q + 1 + side);      // left: floats 0..5, right: floats 6..11
-                    float bmin[3], bmax[3];
-                    if (side == 0u) { bmin[0] = x.x; bmin[1] = x.y; bmin[2] = x.z; bmax[0] = x.w; bmax[1] = y.x; bmax[2] = y.y; }
-                    else { bmin[0] = x.z; bmin[1] = x.w; bmin[2] = y.x; bmax[0] = y.y; bmax[1] = y.z; bmax[2] = y.w; }
-                    const BoxBracket bb = box_filter(r, bmin, bmax);
-                    const bool no = bracket_geom_no(bb) | bracket_t_no(bb, r.t), yes = bracket_geom_yes(bb) & bracket_t_yes(bb, r.t);
-                    acc = yes;
-                    if (!(no | yes)) {
-                        if (COUNT) lc.box_exact++;
-                        acc = box_accept(exact_child(P.pairs64, pid, side, r.r64), r.t);
-                    }
-                }
-                if (acc) {
-                    for (uint32_t i = 0; i < cur_cnt; i++) {
-                        uint32_t pos = cur_ref + i;
-                        if (COUNT) lc.tri++;
-                        const TriHit th = leaf_triangle<false, COUNT>(P, r, pos, lc);
-                        if (th.hit) {
-                            if (th.t > kEps) r.t = macro_min(r.t, th.t);               // bvh.cpp:161
-                            if (r.t != kRayTInit && r.t < tclosest) {                  // bvh.cpp:212
-                                closest_pos = pos; tclosest = r.t;
-                            }
-                        }
-                    }
-                }
-            } else {
-                CT_CHECK(cur_ref < P.n_pairs);
-                DevPair32 pr;
-                load_pair32(P.pairs32, cur_ref, pr);
-                if (COUNT) lc.box += 2;
-                float l_lo, r_lo;
-                const bool hit_l = box_maybe_lo<false>(r, pr.lmin, pr.lmax, l_lo), hit_r = box_maybe_lo<false>(r, pr.rmin, pr.rmax, r_lo);
-                if (hit_l & hit_r) {
-                    CT_CHECK(sp < kStackMax);
-                    stk_ref[sp] = pr.r_ref; stk_cnt[sp] = pr.r_cnt; stk_lo[sp] = r_lo; stk_src[sp] = cur_ref;
-                    sp++;
-                }
-                if (hit_l | hit_r) {
-                    cur_code = 2u * cur_ref + (hit_l ? 0u : 1u);
-                    cur_ref = hit_l ? pr.l_ref : pr.r_ref; cur_cnt = hit_l ? pr.l_cnt : pr.r_cnt;
-                    need_pop = false;
-                }
-            }
-            if (need_pop) {
-                live = false;
-                while (sp > 0) {
-                    --sp;
-                    if (stk_lo[sp] >= r.t) continue;                          // tmin >= its lower bracket end >= ray.t: bvh.cpp:178 rejects it now
-                    cur_ref = stk_ref[sp]; cur_cnt = stk_cnt[sp]; cur_code = 2u * stk_src[sp] + 1u; live = true;
-                    break;
-                }
-            }
-        }
-    }
-    if (!active) return kTravMiss;
-    return r.t != kRayTInit ? kTravHit : kTravMiss;
-}
-
-// The same walk with LANE REFILL (north_star: "__ballot_sync / __shfl_sync compaction for ray regrouping"): the warp
-// does not wait for the slowest ray of a group of 32.  A lane whose walk has ended hands its result to the job and falls
-// idle; as soon as kRefillLanes lanes are idle (one ballot per iteration) the job deals new rays to exactly those lanes --
-// ranked with a prefix popcount over the idle mask -- whose set-up then runs for that many lanes at once.  Per ray nothing
-// changes (same visits, same order, same arithmetic); what changes is which rays share a warp at any moment.  Besides the
-// fuller warps this removes the per-group barrier, so a kernel ends with its longest single WALK, not its slowest group.
-// A JOB supplies the rays and takes the results:
-//     bool refill(P, idle_mask, got, r, r64)   warp-uniform.  May hand a ray to any lane of idle_mask: sets got and fills
-//                                              r / r64 (tray_setup).  Returns false once the source is exhausted.
-//     void finish(P, found, tc, pos)           per lane, when its walk has ended.
-#ifndef CT_REFILL_T
-#define CT_REFILL_T 0                 // 0: off (k_primary walks whole chunks); 1..32: idle lanes that trigger a refill
-#endif
-constexpr int kRefillLanes = CT_REFILL_T > 0 ? CT_REFILL_T : 32;
-template <bool COUNT, class Job>
-CT_DEV void traverse_closest_refill(const Params &P, Job &job, LocalCount &lc) {
-    uint32_t stk_ref[kStackMax], stk_cnt[kStackMax], stk_src[kStackMax];
-    float stk_lo[kStackMax], stk_hi[kStackMax];
-    int sp = 0;
-    float tclosest = kFinf;
-    uint32_t closest_pos = kNoPos, cur_ref = 0u, cur_cnt = 0u;
-    bool live = false;                                        // this lane holds a ray whose walk is not over
-    double r64[kRay64];
-    TRay r;
-    r.t = 0.0f; r.filt = r.tfilt = false; r.r64 = r64;
-    bool more = true;                                         // warp-uniform: the source may still hold rays
-    while (true) {
-        const uint32_t idle = __ballot_sync(kFullMask, !live);
-        if (more && __popc(idle) >= kRefillLanes) {
-            bool got = false;
-            more = job.refill(P, idle, got, r, r64);
-            if (got) {
-                sp = 0; tclosest = kFinf; closest_pos = kNoPos;                // raythread.cpp:204-205
-                cur_ref = P.root_ref; cur_cnt = P.root_cnt;
-                if (COUNT) lc.box++;
-                live = root_accept(P, r);
-                if (!live) job.finish(P, false, tclosest, closest_pos);      // missed the root box: found = false
-            }
-            continue;
-        }
-        if (idle == kFullMask) break;
         if (live) {
             bool need_pop = true;
             if (cur_cnt > 0) {
@@ -463,6 +219,7 @@ CT_DEV void traverse_closest_refill(const Params &P, Job &job, LocalCount &lc) {
                 }
             } else {
                 CT_CHECK(cur_ref < P.n_pairs);
+                if (BUDGETED && ++visits > budget) { over = true; live = false; continue; }      // a long walk: the caller parks the ray (k_primary<COUNT, true>)
                 DevPair32 pr;
                 load_pair32(P.pairs32, cur_ref, pr);
                 if (COUNT) lc.box += 2;
@@ -470,8 +227,11 @@ CT_DEV void traverse_closest_refill(const Params &P, Job &job, LocalCount &lc) {
                 pair_accept<COUNT>(P, r, cur_ref, pr, hit_l, hit_r, r_lo, r_hi, lc);
                 if (hit_l & hit_r) {
                     CT_CHECK(sp < kStackMax);
-                    stk_ref[sp] = pr.r_ref; stk_cnt[sp] = pr.r_cnt;
-                    stk_lo[sp] = r_lo; stk_hi[sp] = r_hi; stk_src[sp] = cur_ref;
+                    if (sp < 0) {
+                        for (int w = 0; w < 5; w++) spill[(5 * sp + w) * kBlockThreads] = 0u;
+                    } else {
+                        stk_ref[sp] = pr.r_ref; stk_cnt[sp] = pr.r_cnt; stk_lo[sp] = r_lo; stk_hi[sp] = r_hi; stk_src[sp] = cur_ref;
+                    }
                     sp++;
                 }
                 if (hit_l | hit_r) {
@@ -492,10 +252,12 @@ CT_DEV void traverse_closest_refill(const Params &P, Job &job, LocalCount &lc) {
                     cur_ref = stk_ref[sp]; cur_cnt = stk_cnt[sp]; live = true;
                     break;
                 }
-                if (!live) job.finish(P, r.t != kRayTInit, tclosest, closest_pos);      // raythread.cpp:227
             }
         }
     }
+    if (!active) return kTravMiss;
+    if (BUDGETED && over) return kTravOverBudget;          // given up after `budget` pair visits: ray.t, tclosest, closest_pos are those of a walk half done
+    return r.t != kRayTInit ? kTravHit : kTravMiss;
 }
 
 // The two early-exit walks.
@@ -604,37 +366,8 @@ CT_DEV int traverse_early(const Params &P, const TRay &r, bool active, const uin
 // A triangle that passes the exact test counts only if the reference's walk reaches its leaf (candidate_reached).
 // WARP-SYNCHRONOUS, same contract as traverse_early; a stack that would overflow ends the walk as kTravOverBudget (the
 // ray is parked and finished on the binary tree).
-// Optional experiment (-DCT_TOP_SMEM=M, north_star: "BVH nodes staged through shared memory or TMA for the top levels"):
-// the first M nodes of the wide tree -- they are numbered breadth first, so these are its top levels -- are copied into
-// shared memory by one bulk-copy (TMA) instruction per CTA and the walk reads them from there.  Off by default: see the
-// staging table in DESIGN.md 5.
-#ifndef CT_TOP_SMEM
-#define CT_TOP_SMEM 0
-#endif
-constexpr uint32_t kTopSmem = CT_TOP_SMEM;
-
-// Stage the top of the wide tree: thread 0 arms an mbarrier with the byte count and issues one cp.async.bulk
-// (global -> shared, completion on the mbarrier); everybody waits on the barrier's phase.  Returns the staged node count.
-CT_DEV uint32_t stage_top_nodes(const Params &P, DevWide *top, unsigned long long *bar, uint32_t n_wide) {
-    const uint32_t n_top = min(kTopSmem, n_wide);
-    if (n_top == 0u) return 0u;
-    const uint32_t bar_a = (uint32_t)__cvta_generic_to_shared(bar), dst_a = (uint32_t)__cvta_generic_to_shared(top);
-    const uint32_t bytes = n_top * (uint32_t)sizeof(DevWide);
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(dst_a), "l"(P.wide), "r"(bytes), "r"(bar_a) : "memory");
-    }
-    asm volatile("{\n .reg .pred p;\n WAIT_TOP:\n mbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n @p bra DONE_TOP;\n bra WAIT_TOP;\n DONE_TOP:\n}" ::"r"(bar_a) : "memory");
-    return n_top;
-}
-
-// THE ANY-HIT WALK'S PER-LANE LISTS LIVE IN SHARED MEMORY (-DCT_SM_WALK=0: in local memory, as in round 1).  As local arrays
+//
+// THE ANY-HIT WALK'S PER-LANE LISTS LIVE IN SHARED MEMORY.  As local arrays (round 1)
 // the pending-children stack and the deferred-leaf list were more than half of the L1's sector traffic in every walk kernel
 // (ncu, k_shadow: 137 M local sectors against 95 M global ones per launch; the lanes of a walking warp sit at different
 // depths, so one STL / LDL touches up to 32 lines), every store went through to L2 (70 M write sectors = 2.2 GB per launch,
@@ -647,9 +380,6 @@ CT_DEV uint32_t stage_top_nodes(const Params &P, DevWide *top, unsigned long lon
 // 1.153 / 6.75 (a shorter leaf list also means earlier leaf phases: occluded rays leave sooner, lit ones pay more phases).
 // The first-line walk (k_bounce) pushes leaves as well (two words per entry) and lost 2-6 % with its lists in shared
 // memory at every size tried -- its rays are less coherent and want the L1 -- so it keeps local arrays.
-#ifndef CT_SM_WALK
-#define CT_SM_WALK 1
-#endif
 #ifndef CT_SM_STACK
 #define CT_SM_STACK 8
 #endif
@@ -662,14 +392,14 @@ constexpr int kWideStack = 64;                 // pending children per lane: (kW
 #endif
 constexpr int kWideLeaves = CT_LINE_LEAVES;     // deferred leaves per lane of a first-line walk; a visit may add kWide
 constexpr int kAnyLeaves = CT_ANY_LEAVES;      // ... of an any-hit walk
-constexpr int kSmStackWords = CT_SM_WALK ? CT_SM_STACK : 0;                 // shared-memory words per lane: stack ...
-constexpr int kSmLeafWords = CT_SM_WALK ? 2 * kAnyLeaves : 0;               // ... and leaf list
-constexpr int kWalkWords = CT_SM_WALK ? kSmStackWords + kSmLeafWords : 1;   // k_shadow declares walk_sm[kWalkWords * kBlockThreads]
+constexpr int kSmStackWords = CT_SM_STACK;                   // shared-memory words per lane: stack ...
+constexpr int kSmLeafWords = 2 * kAnyLeaves;                // ... and leaf list
+constexpr int kWalkWords = kSmStackWords + kSmLeafWords;    // k_shadow declares walk_sm[kWalkWords * kBlockThreads]
 template <TraverseMode MODE, bool COUNT>
 CT_DEV int traverse_wide(const Params &P, const TRay &r, bool active, const uint32_t budget, float &tclosest, uint32_t &closest_pos, LocalCount &lc,
-                         uint32_t *sm, const DevWide *top = nullptr, uint32_t n_top = 0u) {
+                         uint32_t *sm) {
     static_assert(MODE != kClosest, "closest-hit rays use traverse_closest");
-    constexpr bool kUseSm = CT_SM_WALK && MODE == kAnyHit;                  // sm: this thread's column of walk_sm (any-hit walks only)
+    constexpr bool kUseSm = MODE == kAnyHit;                                // sm: this thread's column of walk_sm (any-hit walks only)
     constexpr int kLeaves = MODE == kAnyHit ? kAnyLeaves : kWideLeaves;
     constexpr int kSmEntries = kUseSm ? kSmStackWords : 0, kSmLeaves = kUseSm ? kAnyLeaves : 0;
     uint2 stk_spill[kWideStack - kSmEntries];             // pushed children (ref, cnt) beyond the shared-memory part
@@ -717,8 +447,6 @@ CT_DEV int traverse_wide(const Params &P, const TRay &r, bool active, const uint
                     spent += cur_cnt;
                 } else {
                     const float4 *q = reinterpret_cast<const float4 *>(P.wide + cur_ref);
-                    const bool staged = kTopSmem > 0u && cur_ref < n_top;             // (generic loads below when the experiment is on)
-                    if (staged) q = reinterpret_cast<const float4 *>(top + cur_ref);
                     if (COUNT) lc.box += kWide;
                     spent += (uint32_t)kWide;
                     if (sp > kWideStack - kWide) { result = kTravOverBudget; state = 0; nleaf = 0; sp = 0; }
@@ -726,8 +454,7 @@ CT_DEV int traverse_wide(const Params &P, const TRay &r, bool active, const uint
 #pragma unroll
                         for (int e = kWide - 1; e >= 0; e--) {             // reverse: the first accepted child is popped first
                             float4 a; uint4 b;
-                            if (kTopSmem > 0u) { a = q[2 * e]; b = *reinterpret_cast<const uint4 *>(q + 2 * e + 1); }
-                            else ldg256(q + 2 * e, a, b);
+                            ldg256(q + 2 * e, a, b);
                             const float bmin[3] = {a.x, a.y, a.z}, bmax[3] = {a.w, __uint_as_float(b.x), __uint_as_float(b.y)};
                             const bool hit = box_maybe<MODE == kAnyHit>(r, bmin, bmax);
                             if (MODE == kAnyHit) {
@@ -771,333 +498,13 @@ CT_DEV int traverse_wide(const Params &P, const TRay &r, bool active, const uint
     return result;
 }
 
-// IntersectBVHClosest over the wide tree.  On a nested tree the closest-hit walk is, like the early-exit walks, a matter of
-// its LEAVES only: with ray.t only ever decreasing,  tmin(ancestor) <= tmin(leaf) < ray.t(at the leaf's visit) <= ray.t(at
-// the ancestor's visit),  so the reference visits a leaf exactly when the leaf's own box passes IntersectAABB against the
-// ray.t of that moment -- i.e. the reference's result is that of scanning the leaves in DFS order, testing each leaf's own
-// box against the current ray.t and, where it passes, its triangles in order (bvh.cpp:198-222).  So:
-//   * the walk enumerates candidate leaves in DFS order with the conservative box_maybe against whatever ray.t it holds
-//     at the time -- never smaller than the reference's at that node, because the leaves processed so far all precede the
-//     node in DFS order -- hence a superset of the leaves the reference visits, in the reference's order;
-//   * leaves are deferred to the list and processed in the leaf phase, oldest first: the exact slab test of the leaf's
-//     own box (certified bracket, fp64 when undecided) against the CURRENT ray.t, then its triangles in order with the
-//     reference's update rules.
-// Same hits, same order, same ray.t / tclosest / closestIndex as traverse_closest; rays that do not allow conservative
-// tests (and walks whose stack would overflow) take traverse_closest.  WARP-SYNCHRONOUS.
-// How long the walk runs ahead of the leaf tests decides how stale the ray.t it prunes with is (a closest-hit walk lives on
-// pruning): a lane defers at most kClosestLeaves leaves, and a leaf phase starts as soon as kClosestLanes lanes hold one.
-#ifndef CT_CLOSEST_LEAVES
-#define CT_CLOSEST_LEAVES 1
-#endif
-#ifndef CT_CLOSEST_LANES
-#define CT_CLOSEST_LANES 24
-#endif
-constexpr int kClosestLeaves = CT_CLOSEST_LEAVES, kClosestLanes = CT_CLOSEST_LANES;
-template <bool COUNT>
-CT_DEV int traverse_wide_closest(const Params &P, TRay &r, bool active, float &tclosest, uint32_t &closest_pos, LocalCount &lc) {
-    uint2 stk[kWideStack];
-    uint2 leaf[kClosestLeaves];
-    int sp = 0, nleaf = 0;
-    uint32_t cur_ref = 0u, cur_cnt = P.root_cnt;
-    if (P.root_cnt > 0u) cur_ref = P.root_ref;
-    int state = 0;
-    bool overflow = false;
-    tclosest = kFinf;          // raythread.cpp:204
-    closest_pos = kNoPos;
-    if (active) {
-        if (COUNT) lc.box++;
-        state = root_accept(P, r) ? 1 : 0;
-    }
-    while (true) {
-        // ---- walk phase: candidate leaves in DFS order
-        while (__any_sync(kFullMask, (state == 1) & (nleaf < kClosestLeaves)) && __popc(__ballot_sync(kFullMask, nleaf > 0)) < kClosestLanes) {
-            if ((state == 1) & (nleaf < kClosestLeaves)) {
-                if (cur_cnt > 0u) {
-                    leaf[nleaf] = make_uint2(cur_ref, cur_cnt); nleaf++;
-                } else if (sp > kWideStack - kWide) {
-                    overflow = true; state = 0; nleaf = 0; sp = 0;
-                } else {
-                    const float4 *q = reinterpret_cast<const float4 *>(P.wide + cur_ref);
-                    if (COUNT) lc.box += kWide;
-#pragma unroll
-                    for (int e = kWide - 1; e >= 0; e--) {                 // reverse: the first accepted child is popped first
-                        float4 a; uint4 b;
-                        ldg256(q + 2 * e, a, b);
-                        const float bmin[3] = {a.x, a.y, a.z}, bmax[3] = {a.w, __uint_as_float(b.x), __uint_as_float(b.y)};
-                        if (box_maybe<false>(r, bmin, bmax)) { stk[sp] = make_uint2(b.z, b.w); sp++; }
-                    }
-                }
-                if (state == 1) {
-                    if (sp == 0) state = 0;
-                    else { --sp; const uint2 t = stk[sp]; cur_ref = t.x; cur_cnt = t.y; }
-                }
-            }
-        }
-        // ---- leaf phase: the deferred leaves in order; per iteration a lane either opens its next leaf (the exact test of
-        // the leaf's own box against the current ray.t) or tests one triangle of the open leaf
-        int li = 0;
-        uint32_t tri = 0;
-        bool open = false;
-        while (__any_sync(kFullMask, li < nleaf)) {
-            if (li < nleaf) {
-                const uint2 lf = leaf[li];
-                if (!open) {
-                    const uint32_t code = __ldg(P.tri_parent + lf.x);
-                    bool acc;
-                    if (code == kNoPos) acc = true;                    // the root itself: accepted before the walk (nothing has changed ray.t since)
-                    else {
-                        const uint32_t pid = code >> 1, side = code & 1u;
-                        const float4 *q = reinterpret_cast<const float4 *>(P.pairs32 + pid);
-                        const float4 x = __ldg(q + side), y = __ldg(q + 1 + side);      // left: floats 0..5, right: floats 6..11
-                        float bmin[3], bmax[3];
-                        if (side == 0u) { bmin[0] = x.x; bmin[1] = x.y; bmin[2] = x.z; bmax[0] = x.w; bmax[1] = y.x; bmax[2] = y.y; }
-                        else { bmin[0] = x.z; bmin[1] = x.w; bmin[2] = y.x; bmax[0] = y.y; bmax[1] = y.z; bmax[2] = y.w; }
-                        const BoxBracket bb = box_filter(r, bmin, bmax);
-                        const bool no = bracket_geom_no(bb) | bracket_t_no(bb, r.t), yes = bracket_geom_yes(bb) & bracket_t_yes(bb, r.t);
-                        acc = yes;
-                        if (!(no | yes)) {
-                            if (COUNT) lc.box_exact++;
-                            acc = box_accept(exact_child(P.pairs64, pid, side, r.r64), r.t);
-                        }
-                    }
-                    if (COUNT) lc.box++;
-                    if (acc) { open = true; tri = 0; } else li++;
-                } else {
-                    const uint32_t pos = lf.x + tri;
-                    if (COUNT) lc.tri++;
-                    const TriHit th = leaf_triangle<false, COUNT>(P, r, pos, lc);
-                    if (th.hit) {
-                        if (th.t > kEps) r.t = macro_min(r.t, th.t);               // bvh.cpp:161
-                        if (r.t != kRayTInit && r.t < tclosest) {                  // bvh.cpp:212
-                            closest_pos = pos; tclosest = r.t;
-                        }
-                    }
-                    if (++tri == lf.y) { open = false; li++; }
-                }
-            }
-        }
-        nleaf = 0;
-        if (!__any_sync(kFullMask, state == 1)) break;
-    }
-    if (!active) return kTravMiss;
-    if (overflow) return kTravOverBudget;
-    return r.t != kRayTInit ? kTravHit : kTravMiss;
-}
-
-// IntersectBVHClosest as an ORDER-FREE search (primary rays, ray.t = 1e30f).  On a nested tree the reference tests a triangle
-// iff its LEAF's own box passes IntersectAABB against the ray.t of that moment (see traverse_wide_closest).  Let G be the
-// triangles with a barycentric pass and 1e-4 < t < 1e30 whose leaf box passes the two conditions that do not involve ray.t,
-// m = min t over G, and sigma the ray's slop bound (tray_nearest_setup:  tmin(leaf of Z) <= t_Z + sigma  for every Z).  Then
-//   * ray.t never drops below m; the first triangle with t = m is tested unless ray.t <= tmin(its leaf) <= m + sigma by
-//     then -- either way the walk ends with ray.t <= m + sigma;
-//   * a triangle with t > tau changes the fate of one with t <= tau only by lowering ray.t to a value that blocks the
-//     latter's leaf, i.e. only if  tmin(that leaf) >= t > tau.
-// So with S = { Z in G : t_Z <= m + sigma }:  if every member of S has tmin(leaf) <= m + sigma, nothing outside S can block
-// a member of S, a tested member of S lowers ray.t below anything outside S, and replaying the reference's update rules
-// (bvh.cpp:161, 178, 212) over S alone, in leaf-position order (= the reference's test order), gives the reference's
-// ray.t, tclosest and closestIndex bit for bit.  Finding S needs no particular order: the walk keeps best = min t so far
-// and prunes a box only when the LOWER end of its near bracket is >= best + 2 sigma: every triangle Z below it has
-// t_Z >= tmin(leaf of Z) - sigma >= tmin(box) - sigma >= best + sigma >= m + sigma (boxes are nested, best >= m; sigma
-// carries slack, so the inequality is strict) and is not in S.  Each barycentric pass within best + sigma becomes a candidate once the exact fp64 test of its own leaf box confirms membership in G (that test also
-// yields the reference's tmin for the replay).  The rare leftovers -- more than kNearCand candidates, a member of S whose
-// leaf starts beyond m + sigma, t >= FINF (raythread.cpp:204's tclosest quirk), a full stack -- return kTravOverBudget
-// and take traverse_closest.  The argument is checked on the CPU by tests/test_free_closest_prototype.py.
-// What the freedom buys: conservative one-sided box tests over the wide tree (half the FMAs of the certified brackets, half
-// the dependent fetches, no fp64 fallback), leaves tested by the warp together, and a walk that may be cut short.
-// WARP-SYNCHRONOUS, same contract as traverse_closest for the rays it decides.
-#ifndef CT_NEAR_LEAVES
-#define CT_NEAR_LEAVES 1
-#endif
-#ifndef CT_NEAR_LANES
-#define CT_NEAR_LANES 24
-#endif
-constexpr int kNearLeaves = CT_NEAR_LEAVES, kNearLanes = CT_NEAR_LANES, kNearCand = 4;      // kNearLeaves = 0: leaves are tested on the spot
-constexpr int kNearLeavesCap = kNearLeaves > 0 ? kNearLeaves : 1;
-template <bool COUNT>
-CT_DEV int traverse_wide_nearest(const Params &P, const TRay &r, bool active, float &tclosest, uint32_t &closest_pos, LocalCount &lc) {
-    uint2 stk[kWideStack];
-    float stk_near[kWideStack];                           // lower end of the pushed child's near bracket
-    uint2 leaf[kNearLeavesCap];
-    float cand_t[kNearCand], cand_tmin[kNearCand];
-    uint32_t cand_pos[kNearCand], cand_code[kNearCand];
-    int sp = 0, nleaf = 0, ncand = 0;
-    float best = kRayTInit, band = kRayTInit, thr = kRayTInit;     // band >= best + sigma, thr >= best + 2 sigma
-    uint32_t cur_ref = 0u, cur_cnt = P.root_cnt;
-    if (P.root_cnt > 0u) cur_ref = P.root_ref;
-    int state = 0;
-    bool undecided = false;
-    tclosest = kFinf;          // raythread.cpp:204
-    closest_pos = kNoPos;
-    if (active) {
-        if (COUNT) lc.box++;
-        state = root_accept(P, r) ? 1 : 0;
-    }
-    auto test_triangle = [&](uint32_t pos) {
-        if (COUNT) lc.tri++;
-        const TriHit th = leaf_triangle<false, COUNT>(P, r, pos, lc);
-        if (th.hit & (th.t > kEps) & (th.t < kRayTInit)) {                     // would lower a ray.t of 1e30f (bvh.cpp:161)
-            if (!(th.t < kFinf)) undecided = true;
-            else if (th.t <= band) {
-                const uint32_t code = __ldg(P.tri_parent + pos);               // the triangle's leaf: 2 * pair + side
-                if (COUNT) lc.box_exact++;
-                const BoxTimes e = code == kNoPos ? box_times(r.r64, P.root_min, P.root_max) : exact_child(P.pairs64, code >> 1, code & 1u, r.r64);
-                if ((e.tmax >= e.tmin) & (e.tmax > 0.0f)) {                    // the leaf is one the reference can reach: Z is in G
-                    if (th.t < best) { best = th.t; band = __fadd_ru(best, r.sg); thr = __fadd_ru(band, r.sg); }
-                    if (ncand == kNearCand) {                                  // drop what has fallen out of the band
-                        int k = 0;
-                        for (int j = 0; j < kNearCand; j++)
-                            if (cand_t[j] <= band) { cand_t[k] = cand_t[j]; cand_tmin[k] = cand_tmin[j]; cand_pos[k] = cand_pos[j]; cand_code[k] = cand_code[j]; k++; }
-                        ncand = k;
-                    }
-                    if (ncand == kNearCand) undecided = true;
-                    else { cand_t[ncand] = th.t; cand_tmin[ncand] = e.tmin; cand_pos[ncand] = pos; cand_code[ncand] = code; ncand++; }
-                }
-            }
-        }
-    };
-    while (true) {
-        // ---- walk phase: one wide-node visit per walking lane and iteration
-        while (__any_sync(kFullMask, (state == 1) & (nleaf < kNearLeavesCap)) && __popc(__ballot_sync(kFullMask, nleaf > 0)) < kNearLanes) {
-            if ((state == 1) & (nleaf < kNearLeavesCap)) {
-                if (cur_cnt > 0u) {
-                    if (kNearLeaves == 0) {                                 // on the spot
-                        for (uint32_t i = 0; i < cur_cnt; i++) test_triangle(cur_ref + i);
-                        if (undecided) { state = 0; sp = 0; }
-                    }
-                    else { leaf[nleaf] = make_uint2(cur_ref, cur_cnt); nleaf++; }
-                } else if (sp > kWideStack - kWide) {
-                    undecided = true; state = 0; nleaf = 0; sp = 0;
-                } else {
-                    const float4 *q = reinterpret_cast<const float4 *>(P.wide + cur_ref);
-                    if (COUNT) lc.box += kWide;
-#pragma unroll
-                    for (int e = kWide - 1; e >= 0; e--) {                 // reverse: the first accepted child is popped first
-                        float4 a; uint4 b;
-                        ldg256(q + 2 * e, a, b);
-                        const float bmax1 = __uint_as_float(b.x), bmax2 = __uint_as_float(b.y);
-                        const bool px = r.rdf[0] > 0.0f, py = r.rdf[1] > 0.0f, pz = r.rdf[2] > 0.0f;
-                        const float n0 = __fmaf_rd(px ? a.x : a.w, r.rdf[0], r.cl[0]), f0 = __fmaf_ru(px ? a.w : a.x, r.rdf[0], r.cu[0]);
-                        const float n1 = __fmaf_rd(py ? a.y : bmax1, r.rdf[1], r.cl[1]), f1 = __fmaf_ru(py ? bmax1 : a.y, r.rdf[1], r.cu[1]);
-                        const float n2 = __fmaf_rd(pz ? a.z : bmax2, r.rdf[2], r.cl[2]), f2 = __fmaf_ru(pz ? bmax2 : a.z, r.rdf[2], r.cu[2]);
-                        const float near_lo = fmaxf(fmaxf(n0, n1), n2), far_hi = fminf(fminf(f0, f1), f2);      // box_maybe's brackets
-                        const bool no = (far_hi < near_lo) | (far_hi <= 0.0f) | (near_lo >= thr);
-                        if (!no) { stk[sp] = make_uint2(b.z, b.w); stk_near[sp] = near_lo; sp++; }
-                    }
-                }
-                if (state == 1) {
-                    state = 0;
-                    while (sp > 0) {                                       // best may have dropped since the child was pushed
-                        --sp;
-                        if (stk_near[sp] >= thr) continue;
-                        const uint2 t = stk[sp]; cur_ref = t.x; cur_cnt = t.y; state = 1;
-                        break;
-                    }
-                }
-            }
-        }
-        // ---- leaf phase: one triangle per lane and iteration
-        int li = 0;
-        uint32_t tri = 0;
-        while (__any_sync(kFullMask, li < nleaf)) {
-            if (li < nleaf) {
-                const uint2 lf = leaf[li];
-                const uint32_t pos = lf.x + tri;
-                test_triangle(pos);
-                if (++tri == lf.y) { tri = 0; li++; }
-            }
-        }
-        nleaf = 0;
-        if (undecided) { state = 0; sp = 0; }
-        if (!__any_sync(kFullMask, state == 1)) break;
-    }
-    if (!active) return kTravMiss;
-    if (undecided) return kTravOverBudget;
-    if (best == kRayTInit) return kTravMiss;                                           // ray.t never changes
-    // ---- S, its precondition, and the replay in leaf-position order
-    int n = 0;
-    for (int j = 0; j < ncand; j++)
-        if (cand_t[j] <= band) { cand_t[n] = cand_t[j]; cand_tmin[n] = cand_tmin[j]; cand_pos[n] = cand_pos[j]; cand_code[n] = cand_code[j]; n++; }
-    for (int j = 0; j < n; j++) if (!(cand_tmin[j] <= band)) return kTravOverBudget;
-    for (int j = 1; j < n; j++) {
-        const float zt = cand_t[j], zm = cand_tmin[j]; const uint32_t zp = cand_pos[j], zc = cand_code[j];
-        int k = j;
-        while (k > 0 && cand_pos[k - 1] > zp) { cand_t[k] = cand_t[k - 1]; cand_tmin[k] = cand_tmin[k - 1]; cand_pos[k] = cand_pos[k - 1]; cand_code[k] = cand_code[k - 1]; k--; }
-        cand_t[k] = zt; cand_tmin[k] = zm; cand_pos[k] = zp; cand_code[k] = zc;
-    }
-    float rt = kRayTInit;
-    uint32_t entered = 0xfffffffeu;                                                    // (no leaf has this code)
-    for (int j = 0; j < n; j++) {
-        if (cand_code[j] != entered) {                                                 // the box is tested once per leaf visit
-            if (!(cand_tmin[j] < rt)) continue;                                        // bvh.cpp:178, the leaf's own box
-            entered = cand_code[j];
-        }
-        rt = macro_min(rt, cand_t[j]);                                                 // bvh.cpp:161
-        if (rt != kRayTInit && rt < tclosest) { closest_pos = cand_pos[j]; tclosest = rt; }   // bvh.cpp:212
-    }
-    return rt != kRayTInit ? kTravHit : kTravMiss;
-}
-
-// The closest-hit walk for every lane's ray: over the wide tree where the ray allows conservative box tests, the binary
-// walk with the reference's verdict at every box otherwise.
-// Measured (DESIGN.md 5): the wide closest-hit walk is 7 % faster than the binary one on the dragon-class frame, 8 % slower
-// on the bunny and 30 % slower on scene_import.json (leaves of up to 54 triangles) -- a closest-hit walk wants its leaves
-// tested at once, which is what the binary walk does.  It is therefore an experiment: -DCT_WIDE_CLOSEST=1 switches it on.
-#ifndef CT_WIDE_CLOSEST
-#define CT_WIDE_CLOSEST 0
-#endif
-#ifndef CT_CONS_CLOSEST
-#define CT_CONS_CLOSEST 0            // 1: the ordered closest-hit walk tests interior boxes conservatively and opens leaves exactly (traverse_closest_cons) -- measured slower, DESIGN.md 5
-#endif
-#ifndef CT_NEAREST
-#define CT_NEAREST 0                 // 1: primary rays take the order-free walk (traverse_wide_nearest) where the ray allows it -- measured slower, DESIGN.md 5
-#endif
-template <bool COUNT, bool BUDGETED = false>
-CT_DEV int traverse_closest_any(const Params &P, TRay &r, bool active, float &tclosest, uint32_t &closest_pos, LocalCount &lc, uint32_t *sm = nullptr,
-                                const uint32_t budget = 0xffffffffu) {
-    if (CT_NEAREST) {
-        // r.sg > 0: tray_nearest_setup found the ray within the limits of the slop analysis (and r.filt); ray.t must be 1e30f
-        const bool fr = active & (r.sg > 0.0f) & (r.t == kRayTInit) & (P.nested != 0u) & (P.wide != nullptr);
-        int res = traverse_wide_nearest<COUNT>(P, r, fr, tclosest, closest_pos, lc);
-        const bool ordered = active & (!fr | (res == kTravOverBudget));
-        if (__any_sync(kFullMask, ordered)) {                          // the ordered walk decides the rest
-            float tc2; uint32_t pos2;
-            const int res2 = traverse_closest<COUNT>(P, r, ordered, tc2, pos2, lc);
-            if (ordered) { res = res2; tclosest = tc2; closest_pos = pos2; }
-        }
-        return res;
-    }
-    if (CT_CONS_CLOSEST) {
-        const bool cons = active & r.filt & (P.nested != 0u);
-        int res = traverse_closest_cons<COUNT>(P, r, cons, tclosest, closest_pos, lc);
-        const bool rest = active & !cons;
-        if (__any_sync(kFullMask, rest)) {                             // zero direction components, trees that are not nested
-            float tc2; uint32_t pos2;
-            const int res2 = traverse_closest<COUNT>(P, r, rest, tc2, pos2, lc);
-            if (rest) { res = res2; tclosest = tc2; closest_pos = pos2; }
-        }
-        return res;
-    }
-    if (!CT_WIDE_CLOSEST) return traverse_closest<COUNT, BUDGETED>(P, r, active, tclosest, closest_pos, lc, sm, budget);
-    const bool cons = r.filt & (P.nested != 0u) & (P.wide != nullptr);
-    const float t0 = r.t;
-    int res = traverse_wide_closest<COUNT>(P, r, active & cons, tclosest, closest_pos, lc);
-    const bool binary = active & (!cons | (res == kTravOverBudget));
-    if (__any_sync(kFullMask, binary)) {
-        float tc2; uint32_t pos2;
-        if (binary) r.t = t0;                                          // (a walk given up half way starts over)
-        const int res2 = traverse_closest<COUNT>(P, r, binary, tc2, pos2, lc);
-        if (binary) { res = res2; tclosest = tc2; closest_pos = pos2; }
-    }
-    return res;
-}
-
 // An early-exit walk for every lane's ray: over the wide tree where the ray allows conservative box tests, with the
 // reference's exact verdicts at every box of the binary tree otherwise (zero direction components, non-nested trees).
 template <TraverseMode MODE, bool COUNT>
 CT_DEV int traverse_early_any(const Params &P, const TRay &r, bool active, const uint32_t budget, float &tclosest, uint32_t &closest_pos, LocalCount &lc,
-                              uint32_t *sm, const DevWide *top = nullptr, uint32_t n_top = 0u) {
+                              uint32_t *sm) {
     const bool cons = r.filt & (P.nested != 0u) & (P.wide != nullptr);
-    int res = traverse_wide<MODE, COUNT>(P, r, active & cons, budget, tclosest, closest_pos, lc, sm, top, n_top);
+    int res = traverse_wide<MODE, COUNT>(P, r, active & cons, budget, tclosest, closest_pos, lc, sm);
     // the binary walk for the other rays, and for rays that may not be parked (no budget) whose wide stack overflowed
     const bool binary = active & (!cons | ((res == kTravOverBudget) & (budget == 0xffffffffu)));
     if (__any_sync(kFullMask, binary)) {

@@ -626,7 +626,7 @@ uint64_t ct_oracle_prehit_check(const ct_oracle_scene *s, uint64_t n, const doub
 }
 
 /* ---- prototype: the WHOLE closest-hit walk as an order-free search + a replay of the near-minimum candidates ----------
- * (what cobbletrace_b200's traverse_wide_nearest does on the device; checked here, on the CPU, against bvh_closest.)
+ * (what cobbletrace_b200's k_primary_split does on the device; checked here, on the CPU, against bvh_closest.)
  * On a nested tree the reference tests triangle Z iff its LEAF's box passes IntersectAABB against the ray.t of that moment
  * (DESIGN.md 2).  With G = the triangles with a barycentric pass and 1e-4 < t < 1e30 in leaves whose box passes the two
  * conditions that do not depend on ray.t, and m = min t over G:

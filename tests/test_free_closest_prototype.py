@@ -1,4 +1,4 @@
-"""The closest-hit walk as an order-free search, checked on the CPU before the kernel (traverse_wide_nearest) relies on it.
+"""The closest-hit walk as an order-free search, checked on the CPU before the kernel (k_primary_split) relies on it.
 oracle/ct_oracle.c holds a prototype: any visit order, boxes pruned with a margin against the best t so far, the candidates
 within a rounding slop of the minimum replayed in leaf order with the reference's update rules -- or "undecided", where the
 caller falls back to the ordered walk.  Every ray the prototype decides must equal the reference-order walk bit for bit

@@ -2,8 +2,7 @@
 
 Every answer is checked bit for bit against the oracle's ClosestIntersection (ray.t = 1e30f: primary found / index / tclosest,
 shadow found; ray.t = 0: reflection found / index / tclosest) and against the KAT entries ct_gpu_debug_primary / ct_gpu_debug_early,
-which run the same path in the caller's order.  Permuting the rays must not change any ray's bits (also with the rays binned
-before the walk, build switch -DCT_RAY_BINS=1)."""
+which run the same path in the caller's order.  Permuting the rays must not change any ray's bits."""
 import ctypes as C
 import os
 import tempfile
