@@ -27,7 +27,7 @@ ABI_SYMBOLS = [
     "ct_gpu_set_stream", "ct_gpu_render_tile", "ct_gpu_readback", "ct_gpu_readback_async", "ct_gpu_readback_wait", "ct_gpu_readback_hits", "ct_gpu_get_counters",
     "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early", "ct_gpu_debug_primary",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
-    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays",
+    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays", "ct_gpu_shade_rays",
 ]
 RAY_KINDS = {"primary": 0, "shadow": 1, "reflection": 2}     # CT_RAY_PRIMARY, CT_RAY_SHADOW, CT_RAY_REFLECTION
 
@@ -70,6 +70,11 @@ class RayQuery(C.Structure):     # == ct_ray_query
     _fields_ = [("struct_size", C.c_uint32), ("kind", C.c_int32), ("n", C.c_uint32), ("_pad", C.c_uint32),
                 ("origins", C.c_void_p), ("directions", C.c_void_p), ("found", C.c_void_p), ("index", C.c_void_p),
                 ("tclosest", C.c_void_p), ("stream", C.c_void_p)]
+
+
+class ShadeQuery(C.Structure):   # == ct_shade_query
+    _fields_ = [("struct_size", C.c_uint32), ("n", C.c_uint32), ("max_depth", C.c_int32), ("_pad", C.c_uint32),
+                ("origins", C.c_void_p), ("directions", C.c_void_p), ("color", C.c_void_p), ("stream", C.c_void_p)]
 
 
 class RayCounters(C.Structure):  # == ct_ray_counters
@@ -141,6 +146,7 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_build_bvh.argtypes = [C.c_int, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, vp]
     L.ct_gpu_debug_scene_array.argtypes = [C.c_int, C.c_char_p, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     L.ct_gpu_trace_rays.argtypes = [C.c_int, C.POINTER(RayQuery)]
+    L.ct_gpu_shade_rays.argtypes = [C.c_int, C.POINTER(ShadeQuery)]
     if path == GPU_LIB:
         _lib = L
     return L
@@ -320,6 +326,23 @@ class GpuRenderer:
     def gather_rows_to(self, dst_device: int, row_start: int, row_end: int):
         _check(self.L, self.L.ct_gpu_gather_rows(self.device, dst_device, row_start, row_end))
 
+    def _check_rays(self, origins, directions, dev):
+        """The rays trace_rays / shade_rays read in place: float64 (n, 3) contiguous tensors on this renderer's device."""
+        import torch
+        for name, a in (("origins", origins), ("directions", directions)):
+            if not isinstance(a, torch.Tensor):
+                raise ValueError(f"{name}: a torch tensor or a numpy array, not {type(a).__name__}")
+            if a.device != dev:
+                raise ValueError(f"{name} is on {a.device}, this renderer traces on {dev}")
+            if a.dtype != torch.float64:
+                raise ValueError(f"{name} is {a.dtype}, rays are float64")
+            if a.dim() != 2 or a.shape[1] != 3:
+                raise ValueError(f"{name} has shape {tuple(a.shape)}, rays are (n, 3)")
+            if not a.is_contiguous():
+                raise ValueError(f"{name} is not contiguous")
+        if origins.shape != directions.shape:
+            raise ValueError(f"origins {tuple(origins.shape)} and directions {tuple(directions.shape)} differ in shape")
+
     # -- ct_gpu_trace_rays ----------------------------------------------------------------------------
     def trace_rays(self, origins, directions, kind: str = "primary"):
         """ClosestIntersection for n rays of one kind the reference casts ("primary": ray.t = 1e30f, the closest hit; "shadow":
@@ -341,19 +364,7 @@ class GpuRenderer:
             torch.cuda.current_stream(dev).synchronize()
             found, index, t = (None if x is None else x.cpu().numpy() for x in out)
             return (found.view(np.uint32), None if index is None else index.view(np.uint32), t)
-        for name, a in (("origins", origins), ("directions", directions)):
-            if not isinstance(a, torch.Tensor):
-                raise ValueError(f"{name}: a torch tensor or a numpy array, not {type(a).__name__}")
-            if a.device != dev:
-                raise ValueError(f"{name} is on {a.device}, this renderer traces on {dev}")
-            if a.dtype != torch.float64:
-                raise ValueError(f"{name} is {a.dtype}, rays are float64")
-            if a.dim() != 2 or a.shape[1] != 3:
-                raise ValueError(f"{name} has shape {tuple(a.shape)}, rays are (n, 3)")
-            if not a.is_contiguous():
-                raise ValueError(f"{name} is not contiguous")
-        if origins.shape != directions.shape:
-            raise ValueError(f"origins {tuple(origins.shape)} and directions {tuple(directions.shape)} differ in shape")
+        self._check_rays(origins, directions, dev)
         n = origins.shape[0]
         found = torch.empty(n, dtype=torch.int32, device=dev)
         index = None if kind == "shadow" else torch.empty(n, dtype=torch.int32, device=dev)
@@ -367,6 +378,35 @@ class GpuRenderer:
         q.stream = torch.cuda.current_stream(dev).cuda_stream or 1      # (handle 0, torch's default stream, is cudaStreamLegacy = 1)
         _check(self.L, self.L.ct_gpu_trace_rays(self.device, C.byref(q)))
         return found, index, t
+
+    # -- ct_gpu_shade_rays ----------------------------------------------------------------------------
+    def shade_rays(self, origins, directions, max_depth: Optional[int] = None):
+        """TraceRay's colour (0x00BBGGRR) for n rays: lighting, shadow rays and `max_depth` levels of reflection (None: the depth
+        the scene was uploaded with), bit for bit; a miss gets the background.  See ct_gpu_shade_rays.
+
+        torch tensors: float64, shape (n, 3), contiguous, on cuda:<device>.  They are read in place, the work runs on
+        torch.cuda.current_stream(device), and the colours come back as an int32 tensor on the device that is valid in that stream's
+        order: the call does not synchronise.  numpy arrays: copied to the device, shaded, synchronised, returned as uint32 numpy.
+        Anything else raises ValueError, as trace_rays does."""
+        import torch
+        if max_depth is not None and (not isinstance(max_depth, (int, np.integer)) or isinstance(max_depth, bool) or not -2**31 <= max_depth < 2**31):
+            raise ValueError(f"max_depth must be an int or None, not {max_depth!r}")
+        dev = torch.device("cuda", self.device)
+        if isinstance(origins, np.ndarray) and isinstance(directions, np.ndarray):
+            o = torch.from_numpy(np.ascontiguousarray(origins, np.float64).reshape(-1, 3)).to(dev)
+            d = torch.from_numpy(np.ascontiguousarray(directions, np.float64).reshape(-1, 3)).to(dev)
+            color = self.shade_rays(o, d, max_depth)
+            torch.cuda.current_stream(dev).synchronize()
+            return color.cpu().numpy().view(np.uint32)
+        self._check_rays(origins, directions, dev)
+        n = origins.shape[0]
+        color = torch.empty(n, dtype=torch.int32, device=dev)
+        q = ShadeQuery()
+        q.struct_size, q.n, q.max_depth = C.sizeof(ShadeQuery), n, -1 if max_depth is None else int(max_depth)
+        q.origins, q.directions, q.color = origins.data_ptr() or None, directions.data_ptr() or None, color.data_ptr() or None
+        q.stream = torch.cuda.current_stream(dev).cuda_stream or 1      # (handle 0, torch's default stream, is cudaStreamLegacy = 1)
+        _check(self.L, self.L.ct_gpu_shade_rays(self.device, C.byref(q)))
+        return color
 
     # -- KAT entry points -----------------------------------------------------------------------------
     def debug_closest(self, origins, directions, t0):

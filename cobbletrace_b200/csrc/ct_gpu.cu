@@ -419,6 +419,219 @@ int debug_query(int device, int kind, uint32_t n, const double *origins, const d
     return CT_OK;
 }
 
+// The per-depth path state the stages of a tile or of a shade query batch work on: [depth][cap] arrays as DeviceState describes
+// them, parking buffers [2 * depth + kind][ovf_cap].  A frame's are allocated at upload, a query's per call (shade_impl).
+struct PathArrays {
+    float *hitb_t_all; uint32_t *hitb_pos_all;
+    double *rays_all; uint32_t *path_slot_all;
+    uint32_t *occ_all, *parent_q_all, *far_all;
+    OvfRay *ovf_all; uint32_t *ovf_huge_all;
+};
+
+// The stages of one tile (render_impl) or of one batch of a shade query (shade_impl, QUERY: the query forms of k_primary, k_shadow,
+// k_shade and k_resolve).  pk: what every launch starts from, pk.max_depth the depth the recursion goes to (0 without a reflective
+// material).  serial: every launch on st in the order written (CT_FLAG_STAGE_TIMING, and queries); otherwise each depth's lighting
+// chain runs on a side stream of its own (s.aux, DESIGN.md 4).  mark(name, depth) is called after each stage enqueued on st (side
+// stream stages: in serial mode only); `launches` counts the rest.
+template <bool QUERY, class Mark>
+int enqueue_stages(DeviceState &s, const Params &pk, const PathArrays &a, bool count, bool serial, cudaStream_t st, Mark &&mark,
+                   unsigned long long &launches) {
+    const int depth_max = pk.max_depth;
+    const int grid = launch_grid(s, 8);
+    int work = 0;
+    // Params as the launches of depth d see them: their own hit records, occlusion masks, ray queue in / out
+    auto view = [&](int d) {
+        Params v = pk;
+        const size_t cap = pk.cap;
+        if (a.hitb_t_all) { v.hitb_t = a.hitb_t_all + cap * d; v.hitb_pos = a.hitb_pos_all + cap * d; }
+        if (a.rays_all) {
+            v.ray_buf[d & 1] = a.rays_all + cap * 6 * d;            v.path_slot[d & 1] = a.path_slot_all + cap * d;
+            v.ray_buf[(d & 1) ^ 1] = a.rays_all + cap * 6 * (d + 1); v.path_slot[(d & 1) ^ 1] = a.path_slot_all + cap * (d + 1);
+            v.parent_q[d & 1] = a.parent_q_all + cap * d; v.parent_q[(d & 1) ^ 1] = a.parent_q_all + cap * (d + 1);
+        }
+        v.occ = a.occ_all + cap * pk.occ_words * d;
+        if (a.far_all) v.far_list = a.far_all + cap * d;
+        return v;
+    };
+    auto overflow = [&](const Params &v0, cudaStream_t q, int mode_anyhit, int ovf_idx, int depth) -> int {   // parked rays of the launch just made
+        if (!s.can_overflow) return CT_OK;
+        Params v = v0;
+        v.ovf = a.ovf_all + (size_t)pk.ovf_cap * ovf_idx; v.ovf_huge = a.ovf_huge_all + (size_t)pk.ovf_cap * ovf_idx;
+        const int g1 = s.n_sm * 2, g2 = s.n_sm * 4;
+        if (mode_anyhit) {
+            if (count) { k_overflow<kAnyHit, true><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kAnyHit, true><<<g2, 256, 0, q>>>(v, ovf_idx); }
+            else { k_overflow<kAnyHit, false><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kAnyHit, false><<<g2, 256, 0, q>>>(v, ovf_idx); }
+        } else {
+            if (count) { k_overflow<kFirstLine, true><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kFirstLine, true><<<g2, 256, 0, q>>>(v, ovf_idx); }
+            else { k_overflow<kFirstLine, false><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kFirstLine, false><<<g2, 256, 0, q>>>(v, ovf_idx); }
+        }
+        launches++;                                         // two kernels, one stage
+        return mark(mode_anyhit ? "overflow_shadow" : "overflow_bounce", depth);
+    };
+    // Two dependency chains per frame (DESIGN.md 4):
+    //   hits      primary -> emit(0) -> bounce(1) -> emit(1) -> bounce(2) -> ...          (main stream)
+    //   lighting  shadow(d) -> shade(d), needs only the hits of depth d                   (one side stream per depth)
+    // so the lighting of depth d overlaps the hit chain of depth d+1 and the lighting of the other depths; the
+    // persistent CTAs of a later kernel move into an SM as those of an earlier one run out of work, which fills
+    // the kernels' tails.  Serial: everything on the main stream instead.
+    // (Queries never count tests: count is false for them, and the query forms have no COUNT instantiations.)
+    {
+        Params v0 = view(0);              // (k_primary also runs the recursion step of depth 0: it needs the depth's queues)
+        // walks longer than primary_budget pair visits are parked (slot 0 of the parking buffers: depth 0 has no bounce launch)
+        // and walked again by k_primary_long, in warps made of long walks only
+        const bool park_primary = s.can_overflow && pk.primary_budget > 0u;
+        v0.ovf = park_primary ? a.ovf_all : nullptr;
+        if (park_primary) {
+            if (count) { if constexpr (!QUERY) k_primary<true, true><<<grid, kBlockThreads, 0, st>>>(v0); }
+            else k_primary<false, true, QUERY><<<grid, kBlockThreads, 0, st>>>(v0);
+        } else {
+            if (count) { if constexpr (!QUERY) k_primary<true, false><<<grid, kBlockThreads, 0, st>>>(v0); }
+            else k_primary<false, false, QUERY><<<grid, kBlockThreads, 0, st>>>(v0);
+        }
+        TRY(mark("primary", 0));
+        if (park_primary) {
+            const bool split = launch_parked_primary(s, v0, count, st, work);
+            if (!split) work++;
+            TRY(mark(split ? "primary_split" : "primary_long", 0));
+        }
+    }
+    for (int d = 0; d <= depth_max; d++) {
+        const Params v = view(d);
+        const int ovf_b = 2 * d, ovf_s = 2 * d + 1;
+        if (d > 0) {
+            Params vb = v;
+            vb.budget = first_line_budget(s);
+            if (s.can_overflow) { vb.ovf = a.ovf_all + (size_t)pk.ovf_cap * ovf_b; vb.ovf_huge = a.ovf_huge_all + (size_t)pk.ovf_cap * ovf_b; }
+            if (count) k_bounce<true><<<grid, kBlockThreads, 0, st>>>(vb, d, work++, ovf_b);
+            else k_bounce<false><<<grid, kBlockThreads, 0, st>>>(vb, d, work++, ovf_b);
+            TRY(mark("bounce", d));
+            TRY(overflow(v, st, 0, ovf_b, d));
+        }
+        cudaStream_t side = serial ? st : s.aux[d % 4];
+        if (!serial) { CU(cudaEventRecord(s.ev_hit[d], st)); CU(cudaStreamWaitEvent(side, s.ev_hit[d], 0)); }
+        if (depth_max > 0) {
+            // TraceRay's recursion step runs inside the hit kernels (emit_paths); what is left for a kernel of its own are the
+            // reflection paths k_bounce had parked, whose hit k_overflow has just delivered
+            if (d > 0 && s.can_overflow) {
+                k_emit<<<s.n_sm * 2, kBlockThreads, 0, st>>>(v, d, work++, a.ovf_all + (size_t)pk.ovf_cap * ovf_b, ovf_b);
+                TRY(mark("emit_late", d));
+            }
+        }
+        if (pk.n_slights > 0) {
+            Params vs = v;
+            if (s.can_overflow) { vs.ovf = a.ovf_all + (size_t)pk.ovf_cap * ovf_s; vs.ovf_huge = a.ovf_huge_all + (size_t)pk.ovf_cap * ovf_s; }
+            if (count) { if constexpr (!QUERY) k_shadow<true><<<grid, kBlockThreads, 0, side>>>(vs, d, work++, ovf_s); }
+            else k_shadow<false, QUERY><<<grid, kBlockThreads, 0, side>>>(vs, d, work++, ovf_s);
+            if (serial) TRY(mark("shadow", d)); else launches++;
+            if (serial) { TRY(overflow(v, side, 1, ovf_s, d)); }
+            else if (s.can_overflow) {
+                Params vo = v;
+                vo.ovf = a.ovf_all + (size_t)pk.ovf_cap * ovf_s; vo.ovf_huge = a.ovf_huge_all + (size_t)pk.ovf_cap * ovf_s;
+                if (count) { k_overflow<kAnyHit, true><<<s.n_sm * 2, kOvfThreads, 0, side>>>(vo, ovf_s); k_overflow_huge<kAnyHit, true><<<s.n_sm * 4, 256, 0, side>>>(vo, ovf_s); }
+                else { k_overflow<kAnyHit, false><<<s.n_sm * 2, kOvfThreads, 0, side>>>(vo, ovf_s); k_overflow_huge<kAnyHit, false><<<s.n_sm * 4, 256, 0, side>>>(vo, ovf_s); }
+                launches += 2;
+            }
+        }
+        if (!serial) {
+            // k_shade(d) may read the shadow verdicts of shallower depths (occlusion_source): they are complete at ev_lit
+            CU(cudaEventRecord(s.ev_lit[d], side));
+            for (int dd = 0; dd < d; dd++) CU(cudaStreamWaitEvent(side, s.ev_lit[dd], 0));
+        }
+        k_shade<QUERY><<<grid, kBlockThreads, 0, side>>>(v, d, work++);
+        if (serial) TRY(mark("shade", d)); else launches++;
+        if (!serial) CU(cudaEventRecord(s.ev_done[d], side));
+    }
+    if (!serial) for (int d = 0; d <= depth_max; d++) CU(cudaStreamWaitEvent(st, s.ev_done[d], 0));
+    if (depth_max > 0) { k_resolve<QUERY><<<s.n_sm * 4, 256, 0, st>>>(pk); TRY(mark("resolve", 0)); }
+    if (pk.supersample) { k_supersample<<<s.n_sm * 4, 256, 0, st>>>(pk); TRY(mark("supersample", 0)); }
+    if (pk.subsample) { k_subsample<<<s.n_sm * 4, 256, 0, st>>>(pk); TRY(mark("subsample", 0)); }
+    return CT_OK;
+}
+
+
+// Rays a shade query takes per batch: its path state is carved for this many, whatever n is (the bound ct_gpu.h states).
+constexpr uint32_t kShadeBatch = 1u << 20;
+
+// ct_gpu_shade_rays: TraceRay (raythread.cpp:353-386) for n caller rays, recursion depth max_depth, through the frame's own stages
+// (enqueue_stages<true>, serialised on st) -- the caller's ray i is depth-0 slot i of its batch, its colour goes to color[i].  The
+// batches of at most kShadeBatch rays reuse one stream-ordered allocation: the path state of every level, carved like upload's, and
+// parking buffers of min(batch, the frame's ovf_cap) rays.  Nothing is synchronised; the scratch is freed in stream order.
+int shade_impl(DeviceState &s, uint32_t n, int max_depth, const double *org, const double *dir, uint32_t *color, cudaStream_t st) {
+    const int depth_max = s.any_reflective ? max_depth : 0;       // render_impl's rule: without a reflective material TraceRay stops at :369
+    const size_t levels = (size_t)depth_max + 1;
+    const uint32_t batch = std::min(n, kShadeBatch);
+    const size_t cap = (batch + kChunkMax - 1u) / kChunkMax * kChunkMax;
+    const uint32_t ovf_cap = s.can_overflow ? std::min<uint32_t>(batch, s.p.ovf_cap) : 0u;
+    const size_t words = s.p.occ_words;
+    char *base = nullptr;
+    size_t used = 0;
+    auto take = [&](size_t bytes) { char *q = base ? base + used : nullptr; used += (bytes + 255u) & ~(size_t)255u; return q; };
+    Params pk = s.p;
+    PathArrays a{};
+    auto carve = [&]() {                                            // (first pass: sizes only)
+        used = 0;
+        pk.sched = (DevSched *)take(sizeof(DevSched)); pk.tot = (DevTotals *)take(sizeof(DevTotals));
+        pk.hit0_t = (float *)take(4 * cap); pk.hit0_pos = (uint32_t *)take(4 * cap);
+        pk.stack_color = (uint32_t *)take(4 * cap * levels);
+        pk.term_level = (uint8_t *)take(cap);
+        pk.own_chunks = (uint32_t *)take(4 * ((cap >> kChunkLocalShift) + 1));
+        a.occ_all = (uint32_t *)take(4 * cap * words * levels);
+        if (ovf_cap) { a.ovf_all = (OvfRay *)take(sizeof(OvfRay) * ovf_cap * 2 * levels); a.ovf_huge_all = (uint32_t *)take(4ull * ovf_cap * 2 * levels); }
+        if (levels > 1) {
+            a.hitb_t_all = (float *)take(4 * cap * levels); a.hitb_pos_all = (uint32_t *)take(4 * cap * levels);
+            pk.stack_refl = (float *)take(4 * cap * levels);
+            a.rays_all = (double *)take(48 * cap * (levels + 1)); a.path_slot_all = (uint32_t *)take(4 * cap * (levels + 1));
+            a.parent_q_all = (uint32_t *)take(4 * cap * (levels + 1));
+            a.far_all = (uint32_t *)take(4 * cap * levels);
+        }
+    };
+    carve();
+    cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&base), used, st);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "cudaMallocAsync(%zu bytes): %s", used, cudaGetErrorString(e));
+    }
+    carve();
+    if (levels == 1) pk.stack_refl = nullptr;
+    pk.max_depth = depth_max;
+    pk.cap = (uint32_t)cap;
+    pk.occ = a.occ_all;
+    pk.parent_q_all = a.parent_q_all; pk.hitb_t_all = a.hitb_t_all; pk.occ_all = a.occ_all;
+    pk.reuse_shadow = (g_shadow_reuse && a.parent_q_all) ? 1u : 0u;
+    pk.ovf = a.ovf_all; pk.ovf_huge = a.ovf_huge_all; pk.ovf_cap = ovf_cap;
+    // one device, its own cursor, chunks of 32 rays: what render_impl sets up for a tile rendered alone, without emulate_ranks
+    pk.steal = &pk.sched->steal_local;
+    pk.chunk_shift = kChunkLocalShift; pk.steal_stride = 1u; pk.part_index = pk.part_count = 0u; pk.run_shift = 0u;
+    pk.fb = pk.fb_out = nullptr; pk.dbg_found = pk.dbg_index = nullptr; pk.dbg_t = nullptr; pk.split_path = nullptr;
+    pk.subsample = pk.supersample = 0;
+    unsigned long long launches = 0;                                // (not the device's: queries leave ct_gpu_kernel_launches alone)
+    int rc = CT_OK;
+    cudaError_t r = cudaMemsetAsync(pk.tot, 0, sizeof(DevTotals), st);
+    for (uint32_t first = 0; r == cudaSuccess && rc == CT_OK && first < n; first += batch) {
+        Params v = pk;
+        v.n_slots = std::min(batch, n - first);
+        v.q_org = org + 3ull * first; v.q_dir = dir + 3ull * first;
+        v.final_color = color + first;
+        if ((r = cudaMemsetAsync(pk.sched, 0, sizeof(DevSched), st)) != cudaSuccess) break;
+        rc = enqueue_stages<true>(s, v, a, false, true, st, [](const char *, int) { return (int)CT_OK; }, launches);
+    }
+    if (r == cudaSuccess) r = cudaGetLastError();
+    const cudaError_t f = cudaFreeAsync(base, st);
+    if (rc != CT_OK) return rc;
+    if (r != cudaSuccess) return fail(CT_ERR_CUDA, "shade query: %s", cudaGetErrorString(r));
+    if (f != cudaSuccess) return fail(CT_ERR_CUDA, "cudaFreeAsync: %s", cudaGetErrorString(f));
+    return CT_OK;
+}
+
+// A query's array: device (or managed) memory of `device`, aligned.  Checked before anything is enqueued.
+int check_device_array(int device, const void *p, size_t align, const char *name) {
+    if ((uintptr_t)p % align) return fail(CT_ERR_INVALID, "%s is not %zu-byte aligned", name, align);
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return fail(CT_ERR_INVALID, "%s: not a CUDA pointer", name); }
+    if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != device)
+        return fail(CT_ERR_INVALID, "%s is not device memory of device %d", name, device);
+    return CT_OK;
+}
 }  // namespace
 
 // ==== exported C ABI ==========================================================================================
@@ -873,12 +1086,10 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
     }
     CU(cudaMemsetAsync(p.sched, 0, sizeof(DevSched), st));
     CU(cudaEventRecord(s.ev0, st));
-    const int grid = launch_grid(s, 8);
-    int work = 0;
     const bool stages = (s.flags & CT_FLAG_STAGE_TIMING) != 0;
     s.n_stages = 0;
     if (stages) CU(cudaEventRecord(s.stage_ev[0], st));
-    auto mark = [&](const char *name, int depth) -> int {          // called after each launch
+    auto mark = [&](const char *name, int depth) -> int {          // called after each launch on st
         s.launches++;
         if (!stages || s.n_stages >= kMaxLaunches) return CT_OK;
         s.stage_name[s.n_stages] = name; s.stage_depth[s.n_stages] = depth;
@@ -886,111 +1097,9 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
         CU(cudaEventRecord(s.stage_ev[s.n_stages], st));
         return CT_OK;
     };
-    // Params as the launches of depth d see them: their own hit records, occlusion masks, ray queue in / out
-    auto view = [&](int d) {
-        Params v = pk;
-        const size_t cap = pk.cap;
-        if (s.hitb_t_all) { v.hitb_t = s.hitb_t_all + cap * d; v.hitb_pos = s.hitb_pos_all + cap * d; }
-        if (s.rays_all) {
-            v.ray_buf[d & 1] = s.rays_all + cap * 6 * d;            v.path_slot[d & 1] = s.path_slot_all + cap * d;
-            v.ray_buf[(d & 1) ^ 1] = s.rays_all + cap * 6 * (d + 1); v.path_slot[(d & 1) ^ 1] = s.path_slot_all + cap * (d + 1);
-            v.parent_q[d & 1] = s.parent_q_all + cap * d; v.parent_q[(d & 1) ^ 1] = s.parent_q_all + cap * (d + 1);
-        }
-        v.occ = s.occ_all + cap * pk.occ_words * d;
-        if (s.far_all) v.far_list = s.far_all + cap * d;
-        return v;
-    };
-    auto overflow = [&](const Params &v0, cudaStream_t q, int mode_anyhit, int ovf_idx, int depth) -> int {   // parked rays of the launch just made
-        if (!s.can_overflow) return CT_OK;
-        Params v = v0;
-        v.ovf = s.ovf_all + (size_t)pk.ovf_cap * ovf_idx; v.ovf_huge = s.ovf_huge_all + (size_t)pk.ovf_cap * ovf_idx;
-        const int g1 = s.n_sm * 2, g2 = s.n_sm * 4;
-        if (mode_anyhit) {
-            if (count) { k_overflow<kAnyHit, true><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kAnyHit, true><<<g2, 256, 0, q>>>(v, ovf_idx); }
-            else { k_overflow<kAnyHit, false><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kAnyHit, false><<<g2, 256, 0, q>>>(v, ovf_idx); }
-        } else {
-            if (count) { k_overflow<kFirstLine, true><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kFirstLine, true><<<g2, 256, 0, q>>>(v, ovf_idx); }
-            else { k_overflow<kFirstLine, false><<<g1, kOvfThreads, 0, q>>>(v, ovf_idx); k_overflow_huge<kFirstLine, false><<<g2, 256, 0, q>>>(v, ovf_idx); }
-        }
-        s.launches++;                                       // two kernels, one stage
-        return mark(mode_anyhit ? "overflow_shadow" : "overflow_bounce", depth);
-    };
-    // Two dependency chains per frame (DESIGN.md 4):
-    //   hits      primary -> emit(0) -> bounce(1) -> emit(1) -> bounce(2) -> ...          (main stream)
-    //   lighting  shadow(d) -> shade(d), needs only the hits of depth d                   (one side stream per depth)
-    // so the lighting of depth d overlaps the hit chain of depth d+1 and the lighting of the other depths; the
-    // persistent CTAs of a later kernel move into an SM as those of an earlier one run out of work, which fills
-    // the kernels' tails.  With CT_FLAG_STAGE_TIMING everything is serialised on the main stream instead.
-    {
-        Params v0 = view(0);              // (k_primary also runs the recursion step of depth 0: it needs the depth's queues)
-        // walks longer than primary_budget pair visits are parked (slot 0 of the parking buffers: depth 0 has no bounce launch)
-        // and walked again by k_primary_long, in warps made of long walks only
-        const bool park_primary = s.can_overflow && pk.primary_budget > 0u;
-        v0.ovf = park_primary ? s.ovf_all : nullptr;
-        if (park_primary) {
-            if (count) k_primary<true, true><<<grid, kBlockThreads, 0, st>>>(v0);
-            else k_primary<false, true><<<grid, kBlockThreads, 0, st>>>(v0);
-        } else {
-            if (count) k_primary<true, false><<<grid, kBlockThreads, 0, st>>>(v0);
-            else k_primary<false, false><<<grid, kBlockThreads, 0, st>>>(v0);
-        }
-        TRY(mark("primary", 0));
-        if (park_primary) {
-            const bool split = launch_parked_primary(s, v0, count, st, work);
-            if (!split) work++;
-            TRY(mark(split ? "primary_split" : "primary_long", 0));
-        }
-    }
-    for (int d = 0; d <= depth_max; d++) {
-        const Params v = view(d);
-        const int ovf_b = 2 * d, ovf_s = 2 * d + 1;
-        if (d > 0) {
-            Params vb = v;
-            vb.budget = first_line_budget(s);
-            if (s.can_overflow) { vb.ovf = s.ovf_all + (size_t)pk.ovf_cap * ovf_b; vb.ovf_huge = s.ovf_huge_all + (size_t)pk.ovf_cap * ovf_b; }
-            if (count) k_bounce<true><<<grid, kBlockThreads, 0, st>>>(vb, d, work++, ovf_b);
-            else k_bounce<false><<<grid, kBlockThreads, 0, st>>>(vb, d, work++, ovf_b);
-            TRY(mark("bounce", d));
-            TRY(overflow(v, st, 0, ovf_b, d));
-        }
-        cudaStream_t side = stages ? st : s.aux[d % 4];
-        if (!stages) { CU(cudaEventRecord(s.ev_hit[d], st)); CU(cudaStreamWaitEvent(side, s.ev_hit[d], 0)); }
-        if (depth_max > 0) {
-            // TraceRay's recursion step runs inside the hit kernels (emit_paths); what is left for a kernel of its own are the
-            // reflection paths k_bounce had parked, whose hit k_overflow has just delivered
-            if (d > 0 && s.can_overflow) {
-                k_emit<<<s.n_sm * 2, kBlockThreads, 0, st>>>(v, d, work++, s.ovf_all + (size_t)pk.ovf_cap * ovf_b, ovf_b);
-                TRY(mark("emit_late", d));
-            }
-        }
-        if (pk.n_slights > 0) {
-            Params vs = v;
-            if (s.can_overflow) { vs.ovf = s.ovf_all + (size_t)pk.ovf_cap * ovf_s; vs.ovf_huge = s.ovf_huge_all + (size_t)pk.ovf_cap * ovf_s; }
-            if (count) k_shadow<true><<<grid, kBlockThreads, 0, side>>>(vs, d, work++, ovf_s);
-            else k_shadow<false><<<grid, kBlockThreads, 0, side>>>(vs, d, work++, ovf_s);
-            if (stages) TRY(mark("shadow", d)); else s.launches++;
-            if (stages) { TRY(overflow(v, side, 1, ovf_s, d)); }
-            else if (s.can_overflow) {
-                Params vo = v;
-                vo.ovf = s.ovf_all + (size_t)pk.ovf_cap * ovf_s; vo.ovf_huge = s.ovf_huge_all + (size_t)pk.ovf_cap * ovf_s;
-                if (count) { k_overflow<kAnyHit, true><<<s.n_sm * 2, kOvfThreads, 0, side>>>(vo, ovf_s); k_overflow_huge<kAnyHit, true><<<s.n_sm * 4, 256, 0, side>>>(vo, ovf_s); }
-                else { k_overflow<kAnyHit, false><<<s.n_sm * 2, kOvfThreads, 0, side>>>(vo, ovf_s); k_overflow_huge<kAnyHit, false><<<s.n_sm * 4, 256, 0, side>>>(vo, ovf_s); }
-                s.launches += 2;
-            }
-        }
-        if (!stages) {
-            // k_shade(d) may read the shadow verdicts of shallower depths (occlusion_source): they are complete at ev_lit
-            CU(cudaEventRecord(s.ev_lit[d], side));
-            for (int dd = 0; dd < d; dd++) CU(cudaStreamWaitEvent(side, s.ev_lit[dd], 0));
-        }
-        k_shade<<<grid, kBlockThreads, 0, side>>>(v, d, work++);
-        if (stages) TRY(mark("shade", d)); else s.launches++;
-        if (!stages) CU(cudaEventRecord(s.ev_done[d], side));
-    }
-    if (!stages) for (int d = 0; d <= depth_max; d++) CU(cudaStreamWaitEvent(st, s.ev_done[d], 0));
-    if (depth_max > 0) { k_resolve<<<s.n_sm * 4, 256, 0, st>>>(pk); TRY(mark("resolve", 0)); }
-    if (pk.supersample) { k_supersample<<<s.n_sm * 4, 256, 0, st>>>(pk); TRY(mark("supersample", 0)); }
-    if (pk.subsample) { k_subsample<<<s.n_sm * 4, 256, 0, st>>>(pk); TRY(mark("subsample", 0)); }
+    const PathArrays arrays{s.hitb_t_all, s.hitb_pos_all, s.rays_all, s.path_slot_all, s.occ_all, s.parent_q_all, s.far_all,
+                            s.ovf_all, s.ovf_huge_all};
+    TRY(enqueue_stages<false>(s, pk, arrays, count, stages, st, mark, s.launches));
     CU(cudaEventRecord(s.ev1, st));
     CU(cudaEventRecord(s.tile_done[s.tiles_submitted % 8], st));
     s.tiles_submitted++;
@@ -1450,18 +1559,29 @@ int ct_gpu_trace_rays(int device, const ct_ray_query *q) {
     if (q->n == 0) return CT_OK;
     const struct { const void *p; size_t align; const char *name; } arrays[] = {
         {q->origins, 8, "origins"}, {q->directions, 8, "directions"}, {q->found, 4, "found"}, {q->index, 4, "index"}, {q->tclosest, 4, "tclosest"}};
-    for (const auto &a : arrays) {
-        if (!a.p) continue;
-        if ((uintptr_t)a.p % a.align) return fail(CT_ERR_INVALID, "%s is not %zu-byte aligned", a.name, a.align);
-        cudaPointerAttributes at{};
-        if (cudaPointerGetAttributes(&at, a.p) != cudaSuccess) { cudaGetLastError(); return fail(CT_ERR_INVALID, "%s: not a CUDA pointer", a.name); }
-        if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != device)
-            return fail(CT_ERR_INVALID, "%s is not device memory of device %d", a.name, device);
-    }
+    for (const auto &a : arrays)
+        if (a.p) TRY(check_device_array(device, a.p, a.align, a.name));
     const cudaStream_t st = q->stream ? static_cast<cudaStream_t>(q->stream) : s.stream;
     const bool shadow = q->kind == CT_RAY_SHADOW;
     return trace_impl(s, q->kind, q->n, q->origins, q->directions, q->found, shadow ? nullptr : q->index, shadow ? nullptr : q->tclosest,
                       nullptr, 0u, st);
+}
+
+int ct_gpu_shade_rays(int device, const ct_shade_query *q) {
+    if (!q || q->struct_size != sizeof(ct_shade_query)) return fail(CT_ERR_INVALID, "ct_shade_query missing or struct_size != %zu", sizeof(ct_shade_query));
+    if (q->n >= (1u << 31)) return fail(CT_ERR_LIMIT, "%u rays: a query takes fewer than 2^31", q->n);
+    if (q->max_depth > 15) return fail(CT_ERR_LIMIT, "max_depth %d outside 0..15 (< 0: the scene's)", q->max_depth);
+    if (q->n > 0 && (!q->origins || !q->directions || !q->color)) return fail(CT_ERR_INVALID, "NULL origins, directions or color with n = %u", q->n);
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    if (q->n == 0) return CT_OK;
+    TRY(check_device_array(device, q->origins, 8, "origins"));
+    TRY(check_device_array(device, q->directions, 8, "directions"));
+    TRY(check_device_array(device, q->color, 4, "color"));
+    const cudaStream_t st = q->stream ? static_cast<cudaStream_t>(q->stream) : s.stream;
+    return shade_impl(s, q->n, q->max_depth < 0 ? s.p.max_depth : q->max_depth, q->origins, q->directions, q->color, st);
 }
 
 static int debug_primitives_impl(int device, uint32_t n, const double *origins, const double *directions, float *ray_t,

@@ -54,8 +54,20 @@ CT_DEV Ray primary_ray_at(const Params &P, float px, float py) {
     return r;
 }
 
+// WHERE A DEPTH-0 RAY COMES FROM AND WHERE ITS COLOUR GOES.  A frame's depth-0 slot is a pixel (or a sample of one) of the tile; a
+// shade query's (QUERY, ct_gpu_shade_rays) is the caller's ray `slot` of the current batch.  Only primary_ray, slot_pixel and
+// store_pixel know the difference: the stage kernels that call them (k_primary, k_shadow, k_shade, k_resolve) take QUERY as a
+// template parameter, everything past depth 0 reads the parking buffers and ray queues and is the same for both.
+
 // Primary ray of depth-0 slot `slot`, whose pixel is (x, y): the pixel centre, or one of its 16 jittered samples.
+// QUERY: the caller's ray, ray.t = 1e30f as TraceRay's callers pass it (raythread.cpp:508).
+template <bool QUERY = false>
 CT_DEV Ray primary_ray(const Params &P, uint32_t slot, int x, int y) {
+    if (QUERY) {
+        Ray r;
+        r.o = ld3(P.q_org + 3ull * slot); r.d = ld3(P.q_dir + 3ull * slot); r.t = kRayTInit;
+        return r;
+    }
     if (!P.supersample) return primary_ray_at(P, (float)x, (float)y);
     float px, py;
     sample_point(x, y, (int)(slot & 15u), px, py);
@@ -65,12 +77,16 @@ CT_DEV Ray primary_ray(const Params &P, uint32_t slot, int x, int y) {
 // slot -> canvas pixel.  A warp owns an 8x4 pixel block (coherent rays); returns false for padding lanes
 // and for pixels PutPixel would drop (draw2d.h:11-14), which are not traced at all (with subsampling a dropped
 // row is still traced -- fb_index = -1 -- because its colour enters the average stored in the row above it).
+// QUERY: slot i of the batch is ray i, valid for i < n_slots; fb_index = -1, and store_pixel writes final_color (the caller's colour
+// array at the batch's first ray) only.
 CT_DEV void store_pixel(const Params &P, uint32_t slot, int fb_index, uint32_t color) {
     if (fb_index >= 0) P.fb_out[fb_index] = color;
     if (P.final_color) P.final_color[slot] = color;
 }
 
+template <bool QUERY = false>
 CT_DEV bool slot_pixel(const Params &P, uint32_t slot, int &x, int &y, int &fb_index) {
+    if (QUERY) { x = y = 0; fb_index = -1; return slot < P.n_slots; }
     if (P.supersample) slot >>= 4;                            // 16 samples per pixel
     uint32_t blk = slot >> 5, lane = slot & 31u;
     int bx = (int)(blk % (uint32_t)P.blocks_x), by = (int)(blk / (uint32_t)P.blocks_x);
@@ -111,14 +127,15 @@ CT_DEV uint32_t depth0_count(const Params &P) { return P.sched->own_count << P.c
 
 // The path with queue index q at `depth`: its ray (direction only for depth 0 is regenerated from the pixel),
 // its closest-hit record and its depth-0 slot.  False for padding lanes / untraced pixels.
+template <bool QUERY = false>
 CT_DEV bool load_path(const Params &P, int depth, uint32_t q, uint32_t &slot, int &fbi, Ray &r, float &tc, uint32_t &pos) {
     if (depth == 0) {
         int x, y;
         slot = own_slot(P, q);
-        if (!slot_pixel(P, slot, x, y, fbi)) return false;
+        if (!slot_pixel<QUERY>(P, slot, x, y, fbi)) return false;
         tc = P.hit0_t[slot]; pos = P.hit0_pos[slot];
         if (pos == kNoPos) return true;                         // a miss: nobody needs its ray again (background pixel)
-        r = primary_ray(P, slot, x, y);
+        r = primary_ray<QUERY>(P, slot, x, y);
     } else {
         const int cur = depth & 1;
         slot = P.path_slot[cur][q];
@@ -279,6 +296,7 @@ struct PrimaryJob {
     uint32_t n_rays = 0;
 
     // One slot per lane (got: the slot is a pixel to trace, r / r64 set up); false once the cursor is exhausted.
+    template <bool QUERY>
     CT_DEV bool refill(const Params &P, bool &got, TRay &r, double *r64) {
         const uint32_t lane = threadIdx.x & 31u;
         if (pend_left == 0u) {
@@ -304,8 +322,8 @@ struct PrimaryJob {
         if (rank < take) {
             slot = pend_slot + rank; q = pend_q + rank;     // q: this path's depth-0 number on this device
             int x, y;
-            if (slot < P.n_slots && slot_pixel(P, slot, x, y, fbi)) {
-                const Ray ray = primary_ray(P, slot, x, y);
+            if (slot < P.n_slots && slot_pixel<QUERY>(P, slot, x, y, fbi)) {
+                const Ray ray = primary_ray<QUERY>(P, slot, x, y);
                 tray_setup(r, ray, P.bound, r64);
                 got = true;
             }
@@ -349,7 +367,8 @@ CT_DEV int primary_walk_or_park(const Params &P, TRay &r, const double *r64, boo
 // 8x4 pixel block: neighbouring rays visit the same nodes; refilling idle lanes from the next chunk instead measured slower,
 // DESIGN.md 5).
 // PARK: walks longer than P.primary_budget pair visits are given up and parked for k_primary_long (option "primary_budget").
-template <bool COUNT, bool PARK>
+// QUERY: the depth-0 rays are a shade query's (see primary_ray).
+template <bool COUNT, bool PARK, bool QUERY = false>
 __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary(const __grid_constant__ Params P) {
     LocalCount lc;
     uint32_t n_refl = 0;
@@ -362,7 +381,7 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary(const __g
         bool got = false;
         double r64[kRay64];
         TRay r;
-        if (!job.refill(P, got, r, r64)) break;
+        if (!job.refill<QUERY>(P, got, r, r64)) break;
         int res; float tc; uint32_t pos;
         const int how = primary_walk_or_park<COUNT, PARK>(P, r, r64, got, job.q, job.slot, n_parked, lc, res, tc, pos);
         const bool done = got && how != kParked, found = res == kTravHit;
@@ -403,6 +422,8 @@ __global__ void __launch_bounds__(kBlockThreads, kMinBlocks) k_primary_long(cons
         float tc; uint32_t pos;
         const bool found = traverse_closest<COUNT>(P, r, active, tc, pos, lc) == kTravHit;
         if (active) {
+            // (the pixel only for CT_FLAG_KEEP_HITS: a shade query's parked rays get a meaningless fbi here, which
+            // store_primary_hit ignores because a query's dbg_* are NULL -- so this kernel needs no QUERY form)
             int x, y, fbi = -1;
             if (!slot_pixel(P, slot, x, y, fbi)) fbi = -1;
             n_rays++;
@@ -605,7 +626,7 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
             found = res == kTravHit; tc = tc2; pos = pos2;
         }
         if (lane == 0) {                                      // lane 0 holds the answer
-            int x, y, fbi = -1;
+            int x, y, fbi = -1;                               // (for CT_FLAG_KEEP_HITS only; a shade query's: see k_primary_long)
             if (!slot_pixel(P, slot, x, y, fbi)) fbi = -1;
             n_rays++;
             store_primary_hit(P, slot, q, fbi, found, tc, pos);
@@ -630,7 +651,7 @@ __global__ void __launch_bounds__(kOvfThreads) k_primary_split(const __grid_cons
 #ifndef CT_SHADOW_BLOCKS
 #define CT_SHADOW_BLOCKS CT_MIN_BLOCKS
 #endif
-template <bool COUNT>
+template <bool COUNT, bool QUERY = false>
 __global__ void __launch_bounds__(kBlockThreads, CT_SHADOW_BLOCKS) k_shadow(const __grid_constant__ Params P, int depth, int work_idx, int ovf_idx) {
     LocalCount lc;
     uint32_t n_shadow = 0, n_parked = 0, n_reused = 0;
@@ -658,7 +679,7 @@ __global__ void __launch_bounds__(kBlockThreads, CT_SHADOW_BLOCKS) k_shadow(cons
             n_shadow++; n_reused++;                                   // (every reflection path is a hit: 0 != 1e30f, raythread.cpp:227)
             active = false;
         }
-        active = active && load_path(P, depth, q, slot, fbi, r, tc, pos) && pos != kNoPos;
+        active = active && load_path<QUERY>(P, depth, q, slot, fbi, r, tc, pos) && pos != kNoPos;
         double r64[kRay64];
         TRay tr;
         uint32_t word = 0, bit = 0;
@@ -733,7 +754,7 @@ CT_DEV void emit_paths(const Params &P, int depth, bool active, uint32_t q, uint
 }
 
 // The same step as a kernel of its own, for the paths whose hit record a hit kernel could not finish itself: the reflection
-// paths k_bounce had parked (late_list; their hit came from k_overflow).
+// paths k_bounce had parked (late_list; their hit came from k_overflow).  Depth >= 1 only, so its load_path needs no QUERY form.
 __global__ void __launch_bounds__(kBlockThreads) k_emit(const __grid_constant__ Params P, int depth, int work_idx, const OvfRay *late_list, int ovf_bounce) {
     uint32_t n_refl = 0;
     const uint32_t n = min(P.sched->ovf_count[ovf_bounce], P.ovf_cap);
@@ -754,6 +775,7 @@ __global__ void __launch_bounds__(kBlockThreads) k_emit(const __grid_constant__ 
 
 // TraceRay's local colour (raythread.cpp:359-366) for the paths alive at `depth`; the shadow verdicts were computed
 // by k_shadow (+ k_overflow).
+template <bool QUERY = false>
 __global__ void __launch_bounds__(kBlockThreads) k_shade(const __grid_constant__ Params P, int depth, int work_idx) {
     const uint32_t n = depth == 0 ? depth0_count(P) : P.sched->queue_count[depth];
     while (true) {
@@ -762,7 +784,7 @@ __global__ void __launch_bounds__(kBlockThreads) k_shade(const __grid_constant__
         uint32_t q = (uint32_t)base + (threadIdx.x & 31u);
         uint32_t slot = q, pos = kNoPos; int fbi = 0;
         Ray r; float tc = 0.0f;
-        if (!(q < n && load_path(P, depth, q, slot, fbi, r, tc, pos))) continue;
+        if (!(q < n && load_path<QUERY>(P, depth, q, slot, fbi, r, tc, pos))) continue;
         uint32_t *sc = P.stack_color + (size_t)depth * P.cap + slot;
         if (pos == kNoPos) {                                           // miss (depth 0 only): raythread.cpp:385
             if (depth == 0) store_pixel(P, slot, fbi, P.background);
@@ -1030,12 +1052,13 @@ __global__ void __launch_bounds__(256) k_overflow_huge(const __grid_constant__ P
 }
 
 // Unwind TraceRay's recursion (raythread.cpp:375-379) for pixels whose chain went past depth 0.
+template <bool QUERY = false>
 __global__ void __launch_bounds__(256) k_resolve(const __grid_constant__ Params P) {
     const uint32_t n = depth0_count(P);
     for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < n; q += gridDim.x * blockDim.x) {
         const uint32_t slot = own_slot(P, q);
         int x, y, fbi;
-        if (!slot_pixel(P, slot, x, y, fbi)) continue;
+        if (!slot_pixel<QUERY>(P, slot, x, y, fbi)) continue;
         int lvl = P.term_level[slot];
         if (lvl == 0) continue;                              // already stored by k_shade
         uint32_t color = P.stack_color[(size_t)lvl * P.cap + slot];

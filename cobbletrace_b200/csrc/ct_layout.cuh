@@ -166,6 +166,9 @@ struct Params {
     const uint32_t *tri_parent;                  // leaf position -> 2 * pair + side of the box of the leaf that holds it (kNoPos: root leaf)
     DevSched *sched;
     DevTotals *tot;
+    // shade queries (ct_gpu_shade_rays; unused by frames): the caller's rays of the current batch, n_slots x 3 doubles each, read as
+    // the depth-0 rays by the QUERY forms of the stage kernels.  Last in the struct: the frame kernels' parameter offsets do not move.
+    const double *q_org, *q_dir;
 };
 
 struct LocalCount { uint32_t box = 0, tri = 0, box_exact = 0, tri_exact = 0; };

@@ -354,6 +354,48 @@ typedef struct ct_ray_query {
 
 int ct_gpu_trace_rays(int device, const ct_ray_query *q);
 
+/* ---- shading queries on device memory -------------------------------------------------------------------------
+ * ct_gpu_shade_rays returns, for n caller rays, the colour the reference's TraceRay (raythread.cpp:353-386) returns for them:
+ * color[i] = TraceRay({origins[i], directions[i], 1e30f}, 1, FINF, max_depth) as 0x00BBGGRR -- lighting, shadow rays and the
+ * reflection recursion included, bit for bit; a ray that hits nothing gets the scene's background.  With no reflective material
+ * in the scene the recursion stops at depth 0, as in frames.  The rays go through a frame's own stages (primary, shadow, shade,
+ * bounce, ..., resolve) in place of the camera's, so any camera model, sample pattern or batch of views can be shaded.
+ * Options apply as they do to frames: traversal_budget, overflow_warp_budget, any_leaves and primary_budget are read at upload,
+ * primary_split and shadow_reuse at the call; emulate_ranks and the shared-frame state (ct_gpu_share_*) are ignored -- a query
+ * shades every ray on this device.
+ *
+ * Every array lives in DEVICE (or managed) memory of `device`: origins and directions n x 3 doubles (8-byte aligned), color n
+ * words (4-byte aligned).  The call is asynchronous: it enqueues its work on `stream` (NULL = the device's render stream, see
+ * ct_gpu_set_stream) and returns; color is valid once the stream reaches that point.  It does not synchronise: its scratch comes
+ * from the stream-ordered allocator and is freed in stream order, nothing is kept between calls, and the caller's stream is left
+ * as it is (no L2 access-policy window).  The stages run one after the other on that stream (a frame overlaps each depth's
+ * lighting with the next depth's hits on side streams the library shares with frames).  Queries read the scene's arrays only:
+ * frames, ct_gpu_get_counters, ct_gpu_kernel_launches, ct_gpu_overflow_stats and ct_gpu_reuse_stats are unchanged by them.  The
+ * scene must outlive the queries in flight (see ct_gpu_trace_rays).
+ *
+ * Scratch: the rays are shaded in batches of up to 2^20 that reuse one allocation, so the scratch does not grow with n.  For a
+ * batch of B = min(n, 2^20) rays (rounded up to 64), L = max_depth + 1 levels (1 without a reflective material) and the scene's
+ * n_lights, counted from the allocation: B x 13 B for L = 1, B x (65 + 76 L) B for L > 1 (hit records, colour and reflection
+ * stacks, ray queues with their slot and parent lists, far lists), plus B x L x 4 B x ceil(n_lights / 32) of occlusion words,
+ * plus, on a scene whose walks can be parked, 2 x L x 68 B x min(B, the frame's parking capacity: 2^18, or 1/16 of the frame's
+ * slots with primary_budget set) of parking buffers -- e.g. about 430 MB at B = 2^20, L = 3, 3 lights.
+ * Returns CT_OK; CT_ERR_INVALID for a NULL q, a wrong struct_size, NULL arrays with n > 0, an array that is not device memory of
+ * `device` (host memory, pageable or pinned, is refused) or is misaligned; CT_ERR_LIMIT for n >= 2^31 or max_depth > 15;
+ * CT_ERR_NO_SCENE -- all checked before anything is enqueued; CT_ERR_OOM when the scratch cannot be allocated (nothing is
+ * enqueued then). */
+typedef struct ct_shade_query {
+    uint32_t struct_size;            /* = sizeof(ct_shade_query) */
+    uint32_t n;                      /* rays; 0 is a no-op */
+    int32_t max_depth;               /* TraceRay's recursionDepth: 0..15, < 0 = the scene's (as uploaded) */
+    uint32_t _pad;
+    const double *origins;           /* n x 3 doubles, device memory of `device` */
+    const double *directions;        /* n x 3 doubles, device memory of `device` */
+    uint32_t *color;                 /* n, device memory: 0x00BBGGRR */
+    void *stream;                    /* cudaStream_t to run on; NULL = the device's render stream (ct_gpu_set_stream) */
+} ct_shade_query;
+
+int ct_gpu_shade_rays(int device, const ct_shade_query *q);
+
 /* Known-answer-test entry: ClosestIntersection (raythread.cpp:197-227) for n arbitrary rays through the
  * uploaded scene.  origins/directions: n x 3 doubles; t0: initial ray_t.t per ray (1e30f primary/shadow,
  * 0 for the reference's reflection rays, raythread.cpp:373).  Outputs may be NULL. */
