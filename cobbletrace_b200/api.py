@@ -27,7 +27,7 @@ ABI_SYMBOLS = [
     "ct_gpu_set_stream", "ct_gpu_render_tile", "ct_gpu_readback", "ct_gpu_readback_async", "ct_gpu_readback_wait", "ct_gpu_readback_hits", "ct_gpu_get_counters",
     "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early", "ct_gpu_debug_primary",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
-    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays", "ct_gpu_shade_rays",
+    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays", "ct_gpu_shade_rays", "ct_gpu_update_triangles",
 ]
 RAY_KINDS = {"primary": 0, "shadow": 1, "reflection": 2}     # CT_RAY_PRIMARY, CT_RAY_SHADOW, CT_RAY_REFLECTION
 
@@ -75,6 +75,11 @@ class RayQuery(C.Structure):     # == ct_ray_query
 class ShadeQuery(C.Structure):   # == ct_shade_query
     _fields_ = [("struct_size", C.c_uint32), ("n", C.c_uint32), ("max_depth", C.c_int32), ("_pad", C.c_uint32),
                 ("origins", C.c_void_p), ("directions", C.c_void_p), ("color", C.c_void_p), ("stream", C.c_void_p)]
+
+
+class TriangleUpdate(C.Structure):   # == ct_triangle_update
+    _fields_ = [("struct_size", C.c_uint32), ("n_triangles", C.c_uint32), ("triangle_stride", C.c_uint32), ("_pad", C.c_uint32),
+                ("triangles", C.c_void_p), ("stream", C.c_void_p)]
 
 
 class RayCounters(C.Structure):  # == ct_ray_counters
@@ -147,6 +152,7 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_debug_scene_array.argtypes = [C.c_int, C.c_char_p, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     L.ct_gpu_trace_rays.argtypes = [C.c_int, C.POINTER(RayQuery)]
     L.ct_gpu_shade_rays.argtypes = [C.c_int, C.POINTER(ShadeQuery)]
+    L.ct_gpu_update_triangles.argtypes = [C.c_int, C.POINTER(TriangleUpdate)]
     if path == GPU_LIB:
         _lib = L
     return L
@@ -177,6 +183,7 @@ class GpuRenderer:
         self.device = int(device)
         self.width = self.height = 0
         self.flags = 0
+        self.n_tri = None
 
     # -- ct_gpu_upload_scene ------------------------------------------------------------------------
     def upload(self, fs: FlatScene, width: int, height: int, max_depth: int = REFERENCE_MAX_DEPTH, flags: int = 0,
@@ -213,8 +220,40 @@ class GpuRenderer:
         d.viewport = (C.c_float * 3)(*viewport)
         d.width, d.height, d.max_depth, d.background = width, height, max_depth, background
         _check(self.L, self.L.ct_gpu_upload_scene(self.device, C.byref(d)))
-        self.width, self.height, self.flags = width, height, flags
+        self.width, self.height, self.flags, self.n_tri = width, height, flags, fs.n_tri
         return self
+
+    # -- ct_gpu_update_triangles ----------------------------------------------------------------------
+    def update_triangles(self, triangles):
+        """Replace the loaded scene's triangles and rebuild the reference's tree over them on the device, in place: afterwards the
+        device holds the scene upload(..., build_bvh=True) would load from them with the scene's materials, lights, camera and frame;
+        the stream set with set_stream, the framebuffer, counters and shared-frame state stay.  See ct_gpu_update_triangles.
+
+        torch tensor: float64, shape (n, 9) or (n, 3, 3) (p1, p2, p3 per triangle), contiguous, on cuda:<device>, n the uploaded
+        scene's triangle count.  It is read in place in torch.cuda.current_stream(device)'s order, so a kernel that wrote it on that
+        stream needs no synchronisation; the call returns when the update is done.  numpy array: copied to the device first.
+        Anything else raises ValueError before the library is called."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        if isinstance(triangles, np.ndarray):
+            triangles = torch.from_numpy(np.ascontiguousarray(triangles, np.float64)).to(dev)
+        if not isinstance(triangles, torch.Tensor):
+            raise ValueError(f"triangles: a torch tensor or a numpy array, not {type(triangles).__name__}")
+        if triangles.device != dev:
+            raise ValueError(f"triangles are on {triangles.device}, this renderer's scene is on {dev}")
+        if triangles.dtype != torch.float64:
+            raise ValueError(f"triangles are {triangles.dtype}, vertices are float64")
+        if tuple(triangles.shape[1:]) not in ((9,), (3, 3)):
+            raise ValueError(f"triangles have shape {tuple(triangles.shape)}, not (n, 9) or (n, 3, 3)")
+        if self.n_tri is not None and triangles.shape[0] != self.n_tri:
+            raise ValueError(f"{triangles.shape[0]} triangles: the uploaded scene has {self.n_tri}")
+        if not triangles.is_contiguous():
+            raise ValueError("triangles are not contiguous")
+        u = TriangleUpdate()
+        u.struct_size, u.n_triangles, u.triangle_stride = C.sizeof(TriangleUpdate), triangles.shape[0], 72
+        u.triangles = triangles.data_ptr() or None
+        u.stream = torch.cuda.current_stream(dev).cuda_stream or 1      # (handle 0, torch's default stream, is cudaStreamLegacy = 1)
+        _check(self.L, self.L.ct_gpu_update_triangles(self.device, C.byref(u)))
 
     def set_camera(self, position, rotation):
         p = np.ascontiguousarray(position, np.float64); r = np.ascontiguousarray(rotation, np.float64).reshape(9)

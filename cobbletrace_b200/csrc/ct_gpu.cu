@@ -119,6 +119,11 @@ struct DeviceState {
     bool copy_pending = false;
     void *hot_base = nullptr; size_t hot_bytes = 0;      // pairs32 + tris32 (one allocation): the L2 access-policy window
     size_t l2_window = 0, l2_set_aside = 0;              // what apply_l2_policy obtained (0: none)
+    // what the tree's allocations hold (ct_gpu_update_triangles reuses them when the new tree fits): bytes of the hot allocation,
+    // pairs64 records, pair_parent entries (its allocation stays when a new tree cannot park: p.pair_parent is then NULL)
+    size_t hot_cap = 0;
+    uint32_t pairs_cap = 0, pair_parent_cap = 0;
+    uint32_t *pair_parent_mem = nullptr;
     std::vector<void *> allocs;
     ct_ray_counters snapshot{};      // totals at the end of the previous counted tile
     unsigned long long rays_overflow = 0, rays_in_place = 0;   // DevTotals' overflow counters as of the last read_totals
@@ -156,14 +161,20 @@ int check_device(int device) {
     return CT_OK;
 }
 
+// Hands the persisting L2 lines back and takes the access-policy window off the library's own stream (a caller's stream may be
+// gone by now: ct_gpu_set_stream clears it when it is replaced).
+void release_l2(DeviceState &s) {
+    if (!s.l2_set_aside) return;
+    cudaStreamAttrValue attr{};
+    attr.accessPolicyWindow.num_bytes = 0;
+    if (s.own_stream) cudaStreamSetAttribute(s.own_stream, cudaStreamAttributeAccessPolicyWindow, &attr);
+    cudaCtxResetPersistingL2Cache();
+    cudaGetLastError();
+    s.l2_set_aside = s.l2_window = 0;
+}
+
 void free_device(DeviceState &s) {
-    if (s.l2_set_aside) {                                  // hand the persisting lines back
-        cudaStreamAttrValue attr{};
-        attr.accessPolicyWindow.num_bytes = 0;
-        if (s.own_stream) cudaStreamSetAttribute(s.own_stream, cudaStreamAttributeAccessPolicyWindow, &attr);   // (a caller's stream may be gone by now: ct_gpu_set_stream clears it when it is replaced)
-        cudaCtxResetPersistingL2Cache();
-        cudaGetLastError();
-    }
+    release_l2(s);
     for (void *q : s.ipc_opened) if (q) cudaIpcCloseMemHandle(q);
     for (void *p : s.allocs) cudaFree(p);
     s.allocs.clear();
@@ -201,6 +212,14 @@ int dev_alloc(DeviceState &s, T **out, size_t count, bool zero = false) {
     if (zero) CU(cudaMemset(p, 0, bytes));
     *out = static_cast<T *>(p);
     return CT_OK;
+}
+
+// frees one allocation of dev_alloc's (cudaFree: waits for the device)
+void dev_release(DeviceState &s, void *p) {
+    if (!p) return;
+    cudaFree(p);
+    const auto it = std::find(s.allocs.begin(), s.allocs.end(), p);
+    if (it != s.allocs.end()) s.allocs.erase(it);
 }
 
 #define TRY(expr) do { int rc_ = (expr); if (rc_ != CT_OK) return rc_; } while (0)
@@ -245,21 +264,154 @@ int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *
     return best;
 }
 
-// Device buffers and a stream that live for one ct_gpu_upload_scene call: the staged copies of the caller's arrays, the tree
-// built with CT_FLAG_BUILD_BVH (arena), the wide tree's scratch.  Freed when the call returns, whatever it returns.
+// Device buffers and a stream that live for one ct_gpu_upload_scene or ct_gpu_update_triangles call: the staged copies of the
+// caller's arrays, the tree built on the device (arena), the wide tree's scratch.  Freed when the call returns, whatever it returns.
+// async: the buffers come from the stream-ordered allocator and are freed in st's order (cudaFree would wait for the whole device;
+// the update's arena is allocated on the caller's stream, which st has waited for).
 struct Staging {
     std::vector<void *> ptrs;
     BbArena arena;
     cudaStream_t st = nullptr;
-    ~Staging() { if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } cudaFree(arena.base); for (void *q : ptrs) cudaFree(q); }
+    bool async = false;
+    cudaEvent_t ready = nullptr;
+    ~Staging() {
+        if (async) {
+            if (arena.base) cudaFreeAsync(arena.base, st);
+            for (void *q : ptrs) cudaFreeAsync(q, st);
+        }
+        if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
+        if (ready) cudaEventDestroy(ready);
+        if (!async) { cudaFree(arena.base); for (void *q : ptrs) cudaFree(q); }
+    }
     template <typename T> cudaError_t alloc(T **out, size_t count) {
         void *q = nullptr;
-        const cudaError_t e = cudaMalloc(&q, std::max<size_t>(count, 1) * sizeof(T));
+        const size_t bytes = std::max<size_t>(count, 1) * sizeof(T);
+        const cudaError_t e = async ? cudaMallocAsync(&q, bytes, st) : cudaMalloc(&q, bytes);
         if (e == cudaSuccess) ptrs.push_back(q);
         *out = static_cast<T *>(q);
         return e;
     }
 };
+
+// ---- the scene built from a tree: one builder for ct_gpu_upload_scene and ct_gpu_update_triangles ------------------------------
+// A binary tree in the reference's layout on the device and what the scene arrays are made from with it.
+struct DeviceTree {
+    const ct_bvh_node *nodes = nullptr;
+    const uint32_t *pid = nullptr;           // interior numbering: pair of an interior node, kLeafMark for a leaf, kNoPos unreachable
+    const uint32_t *tri_index = nullptr;
+    const unsigned char *tris = nullptr;     // the triangles at `stride`
+    uint32_t stride = 72, n_nodes = 0, n_pairs = 0;
+    ct_bvh_node root{};
+    int depth = 0;
+    DevWide *wide = nullptr;                 // the early-exit walks' wide tree, in scratch (collapse_wide)
+    uint32_t n_wide = 0;
+};
+
+// The reference's BuildBVH over the n triangles in bf.raw on stg.st (bb_build), then the interior numbering k_build_pairs takes
+// (k_pid_flags, bb_scan, k_pid_leaves).  Synchronises stg.st once per level.  A tree deeper than the device traversal stack is
+// CT_ERR_LIMIT, before anything else is allocated.
+int build_device_tree(Staging &stg, const BbBuffers &bf, uint32_t stride, uint32_t n, int n_sm, DeviceTree &t) {
+    CU(bb_build(bf, stride, n, n_sm, stg.st, &t.n_nodes, &t.depth));
+    CU(cudaMemcpyAsync(&t.root, bf.out, sizeof t.root, cudaMemcpyDeviceToHost, stg.st));
+    CU(cudaStreamSynchronize(stg.st));
+    if (t.depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", t.depth, kStackMax);
+    t.n_pairs = (t.n_nodes - 1u) / 2u;                                      // every node is reachable: 1 + 2 * interior nodes
+    uint32_t *pid = nullptr, *ptile = nullptr;                              // interior numbering: a scan over the node order
+    CU(stg.alloc(&pid, (size_t)t.n_nodes + 1)); CU(stg.alloc(&ptile, ((size_t)t.n_nodes + 1) / kBbScanTile + 1));
+    const int blocks = std::max(1, std::min(n_sm * 8, (int)((t.n_nodes + kBbThreads) / kBbThreads)));
+    k_pid_flags<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, t.n_nodes, pid);
+    CU(bb_scan(pid, t.n_nodes, ptile, stg.st));
+    k_pid_leaves<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, t.n_nodes, pid);
+    CU(cudaGetLastError());
+    t.nodes = bf.out; t.pid = pid; t.tri_index = bf.tri_index; t.tris = bf.raw; t.stride = stride;
+    return CT_OK;
+}
+
+// The early-exit walks' wide tree into scratch (none for a leaf root).  Synchronises stg.st.
+int collapse_wide(Staging &stg, DeviceTree &t, int n_sm) {
+    if (t.root.triangle_count == 0) {
+        uint32_t *root_of = nullptr, *wcnt = nullptr, *wtile = nullptr;
+        CU(stg.alloc(&t.wide, t.n_pairs)); CU(stg.alloc(&root_of, (size_t)t.n_pairs + 1)); CU(stg.alloc(&wcnt, (size_t)t.n_pairs + 1));
+        CU(stg.alloc(&wtile, ((size_t)t.n_pairs + 1) / kBbScanTile + 1));
+        CU(build_wide(t.nodes, root_of, wcnt, wtile, t.wide, n_sm, stg.st, &t.n_wide));
+    }
+    CU(cudaStreamSynchronize(stg.st));
+    return CT_OK;
+}
+
+// The records every walk step reads -- the wide tree, fp32 child pairs and fp32 triangles -- share ONE allocation, so that a single
+// L2 access-policy window can cover them (apply_l2_policy): wide at 0, pairs32 at pairs_at, tris32 at tris_at.
+struct HotLayout { size_t pairs_at, tris_at, bytes; };
+HotLayout hot_layout(uint32_t n_wide, uint32_t n_pairs, uint32_t n_tri) {
+    const size_t pair_bytes = ((size_t)std::max<uint32_t>(n_pairs, 1) * sizeof(DevPair32) + 255u) & ~(size_t)255u;
+    const size_t wide_bytes = ((size_t)n_wide * sizeof(DevWide) + 255u) & ~(size_t)255u;
+    return {wide_bytes, wide_bytes + pair_bytes, wide_bytes + pair_bytes + (size_t)n_tri * sizeof(DevTri32)};
+}
+
+// Parked rays: only when a DFS can run past the visit budget at all.
+bool walks_can_park(const Params &p, uint32_t n_nodes) { return (uint64_t)n_nodes + p.n_tri > p.budget; }
+
+// Parked rays per launch: 2^18 (16 MB) -- with primary walks parked as well (option "primary_budget": 2-3 % of a dragon-class
+// frame's primary rays) 1/16 of the frame's paths where that is more; a full buffer means finishing rays in place, which must
+// stay hypothetical.
+uint32_t parking_cap(const Params &p) { return p.primary_budget > 0u ? std::max<uint32_t>(1u << 18, p.cap / 16u) : 1u << 18; }
+
+// Where the scene arrays go.  pair_parent may be NULL (no walk can be parked).
+struct SceneArrays { unsigned char *hot; DevPair64 *pairs64; uint32_t *pair_parent, *tri_parent; DevTri *tris; };
+
+// The scene arrays from tree t (k_build_pairs, k_build_tris, the wide tree copied into the hot allocation at hot_layout's offsets)
+// and what the build reports about them.  materials: the scene's, by original id, already on the device.  The scratch is taken
+// before anything is written; the rest is enqueued on st, which is synchronised.
+int build_scene_arrays(Staging &stg, cudaStream_t st, const DeviceTree &t, const ct_material *materials, uint32_t n_tri, const SceneArrays &out,
+                       int n_sm, BuildReport *rep) {
+    uint32_t *seen = nullptr; BuildReport *drep = nullptr;
+    const size_t seen_words = ((size_t)n_tri + 31u) / 32u;
+    CU(stg.alloc(&drep, 1));
+    CU(stg.alloc(&seen, seen_words));
+    const HotLayout hl = hot_layout(t.n_wide, t.n_pairs, n_tri);
+    DevPair32 *dp32 = reinterpret_cast<DevPair32 *>(out.hot + hl.pairs_at);
+    DevTri32 *dt32 = reinterpret_cast<DevTri32 *>(out.hot + hl.tris_at);
+    if (t.n_wide) CU(cudaMemcpyAsync(out.hot, t.wide, (size_t)t.n_wide * sizeof(DevWide), cudaMemcpyDeviceToDevice, st));
+    CU(cudaMemsetAsync(seen, 0, seen_words * 4, st));
+    *rep = BuildReport{};
+    rep->bad_pos = kNoPos; rep->pos0 = kNoPos;
+    CU(cudaMemcpyAsync(drep, rep, sizeof *rep, cudaMemcpyHostToDevice, st));
+    if (out.pair_parent) CU(cudaMemsetAsync(out.pair_parent, 0xff, (size_t)std::max<uint32_t>(t.n_pairs, 1) * 4, st));
+    CU(cudaMemsetAsync(out.tri_parent, 0xff, (size_t)n_tri * 4, st));
+    const int build_blocks = n_sm * 8;
+    k_build_pairs<<<build_blocks, 256, 0, st>>>(t.nodes, t.pid, t.n_nodes, dp32, out.pairs64, out.pair_parent, out.tri_parent, n_tri, drep);
+    k_build_tris<<<build_blocks, 256, 0, st>>>(t.tris, t.stride, t.tri_index, materials, n_tri, out.tris, dt32, seen, drep);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(rep, drep, sizeof *rep, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return CT_OK;
+}
+
+// What the frame kernels read about the tree, from t and its build report; pointers into out as build_scene_arrays wrote them.
+void set_tree(DeviceState &s, const DeviceTree &t, const SceneArrays &out, const BuildReport &rep) {
+    Params &p = s.p;
+    const HotLayout hl = hot_layout(t.n_wide, t.n_pairs, p.n_tri);
+    p.root_cnt = t.root.triangle_count;
+    p.root_ref = t.root.triangle_count ? t.root.first_triangle_index : 0u;      // an interior root is pair 0
+    p.n_pairs = t.n_pairs;
+    p.n_nodes = t.n_nodes;
+    p.wide = t.n_wide ? reinterpret_cast<const DevWide *>(out.hot) : nullptr;
+    p.n_wide = t.n_wide;
+    p.pos_of_tri0 = rep.pos0;
+    p.nested = (!rep.not_nested && !rep.boxes_bad) ? 1u : 0u;
+    for (int a = 0; a < 3; a++) {
+        double bound;
+        memcpy(&bound, &rep.bound_bits[a], sizeof bound);
+        p.bound[a] = (!rep.boxes_bad && bound < 1e30) ? bound : INFINITY;
+        p.root_min[a] = t.root.aabb_min[a]; p.root_max[a] = t.root.aabb_max[a];
+        p.root_min32[a] = (float)p.root_min[a]; p.root_max32[a] = (float)p.root_max[a];
+    }
+    p.pairs32 = reinterpret_cast<const DevPair32 *>(out.hot + hl.pairs_at); p.pairs64 = out.pairs64;
+    p.tris = out.tris; p.tris32 = reinterpret_cast<const DevTri32 *>(out.hot + hl.tris_at);
+    p.pair_parent = out.pair_parent; p.tri_parent = out.tri_parent;
+    s.hot_base = out.hot; s.hot_bytes = hl.bytes;
+    s.depth = t.depth;
+}
 
 int launch_grid(const DeviceState &s, int blocks_per_sm) { return s.n_sm * blocks_per_sm; }
 
@@ -291,16 +443,17 @@ bool launch_parked_primary(const DeviceState &s, const Params &v, bool count, cu
 // stream the tile's kernels run on; hitRatio scales the window down to the set-aside size when the scene is larger.
 int apply_l2_policy(DeviceState &s, int device, cudaStream_t st) {
     if (!g_l2_persist || !s.hot_base || s.hot_bytes == 0) return CT_OK;
-    cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, device));
-    if (prop.persistingL2CacheMaxSize <= 0 || prop.accessPolicyMaxWindowSize <= 0) return CT_OK;
+    int persisting_max = 0, window_max = 0;           // (two attributes: cudaGetDeviceProperties takes milliseconds)
+    CU(cudaDeviceGetAttribute(&persisting_max, cudaDevAttrMaxPersistingL2CacheSize, device));
+    CU(cudaDeviceGetAttribute(&window_max, cudaDevAttrMaxAccessPolicyWindowSize, device));
+    if (persisting_max <= 0 || window_max <= 0) return CT_OK;
     if (s.l2_set_aside == 0) {
-        const size_t want = std::min<size_t>(s.hot_bytes, (size_t)prop.persistingL2CacheMaxSize);
+        const size_t want = std::min<size_t>(s.hot_bytes, (size_t)persisting_max);
         if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) != cudaSuccess) { cudaGetLastError(); return CT_OK; }
         size_t got = 0;
         cudaDeviceGetLimit(&got, cudaLimitPersistingL2CacheSize);
         s.l2_set_aside = got;
-        s.l2_window = std::min<size_t>(s.hot_bytes, (size_t)prop.accessPolicyMaxWindowSize);
+        s.l2_window = std::min<size_t>(s.hot_bytes, (size_t)window_max);
     }
     if (s.l2_set_aside == 0) return CT_OK;
     cudaStreamAttrValue attr{};
@@ -689,10 +842,7 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     const size_t tri_bytes = (size_t)(d->n_triangles - 1) * d->triangle_stride + 72;      // the last triangle may end at its third vertex
     Staging stg;
     CU(cudaStreamCreateWithFlags(&stg.st, cudaStreamNonBlocking));
-    const ct_bvh_node *raw_nodes = nullptr; const uint32_t *raw_idx = nullptr; const unsigned char *raw_tris = nullptr;
-    uint32_t *raw_pid = nullptr;
-    uint32_t n_nodes = d->n_nodes, n_pairs = 0;
-    ct_bvh_node root{};
+    DeviceTree t;
     if (build) {
         BbBuffers bf;
         bb_carve(stg.arena, d->n_triangles, tri_bytes, bf);
@@ -700,46 +850,27 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
         stg.arena.used = 0;
         bb_carve(stg.arena, d->n_triangles, tri_bytes, bf);
         CU(cudaMemcpyAsync(bf.raw, d->triangles, tri_bytes, cudaMemcpyHostToDevice, stg.st));
-        CU(bb_build(bf, d->triangle_stride, d->n_triangles, n_sm, stg.st, &n_nodes, &depth));
-        CU(cudaMemcpyAsync(&root, bf.out, sizeof root, cudaMemcpyDeviceToHost, stg.st));
-        CU(cudaStreamSynchronize(stg.st));
+        TRY(build_device_tree(stg, bf, d->triangle_stride, d->n_triangles, n_sm, t));
         lap("BVH built on the device");
-        if (depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", depth, kStackMax);
-        n_pairs = (n_nodes - 1u) / 2u;                                      // every node is reachable: 1 + 2 * interior nodes
-        uint32_t *ptile = nullptr;                                          // interior numbering: a scan over the node order
-        CU(stg.alloc(&raw_pid, (size_t)n_nodes + 1)); CU(stg.alloc(&ptile, ((size_t)n_nodes + 1) / kBbScanTile + 1));
-        const int blocks = std::max(1, std::min(n_sm * 8, (int)((n_nodes + kBbThreads) / kBbThreads)));
-        k_pid_flags<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, n_nodes, raw_pid);
-        CU(bb_scan(raw_pid, n_nodes, ptile, stg.st));
-        k_pid_leaves<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, n_nodes, raw_pid);
-        CU(cudaGetLastError());
-        raw_nodes = bf.out; raw_idx = bf.tri_index; raw_tris = bf.raw;
     } else {
-        root = d->nodes[0];
+        t.root = d->nodes[0];
+        t.n_nodes = d->n_nodes; t.depth = depth; t.stride = d->triangle_stride;
         // nodes: reference layout -> per-interior-node child pairs, built on the device from the raw arrays (k_build_pairs); the host
         // only numbers the interior nodes it validated
         std::vector<uint32_t> pid_of(d->n_nodes, kNoPos);
         for (uint32_t i = 0; i < d->n_nodes; i++)
-            if (reachable[i]) pid_of[i] = d->nodes[i].triangle_count == 0 ? n_pairs++ : kLeafMark;      // unreachable slots get no record and write nothing
-        ct_bvh_node *rn = nullptr; uint32_t *ri = nullptr; unsigned char *rt = nullptr;
-        CU(stg.alloc(&rn, d->n_nodes)); CU(stg.alloc(&raw_pid, d->n_nodes)); CU(stg.alloc(&ri, d->n_triangles)); CU(stg.alloc(&rt, tri_bytes));
+            if (reachable[i]) pid_of[i] = d->nodes[i].triangle_count == 0 ? t.n_pairs++ : kLeafMark;      // unreachable slots get no record and write nothing
+        ct_bvh_node *rn = nullptr; uint32_t *rp = nullptr, *ri = nullptr; unsigned char *rt = nullptr;
+        CU(stg.alloc(&rn, d->n_nodes)); CU(stg.alloc(&rp, d->n_nodes)); CU(stg.alloc(&ri, d->n_triangles)); CU(stg.alloc(&rt, tri_bytes));
         CU(cudaMemcpyAsync(rn, d->nodes, (size_t)d->n_nodes * sizeof(ct_bvh_node), cudaMemcpyHostToDevice, stg.st));
-        CU(cudaMemcpyAsync(raw_pid, pid_of.data(), (size_t)d->n_nodes * 4, cudaMemcpyHostToDevice, stg.st));
+        CU(cudaMemcpyAsync(rp, pid_of.data(), (size_t)d->n_nodes * 4, cudaMemcpyHostToDevice, stg.st));
         CU(cudaMemcpyAsync(ri, d->tri_indexes, (size_t)d->n_triangles * 4, cudaMemcpyHostToDevice, stg.st));
         CU(cudaMemcpyAsync(rt, d->triangles, tri_bytes, cudaMemcpyHostToDevice, stg.st));
-        raw_nodes = rn; raw_idx = ri; raw_tris = rt;
+        t.nodes = rn; t.pid = rp; t.tri_index = ri; t.tris = rt;
         lap("interior-node numbering (host)");
     }
     // the early-exit walks' wide tree, into scratch first: its size decides the layout of the hot allocation below
-    DevWide *wide_tmp = nullptr;
-    uint32_t n_wide = 0;
-    if (root.triangle_count == 0) {
-        uint32_t *root_of = nullptr, *wcnt = nullptr, *wtile = nullptr;
-        CU(stg.alloc(&wide_tmp, n_pairs)); CU(stg.alloc(&root_of, (size_t)n_pairs + 1)); CU(stg.alloc(&wcnt, (size_t)n_pairs + 1));
-        CU(stg.alloc(&wtile, ((size_t)n_pairs + 1) / kBbScanTile + 1));
-        CU(build_wide(raw_nodes, root_of, wcnt, wtile, wide_tmp, n_sm, stg.st, &n_wide));
-    }
-    CU(cudaStreamSynchronize(stg.st));
+    TRY(collapse_wide(stg, t, n_sm));
     lap("wide tree (device)");
 
     free_device(s);
@@ -759,72 +890,32 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     s.p.primary_budget = g_primary_budget_option < 0 ? 0u : g_primary_budget_option > 0 ? (uint32_t)std::min<long long>(g_primary_budget_option, 1ll << 30) : kDefaultPrimaryBudget;
     s.flags = d->flags;
     s.leaf_dfs_order = dfs_order;
-    s.depth = depth;
 
     Params &p = s.p;
     p.n_tri = d->n_triangles; p.n_lights = d->n_lights;
-    p.root_cnt = root.triangle_count;
-    p.root_ref = root.triangle_count ? root.first_triangle_index : 0u;      // an interior root is pair 0
-    p.n_pairs = n_pairs;
-    p.n_nodes = n_nodes;
-    s.can_overflow = (uint64_t)n_nodes + d->n_triangles > p.budget;      // parked rays: only when a DFS can run past the budget at all
+    s.can_overflow = walks_can_park(p, t.n_nodes);
 
-    DevPair32 *dp32 = nullptr; DevPair64 *dp64 = nullptr; DevTri *dt = nullptr; DevTri32 *dt32 = nullptr; ct_material *dm = nullptr;
-    uint32_t *dpp = nullptr, *dtp = nullptr;
-    {
-        // the records every walk step reads -- fp32 child pairs and fp32 triangles -- share ONE allocation, so that a single
-        // L2 access-policy window can cover them (apply_l2_policy)
-        const size_t pair_bytes = ((size_t)std::max<uint32_t>(n_pairs, 1) * sizeof(DevPair32) + 255u) & ~(size_t)255u;
-        const size_t wide_bytes = ((size_t)n_wide * sizeof(DevWide) + 255u) & ~(size_t)255u;
-        unsigned char *hot = nullptr;
-        s.hot_bytes = wide_bytes + pair_bytes + (size_t)d->n_triangles * sizeof(DevTri32);
-        TRY(dev_alloc(s, &hot, s.hot_bytes));
-        s.hot_base = hot;
-        if (n_wide) {
-            CU(cudaMemcpyAsync(hot, wide_tmp, (size_t)n_wide * sizeof(DevWide), cudaMemcpyDeviceToDevice, s.stream));
-            p.wide = reinterpret_cast<const DevWide *>(hot);
-            p.n_wide = n_wide;
-        }
-        dp32 = reinterpret_cast<DevPair32 *>(hot + wide_bytes); dt32 = reinterpret_cast<DevTri32 *>(hot + wide_bytes + pair_bytes);
-    }
-    TRY(dev_alloc(s, &dp64, std::max<uint32_t>(n_pairs, 1)));
-    TRY(dev_alloc(s, &dt, d->n_triangles)); TRY(dev_alloc(s, &dm, d->n_triangles));
-    TRY(dev_alloc(s, &dtp, d->n_triangles));
-    if (s.can_overflow) TRY(dev_alloc(s, &dpp, std::max<uint32_t>(n_pairs, 1)));
+    SceneArrays out{};
+    ct_material *dm = nullptr;
+    const uint32_t pairs = std::max<uint32_t>(t.n_pairs, 1);
+    s.hot_cap = hot_layout(t.n_wide, t.n_pairs, d->n_triangles).bytes;
+    TRY(dev_alloc(s, &out.hot, s.hot_cap));
+    TRY(dev_alloc(s, &out.pairs64, pairs)); s.pairs_cap = pairs;
+    TRY(dev_alloc(s, &out.tris, d->n_triangles)); TRY(dev_alloc(s, &dm, d->n_triangles));
+    TRY(dev_alloc(s, &out.tri_parent, d->n_triangles));
+    if (s.can_overflow) { TRY(dev_alloc(s, &out.pair_parent, pairs)); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
     BuildReport rep{};
     {
-        uint32_t *seen = nullptr; BuildReport *drep = nullptr;
-        auto staged = [&](cudaError_t e) { if (e != cudaSuccess) free_device(s); return e; };
-        CU(staged(stg.alloc(&drep, 1)));
-        const size_t seen_words = ((size_t)d->n_triangles + 31u) / 32u;
-        CU(staged(stg.alloc(&seen, seen_words)));
-        CU(staged(cudaMemsetAsync(seen, 0, seen_words * 4, s.stream)));
-        rep.bad_pos = kNoPos; rep.pos0 = kNoPos;
-        CU(staged(cudaMemcpyAsync(drep, &rep, sizeof rep, cudaMemcpyHostToDevice, s.stream)));
-        if (dpp) CU(staged(cudaMemsetAsync(dpp, 0xff, (size_t)std::max<uint32_t>(n_pairs, 1) * 4, s.stream)));
-        CU(staged(cudaMemsetAsync(dtp, 0xff, (size_t)d->n_triangles * 4, s.stream)));
-        const int build_blocks = s.n_sm * 8;
-        k_build_pairs<<<build_blocks, 256, 0, s.stream>>>(raw_nodes, raw_pid, n_nodes, dp32, dp64, dpp, dtp, d->n_triangles, drep);
-        CU(staged(cudaMemcpyAsync(dm, d->materials, (size_t)d->n_triangles * sizeof(ct_material), cudaMemcpyHostToDevice, s.stream)));
-        k_build_tris<<<build_blocks, 256, 0, s.stream>>>(raw_tris, (uint32_t)d->triangle_stride, raw_idx, dm, d->n_triangles, dt, dt32, seen, drep);
-        CU(staged(cudaGetLastError()));
-        CU(staged(cudaMemcpyAsync(&rep, drep, sizeof rep, cudaMemcpyDeviceToHost, s.stream)));
-        CU(staged(cudaStreamSynchronize(s.stream)));
+        const cudaError_t e = cudaMemcpyAsync(dm, d->materials, (size_t)d->n_triangles * sizeof(ct_material), cudaMemcpyHostToDevice, s.stream);
+        if (e != cudaSuccess) { free_device(s); CU(e); }
+        const int rc = build_scene_arrays(stg, s.stream, t, dm, d->n_triangles, out, s.n_sm, &rep);
+        if (rc != CT_OK) { free_device(s); return rc; }
     }
     if (rep.bad_pos != kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes[%u] = %u out of range", rep.bad_pos, build ? 0u : d->tri_indexes[rep.bad_pos]); }
     if (rep.duplicate || rep.pos0 == kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes is not a permutation of 0..n_triangles-1 (an index occurs twice)"); }
-    p.pos_of_tri0 = rep.pos0;
-    p.nested = (!rep.not_nested && !rep.boxes_bad) ? 1u : 0u;
     s.any_reflective = rep.any_reflective != 0;
-    for (int a = 0; a < 3; a++) {
-        double bound;
-        memcpy(&bound, &rep.bound_bits[a], sizeof bound);
-        p.bound[a] = (!rep.boxes_bad && bound < 1e30) ? bound : INFINITY;
-        p.root_min[a] = root.aabb_min[a]; p.root_max[a] = root.aabb_max[a];
-        p.root_min32[a] = (float)p.root_min[a]; p.root_max32[a] = (float)p.root_max[a];
-    }
-    p.pairs32 = dp32; p.pairs64 = dp64; p.tris = dt; p.tris32 = dt32; p.materials = dm;
-    p.pair_parent = dpp; p.tri_parent = dtp;
+    set_tree(s, t, out, rep);
+    p.materials = dm;
     lap("scene arrays built on the device");
     std::vector<DevLight> lights(std::max<uint32_t>(d->n_lights, 1));
     for (uint32_t i = 0; i < d->n_lights; i++) {
@@ -882,11 +973,7 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     TRY(dev_alloc(s, &s.occ_all, (size_t)p.cap * p.occ_words * levels, true));
     p.occ = s.occ_all;
     if (s.can_overflow) {
-        // parked rays per launch: 2^18 (16 MB) -- with primary walks parked as well (option "primary_budget": 2-3 % of a dragon-class
-        // frame's primary rays) 1/16 of the frame's paths where that is more; a full buffer means finishing rays in place, which
-        // must stay hypothetical
-        p.ovf_cap = 1u << 18;
-        if (p.primary_budget > 0u) p.ovf_cap = std::max<uint32_t>(p.ovf_cap, p.cap / 16u);
+        p.ovf_cap = parking_cap(p);
         TRY(dev_alloc(s, &s.ovf_all, (size_t)p.ovf_cap * 2 * levels));
         TRY(dev_alloc(s, &s.ovf_huge_all, (size_t)p.ovf_cap * 2 * levels));
         p.ovf = s.ovf_all; p.ovf_huge = s.ovf_huge_all;
@@ -966,6 +1053,123 @@ int ct_gpu_build_bvh(int device, uint32_t n_triangles, const void *triangles, ui
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
     lap("tree to the host");
     return (int)n_nodes;
+}
+
+// The scene ct_gpu_upload_scene with CT_FLAG_BUILD_BVH would load from the caller's triangles and the loaded scene's materials,
+// lights, camera and frame, built by the same functions into the loaded scene's arrays: the tree in scratch first (a refused or
+// failed build changes nothing), then -- after the device has finished the work in flight -- the scene arrays over the live ones.
+// Everything else the device holds stays.
+int ct_gpu_update_triangles(int device, const ct_triangle_update *u) {
+    if (!u || u->struct_size != sizeof(ct_triangle_update)) return fail(CT_ERR_INVALID, "ct_triangle_update missing or struct_size != %zu", sizeof(ct_triangle_update));
+    if (!u->triangles) return fail(CT_ERR_INVALID, "NULL triangles");
+    if (u->triangle_stride < 72 || u->triangle_stride % 8) return fail(CT_ERR_INVALID, "triangle_stride must be >= 72 and a multiple of 8");
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    std::lock_guard<std::mutex> lock(g_mutex);
+    DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    Params &p = s.p;
+    if (u->n_triangles != p.n_tri) return fail(CT_ERR_INVALID, "%u triangles: the loaded scene has %u (a re-upload changes the count)", u->n_triangles, p.n_tri);
+    TRY(check_device_array(device, u->triangles, 8, "triangles"));
+    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
+    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
+    const double t_begin = now_ms();
+    double t_mark = t_begin;
+    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_update_triangles: %-28s %7.2f ms\n", what, t - t_mark); t_mark = t; } };
+    const cudaStream_t st = u->stream ? static_cast<cudaStream_t>(u->stream) : s.stream;
+    const uint32_t n = p.n_tri;
+    const size_t tri_bytes = (size_t)(n - 1) * u->triangle_stride + 72;      // the last triangle may end at its third vertex
+
+    // the caller's triangles into the build's arena in `st`'s order; the build runs on the scratch stream behind them
+    Staging stg;
+    stg.async = true;
+    CU(cudaStreamCreateWithFlags(&stg.st, cudaStreamNonBlocking));
+    CU(cudaEventCreateWithFlags(&stg.ready, cudaEventDisableTiming));
+    BbBuffers bf;
+    bb_carve(stg.arena, n, tri_bytes, bf);
+    {
+        const cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&stg.arena.base), stg.arena.used, st);
+        if (e != cudaSuccess) { cudaGetLastError(); stg.arena.base = nullptr; CU(e); }
+    }
+    stg.arena.used = 0;
+    bb_carve(stg.arena, n, tri_bytes, bf);
+    {
+        const cudaError_t c = cudaMemcpyAsync(bf.raw, u->triangles, tri_bytes, cudaMemcpyDeviceToDevice, st);
+        cudaError_t w = cudaEventRecord(stg.ready, st);
+        if (w == cudaSuccess) w = cudaStreamWaitEvent(stg.st, stg.ready, 0);
+        if (w != cudaSuccess) cudaStreamSynchronize(st);              // the arena is freed in stg.st's order: after the copy
+        CU(c); CU(w);
+    }
+    DeviceTree t;
+    TRY(build_device_tree(stg, bf, u->triangle_stride, n, s.n_sm, t));
+    lap("BVH built on the device");
+    TRY(collapse_wide(stg, t, s.n_sm));
+    lap("wide tree (device)");
+
+    // The live allocations the new tree needs: the hot allocation, pairs64 and pair_parent are reused where the new records fit,
+    // the parking buffers appear when walks can be parked for the first time.  New ones are taken before anything is written.
+    const HotLayout hl = hot_layout(t.n_wide, t.n_pairs, n);
+    const uint32_t pairs = std::max<uint32_t>(t.n_pairs, 1);
+    const bool can_overflow = walks_can_park(p, t.n_nodes);
+    SceneArrays out{};
+    out.hot = hl.bytes <= s.hot_cap ? static_cast<unsigned char *>(s.hot_base) : nullptr;
+    out.pairs64 = pairs <= s.pairs_cap ? const_cast<DevPair64 *>(p.pairs64) : nullptr;
+    out.pair_parent = !can_overflow ? nullptr : pairs <= s.pair_parent_cap ? s.pair_parent_mem : nullptr;
+    out.tri_parent = const_cast<uint32_t *>(p.tri_parent);
+    out.tris = const_cast<DevTri *>(p.tris);
+    const bool new_hot = !out.hot, new_pairs = !out.pairs64, new_parent = can_overflow && !out.pair_parent, new_parking = can_overflow && !s.ovf_all;
+    OvfRay *ovf = nullptr; uint32_t *ovf_huge = nullptr;
+    const uint32_t ovf_cap = new_parking ? parking_cap(p) : p.ovf_cap;
+    auto take = [&]() -> int {
+        if (new_hot) TRY(dev_alloc(s, &out.hot, hl.bytes));
+        if (new_pairs) TRY(dev_alloc(s, &out.pairs64, pairs));
+        if (new_parent) TRY(dev_alloc(s, &out.pair_parent, pairs));
+        if (new_parking) { TRY(dev_alloc(s, &ovf, (size_t)ovf_cap * 2 * s.levels)); TRY(dev_alloc(s, &ovf_huge, (size_t)ovf_cap * 2 * s.levels)); }
+        return CT_OK;
+    };
+    auto give_back = [&]() {                                         // the new allocations of a call that fails
+        if (new_hot) dev_release(s, out.hot);
+        if (new_pairs) dev_release(s, out.pairs64);
+        if (new_parent) dev_release(s, out.pair_parent);
+        dev_release(s, ovf); dev_release(s, ovf_huge);
+    };
+    int rc = take();
+    if (rc != CT_OK) { give_back(); return rc; }
+    lap("allocation");
+
+    // frames and queries in flight finish on the previous geometry (the rule of a re-upload, whose cudaFree waits for the device)
+    {
+        const cudaError_t e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) { give_back(); CU(e); }
+    }
+    BuildReport rep{};
+    rc = build_scene_arrays(stg, stg.st, t, p.materials, n, out, s.n_sm, &rep);
+    if (rc != CT_OK) {
+        // nothing was written when the scratch could not be taken; past that point only a CUDA failure gets here
+        give_back();
+        return rc;
+    }
+    lap("scene arrays built on the device");
+    void *const old_hot = s.hot_base;
+    const size_t old_hot_bytes = s.hot_bytes;
+    if (new_hot) { dev_release(s, s.hot_base); s.hot_cap = hl.bytes; }
+    if (new_pairs) { dev_release(s, const_cast<DevPair64 *>(p.pairs64)); s.pairs_cap = pairs; }
+    if (new_parent) { dev_release(s, s.pair_parent_mem); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
+    if (new_parking) { s.ovf_all = ovf; s.ovf_huge_all = ovf_huge; p.ovf_cap = ovf_cap; p.ovf = ovf; p.ovf_huge = ovf_huge; }
+    s.can_overflow = can_overflow;
+    s.leaf_dfs_order = true;                                         // BuildBVH's leaves come in DFS order (bvh.cpp:70-97)
+    set_tree(s, t, out, rep);
+    lap("previous allocations freed");
+    if (s.hot_base != old_hot || s.hot_bytes != old_hot_bytes) {
+        // the window over the hot records, sized as an upload sizes it, on every stream the frames run on
+        release_l2(s);
+        TRY(apply_l2_policy(s, device, s.own_stream));
+        if (s.stream != s.own_stream) TRY(apply_l2_policy(s, device, s.stream));
+        for (cudaStream_t a : s.aux) TRY(apply_l2_policy(s, device, a));
+        lap("L2 window re-applied");
+    }
+    if (timing) fprintf(stderr, "ct_gpu_update_triangles: %u nodes, depth %d, L2 window %zu bytes; total %.2f ms\n", t.n_nodes, t.depth, s.l2_window, now_ms() - t_begin);
+    return CT_OK;
 }
 
 int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t capacity, size_t *bytes) {

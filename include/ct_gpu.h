@@ -396,6 +396,45 @@ typedef struct ct_shade_query {
 
 int ct_gpu_shade_rays(int device, const ct_shade_query *q);
 
+/* ---- moving a loaded scene's triangles on the device ----------------------------------------------------------------
+ * ct_gpu_update_triangles replaces the triangles of the scene loaded on `device` with n_triangles new ones held in device memory
+ * -- a mesh deformed or animated on the GPU -- and rebuilds the reference's tree (InitializeBVHState + BuildBVH, bvh.cpp:16-120)
+ * over them, on the device, in place.
+ *
+ * Result: afterwards the device holds exactly the scene ct_gpu_upload_scene with CT_FLAG_BUILD_BVH would load from these triangles
+ * plus the scene's current materials, lights, camera, frame size, depth and flags: every array ct_gpu_debug_scene_array exports is
+ * equal byte for byte, "summary" included, whether the scene was uploaded with a caller's tree or with the flag (after an update
+ * the tree is always BuildBVH's, leaf_dfs_order 1).  Frames and queries that follow equal the reference's on the new triangles.
+ *
+ * What it keeps -- the update is not an upload: the materials, lights, camera and frame settings; the stream set with
+ * ct_gpu_set_stream; a shared-frame attach, partition and frame count (ct_gpu_share_*); the framebuffer, which holds the previous
+ * frame's pixels until the next render, and the rows ct_gpu_readback copies; ct_gpu_get_counters, ct_gpu_kernel_launches,
+ * ct_gpu_overflow_stats and ct_gpu_reuse_stats.  Options read at upload (traversal_budget, overflow_warp_budget, any_leaves,
+ * primary_budget) keep their upload-time values.  The triangle count, materials and lights cannot change: re-upload for that.
+ *
+ * Order: the triangles are read in `stream`'s order (NULL = the render stream, see ct_gpu_set_stream), so work that wrote them on
+ * that stream needs no synchronisation by the caller.  The new tree is built into scratch from the stream-ordered allocator first;
+ * then the call waits for all work on the device -- frames and queries in flight finish on the old geometry, as they do when a
+ * re-upload frees the previous scene -- and overwrites the live arrays, reusing their allocations where the new tree fits.  The
+ * call is synchronous: when it returns, `triangles` may be overwritten or freed.  Every participant of a shared frame must update
+ * its triangles the same way before the next shared frame; the library does not check this.
+ *
+ * Returns CT_OK; CT_ERR_INVALID for a NULL u, a wrong struct_size, NULL triangles, n_triangles other than the loaded scene's, a
+ * triangle_stride below 72 or not a multiple of 8, triangles that are not device memory of `device` (host memory, pageable or
+ * pinned, is refused) or not 8-byte aligned; CT_ERR_NO_SCENE -- all checked before anything is enqueued or changed.  A new tree
+ * deeper than the device traversal stack (96) returns CT_ERR_LIMIT and a failed allocation CT_ERR_OOM; in both cases the previous
+ * triangles stay loaded and render as before. */
+typedef struct ct_triangle_update {
+    uint32_t struct_size;            /* = sizeof(ct_triangle_update) */
+    uint32_t n_triangles;            /* must equal the loaded scene's */
+    uint32_t triangle_stride;        /* as ct_scene_desc: >= 72, a multiple of 8 */
+    uint32_t _pad;
+    const void *triangles;           /* device memory of `device`: 9 doubles p1,p2,p3 at the start of each record, 8-byte aligned */
+    void *stream;                    /* cudaStream_t the triangles are read in the order of; NULL = the render stream */
+} ct_triangle_update;
+
+int ct_gpu_update_triangles(int device, const ct_triangle_update *u);
+
 /* Known-answer-test entry: ClosestIntersection (raythread.cpp:197-227) for n arbitrary rays through the
  * uploaded scene.  origins/directions: n x 3 doubles; t0: initial ray_t.t per ray (1e30f primary/shadow,
  * 0 for the reference's reflection rays, raythread.cpp:373).  Outputs may be NULL. */
