@@ -27,7 +27,7 @@ ABI_SYMBOLS = [
     "ct_gpu_set_stream", "ct_gpu_render_tile", "ct_gpu_readback", "ct_gpu_readback_async", "ct_gpu_readback_wait", "ct_gpu_readback_hits", "ct_gpu_get_counters",
     "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early", "ct_gpu_debug_primary",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
-    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays", "ct_gpu_shade_rays", "ct_gpu_update_triangles",
+    "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays", "ct_gpu_shade_rays", "ct_gpu_update_triangles", "ct_gpu_debug_shading",
 ]
 RAY_KINDS = {"primary": 0, "shadow": 1, "reflection": 2}     # CT_RAY_PRIMARY, CT_RAY_SHADOW, CT_RAY_REFLECTION
 
@@ -137,6 +137,7 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_debug_primary.argtypes = [C.c_int, C.c_uint32, vp, vp, C.c_uint32, vp, vp, vp, vp]
     L.ct_gpu_debug_primitives.argtypes = [C.c_int, C.c_uint32, vp, vp, vp, vp, vp, vp, vp, vp]
     L.ct_gpu_debug_filter.argtypes = [C.c_int, C.c_uint32, vp, vp, vp, vp, vp, vp, C.c_double, vp]
+    L.ct_gpu_debug_shading.argtypes = [C.c_int, C.c_uint32] + [vp] * 13
     L.ct_gpu_filter_stats.argtypes = [C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.ct_gpu_reuse_stats.argtypes = [C.c_int, C.POINTER(C.c_uint64)]
     L.ct_gpu_share_export.argtypes = [C.c_int, C.POINTER(Share)]
@@ -493,6 +494,27 @@ class GpuRenderer:
         n = o.shape[0]
         out = np.zeros(n, np.uint32)
         _check(self.L, self.L.ct_gpu_debug_filter(self.device, n, _ptr(o), _ptr(d), _ptr(rt), _ptr(tr), _ptr(mn), _ptr(mx), float(bound_scale), _ptr(out)))
+        return out
+
+    def debug_shading(self, color=None, intensity=None, lc=None, rc=None, reflection=None, x=None, e=None, acc=None, li=None):
+        """ct_gpu_debug_shading: the shading arithmetic on independent cases.  Each family is computed when its inputs are given:
+        (color, intensity) -> shaded uint32, (lc, rc, reflection) -> blended uint32, (x, e) -> pow float64, and with (acc, li) too the
+        specular accumulation float32.  Returns a dict of the families computed."""
+        u32 = lambda a: None if a is None else np.ascontiguousarray(a, np.uint32).ravel()
+        f32 = lambda a: None if a is None else np.ascontiguousarray(a, np.float32).ravel()
+        ins = dict(color=u32(color), intensity=f32(intensity), lc=u32(lc), rc=u32(rc), reflection=f32(reflection), x=f32(x),
+                   e=None if e is None else np.ascontiguousarray(e, np.int32).ravel(), acc=f32(acc), li=f32(li))
+        sizes = {a.size for a in ins.values() if a is not None}
+        if len(sizes) != 1:
+            raise ValueError("debug_shading: give at least one family, every input of the same length")
+        n = sizes.pop()
+        fam = {"shaded": ("color", "intensity"), "blended": ("lc", "rc", "reflection"), "pow": ("x", "e"), "acc": ("x", "e", "acc", "li")}
+        out = {k: np.zeros(n, np.float64 if k == "pow" else np.float32 if k == "acc" else np.uint32)
+               for k, need in fam.items() if all(ins[a] is not None for a in need)}
+        _check(self.L, self.L.ct_gpu_debug_shading(self.device, n, _ptr(ins["color"]), _ptr(ins["intensity"]), _ptr(out.get("shaded")),
+                                                   _ptr(ins["lc"]), _ptr(ins["rc"]), _ptr(ins["reflection"]), _ptr(out.get("blended")),
+                                                   _ptr(ins["x"]), _ptr(ins["e"]), _ptr(out.get("pow")), _ptr(ins["acc"]), _ptr(ins["li"]),
+                                                   _ptr(out.get("acc"))))
         return out
 
     def debug_scene_array(self, name: str) -> np.ndarray:

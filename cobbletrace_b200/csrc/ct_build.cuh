@@ -99,7 +99,7 @@ __global__ void __launch_bounds__(256) k_build_tris(const unsigned char *__restr
         t32.k2 = __double2float_ru(k2); t32.k3 = __double2float_ru(k3);
         tris[pos] = t;
         tris32[pos] = t32;
-        if (materials[k].reflection > 0.0f) refl = true;
+        if (!(materials[k].reflection <= 0.0f)) refl = true;       // NaN too: TraceRay recurses unless reflection <= 0 (:369)
     }
     if (__any_sync(0xffffffffu, refl) && (threadIdx.x & 31u) == 0) atomicOr(&rep->any_reflective, 1u);
 }

@@ -349,11 +349,14 @@ CT_DEV V3 reflect_ray(V3 rv, V3 n) {
 
 // pow(x, n) for ComputeLighting's specular term (raythread.cpp:321: pow(float, int) resolves to the double pow of glibc,
 // whose result is the correctly rounded x^n except within ~2^-15 ulp of a rounding boundary -- its error bound is
-// 0.52 ulp).  CUDA's pow() is documented at up to 2 ulp, so it is not used: for the integer exponents scene files hold
-// (material_t.specular is an int) x^n is computed by square-and-multiply in double-double arithmetic (error < 2^-95
-// relative for n <= 2^20) and rounded once, i.e. the correctly rounded value, which is what glibc returns in all but
-// astronomically rare cases; the double then enters a float accumulator, which discards its last 29 bits anyway.
-// Arguments outside the analysed range (x <= 0, huge or negative n, results near the subnormal range) use pow().
+// 0.52 ulp).  CUDA's pow() is documented at up to 2 ulp and does differ from glibc on reachable arguments (DESIGN 2), so
+// for the integer exponents scene files hold (material_t.specular is an int) x^|n| is computed by square-and-multiply in
+// double-double arithmetic, inverted in double-double for n < 0, and rounded once.  Each dd_mul / dd_recip is within
+// 2^-104 relative, a squaring doubles the relative error it is given, so for |n| <= 2^31 the result is within 2^-72
+// relative of x^n: the correctly rounded value unless x^n lies within 2^-19 ulp of a rounding boundary, and glibc's
+// value wherever glibc is correctly rounded.  pow() is left to arguments that no float qv reaches with a finite result
+// (x <= 2^-1000: 0, NaN) and to results outside [2^-900, 2^900] (an intermediate leaves that range), whose products
+// with a float intensity never move the float accumulator.
 struct DD { double hi, lo; };
 CT_DEV DD dd_mul(DD a, DD b) {
     const double p = __dmul_rn(a.hi, b.hi);
@@ -362,15 +365,31 @@ CT_DEV DD dd_mul(DD a, DD b) {
     const double hi = __dadd_rn(p, c);
     return {hi, __dadd_rn(__dsub_rn(p, hi), c)};                                 // fast two-sum: |p| >= |c|
 }
+// 1 / (a.hi + a.lo): q = fl(1/a.hi), then one Newton step with the exact remainder 1 - q a.hi
+CT_DEV DD dd_recip(DD a) {
+    const double q = __ddiv_rn(1.0, a.hi);
+    const double rem = __fma_rn(-q, a.lo, __fma_rn(-q, a.hi, 1.0));
+    const double c = __dmul_rn(rem, q);
+    const double hi = __dadd_rn(q, c);
+    return {hi, __dadd_rn(__dsub_rn(q, hi), c)};
+}
 CT_DEV double pow_int(double x, int n) {
-    if (!(x > 0x1p-1000) || !(x < 0x1p1000) || n < 0 || n > (1 << 20)) return pow(x, (double)n);
+    if (!(x > 0x1p-1000) || !(x < 0x1p1000)) return pow(x, (double)n);
     DD r = {1.0, 0.0}, b = {x, 0.0};
-    for (uint32_t k = (uint32_t)n; k; k >>= 1) {
+    for (uint32_t k = n < 0 ? 0u - (uint32_t)n : (uint32_t)n; k; k >>= 1) {
         if (k & 1u) r = dd_mul(r, b);
         if (k > 1u) b = dd_mul(b, b);
-        if (!(fabs(b.hi) > 0x1p-900) || !(fabs(b.hi) < 0x1p900) || !(fabs(r.hi) > 0x1p-900)) return pow(x, (double)n);   // leaves the range in which the error terms are normal numbers
+        if (!(fabs(b.hi) > 0x1p-900) || !(fabs(b.hi) < 0x1p900) || !(fabs(r.hi) > 0x1p-900) || !(fabs(r.hi) < 0x1p900))
+            return pow(x, (double)n);                                            // leaves the range in which the error terms are normal numbers
     }
+    if (n < 0) r = dd_recip(r);
     return __dadd_rn(r.hi, r.lo);
+}
+
+// raythread.cpp:321: intensity += li * pow(q, specular) -- the product in double, the sum rounded back to the float accumulator.
+CT_DEV float specular_add(float intensity, float li, float q, int specular) {
+    const double term = __dmul_rn((double)li, pow_int((double)q, specular));
+    return __double2float_rn(__dadd_rn((double)intensity, term));
 }
 
 // ---- color.h ------------------------------------------------------------------------------------
@@ -422,6 +441,13 @@ CT_DEV uint32_t shade_color(uint32_t color, float intensity) {
     return (b8 << 16) | (g8 << 8) | r8;
 }
 
+// The low byte of the reference's (int)c on x86-64: cvttsd2si truncates toward zero and returns the "integer indefinite" value
+// 0x80000000 (low byte 0) for a NaN and for every c outside (-2^31 - 1, 2^31).  PTX's cvt.rzi.s32.f64 saturates instead
+// (c >= 2^31 gives 0x7fffffff, low byte 0xff), so those values are mapped here.
+CT_DEV uint32_t x86_double_to_int_low8(double c) {
+    return (c > -2147483649.0 && c < 2147483648.0) ? ((uint32_t)__double2int_rz(c) & 0xffu) : 0u;
+}
+
 // raythread.cpp:375-379: local*(1-r) + reflected*r per channel in double, truncated to uint8_t
 CT_DEV uint32_t blend_color(uint32_t lc, uint32_t rc, float reflection) {
     double wl = (double)__fsub_rn(1.0f, reflection), wr = (double)reflection;
@@ -430,7 +456,7 @@ CT_DEV uint32_t blend_color(uint32_t lc, uint32_t rc, float reflection) {
     for (int sh = 0; sh <= 16; sh += 8) {
         double l = (double)((lc >> sh) & 0xffu), r = (double)((rc >> sh) & 0xffu);
         double c = __dadd_rn(__dmul_rn(wl, l), __dmul_rn(wr, r));
-        out |= ((uint32_t)__double2int_rz(c) & 0xffu) << sh;
+        out |= x86_double_to_int_low8(c) << sh;
     }
     return out;
 }

@@ -1833,6 +1833,48 @@ int ct_gpu_debug_filter(int device, uint32_t n, const double *origins, const dou
     return debug_primitives_impl(device, n, origins, directions, const_cast<float *>(ray_t), tri, bmin, bmax, nullptr, nullptr, verdict, bound_scale, true);
 }
 
+int ct_gpu_debug_shading(int device, uint32_t n, const uint32_t *color, const float *intensity, uint32_t *shaded,
+                         const uint32_t *lc, const uint32_t *rc, const float *reflection, uint32_t *blended,
+                         const float *x, const int32_t *e, double *pow_out, const float *acc, const float *li, float *acc_out) {
+    if ((shaded && (!color || !intensity)) || (blended && (!lc || !rc || !reflection)) || ((pow_out || acc_out) && (!x || !e)) ||
+        (acc_out && (!acc || !li)))
+        return fail(CT_ERR_INVALID, "NULL input for a requested output");
+    TRY(check_device(device));
+    if (n == 0) return CT_OK;
+    std::vector<void *> bufs;
+    int rc_ = CT_OK;
+    auto cleanup = [&]() { for (void *p : bufs) cudaFree(p); };
+#define CUX(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc_ = fail(CT_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); cleanup(); return rc_; } } while (0)
+    // a device copy of n elements of `src` (uploaded when given), nullptr when the family is not requested
+    auto dev = [&](const void *src, size_t elem, bool want, void **out) -> cudaError_t {
+        *out = nullptr;
+        if (!want) return cudaSuccess;
+        cudaError_t err = cudaMalloc(out, elem * n);
+        if (err != cudaSuccess) return err;
+        bufs.push_back(*out);
+        return src ? cudaMemcpy(*out, src, elem * n, cudaMemcpyHostToDevice) : cudaSuccess;
+    };
+    const bool want_pow = pow_out || acc_out;
+    void *d_color, *d_int, *d_shaded, *d_lc, *d_rc, *d_refl, *d_blended, *d_x, *d_e, *d_pow, *d_acc, *d_li, *d_acc_out;
+    CUX(dev(color, 4, shaded, &d_color)); CUX(dev(intensity, 4, shaded, &d_int)); CUX(dev(nullptr, 4, shaded, &d_shaded));
+    CUX(dev(lc, 4, blended, &d_lc)); CUX(dev(rc, 4, blended, &d_rc)); CUX(dev(reflection, 4, blended, &d_refl)); CUX(dev(nullptr, 4, blended, &d_blended));
+    CUX(dev(x, 4, want_pow, &d_x)); CUX(dev(e, 4, want_pow, &d_e)); CUX(dev(nullptr, 8, pow_out, &d_pow));
+    CUX(dev(acc, 4, acc_out, &d_acc)); CUX(dev(li, 4, acc_out, &d_li)); CUX(dev(nullptr, 4, acc_out, &d_acc_out));
+    k_debug_shading<<<(n + 255) / 256, 256>>>(n, (const uint32_t *)d_color, (const float *)d_int, (uint32_t *)d_shaded,
+                                               (const uint32_t *)d_lc, (const uint32_t *)d_rc, (const float *)d_refl, (uint32_t *)d_blended,
+                                               (const float *)d_x, (const int32_t *)d_e, (double *)d_pow, (const float *)d_acc, (const float *)d_li,
+                                               (float *)d_acc_out);
+    CUX(cudaGetLastError());
+    CUX(cudaDeviceSynchronize());
+    if (shaded) CUX(cudaMemcpy(shaded, d_shaded, 4ull * n, cudaMemcpyDeviceToHost));
+    if (blended) CUX(cudaMemcpy(blended, d_blended, 4ull * n, cudaMemcpyDeviceToHost));
+    if (pow_out) CUX(cudaMemcpy(pow_out, d_pow, 8ull * n, cudaMemcpyDeviceToHost));
+    if (acc_out) CUX(cudaMemcpy(acc_out, d_acc_out, 4ull * n, cudaMemcpyDeviceToHost));
+    cleanup();
+#undef CUX
+    return CT_OK;
+}
+
 int ct_gpu_shutdown(int device) {
     if (device < 0 || device >= kMaxDevices) return fail(CT_ERR_NO_DEVICE, "device %d out of range", device);
     DEVICE_GUARD(device);

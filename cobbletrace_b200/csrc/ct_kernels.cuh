@@ -713,7 +713,7 @@ CT_DEV void emit_paths(const Params &P, int depth, bool active, uint32_t q, uint
         float reflection = 0.0f;
         if (pos != kNoPos) reflection = P.materials[P.tris[pos].orig].reflection;
         const int remaining = P.max_depth - depth;                      // recursionDepth of this TraceRay call
-        if (pos == kNoPos || remaining <= 0 || !(reflection > 0.0f)) {  // miss :385 / :369 (reflection <= 0, NaN-safe)
+        if (pos == kNoPos || remaining <= 0 || reflection <= 0.0f) {     // miss :385 / :369 (a NaN reflection recurses)
             P.term_level[slot] = (uint8_t)depth;
         } else {
             V3 p1, e1, e2;
@@ -818,15 +818,14 @@ __global__ void __launch_bounds__(kBlockThreads) k_shade(const __grid_constant__
                 float rdv = vdot(refl, view);
                 if (rdv > 0.0f) {                                        // :319-321 double pow, += rounds to float
                     float qv = __fdiv_rn(rdv, __fmul_rn(vmag(refl), vmag(view)));
-                    double term = __dmul_rn((double)li, pow_int((double)qv, mat.specular));
-                    intensity = __double2float_rn(__dadd_rn((double)intensity, term));
+                    intensity = specular_add(intensity, li, qv, mat.specular);
                 }
             }
         }
         uint32_t local = shade_color(mat.color, intensity);
         *sc = local;
         // a depth-0 path that ends here (:369) is the pixel; longer chains are blended by k_resolve
-        if (depth == 0 && (P.max_depth <= 0 || !(mat.reflection > 0.0f))) store_pixel(P, slot, fbi, local);
+        if (depth == 0 && (P.max_depth <= 0 || mat.reflection <= 0.0f)) store_pixel(P, slot, fbi, local);
     }
 }
 
@@ -1289,6 +1288,18 @@ __global__ void k_debug_primitives(uint32_t n,const double *org, const double *d
     if (hit && t > kEps) r.t = macro_min(r.t, t);
     tri_hit[i] = hit ? 1u : 0u;
     ray_t[i] = r.t;
+}
+
+// The shading arithmetic of k_shade / k_resolve on n independent cases (ct_gpu_debug_shading); a NULL output skips its family.
+__global__ void k_debug_shading(uint32_t n, const uint32_t *color, const float *intensity, uint32_t *shaded,
+                                const uint32_t *lc, const uint32_t *rc, const float *reflection, uint32_t *blended,
+                                const float *x, const int32_t *e, double *pw, const float *acc, const float *li, float *acc_out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    if (shaded) shaded[i] = shade_color(color[i], intensity[i]);
+    if (blended) blended[i] = blend_color(lc[i], rc[i], reflection[i]);
+    if (pw) pw[i] = pow_int((double)x[i], e[i]);
+    if (acc_out) acc_out[i] = specular_add(acc[i], li[i], x[i], e[i]);
 }
 
 }  // namespace

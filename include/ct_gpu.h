@@ -480,6 +480,17 @@ int ct_gpu_debug_primitives(int device, uint32_t n, const double *origins, const
 int ct_gpu_debug_filter(int device, uint32_t n, const double *origins, const double *directions, const float *ray_t,
                         const double *tri, const double *bmin, const double *bmax, double bound_scale, uint32_t *verdict);
 
+/* Known-answer-test entry for the shading arithmetic of ComputeLighting / TraceRay (raythread.cpp:321, :365, :375-379): n
+ * independent cases, host arrays, synchronous; no scene is needed.  For each case i, with the functions the frame kernels call:
+ *   shaded[i]  = the colour ColorToHsv(color[i]) with v = intensity[i] gives back (HsvToColor), 0x00BBGGRR;
+ *   blended[i] = lc[i] * (1 - reflection[i]) + rc[i] * reflection[i] per channel, truncated to uint8_t;
+ *   pow_out[i] = pow(x[i], e[i]) in double (the specular term);
+ *   acc_out[i] = float(double(acc[i]) + double(li[i]) * pow(x[i], e[i])), the specular accumulation.
+ * Any output may be NULL (its inputs may then be NULL too). */
+int ct_gpu_debug_shading(int device, uint32_t n, const uint32_t *color, const float *intensity, uint32_t *shaded,
+                         const uint32_t *lc, const uint32_t *rc, const float *reflection, uint32_t *blended,
+                         const float *x, const int32_t *e, double *pow_out, const float *acc, const float *li, float *acc_out);
+
 /* Frees everything held for `device` (the reference never frees; this makes the library re-entrant). */
 int ct_gpu_shutdown(int device);
 
