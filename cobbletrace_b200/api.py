@@ -28,7 +28,9 @@ ABI_SYMBOLS = [
     "ct_gpu_last_tile_ms", "ct_gpu_sync", "ct_gpu_throttle", "ct_gpu_kernel_launches", "ct_gpu_last_tile_stages", "ct_gpu_framebuffer", "ct_gpu_gather_rows", "ct_gpu_debug_closest", "ct_gpu_debug_early", "ct_gpu_debug_primary",
     "ct_gpu_debug_primitives", "ct_gpu_debug_filter", "ct_gpu_filter_stats", "ct_gpu_reuse_stats", "ct_gpu_shutdown", "ct_gpu_share_export", "ct_gpu_share_attach", "ct_gpu_share_reset", "ct_gpu_share_partition", "ct_gpu_mark_rows", "ct_gpu_render_shared", "ct_gpu_set_option", "ct_gpu_overflow_stats",
     "ct_gpu_build_bvh", "ct_gpu_debug_scene_array", "ct_gpu_trace_rays", "ct_gpu_shade_rays", "ct_gpu_update_triangles", "ct_gpu_debug_shading",
+    "ct_gpu_update_scene",
 ]
+CT_UPDATE_TRIANGLES, CT_UPDATE_MATERIALS, CT_UPDATE_LIGHTS = 1, 2, 4
 RAY_KINDS = {"primary": 0, "shadow": 1, "reflection": 2}     # CT_RAY_PRIMARY, CT_RAY_SHADOW, CT_RAY_REFLECTION
 
 
@@ -82,6 +84,17 @@ class TriangleUpdate(C.Structure):   # == ct_triangle_update
                 ("triangles", C.c_void_p), ("stream", C.c_void_p)]
 
 
+class SceneUpdate(C.Structure):  # == ct_scene_update
+    _fields_ = [("struct_size", C.c_uint32), ("what", C.c_uint32), ("n_triangles", C.c_uint32), ("triangle_stride", C.c_uint32),
+                ("n_lights", C.c_uint32), ("_pad", C.c_uint32), ("triangles", C.c_void_p), ("materials", C.c_void_p),
+                ("lights", C.c_void_p), ("stream", C.c_void_p)]
+
+
+class PathSummary(C.Structure):  # == ct_path_summary (ct_gpu_debug_scene_array "path_state")
+    _fields_ = [(k, C.c_uint32) for k in ("n_triangles", "n_lights", "n_shadow_lights", "occ_words", "any_leaves", "any_reflective",
+                                          "levels", "ovf_cap")]
+
+
 class RayCounters(C.Structure):  # == ct_ray_counters
     _fields_ = [("rays_primary", C.c_uint64), ("rays_shadow", C.c_uint64), ("rays_reflection", C.c_uint64),
                 ("box_tests", C.c_uint64), ("tri_tests", C.c_uint64)]
@@ -100,6 +113,11 @@ SUMMARY_DT = np.dtype([("n_pairs", "<u4"), ("n_wide", "<u4"), ("root_ref", "<u4"
                        ("leaf_dfs_order", "<u4"), ("can_overflow", "<u4"), ("bound", "<f8", 3), ("depth", "<i4"), ("pad", "<u4")])
 assert SUMMARY_DT.itemsize == 64
 SCENE_ARRAYS = ("wide", "pairs32", "pairs64", "tris32", "tris", "materials", "pair_parent", "tri_parent", "summary")
+# == ct_path_summary (ct_gpu_debug_scene_array "path_state")
+PATH_DT = np.dtype([(k, "<u4") for k, _ in PathSummary._fields_])
+assert PATH_DT.itemsize == C.sizeof(PathSummary) == 32
+# everything a loaded scene's frames read: the arrays, the device's light records and what the path state was sized from
+SCENE_STATE = SCENE_ARRAYS + ("lights", "shadow_lights", "path_state")
 
 _lib = None
 
@@ -154,6 +172,7 @@ def load_library(path: Optional[str] = None):
     L.ct_gpu_trace_rays.argtypes = [C.c_int, C.POINTER(RayQuery)]
     L.ct_gpu_shade_rays.argtypes = [C.c_int, C.POINTER(ShadeQuery)]
     L.ct_gpu_update_triangles.argtypes = [C.c_int, C.POINTER(TriangleUpdate)]
+    L.ct_gpu_update_scene.argtypes = [C.c_int, C.POINTER(SceneUpdate)]
     if path == GPU_LIB:
         _lib = L
     return L
@@ -236,6 +255,20 @@ class GpuRenderer:
         Anything else raises ValueError before the library is called."""
         import torch
         dev = torch.device("cuda", self.device)
+        triangles = self._device_triangles(triangles, dev)
+        if self.n_tri is not None and triangles.shape[0] != self.n_tri:
+            raise ValueError(f"{triangles.shape[0]} triangles: the uploaded scene has {self.n_tri}")
+        u = TriangleUpdate()
+        u.struct_size, u.n_triangles, u.triangle_stride = C.sizeof(TriangleUpdate), triangles.shape[0], 72
+        u.triangles = triangles.data_ptr() or None
+        u.stream = torch.cuda.current_stream(dev).cuda_stream or 1      # (handle 0, torch's default stream, is cudaStreamLegacy = 1)
+        _check(self.L, self.L.ct_gpu_update_triangles(self.device, C.byref(u)))
+
+    @staticmethod
+    def _device_triangles(triangles, dev):
+        """The triangles update_triangles / update_scene read in place: a float64 (n, 9) or (n, 3, 3) contiguous tensor on `dev`
+        (numpy: copied there)."""
+        import torch
         if isinstance(triangles, np.ndarray):
             triangles = torch.from_numpy(np.ascontiguousarray(triangles, np.float64)).to(dev)
         if not isinstance(triangles, torch.Tensor):
@@ -246,15 +279,112 @@ class GpuRenderer:
             raise ValueError(f"triangles are {triangles.dtype}, vertices are float64")
         if tuple(triangles.shape[1:]) not in ((9,), (3, 3)):
             raise ValueError(f"triangles have shape {tuple(triangles.shape)}, not (n, 9) or (n, 3, 3)")
-        if self.n_tri is not None and triangles.shape[0] != self.n_tri:
-            raise ValueError(f"{triangles.shape[0]} triangles: the uploaded scene has {self.n_tri}")
         if not triangles.is_contiguous():
             raise ValueError("triangles are not contiguous")
-        u = TriangleUpdate()
-        u.struct_size, u.n_triangles, u.triangle_stride = C.sizeof(TriangleUpdate), triangles.shape[0], 72
-        u.triangles = triangles.data_ptr() or None
+        return triangles
+
+    @staticmethod
+    def _columns(what, parts, names, dtypes, widths, dev):
+        """A tuple of tensors on `dev`, one per record field: 1-D (width 0) or (n, width), of the given dtypes, of one length n."""
+        import torch
+        if not isinstance(parts, (tuple, list)) or len(parts) != len(names):
+            raise ValueError(f"{what}: a numpy record array or a tuple ({', '.join(names)}) of tensors")
+        n = None
+        for name, a, ok, w in zip(names, parts, dtypes, widths):
+            if not isinstance(a, torch.Tensor):
+                raise ValueError(f"{what} {name}: a torch tensor, not {type(a).__name__}")
+            if a.device != dev:
+                raise ValueError(f"{what} {name} is on {a.device}, this renderer's scene is on {dev}")
+            if a.dtype not in ok:
+                raise ValueError(f"{what} {name} is {a.dtype}, not {' or '.join(map(str, ok))}")
+            if a.shape[1:] != ((w,) if w else ()) or a.dim() != (2 if w else 1):
+                raise ValueError(f"{what} {name} has shape {tuple(a.shape)}, not (n{', %d' % w if w else ''})")
+            if n is not None and a.shape[0] != n:
+                raise ValueError(f"{what}: {name} has {a.shape[0]} entries, {names[0]} {n}")
+            n = a.shape[0]
+        return n
+
+    def _device_materials(self, materials, dev):
+        """ct_material records (12 bytes) on `dev`: from a numpy MAT_DT array (copied), or packed on the current stream from
+        (color uint32 or int64 -- its low 32 bits --, specular int32, reflection float32) tensors."""
+        import torch
+        if isinstance(materials, np.ndarray):
+            if materials.dtype != MAT_DT or materials.ndim != 1:
+                raise ValueError(f"materials: a 1-D array of api.MAT_DT, not {materials.dtype} of shape {materials.shape}")
+            return torch.from_numpy(np.ascontiguousarray(materials).view(np.uint8)).to(dev).view(-1, 12), materials.shape[0]
+        n = self._columns("materials", materials, ("color", "specular", "reflection"),
+                          ((torch.uint32, torch.int64), (torch.int32,), (torch.float32,)), (0, 0, 0), dev)
+        color, specular, reflection = materials
+        if color.dtype == torch.int64:
+            color = color & 0xFFFFFFFF
+            color = torch.where(color >= 2**31, color - 2**32, color).to(torch.int32)
+        else:
+            color = color.view(torch.int32)
+        return torch.stack([color, specular, reflection.view(torch.int32)], 1).contiguous(), n
+
+    def _device_lights(self, lights, dev):
+        """ct_light records (56 bytes) on `dev`: from a numpy LIGHT_DT array (copied), or packed on the current stream from
+        (type int32 or int64, intensity float32, pos float64 (n, 3), dir float64 (n, 3)) tensors."""
+        import torch
+        if isinstance(lights, np.ndarray):
+            if lights.dtype != LIGHT_DT or lights.ndim != 1:
+                raise ValueError(f"lights: a 1-D array of api.LIGHT_DT, not {lights.dtype} of shape {lights.shape}")
+            return torch.from_numpy(np.ascontiguousarray(lights).view(np.uint8)).to(dev).view(-1, 56), lights.shape[0]
+        n = self._columns("lights", lights, ("type", "intensity", "pos", "dir"),
+                          ((torch.int32, torch.int64), (torch.float32,), (torch.float64,), (torch.float64,)), (0, 0, 3, 3), dev)
+        ltype, intensity, pos, direction = lights
+        if n == 0:
+            return torch.empty((0, 56), dtype=torch.uint8, device=dev), 0
+        parts = [(ltype.to(torch.int32), 4), (intensity, 4), (pos, 24), (direction, 24)]      # ct_light: type, intensity, position, direction
+        return torch.cat([a.contiguous().view(torch.uint8).view(n, w) for a, w in parts], 1), n
+
+    # -- ct_gpu_update_scene --------------------------------------------------------------------------
+    def update_scene(self, triangles=None, materials=None, lights=None):
+        """Replace any of the loaded scene's triangles (of any count), materials and lights from device memory: afterwards the device
+        holds the scene upload(..., build_bvh=True) would load from the new parts and the loaded ones left out, with the scene's camera
+        and frame; the stream set with set_stream, the framebuffer, counters and shared-frame state stay.  See ct_gpu_update_scene.
+
+        triangles: as update_triangles takes them, of any count; a new count needs new materials too.
+        materials: a numpy MAT_DT array, or a (color, specular, reflection) tuple of 1-D tensors on cuda:<device> -- color uint32 or
+                   int64 (its low 32 bits, 0x00BBGGRR), specular int32, reflection float32 -- one per triangle, by triangle id.
+        lights:    a numpy LIGHT_DT array, or a (type, intensity, pos, dir) tuple of tensors on cuda:<device> -- type int32 or int64,
+                   intensity float32, pos and dir float64 (n, 3) -- in file order; an empty one removes every light.
+        Tensors are packed into the library's records on torch.cuda.current_stream(device) and read in that stream's order, so a
+        kernel that wrote them there needs no synchronisation; numpy arrays are copied to the device first.  The call returns when the
+        update is done.  Anything malformed raises ValueError before the library is called."""
+        import torch
+        if triangles is None and materials is None and lights is None:
+            raise ValueError("update_scene: give triangles, materials or lights")
+        dev = torch.device("cuda", self.device)
+        u = SceneUpdate()
+        u.struct_size = C.sizeof(SceneUpdate)
+        keep = []                                                       # the packed inputs live until the call returns
+        n = self.n_tri
+        if triangles is not None:
+            t = self._device_triangles(triangles, dev)
+            u.what |= CT_UPDATE_TRIANGLES
+            n, u.triangle_stride, u.triangles = t.shape[0], 72, t.data_ptr() or None
+            if n == 0:
+                raise ValueError("triangles: a scene has at least one triangle")
+            keep.append(t)
+        if materials is not None:
+            m, n_mat = self._device_materials(materials, dev)
+            if n_mat != n:
+                raise ValueError(f"{n_mat} materials for {n} triangles")
+            u.what |= CT_UPDATE_MATERIALS
+            u.materials = m.data_ptr() or None
+            keep.append(m)
+        elif n != self.n_tri:
+            raise ValueError(f"{n} triangles: the uploaded scene has {self.n_tri}; a new count needs new materials")
+        u.n_triangles = n or 0
+        if lights is not None:
+            lt, n_lit = self._device_lights(lights, dev)
+            u.what |= CT_UPDATE_LIGHTS
+            u.n_lights, u.lights = n_lit, (lt.data_ptr() or None) if n_lit else None
+            keep.append(lt)
         u.stream = torch.cuda.current_stream(dev).cuda_stream or 1      # (handle 0, torch's default stream, is cudaStreamLegacy = 1)
-        _check(self.L, self.L.ct_gpu_update_triangles(self.device, C.byref(u)))
+        _check(self.L, self.L.ct_gpu_update_scene(self.device, C.byref(u)))
+        self.n_tri = n
 
     def set_camera(self, position, rotation):
         p = np.ascontiguousarray(position, np.float64); r = np.ascontiguousarray(rotation, np.float64).reshape(9)
@@ -518,12 +648,15 @@ class GpuRenderer:
         return out
 
     def debug_scene_array(self, name: str) -> np.ndarray:
-        """ct_gpu_debug_scene_array: the bytes of one array the upload built (api.SCENE_ARRAYS); "summary" as a SUMMARY_DT record."""
+        """ct_gpu_debug_scene_array: the bytes of one array the upload built (api.SCENE_STATE); "summary" as a SUMMARY_DT record,
+        "path_state" as a PATH_DT record."""
         n = C.c_size_t()
         _check(self.L, self.L.ct_gpu_debug_scene_array(self.device, name.encode(), None, 0, C.byref(n)))
         out = np.zeros(n.value, np.uint8)
         _check(self.L, self.L.ct_gpu_debug_scene_array(self.device, name.encode(), _ptr(out), out.size, C.byref(n)))
-        return out.view(SUMMARY_DT)[0] if name == "summary" else out
+        if name == "summary":
+            return out.view(SUMMARY_DT)[0]
+        return out.view(PATH_DT)[0] if name == "path_state" else out
 
     def filter_stats(self):
         """(box tests, triangle tests) the fp32 filters left to the fp64 arithmetic (needs CT_FLAG_COUNT_TESTS)."""

@@ -23,6 +23,10 @@ struct BuildReport {
     uint32_t duplicate;                  // a tri_indexes value occurs twice (with every value in range: not a permutation)
 };
 
+// TraceRay recurses unless reflection <= 0 (raythread.cpp:369): a NaN reflection reflects too.  The one test of whether a material
+// makes the scene reflective, for k_build_tris and k_any_reflective.
+__device__ __forceinline__ bool reflects(const ct_material &m) { return !(m.reflection <= 0.0f); }
+
 __global__ void __launch_bounds__(256) k_build_pairs(const ct_bvh_node *__restrict__ nodes, const uint32_t *__restrict__ pid_of, uint32_t n_nodes,
                                                      DevPair32 *__restrict__ pairs32, DevPair64 *__restrict__ pairs64,
                                                      uint32_t *__restrict__ pair_parent, uint32_t *__restrict__ tri_parent, uint32_t n_tri, BuildReport *rep) {
@@ -99,9 +103,59 @@ __global__ void __launch_bounds__(256) k_build_tris(const unsigned char *__restr
         t32.k2 = __double2float_ru(k2); t32.k3 = __double2float_ru(k3);
         tris[pos] = t;
         tris32[pos] = t32;
-        if (!(materials[k].reflection <= 0.0f)) refl = true;       // NaN too: TraceRay recurses unless reflection <= 0 (:369)
+        if (reflects(materials[k])) refl = true;
     }
     if (__any_sync(0xffffffffu, refl) && (threadIdx.x & 31u) == 0) atomicOr(&rep->any_reflective, 1u);
+}
+
+// Whether any of n materials reflects (ct_gpu_update_scene with new materials and no new triangles): *out |= 1.
+__global__ void __launch_bounds__(256) k_any_reflective(const ct_material *__restrict__ materials, uint32_t n, uint32_t *out) {
+    bool refl = false;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        if (reflects(materials[i])) refl = true;
+    if (__any_sync(0xffffffffu, refl) && (threadIdx.x & 31u) == 0) atomicOr(out, 1u);
+}
+
+// The one light conversion of ct_gpu_upload_scene and ct_gpu_update_scene: n lights in file order -> DevLight, and the lights that
+// cast shadow rays -> DevShadowLight, compacted in file order (the fp32 accumulation of ComputeLighting follows it).  Ambient lights
+// cast none (raythread.cpp:284-286); a point light's ray goes to its position (:288), every other type is directional (:293).
+// One block of 256 threads: the compaction is a running count, a ballot per warp and the warps' sums per round of 256 lights.
+// *n_slights: the shadow lights written.
+__global__ void __launch_bounds__(256) k_build_lights(const ct_light *__restrict__ in, uint32_t n, DevLight *__restrict__ lights,
+                                                      DevShadowLight *__restrict__ slights, uint32_t *__restrict__ n_slights) {
+    __shared__ uint32_t warp_sum[8];
+    __shared__ uint32_t base;
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) base = 0;
+    __syncthreads();
+    for (uint32_t first = 0; first < n; first += blockDim.x) {
+        const uint32_t i = first + threadIdx.x;
+        ct_light L{};
+        bool casts = false;
+        if (i < n) {
+            L = in[i];
+            DevLight d;
+            d.type = L.type; d.intensity = L.intensity;
+            for (int a = 0; a < 3; a++) { d.pos[a] = L.position[a]; d.dir[a] = L.direction[a]; }
+            lights[i] = d;
+            casts = L.type != CT_LIGHT_AMBIENT;
+        }
+        const uint32_t ballot = __ballot_sync(0xffffffffu, casts);
+        if (lane == 0) warp_sum[warp] = __popc(ballot);
+        __syncthreads();
+        uint32_t at = base + __popc(ballot & ((1u << lane) - 1u));
+        for (uint32_t w = 0; w < warp; w++) at += warp_sum[w];
+        if (casts) {
+            DevShadowLight sl;
+            sl.type = L.type; sl.index = i;
+            for (int a = 0; a < 3; a++) sl.v[a] = L.type == CT_LIGHT_POINT ? L.position[a] : L.direction[a];
+            slights[at] = sl;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) for (uint32_t w = 0; w < blockDim.x / 32u; w++) base += warp_sum[w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *n_slights = base;
 }
 
 // ---- the early-exit walks' wide tree (DevWide), built from the binary tree on the device --------------------------------

@@ -69,6 +69,12 @@ int fail(int code, const char *fmt, ...) {
             return fail(e_ == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); \
     } while (0)
 
+// The per-depth path state of the frames and their parking buffers, one allocation each (path_take / path_commit).
+enum PathArray {
+    PA_HIT0_T, PA_HIT0_POS, PA_STACK_COLOR, PA_TERM_LEVEL, PA_OCC, PA_OVF, PA_OVF_HUGE,
+    PA_HITB_T, PA_HITB_POS, PA_STACK_REFL, PA_RAYS, PA_PATH_SLOT, PA_PARENT_Q, PA_FAR, kPathArrays
+};
+
 struct DeviceState {
     bool loaded = false;
     Params p{};
@@ -124,6 +130,12 @@ struct DeviceState {
     size_t hot_cap = 0;
     uint32_t pairs_cap = 0, pair_parent_cap = 0;
     uint32_t *pair_parent_mem = nullptr;
+    // records the per-triangle arrays (tris, tri_parent, materials) and the two light arrays have room for (ct_gpu_update_scene
+    // reuses them when the new ones fit)
+    uint32_t tri_cap = 0, light_cap = 0;
+    void *path_mem[kPathArrays] = {};    // the path state: allocation and its bytes, by PathArray (NULL / 0: not allocated)
+    size_t path_cap[kPathArrays] = {};
+    long long any_leaves_option = 0;     // option "any_leaves" as it was at upload (ct_gpu_update_scene applies the rule with it)
     std::vector<void *> allocs;
     ct_ray_counters snapshot{};      // totals at the end of the previous counted tile
     unsigned long long rays_overflow = 0, rays_in_place = 0;   // DevTotals' overflow counters as of the last read_totals
@@ -349,12 +361,96 @@ HotLayout hot_layout(uint32_t n_wide, uint32_t n_pairs, uint32_t n_tri) {
 }
 
 // Parked rays: only when a DFS can run past the visit budget at all.
-bool walks_can_park(const Params &p, uint32_t n_nodes) { return (uint64_t)n_nodes + p.n_tri > p.budget; }
+bool walks_can_park(const Params &p, uint32_t n_nodes, uint32_t n_tri) { return (uint64_t)n_nodes + n_tri > p.budget; }
 
 // Parked rays per launch: 2^18 (16 MB) -- with primary walks parked as well (option "primary_budget": 2-3 % of a dragon-class
 // frame's primary rays) 1/16 of the frame's paths where that is more; a full buffer means finishing rays in place, which must
 // stay hypothetical.
 uint32_t parking_cap(const Params &p) { return p.primary_budget > 0u ? std::max<uint32_t>(1u << 18, p.cap / 16u) : 1u << 18; }
+
+// The any-hit walk's leaf-list length trades the lit rays' phase overhead against the occluded rays' early exit: measured 12 best for
+// the 3-light dragon frame (k_shadow 1.11 ms against 1.15 at 8), 8 for the 66-light scene (6.75 ms against 7.14 at 12) -- a shading point
+// inside a sphere of lights has half of them behind its own surface.  Option "any_leaves" (as read at upload) overrides; 0 = this rule.
+uint32_t any_leaves_for(long long option, uint32_t n_slights) { return option > 0 ? (uint32_t)option : (n_slights >= 16u ? 8u : 12u); }
+
+// Words of occlusion bits per path: one bit per light, shadow-casting or not (k_shadow's bit is the light's number).
+uint32_t occ_words_for(uint32_t n_lights) { return std::max<uint32_t>((n_lights + 31u) / 32u, 1u); }
+
+// ---- the frames' path state: one layout for ct_gpu_upload_scene and ct_gpu_update_scene ----------------------------------------
+// Bytes of each PathArray for paths of `levels` depths (max_depth + 1 with a reflective material, else 1), occ_words words of
+// occlusion bits per path and parking buffers of ovf_cap rays per launch (0: no walk can be parked); 0 = not allocated.
+void path_bytes(uint32_t cap, int levels, uint32_t occ_words, uint32_t ovf_cap, size_t out[kPathArrays]) {
+    const size_t c = cap, L = (size_t)levels, deep = levels > 1 ? 1u : 0u, park = ovf_cap;
+    out[PA_HIT0_T] = 4 * c; out[PA_HIT0_POS] = 4 * c;
+    out[PA_STACK_COLOR] = 4 * c * L; out[PA_TERM_LEVEL] = c;
+    out[PA_OCC] = 4 * c * occ_words * L;
+    out[PA_OVF] = sizeof(OvfRay) * park * 2 * L; out[PA_OVF_HUGE] = 4 * park * 2 * L;
+    out[PA_HITB_T] = out[PA_HITB_POS] = out[PA_STACK_REFL] = out[PA_FAR] = deep * 4 * c * L;
+    out[PA_RAYS] = deep * 48 * c * (L + 1);
+    out[PA_PATH_SLOT] = out[PA_PARENT_Q] = deep * 4 * c * (L + 1);
+}
+
+// What path_take planned: each array's bytes and the allocations taken for the arrays whose allocation was too small.
+struct PathPlan {
+    size_t bytes[kPathArrays] = {};
+    void *fresh[kPathArrays] = {};
+    int levels = 1;
+    uint32_t occ_words = 1, ovf_cap = 0;
+};
+
+// Allocates every path array whose new size does not fit its allocation; nothing is written or released.  Every [depth][cap] array is
+// addressed by cap, occ_words and ovf_cap alone, so a larger allocation serves as it is.
+int path_take(DeviceState &s, int levels, uint32_t occ_words, uint32_t ovf_cap, PathPlan &pl) {
+    pl.levels = levels; pl.occ_words = occ_words; pl.ovf_cap = ovf_cap;
+    path_bytes(s.p.cap, levels, occ_words, ovf_cap, pl.bytes);
+    for (int i = 0; i < kPathArrays; i++)
+        if (pl.bytes[i] > s.path_cap[i]) TRY(dev_alloc(s, reinterpret_cast<unsigned char **>(&pl.fresh[i]), pl.bytes[i]));
+    return CT_OK;
+}
+
+void path_give_back(DeviceState &s, PathPlan &pl) {
+    for (void *&q : pl.fresh) { dev_release(s, q); q = nullptr; }
+}
+
+// Installs the plan: releases the allocations it replaces and those no longer needed (the arrays of deeper levels without a reflective
+// material, the parking buffers when no walk can be parked), zeroes the occlusion words and term_level as an upload does (on st, which
+// is synchronised) and points the frame state at the arrays.
+int path_commit(DeviceState &s, PathPlan &pl, cudaStream_t st) {
+    for (int i = 0; i < kPathArrays; i++) {
+        if (!pl.fresh[i] && pl.bytes[i] != 0) continue;
+        dev_release(s, s.path_mem[i]);
+        s.path_mem[i] = pl.fresh[i]; s.path_cap[i] = pl.fresh[i] ? pl.bytes[i] : 0;
+        pl.fresh[i] = nullptr;
+    }
+    CU(cudaMemsetAsync(s.path_mem[PA_TERM_LEVEL], 0, pl.bytes[PA_TERM_LEVEL], st));
+    CU(cudaMemsetAsync(s.path_mem[PA_OCC], 0, pl.bytes[PA_OCC], st));
+    CU(cudaStreamSynchronize(st));
+    Params &p = s.p;
+    void *const *m = s.path_mem;
+    p.hit0_t = static_cast<float *>(m[PA_HIT0_T]); p.hit0_pos = static_cast<uint32_t *>(m[PA_HIT0_POS]);
+    p.stack_color = static_cast<uint32_t *>(m[PA_STACK_COLOR]); p.term_level = static_cast<uint8_t *>(m[PA_TERM_LEVEL]);
+    p.stack_refl = static_cast<float *>(m[PA_STACK_REFL]);
+    s.occ_all = static_cast<uint32_t *>(m[PA_OCC]);
+    s.ovf_all = static_cast<OvfRay *>(m[PA_OVF]); s.ovf_huge_all = static_cast<uint32_t *>(m[PA_OVF_HUGE]);
+    s.hitb_t_all = static_cast<float *>(m[PA_HITB_T]); s.hitb_pos_all = static_cast<uint32_t *>(m[PA_HITB_POS]);
+    s.rays_all = static_cast<double *>(m[PA_RAYS]); s.path_slot_all = static_cast<uint32_t *>(m[PA_PATH_SLOT]);
+    s.parent_q_all = static_cast<uint32_t *>(m[PA_PARENT_Q]); s.far_all = static_cast<uint32_t *>(m[PA_FAR]);
+    p.occ = s.occ_all; p.occ_words = pl.occ_words;
+    p.ovf = s.ovf_all; p.ovf_huge = s.ovf_huge_all; p.ovf_cap = pl.ovf_cap;
+    s.levels = pl.levels;
+    return CT_OK;
+}
+
+// k_build_lights over the n lights at `in` (device memory) into lights / slights on st; *n_slights: the shadow lights.  Synchronises st.
+int build_lights(Staging &stg, cudaStream_t st, const ct_light *in, uint32_t n, DevLight *lights, DevShadowLight *slights, uint32_t *n_slights) {
+    uint32_t *count = nullptr;
+    CU(stg.alloc(&count, 1));
+    k_build_lights<<<1, 256, 0, st>>>(in, n, lights, slights, count);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(n_slights, count, sizeof *n_slights, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return CT_OK;
+}
 
 // Where the scene arrays go.  pair_parent may be NULL (no walk can be parked).
 struct SceneArrays { unsigned char *hot; DevPair64 *pairs64; uint32_t *pair_parent, *tri_parent; DevTri *tris; };
@@ -891,9 +987,11 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     s.flags = d->flags;
     s.leaf_dfs_order = dfs_order;
 
+    s.any_leaves_option = g_any_leaves;
+
     Params &p = s.p;
     p.n_tri = d->n_triangles; p.n_lights = d->n_lights;
-    s.can_overflow = walks_can_park(p, t.n_nodes);
+    s.can_overflow = walks_can_park(p, t.n_nodes, p.n_tri);
 
     SceneArrays out{};
     ct_material *dm = nullptr;
@@ -903,6 +1001,7 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     TRY(dev_alloc(s, &out.pairs64, pairs)); s.pairs_cap = pairs;
     TRY(dev_alloc(s, &out.tris, d->n_triangles)); TRY(dev_alloc(s, &dm, d->n_triangles));
     TRY(dev_alloc(s, &out.tri_parent, d->n_triangles));
+    s.tri_cap = d->n_triangles;
     if (s.can_overflow) { TRY(dev_alloc(s, &out.pair_parent, pairs)); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
     BuildReport rep{};
     {
@@ -917,31 +1016,15 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     set_tree(s, t, out, rep);
     p.materials = dm;
     lap("scene arrays built on the device");
-    std::vector<DevLight> lights(std::max<uint32_t>(d->n_lights, 1));
-    for (uint32_t i = 0; i < d->n_lights; i++) {
-        lights[i].type = d->lights[i].type; lights[i].intensity = d->lights[i].intensity;
-        for (int a = 0; a < 3; a++) { lights[i].pos[a] = d->lights[i].position[a]; lights[i].dir[a] = d->lights[i].direction[a]; }
-    }
-    std::vector<DevShadowLight> slights;
-    for (uint32_t i = 0; i < d->n_lights; i++) {
-        if (d->lights[i].type == CT_LIGHT_AMBIENT) continue;            // raythread.cpp:284-286: no shadow ray
-        DevShadowLight sl{};
-        sl.type = d->lights[i].type; sl.index = i;
-        const double *v = (sl.type == CT_LIGHT_POINT) ? d->lights[i].position : d->lights[i].direction;   // :288 / :293 (every non-point light is directional)
-        for (int a = 0; a < 3; a++) sl.v[a] = v[a];
-        slights.push_back(sl);
-    }
-    p.n_slights = (uint32_t)slights.size();
-    // the any-hit walk's leaf-list length trades the lit rays' phase overhead against the occluded rays' early exit: measured 12 best for
-    // the 3-light dragon frame (k_shadow 1.11 ms against 1.15 at 8), 8 for the 66-light scene (6.75 ms against 7.14 at 12) -- a shading point
-    // inside a sphere of lights has half of them behind its own surface.  Option "any_leaves" overrides (0 = this rule).
-    p.any_leaves = g_any_leaves > 0 ? (uint32_t)g_any_leaves : (p.n_slights >= 16u ? 8u : 12u);
-    p.occ_words = std::max<uint32_t>((d->n_lights + 31u) / 32u, 1u);
-    DevLight *dl = nullptr; DevShadowLight *dsl = nullptr;
-    TRY(dev_alloc(s, &dl, lights.size()));
-    TRY(dev_alloc(s, &dsl, slights.size()));
-    if (!slights.empty()) CU(cudaMemcpy(dsl, slights.data(), slights.size() * sizeof(DevShadowLight), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(dl, lights.data(), lights.size() * sizeof(DevLight), cudaMemcpyHostToDevice));
+    // the lights: the caller's records to the device, converted there by the kernel ct_gpu_update_scene runs on new lights
+    DevLight *dl = nullptr; DevShadowLight *dsl = nullptr; ct_light *lights_in = nullptr;
+    s.light_cap = std::max<uint32_t>(d->n_lights, 1);
+    TRY(dev_alloc(s, &dl, s.light_cap));
+    TRY(dev_alloc(s, &dsl, s.light_cap));
+    CU(stg.alloc(&lights_in, d->n_lights));
+    if (d->n_lights) CU(cudaMemcpyAsync(lights_in, d->lights, (size_t)d->n_lights * sizeof(ct_light), cudaMemcpyHostToDevice, stg.st));
+    TRY(build_lights(stg, stg.st, lights_in, d->n_lights, dl, dsl, &p.n_slights));
+    p.any_leaves = any_leaves_for(s.any_leaves_option, p.n_slights);
     p.slights = dsl; p.lights = dl;
 
     memcpy(p.cam, d->camera_position, sizeof p.cam);
@@ -965,25 +1048,10 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
         p.cap = (uint32_t)((slots + kChunkMax - 1u) / kChunkMax * kChunkMax);
     }
 
-    const int levels = s.any_reflective ? d->max_depth + 1 : 1;
-    TRY(dev_alloc(s, &p.hit0_t, p.cap)); TRY(dev_alloc(s, &p.hit0_pos, p.cap));
-    TRY(dev_alloc(s, &p.stack_color, (size_t)p.cap * levels));
-    TRY(dev_alloc(s, &p.term_level, p.cap, true));
-    s.levels = levels;
-    TRY(dev_alloc(s, &s.occ_all, (size_t)p.cap * p.occ_words * levels, true));
-    p.occ = s.occ_all;
-    if (s.can_overflow) {
-        p.ovf_cap = parking_cap(p);
-        TRY(dev_alloc(s, &s.ovf_all, (size_t)p.ovf_cap * 2 * levels));
-        TRY(dev_alloc(s, &s.ovf_huge_all, (size_t)p.ovf_cap * 2 * levels));
-        p.ovf = s.ovf_all; p.ovf_huge = s.ovf_huge_all;
-    }
-    if (levels > 1) {
-        TRY(dev_alloc(s, &s.hitb_t_all, (size_t)p.cap * levels)); TRY(dev_alloc(s, &s.hitb_pos_all, (size_t)p.cap * levels));
-        TRY(dev_alloc(s, &p.stack_refl, (size_t)p.cap * levels));
-        TRY(dev_alloc(s, &s.rays_all, (size_t)p.cap * 6 * (levels + 1))); TRY(dev_alloc(s, &s.path_slot_all, (size_t)p.cap * (levels + 1)));
-        TRY(dev_alloc(s, &s.parent_q_all, (size_t)p.cap * (levels + 1)));
-        TRY(dev_alloc(s, &s.far_all, (size_t)p.cap * levels));
+    {
+        PathPlan pl;
+        TRY(path_take(s, s.any_reflective ? d->max_depth + 1 : 1, occ_words_for(d->n_lights), s.can_overflow ? parking_cap(p) : 0u, pl));
+        TRY(path_commit(s, pl, s.stream));
     }
     TRY(dev_alloc(s, &p.fb, (size_t)d->width * d->height, true));       // calloc'd like cobbletrace.cpp:57
     p.subsample = (d->flags & CT_FLAG_SUBSAMPLING) ? 1 : 0;
@@ -1055,110 +1123,194 @@ int ct_gpu_build_bvh(int device, uint32_t n_triangles, const void *triangles, ui
     return (int)n_nodes;
 }
 
-// The scene ct_gpu_upload_scene with CT_FLAG_BUILD_BVH would load from the caller's triangles and the loaded scene's materials,
-// lights, camera and frame, built by the same functions into the loaded scene's arrays: the tree in scratch first (a refused or
-// failed build changes nothing), then -- after the device has finished the work in flight -- the scene arrays over the live ones.
-// Everything else the device holds stays.
-int ct_gpu_update_triangles(int device, const ct_triangle_update *u) {
-    if (!u || u->struct_size != sizeof(ct_triangle_update)) return fail(CT_ERR_INVALID, "ct_triangle_update missing or struct_size != %zu", sizeof(ct_triangle_update));
-    if (!u->triangles) return fail(CT_ERR_INVALID, "NULL triangles");
-    if (u->triangle_stride < 72 || u->triangle_stride % 8) return fail(CT_ERR_INVALID, "triangle_stride must be >= 72 and a multiple of 8");
+// The scene ct_gpu_upload_scene with CT_FLAG_BUILD_BVH would load from the caller's new triangles, materials and / or lights and the
+// loaded scene's other parts, camera and frame, built by the upload's functions (ct_gpu_update_scene; ct_gpu_update_triangles is
+// what = CT_UPDATE_TRIANGLES).  Everything new is computed into scratch and every allocation it needs is taken first -- a refused or
+// failed build changes nothing; then, after the device has finished the work in flight, it is written over the live state, reusing the
+// allocations where the new records fit.  Everything else the device holds stays.
+static int update_impl(int device, const ct_scene_update &u, const char *who) {
+    if (u.what == 0 || (u.what & ~(uint32_t)(CT_UPDATE_TRIANGLES | CT_UPDATE_MATERIALS | CT_UPDATE_LIGHTS)))
+        return fail(CT_ERR_INVALID, "what = %#x: a non-empty mask of CT_UPDATE_TRIANGLES, CT_UPDATE_MATERIALS, CT_UPDATE_LIGHTS", u.what);
+    const bool new_tri = (u.what & CT_UPDATE_TRIANGLES) != 0, new_mat = (u.what & CT_UPDATE_MATERIALS) != 0, new_lit = (u.what & CT_UPDATE_LIGHTS) != 0;
+    if (new_tri || new_mat) {
+        if (u.n_triangles == 0) return fail(CT_ERR_INVALID, "a scene has at least one triangle");
+        if (u.n_triangles >= (1u << 31)) return fail(CT_ERR_LIMIT, "%u triangles: the device build takes fewer than 2^31", u.n_triangles);
+    }
+    if (new_tri && !u.triangles) return fail(CT_ERR_INVALID, "NULL triangles");
+    if (new_tri && (u.triangle_stride < 72 || u.triangle_stride % 8)) return fail(CT_ERR_INVALID, "triangle_stride must be >= 72 and a multiple of 8");
+    if (new_mat && !u.materials) return fail(CT_ERR_INVALID, "NULL materials");
+    if (new_lit && u.n_lights && !u.lights) return fail(CT_ERR_INVALID, "n_lights = %u but lights == NULL", u.n_lights);
     TRY(check_device(device));
     DEVICE_GUARD(device);
     std::lock_guard<std::mutex> lock(g_mutex);
     DeviceState &s = g_dev[device];
     if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
     Params &p = s.p;
-    if (u->n_triangles != p.n_tri) return fail(CT_ERR_INVALID, "%u triangles: the loaded scene has %u (a re-upload changes the count)", u->n_triangles, p.n_tri);
-    TRY(check_device_array(device, u->triangles, 8, "triangles"));
+    const uint32_t n = (new_tri || new_mat) ? u.n_triangles : p.n_tri;
+    if (n != p.n_tri && !new_tri) return fail(CT_ERR_INVALID, "%u materials: the loaded scene has %u triangles (new materials alone keep the count)", n, p.n_tri);
+    if (n != p.n_tri && !new_mat)
+        return fail(CT_ERR_INVALID, "%u triangles: the loaded scene has %u (a new count needs new materials: CT_UPDATE_MATERIALS)", n, p.n_tri);
+    if (new_tri) TRY(check_device_array(device, u.triangles, 8, "triangles"));
+    if (new_mat) TRY(check_device_array(device, u.materials, 4, "materials"));
+    if (new_lit && u.n_lights) TRY(check_device_array(device, u.lights, 8, "lights"));
     const bool timing = getenv("CT_GPU_TIMING") != nullptr;
     auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
     const double t_begin = now_ms();
     double t_mark = t_begin;
-    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_update_triangles: %-28s %7.2f ms\n", what, t - t_mark); t_mark = t; } };
-    const cudaStream_t st = u->stream ? static_cast<cudaStream_t>(u->stream) : s.stream;
-    const uint32_t n = p.n_tri;
-    const size_t tri_bytes = (size_t)(n - 1) * u->triangle_stride + 72;      // the last triangle may end at its third vertex
+    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "%s: %-28s %7.2f ms\n", who, what, t - t_mark); t_mark = t; } };
+    const cudaStream_t st = u.stream ? static_cast<cudaStream_t>(u.stream) : s.stream;
+    const uint32_t n_lights = new_lit ? u.n_lights : p.n_lights;
 
-    // the caller's triangles into the build's arena in `st`'s order; the build runs on the scratch stream behind them
+    // The caller's arrays into scratch in `st`'s order (allocated there too); the build runs on the scratch stream behind them.
     Staging stg;
     stg.async = true;
     CU(cudaStreamCreateWithFlags(&stg.st, cudaStreamNonBlocking));
     CU(cudaEventCreateWithFlags(&stg.ready, cudaEventDisableTiming));
     BbBuffers bf;
-    bb_carve(stg.arena, n, tri_bytes, bf);
+    ct_material *mat_in = nullptr;
+    ct_light *lit_in = nullptr;
     {
-        const cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&stg.arena.base), stg.arena.used, st);
-        if (e != cudaSuccess) { cudaGetLastError(); stg.arena.base = nullptr; CU(e); }
-    }
-    stg.arena.used = 0;
-    bb_carve(stg.arena, n, tri_bytes, bf);
-    {
-        const cudaError_t c = cudaMemcpyAsync(bf.raw, u->triangles, tri_bytes, cudaMemcpyDeviceToDevice, st);
-        cudaError_t w = cudaEventRecord(stg.ready, st);
-        if (w == cudaSuccess) w = cudaStreamWaitEvent(stg.st, stg.ready, 0);
-        if (w != cudaSuccess) cudaStreamSynchronize(st);              // the arena is freed in stg.st's order: after the copy
-        CU(c); CU(w);
+        auto stage = [&]() -> cudaError_t {
+            cudaError_t e = cudaSuccess;
+            if (new_tri) {
+                const size_t tri_bytes = (size_t)(n - 1) * u.triangle_stride + 72;      // the last triangle may end at its third vertex
+                bb_carve(stg.arena, n, tri_bytes, bf);
+                if ((e = cudaMallocAsync(reinterpret_cast<void **>(&stg.arena.base), stg.arena.used, st)) != cudaSuccess) { stg.arena.base = nullptr; return e; }
+                stg.arena.used = 0;
+                bb_carve(stg.arena, n, tri_bytes, bf);
+                if ((e = cudaMemcpyAsync(bf.raw, u.triangles, tri_bytes, cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+            }
+            if (new_mat) {
+                if ((e = cudaMallocAsync(reinterpret_cast<void **>(&mat_in), (size_t)n * sizeof(ct_material), st)) != cudaSuccess) return e;
+                stg.ptrs.push_back(mat_in);
+                if ((e = cudaMemcpyAsync(mat_in, u.materials, (size_t)n * sizeof(ct_material), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+            }
+            if (new_lit) {
+                if ((e = cudaMallocAsync(reinterpret_cast<void **>(&lit_in), (size_t)std::max<uint32_t>(n_lights, 1) * sizeof(ct_light), st)) != cudaSuccess) return e;
+                stg.ptrs.push_back(lit_in);
+                if (n_lights && (e = cudaMemcpyAsync(lit_in, u.lights, (size_t)n_lights * sizeof(ct_light), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+            }
+            if ((e = cudaEventRecord(stg.ready, st)) != cudaSuccess) return e;
+            return cudaStreamWaitEvent(stg.st, stg.ready, 0);
+        };
+        const cudaError_t e = stage();
+        if (e != cudaSuccess) { cudaGetLastError(); cudaStreamSynchronize(st); CU(e); }    // the scratch is freed in stg.st's order
     }
     DeviceTree t;
-    TRY(build_device_tree(stg, bf, u->triangle_stride, n, s.n_sm, t));
-    lap("BVH built on the device");
-    TRY(collapse_wide(stg, t, s.n_sm));
-    lap("wide tree (device)");
+    if (new_tri) {
+        TRY(build_device_tree(stg, bf, u.triangle_stride, n, s.n_sm, t));
+        lap("BVH built on the device");
+        TRY(collapse_wide(stg, t, s.n_sm));
+        lap("wide tree (device)");
+    }
+    // What the frames derive from the materials and lights: whether any material reflects (the path state's depth), the lights and
+    // the compacted shadow lights (the path state's occlusion words, the any-hit walk's leaf list)
+    bool any_reflective = s.any_reflective;
+    if (new_mat) {
+        uint32_t *flag = nullptr, h = 0;
+        CU(stg.alloc(&flag, 1));
+        CU(cudaMemsetAsync(flag, 0, sizeof *flag, stg.st));
+        k_any_reflective<<<std::max(1, std::min(s.n_sm * 8, (int)((n + 255u) / 256u))), 256, 0, stg.st>>>(mat_in, n, flag);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(&h, flag, sizeof h, cudaMemcpyDeviceToHost, stg.st));
+        CU(cudaStreamSynchronize(stg.st));
+        any_reflective = h != 0;
+    }
+    DevLight *lit_new = nullptr; DevShadowLight *slit_new = nullptr;
+    uint32_t n_slights = p.n_slights;
+    if (new_lit) {
+        CU(stg.alloc(&lit_new, std::max<uint32_t>(n_lights, 1))); CU(stg.alloc(&slit_new, std::max<uint32_t>(n_lights, 1)));
+        TRY(build_lights(stg, stg.st, lit_in, n_lights, lit_new, slit_new, &n_slights));
+        lap("materials and lights (device)");
+    }
 
-    // The live allocations the new tree needs: the hot allocation, pairs64 and pair_parent are reused where the new records fit,
-    // the parking buffers appear when walks can be parked for the first time.  New ones are taken before anything is written.
-    const HotLayout hl = hot_layout(t.n_wide, t.n_pairs, n);
-    const uint32_t pairs = std::max<uint32_t>(t.n_pairs, 1);
-    const bool can_overflow = walks_can_park(p, t.n_nodes);
+    // The live allocations the new state needs, taken before anything is written: the tree's (hot allocation, pairs64, pair_parent),
+    // the per-triangle and light arrays when the new count is larger, the path state when its depth, occlusion words or parking grow.
+    const bool can_overflow = new_tri ? walks_can_park(p, t.n_nodes, n) : s.can_overflow;
+    const bool grow_tri = n > s.tri_cap, grow_lit = n_lights > s.light_cap;
+    HotLayout hl{};
+    uint32_t pairs = 0;
     SceneArrays out{};
-    out.hot = hl.bytes <= s.hot_cap ? static_cast<unsigned char *>(s.hot_base) : nullptr;
-    out.pairs64 = pairs <= s.pairs_cap ? const_cast<DevPair64 *>(p.pairs64) : nullptr;
-    out.pair_parent = !can_overflow ? nullptr : pairs <= s.pair_parent_cap ? s.pair_parent_mem : nullptr;
-    out.tri_parent = const_cast<uint32_t *>(p.tri_parent);
-    out.tris = const_cast<DevTri *>(p.tris);
-    const bool new_hot = !out.hot, new_pairs = !out.pairs64, new_parent = can_overflow && !out.pair_parent, new_parking = can_overflow && !s.ovf_all;
-    OvfRay *ovf = nullptr; uint32_t *ovf_huge = nullptr;
-    const uint32_t ovf_cap = new_parking ? parking_cap(p) : p.ovf_cap;
+    bool fresh_hot = false, fresh_pairs = false, fresh_parent = false;
+    ct_material *mat_fresh = nullptr; DevLight *dl_fresh = nullptr; DevShadowLight *dsl_fresh = nullptr;
+    PathPlan pl;
     auto take = [&]() -> int {
-        if (new_hot) TRY(dev_alloc(s, &out.hot, hl.bytes));
-        if (new_pairs) TRY(dev_alloc(s, &out.pairs64, pairs));
-        if (new_parent) TRY(dev_alloc(s, &out.pair_parent, pairs));
-        if (new_parking) { TRY(dev_alloc(s, &ovf, (size_t)ovf_cap * 2 * s.levels)); TRY(dev_alloc(s, &ovf_huge, (size_t)ovf_cap * 2 * s.levels)); }
+        if (new_tri) {
+            hl = hot_layout(t.n_wide, t.n_pairs, n);
+            pairs = std::max<uint32_t>(t.n_pairs, 1);
+            out.hot = hl.bytes <= s.hot_cap ? static_cast<unsigned char *>(s.hot_base) : nullptr;
+            out.pairs64 = pairs <= s.pairs_cap ? const_cast<DevPair64 *>(p.pairs64) : nullptr;
+            out.pair_parent = !can_overflow ? nullptr : pairs <= s.pair_parent_cap ? s.pair_parent_mem : nullptr;
+            out.tri_parent = grow_tri ? nullptr : const_cast<uint32_t *>(p.tri_parent);
+            out.tris = grow_tri ? nullptr : const_cast<DevTri *>(p.tris);
+            fresh_hot = !out.hot; fresh_pairs = !out.pairs64; fresh_parent = can_overflow && !out.pair_parent;
+            if (fresh_hot) TRY(dev_alloc(s, &out.hot, hl.bytes));
+            if (fresh_pairs) TRY(dev_alloc(s, &out.pairs64, pairs));
+            if (fresh_parent) TRY(dev_alloc(s, &out.pair_parent, pairs));
+            if (grow_tri) { TRY(dev_alloc(s, &out.tris, n)); TRY(dev_alloc(s, &out.tri_parent, n)); }
+        }
+        if (grow_tri) TRY(dev_alloc(s, &mat_fresh, n));                    // (a larger count comes with new materials)
+        if (grow_lit) { TRY(dev_alloc(s, &dl_fresh, n_lights)); TRY(dev_alloc(s, &dsl_fresh, n_lights)); }
+        TRY(path_take(s, any_reflective ? p.max_depth + 1 : 1, occ_words_for(n_lights), can_overflow ? parking_cap(p) : 0u, pl));
         return CT_OK;
     };
-    auto give_back = [&]() {                                         // the new allocations of a call that fails
-        if (new_hot) dev_release(s, out.hot);
-        if (new_pairs) dev_release(s, out.pairs64);
-        if (new_parent) dev_release(s, out.pair_parent);
-        dev_release(s, ovf); dev_release(s, ovf_huge);
+    auto give_back = [&]() {                                             // the new allocations of a call that fails
+        if (fresh_hot) dev_release(s, out.hot);
+        if (fresh_pairs) dev_release(s, out.pairs64);
+        if (fresh_parent) dev_release(s, out.pair_parent);
+        if (grow_tri && new_tri) { dev_release(s, out.tris); dev_release(s, out.tri_parent); }
+        dev_release(s, mat_fresh); dev_release(s, dl_fresh); dev_release(s, dsl_fresh);
+        path_give_back(s, pl);
     };
     int rc = take();
     if (rc != CT_OK) { give_back(); return rc; }
     lap("allocation");
 
-    // frames and queries in flight finish on the previous geometry (the rule of a re-upload, whose cudaFree waits for the device)
+    // frames and queries in flight finish on the previous scene (the rule of a re-upload, whose cudaFree waits for the device)
     {
         const cudaError_t e = cudaDeviceSynchronize();
         if (e != cudaSuccess) { give_back(); CU(e); }
     }
+    // Past this point only a CUDA failure returns early (nothing was written when build_scene_arrays cannot take its scratch).
     BuildReport rep{};
-    rc = build_scene_arrays(stg, stg.st, t, p.materials, n, out, s.n_sm, &rep);
-    if (rc != CT_OK) {
-        // nothing was written when the scratch could not be taken; past that point only a CUDA failure gets here
-        give_back();
-        return rc;
+    if (new_tri) {
+        rc = build_scene_arrays(stg, stg.st, t, new_mat ? mat_in : p.materials, n, out, s.n_sm, &rep);
+        if (rc != CT_OK) { give_back(); return rc; }
+        lap("scene arrays built on the device");
     }
-    lap("scene arrays built on the device");
+    ct_material *const mats = grow_tri ? mat_fresh : const_cast<ct_material *>(p.materials);
+    DevLight *const dl = grow_lit ? dl_fresh : const_cast<DevLight *>(p.lights);
+    DevShadowLight *const dsl = grow_lit ? dsl_fresh : const_cast<DevShadowLight *>(p.slights);
+    {
+        cudaError_t e = cudaSuccess;
+        if (new_mat) e = cudaMemcpyAsync(mats, mat_in, (size_t)n * sizeof(ct_material), cudaMemcpyDeviceToDevice, stg.st);
+        if (e == cudaSuccess && new_lit && n_lights) e = cudaMemcpyAsync(dl, lit_new, (size_t)n_lights * sizeof(DevLight), cudaMemcpyDeviceToDevice, stg.st);
+        if (e == cudaSuccess && new_lit && n_slights) e = cudaMemcpyAsync(dsl, slit_new, (size_t)n_slights * sizeof(DevShadowLight), cudaMemcpyDeviceToDevice, stg.st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(stg.st);
+        if (e != cudaSuccess) { give_back(); CU(e); }
+    }
+
+    // The new state in place of the old: the replaced allocations go back, the frames' parameters follow.
     void *const old_hot = s.hot_base;
     const size_t old_hot_bytes = s.hot_bytes;
-    if (new_hot) { dev_release(s, s.hot_base); s.hot_cap = hl.bytes; }
-    if (new_pairs) { dev_release(s, const_cast<DevPair64 *>(p.pairs64)); s.pairs_cap = pairs; }
-    if (new_parent) { dev_release(s, s.pair_parent_mem); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
-    if (new_parking) { s.ovf_all = ovf; s.ovf_huge_all = ovf_huge; p.ovf_cap = ovf_cap; p.ovf = ovf; p.ovf_huge = ovf_huge; }
+    if (new_tri) {
+        if (fresh_hot) { dev_release(s, s.hot_base); s.hot_cap = hl.bytes; }
+        if (fresh_pairs) { dev_release(s, const_cast<DevPair64 *>(p.pairs64)); s.pairs_cap = pairs; }
+        if (fresh_parent) { dev_release(s, s.pair_parent_mem); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
+        if (grow_tri) { dev_release(s, const_cast<DevTri *>(p.tris)); dev_release(s, const_cast<uint32_t *>(p.tri_parent)); }
+    }
+    if (grow_tri) { dev_release(s, const_cast<ct_material *>(p.materials)); s.tri_cap = n; }
+    if (grow_lit) { dev_release(s, const_cast<DevLight *>(p.lights)); dev_release(s, const_cast<DevShadowLight *>(p.slights)); s.light_cap = n_lights; }
+    p.materials = mats; p.lights = dl; p.slights = dsl;
+    p.n_tri = n; p.n_lights = n_lights; p.n_slights = n_slights;
+    p.any_leaves = any_leaves_for(s.any_leaves_option, n_slights);
+    s.any_reflective = any_reflective;
     s.can_overflow = can_overflow;
-    s.leaf_dfs_order = true;                                         // BuildBVH's leaves come in DFS order (bvh.cpp:70-97)
-    set_tree(s, t, out, rep);
+    TRY(path_commit(s, pl, stg.st));
+    if (new_tri) {
+        s.leaf_dfs_order = true;                                         // BuildBVH's leaves come in DFS order (bvh.cpp:70-97)
+        set_tree(s, t, out, rep);
+    }
     lap("previous allocations freed");
     if (s.hot_base != old_hot || s.hot_bytes != old_hot_bytes) {
         // the window over the hot records, sized as an upload sizes it, on every stream the frames run on
@@ -1168,8 +1320,30 @@ int ct_gpu_update_triangles(int device, const ct_triangle_update *u) {
         for (cudaStream_t a : s.aux) TRY(apply_l2_policy(s, device, a));
         lap("L2 window re-applied");
     }
-    if (timing) fprintf(stderr, "ct_gpu_update_triangles: %u nodes, depth %d, L2 window %zu bytes; total %.2f ms\n", t.n_nodes, t.depth, s.l2_window, now_ms() - t_begin);
+    if (timing) fprintf(stderr, "%s: %u triangles, %u lights, %d levels, L2 window %zu bytes; total %.2f ms\n", who, n, n_lights, s.levels,
+                        s.l2_window, now_ms() - t_begin);
     return CT_OK;
+}
+
+int ct_gpu_update_scene(int device, const ct_scene_update *u) {
+    if (!u || u->struct_size != sizeof(ct_scene_update)) return fail(CT_ERR_INVALID, "ct_scene_update missing or struct_size != %zu", sizeof(ct_scene_update));
+    return update_impl(device, *u, "ct_gpu_update_scene");
+}
+
+// The CT_UPDATE_TRIANGLES case of ct_gpu_update_scene, with its own refusals: the count must be the loaded scene's.
+int ct_gpu_update_triangles(int device, const ct_triangle_update *u) {
+    if (!u || u->struct_size != sizeof(ct_triangle_update)) return fail(CT_ERR_INVALID, "ct_triangle_update missing or struct_size != %zu", sizeof(ct_triangle_update));
+    if (!u->triangles) return fail(CT_ERR_INVALID, "NULL triangles");
+    if (u->triangle_stride < 72 || u->triangle_stride % 8) return fail(CT_ERR_INVALID, "triangle_stride must be >= 72 and a multiple of 8");
+    TRY(check_device(device));
+    DEVICE_GUARD(device);
+    const DeviceState &s = g_dev[device];
+    if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
+    if (u->n_triangles != s.p.n_tri) return fail(CT_ERR_INVALID, "%u triangles: the loaded scene has %u (ct_gpu_update_scene changes the count)", u->n_triangles, s.p.n_tri);
+    ct_scene_update v{};
+    v.struct_size = sizeof v; v.what = CT_UPDATE_TRIANGLES;
+    v.n_triangles = u->n_triangles; v.triangle_stride = u->triangle_stride; v.triangles = u->triangles; v.stream = u->stream;
+    return update_impl(device, v, "ct_gpu_update_triangles");
 }
 
 int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t capacity, size_t *bytes) {
@@ -1180,6 +1354,7 @@ int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t cap
     if (!s.loaded) return fail(CT_ERR_NO_SCENE, "no scene uploaded on device %d", device);
     const Params &p = s.p;
     ct_scene_summary sum{};
+    ct_path_summary ps{};
     const void *src = nullptr;
     size_t n = 0;
     const std::string nm(name);
@@ -1197,6 +1372,13 @@ int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t cap
         for (int a = 0; a < 3; a++) sum.bound[a] = p.bound[a];
         sum.depth = s.depth;
         n = sizeof sum;
+    }
+    else if (nm == "lights") { src = p.lights; n = (size_t)p.n_lights * sizeof(DevLight); }
+    else if (nm == "shadow_lights") { src = p.slights; n = (size_t)p.n_slights * sizeof(DevShadowLight); }
+    else if (nm == "path_state") {
+        ps.n_triangles = p.n_tri; ps.n_lights = p.n_lights; ps.n_shadow_lights = p.n_slights; ps.occ_words = p.occ_words;
+        ps.any_leaves = p.any_leaves; ps.any_reflective = s.any_reflective ? 1u : 0u; ps.levels = (uint32_t)s.levels; ps.ovf_cap = p.ovf_cap;
+        n = sizeof ps;
     } else {
         return fail(CT_ERR_INVALID, "unknown scene array \"%s\"", name);
     }
@@ -1204,6 +1386,7 @@ int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t cap
     if (!dst || n == 0) return CT_OK;
     if (capacity < n) return fail(CT_ERR_INVALID, "%s needs %zu bytes, capacity is %zu", name, n, capacity);
     if (nm == "summary") { memcpy(dst, &sum, n); return CT_OK; }
+    if (nm == "path_state") { memcpy(dst, &ps, n); return CT_OK; }
     CU(cudaMemcpyAsync(dst, src, n, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaStreamSynchronize(s.stream));
     return CT_OK;

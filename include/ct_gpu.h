@@ -154,9 +154,23 @@ typedef struct ct_scene_summary {
     uint32_t _pad;
 } ct_scene_summary;
 
+/* What the frames' path state was sized from, for tests that compare two uploads (ct_gpu_debug_scene_array "path_state"). */
+typedef struct ct_path_summary {
+    uint32_t n_triangles;
+    uint32_t n_lights;
+    uint32_t n_shadow_lights;  /* lights that cast shadow rays (all but the ambient ones) */
+    uint32_t occ_words;        /* words of occlusion bits per path: ceil(n_lights / 32), at least 1 */
+    uint32_t any_leaves;       /* leaf-list entries of the any-hit walk (option "any_leaves" as read at upload, or its rule) */
+    uint32_t any_reflective;   /* some material has reflection > 0 or NaN: paths recurse */
+    uint32_t levels;           /* path depths the per-depth arrays hold: max_depth + 1 with any_reflective, else 1 */
+    uint32_t ovf_cap;          /* rays per parking buffer (0: no walk can be parked, no parking buffers) */
+} ct_path_summary;
+
 /* Debug export: copies one of the arrays ct_gpu_upload_scene built into dst and sets *bytes to its size.  Names: "wide",
  * "pairs32", "pairs64", "tris32", "tris", "materials", "pair_parent" (0 bytes when no walk can be parked), "tri_parent",
- * "summary" (a ct_scene_summary).  dst == NULL only reports *bytes; capacity < *bytes is CT_ERR_INVALID.  Synchronises. */
+ * "summary" (a ct_scene_summary), "lights" (the device's light records, file order), "shadow_lights" (the records of the lights
+ * that cast shadow rays, file order), "path_state" (a ct_path_summary).  dst == NULL only reports *bytes; capacity < *bytes is
+ * CT_ERR_INVALID.  Synchronises. */
 int ct_gpu_debug_scene_array(int device, const char *name, void *dst, size_t capacity, size_t *bytes);
 
 /* Replaces the camera half of HandleUpdates (raythread.cpp:557-572) for an already uploaded scene. */
@@ -410,7 +424,8 @@ int ct_gpu_shade_rays(int device, const ct_shade_query *q);
  * ct_gpu_set_stream; a shared-frame attach, partition and frame count (ct_gpu_share_*); the framebuffer, which holds the previous
  * frame's pixels until the next render, and the rows ct_gpu_readback copies; ct_gpu_get_counters, ct_gpu_kernel_launches,
  * ct_gpu_overflow_stats and ct_gpu_reuse_stats.  Options read at upload (traversal_budget, overflow_warp_budget, any_leaves,
- * primary_budget) keep their upload-time values.  The triangle count, materials and lights cannot change: re-upload for that.
+ * primary_budget) keep their upload-time values.  ct_gpu_update_scene below also changes the triangle count, materials and lights;
+ * this call is its what = CT_UPDATE_TRIANGLES case with the count held fixed.
  *
  * Order: the triangles are read in `stream`'s order (NULL = the render stream, see ct_gpu_set_stream), so work that wrote them on
  * that stream needs no synchronisation by the caller.  The new tree is built into scratch from the stream-ordered allocator first;
@@ -434,6 +449,54 @@ typedef struct ct_triangle_update {
 } ct_triangle_update;
 
 int ct_gpu_update_triangles(int device, const ct_triangle_update *u);
+
+/* ---- editing a loaded scene on the device ---------------------------------------------------------------------------
+ * ct_gpu_update_scene replaces any of three parts of the scene loaded on `device` with new ones held in device memory: the
+ * triangles (of any count: objects spawned or removed, a tessellation level changed), the materials (an object recoloured) and the
+ * lights (a light moved, added or removed) -- geometry, colours and lights generated or animated on the GPU, without a host round trip.
+ *
+ * Result: afterwards the device holds exactly the scene ct_gpu_upload_scene with CT_FLAG_BUILD_BVH would load from the new parts
+ * plus the loaded ones `what` leaves out, with the scene's current camera, frame size, depth, flags, background and viewport, and the
+ * options read at upload as they were at upload: every array ct_gpu_debug_scene_array exports is equal byte for byte, "summary",
+ * "lights", "shadow_lights" and "path_state" included.  New triangles get BuildBVH's tree (InitializeBVHState + BuildBVH,
+ * bvh.cpp:16-120), built on the device; new materials alone or new lights alone leave the tree as it is.  Frames and queries that
+ * follow equal the reference's on the edited scene.
+ *
+ * What it keeps, as ct_gpu_update_triangles does: the camera and frame settings; the stream set with ct_gpu_set_stream; a shared-frame
+ * attach, partition and frame count (ct_gpu_share_*); the framebuffer, which holds the previous frame's pixels until the next render,
+ * and the rows ct_gpu_readback copies; ct_gpu_get_counters, ct_gpu_kernel_launches, ct_gpu_overflow_stats and ct_gpu_reuse_stats.
+ * Frame size, depth and flags do not change: re-upload for those.
+ *
+ * Order: the inputs are read in `stream`'s order (NULL = the render stream, see ct_gpu_set_stream), so work that wrote them on that
+ * stream needs no synchronisation by the caller.  The new state is built into scratch first; then the call waits for all work on the
+ * device -- frames and queries in flight finish on the old scene -- and overwrites the live state, reusing each allocation where the
+ * new records fit.  The call is synchronous: when it returns, the inputs may be overwritten or freed.  Every participant of a shared
+ * frame must apply the same update before the next shared frame; the library does not check this.
+ *
+ * Returns CT_OK; CT_ERR_INVALID for a NULL u, a wrong struct_size, what == 0 or unknown bits; with CT_UPDATE_TRIANGLES or
+ * CT_UPDATE_MATERIALS n_triangles == 0; with CT_UPDATE_TRIANGLES NULL triangles or a triangle_stride below 72 or not a multiple of 8;
+ * with CT_UPDATE_MATERIALS NULL materials; a count other than the loaded scene's without both CT_UPDATE_TRIANGLES and
+ * CT_UPDATE_MATERIALS (materials are per triangle); with CT_UPDATE_LIGHTS n_lights > 0 and NULL lights; an input that is not device
+ * memory of `device` (host memory, pageable or pinned, is refused) or is misaligned (triangles and lights 8 bytes, materials 4);
+ * CT_ERR_LIMIT for n_triangles >= 2^31; CT_ERR_NO_SCENE -- all checked before anything is enqueued or changed.  A new tree deeper
+ * than the device traversal stack (96) returns CT_ERR_LIMIT and a failed allocation CT_ERR_OOM; in both cases the previous scene
+ * stays loaded and renders as before. */
+enum { CT_UPDATE_TRIANGLES = 1u, CT_UPDATE_MATERIALS = 2u, CT_UPDATE_LIGHTS = 4u };
+
+typedef struct ct_scene_update {
+    uint32_t struct_size;            /* = sizeof(ct_scene_update) */
+    uint32_t what;                   /* CT_UPDATE_* mask, != 0 */
+    uint32_t n_triangles;            /* CT_UPDATE_TRIANGLES and / or CT_UPDATE_MATERIALS: the new count */
+    uint32_t triangle_stride;        /* CT_UPDATE_TRIANGLES: as ct_scene_desc, >= 72, a multiple of 8 */
+    uint32_t n_lights;               /* CT_UPDATE_LIGHTS: the new count, 0 allowed (no lights) */
+    uint32_t _pad;
+    const void *triangles;           /* device memory: 9 doubles p1,p2,p3 at the start of each record, 8-byte aligned */
+    const ct_material *materials;    /* device memory: n_triangles records, by triangle id (GetSceneTriangles order), 4-byte aligned */
+    const ct_light *lights;          /* device memory: n_lights records, file order, 8-byte aligned (NULL only when n_lights == 0) */
+    void *stream;                    /* cudaStream_t the inputs are read in the order of; NULL = the render stream */
+} ct_scene_update;
+
+int ct_gpu_update_scene(int device, const ct_scene_update *u);
 
 /* Known-answer-test entry: ClosestIntersection (raythread.cpp:197-227) for n arbitrary rays through the
  * uploaded scene.  origins/directions: n x 3 doubles; t0: initial ray_t.t per ray (1e30f primary/shadow,
