@@ -18,13 +18,12 @@ struct BuildReport {
     uint32_t boxes_bad;                  // some box is unordered or not finite
     uint32_t bad_pos;                    // a tri_indexes entry out of range (kNoPos: none)
     uint32_t pos0;                       // leaf position of triangle 0
-    uint32_t any_reflective;
     uint32_t not_nested;                 // some child's box is not inside its parent's box
     uint32_t duplicate;                  // a tri_indexes value occurs twice (with every value in range: not a permutation)
 };
 
 // TraceRay recurses unless reflection <= 0 (raythread.cpp:369): a NaN reflection reflects too.  The one test of whether a material
-// makes the scene reflective, for k_build_tris and k_any_reflective.
+// makes the scene reflective (k_any_reflective).
 __device__ __forceinline__ bool reflects(const ct_material &m) { return !(m.reflection <= 0.0f); }
 
 __global__ void __launch_bounds__(256) k_build_pairs(const ct_bvh_node *__restrict__ nodes, const uint32_t *__restrict__ pid_of, uint32_t n_nodes,
@@ -76,9 +75,7 @@ __global__ void __launch_bounds__(256) k_build_pairs(const ct_bvh_node *__restri
 }
 
 __global__ void __launch_bounds__(256) k_build_tris(const unsigned char *__restrict__ raw, uint32_t stride, const uint32_t *__restrict__ tri_indexes,
-                                                    const ct_material *__restrict__ materials, uint32_t n_tri,
-                                                    DevTri *__restrict__ tris, DevTri32 *__restrict__ tris32, uint32_t *__restrict__ seen, BuildReport *rep) {
-    bool refl = false;
+                                                    uint32_t n_tri, DevTri *__restrict__ tris, DevTri32 *__restrict__ tris32, uint32_t *__restrict__ seen, BuildReport *rep) {
     auto dmax = [](double a, double b) { return (a < b) ? b : a; };      // std::max: a NaN component is skipped
     for (uint32_t pos = blockIdx.x * blockDim.x + threadIdx.x; pos < n_tri; pos += gridDim.x * blockDim.x) {
         const uint32_t k = tri_indexes[pos];
@@ -103,12 +100,10 @@ __global__ void __launch_bounds__(256) k_build_tris(const unsigned char *__restr
         t32.k2 = __double2float_ru(k2); t32.k3 = __double2float_ru(k3);
         tris[pos] = t;
         tris32[pos] = t32;
-        if (reflects(materials[k])) refl = true;
     }
-    if (__any_sync(0xffffffffu, refl) && (threadIdx.x & 31u) == 0) atomicOr(&rep->any_reflective, 1u);
 }
 
-// Whether any of n materials reflects (ct_gpu_update_scene with new materials and no new triangles): *out |= 1.
+// Whether any of n materials reflects (install_scene, whenever the materials are new): *out |= 1.
 __global__ void __launch_bounds__(256) k_any_reflective(const ct_material *__restrict__ materials, uint32_t n, uint32_t *out) {
     bool refl = false;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)

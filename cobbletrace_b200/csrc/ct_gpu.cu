@@ -75,6 +75,17 @@ enum PathArray {
     PA_HITB_T, PA_HITB_POS, PA_STACK_REFL, PA_RAYS, PA_PATH_SLOT, PA_PARENT_Q, PA_FAR, kPathArrays
 };
 
+// The per-depth path state the stages of a tile or of a shade query batch work on: [depth][cap] arrays (rays: [depth][cap * 6], occ:
+// [depth][cap * occ_words]), parking buffers [2 * depth + kind][ovf_cap].  A frame's are DeviceState::path (path_commit), a query's
+// are carved per call (shade_impl).  Render_impl hands each launch a Params view of its depth, so that the shadow / shade chain of
+// one depth can run on its own stream next to the bounce chain of the next.
+struct PathArrays {
+    float *hitb_t_all; uint32_t *hitb_pos_all;
+    double *rays_all; uint32_t *path_slot_all;
+    uint32_t *occ_all, *parent_q_all, *far_all;     // parent_q: parent path of a reflection path (k_emit); far: k_bounce's far lists
+    OvfRay *ovf_all; uint32_t *ovf_huge_all;
+};
+
 struct DeviceState {
     bool loaded = false;
     Params p{};
@@ -96,16 +107,9 @@ struct DeviceState {
     // property reflection rays are never parked and parked primary rays go to k_primary_long (first_line_budget, render_impl)
     bool leaf_dfs_order = true;
     int depth = 0;                   // the tree's depth (the reference's DFS stack entries)
-    // per-depth path state (render_impl hands each launch a Params view of its depth, so that the shadow / shade
-    // chain of one depth can run on its own stream next to the bounce chain of the next)
-    float *hitb_t_all = nullptr; uint32_t *hitb_pos_all = nullptr;      // [depth][cap]
-    double *rays_all = nullptr; uint32_t *path_slot_all = nullptr;      // [depth][cap * 6], [depth][cap]
-    uint32_t *occ_all = nullptr;                                        // [depth][cap * occ_words]
-    uint32_t *parent_q_all = nullptr;                                   // [depth][cap]: parent path of a reflection path (k_emit)
-    uint32_t *far_all = nullptr;                                        // [depth][cap]: k_bounce's far lists
+    PathArrays path{};               // the frames' per-depth path state
     cudaEvent_t ev_lit[16] = {};                                        // shadow verdicts of depth d complete (k_shade of deeper levels may read them)
     unsigned long long rays_shadow_reused = 0;
-    OvfRay *ovf_all = nullptr; uint32_t *ovf_huge_all = nullptr;        // [2 * depth + kind][ovf_cap]
     int levels = 1;
     cudaStream_t aux[4] = {};
     cudaEvent_t ev_hit[16] = {}, ev_done[16] = {};
@@ -125,13 +129,13 @@ struct DeviceState {
     bool copy_pending = false;
     void *hot_base = nullptr; size_t hot_bytes = 0;      // pairs32 + tris32 (one allocation): the L2 access-policy window
     size_t l2_window = 0, l2_set_aside = 0;              // what apply_l2_policy obtained (0: none)
-    // what the tree's allocations hold (ct_gpu_update_triangles reuses them when the new tree fits): bytes of the hot allocation,
-    // pairs64 records, pair_parent entries (its allocation stays when a new tree cannot park: p.pair_parent is then NULL)
+    // what the tree's allocations hold (install_scene reuses them when the new tree fits; 0 after free_device): bytes of the hot
+    // allocation, pairs64 records, pair_parent entries (its allocation stays when a new tree cannot park: p.pair_parent is then NULL)
     size_t hot_cap = 0;
     uint32_t pairs_cap = 0, pair_parent_cap = 0;
     uint32_t *pair_parent_mem = nullptr;
-    // records the per-triangle arrays (tris, tri_parent, materials) and the two light arrays have room for (ct_gpu_update_scene
-    // reuses them when the new ones fit)
+    // records the per-triangle arrays (tris, tri_parent, materials) and the two light arrays have room for (install_scene reuses
+    // them when the new ones fit)
     uint32_t tri_cap = 0, light_cap = 0;
     void *path_mem[kPathArrays] = {};    // the path state: allocation and its bytes, by PathArray (NULL / 0: not allocated)
     size_t path_cap[kPathArrays] = {};
@@ -236,6 +240,37 @@ void dev_release(DeviceState &s, void *p) {
 
 #define TRY(expr) do { int rc_ = (expr); if (rc_ != CT_OK) return rc_; } while (0)
 
+// CT_GPU_TIMING: host-clock laps of one call on stderr, "ct_gpu_<entry>: <what> <ms> ms" (tools/exp_device_bvh.py and
+// tools/exp_update_triangles.py parse the lines).
+struct Laps {
+    const char *who;
+    const bool on = getenv("CT_GPU_TIMING") != nullptr;
+    static double now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
+    const double begin = now();
+    double mark = begin;
+    void operator()(const char *what) {
+        if (!on) return;
+        const double t = now();
+        fprintf(stderr, "%s: %-28s %7.2f ms\n", who, what, t - mark);
+        mark = t;
+    }
+};
+
+// One scratch allocation handed out by carve(a): a first pass with a.base NULL sizes it, the second carves the allocation.  async: in
+// st's order (cudaMallocAsync), else cudaMalloc.
+template <class Carve> cudaError_t carve_alloc(BbArena &a, bool async, cudaStream_t st, Carve &&carve) {
+    a = BbArena{};
+    carve(a);
+    const cudaError_t e = async ? cudaMallocAsync(&a.base, a.used, st) : cudaMalloc(&a.base, a.used);
+    if (e != cudaSuccess) { a.base = nullptr; return e; }
+    a.used = 0;
+    carve(a);
+    return cudaSuccess;
+}
+
+// Bytes of n triangles at `stride`: the last triangle may end at its third vertex.
+size_t tri_bytes(uint32_t n, uint32_t stride) { return (size_t)(n - 1) * stride + 72; }
+
 
 // depth of the reference's DFS (stack entries needed) -- iterative to survive degenerate trees.  Also marks the nodes the
 // DFS reaches (array slots nobody points at may hold anything) and rejects leaves whose triangle ranges overlap.  The walk visits
@@ -276,10 +311,10 @@ int bvh_depth(const ct_bvh_node *nodes, uint32_t n_nodes, uint32_t n_tri, bool *
     return best;
 }
 
-// Device buffers and a stream that live for one ct_gpu_upload_scene or ct_gpu_update_triangles call: the staged copies of the
-// caller's arrays, the tree built on the device (arena), the wide tree's scratch.  Freed when the call returns, whatever it returns.
-// async: the buffers come from the stream-ordered allocator and are freed in st's order (cudaFree would wait for the whole device;
-// the update's arena is allocated on the caller's stream, which st has waited for).
+// Device buffers and a stream that live for one ct_gpu_upload_scene, ct_gpu_update_scene or ct_gpu_build_bvh call: the staged copies
+// of the caller's arrays, the tree built on the device (arena), the wide tree's scratch.  Freed when the call returns, whatever it
+// returns.  async: the buffers come from the stream-ordered allocator and are freed in st's order (cudaFree would wait for the whole
+// device; the update stages the caller's arrays in the caller's stream, `on`, which st waits for).
 struct Staging {
     std::vector<void *> ptrs;
     BbArena arena;
@@ -295,17 +330,21 @@ struct Staging {
         if (ready) cudaEventDestroy(ready);
         if (!async) { cudaFree(arena.base); for (void *q : ptrs) cudaFree(q); }
     }
-    template <typename T> cudaError_t alloc(T **out, size_t count) {
+    template <typename T> cudaError_t alloc(T **out, size_t count, cudaStream_t on = nullptr) {
         void *q = nullptr;
         const size_t bytes = std::max<size_t>(count, 1) * sizeof(T);
-        const cudaError_t e = async ? cudaMallocAsync(&q, bytes, st) : cudaMalloc(&q, bytes);
+        const cudaError_t e = async ? cudaMallocAsync(&q, bytes, on ? on : st) : cudaMalloc(&q, bytes);
         if (e == cudaSuccess) ptrs.push_back(q);
         *out = static_cast<T *>(q);
         return e;
     }
+    // The device build's buffers for n triangles at `stride` (bb_carve) as the arena.
+    cudaError_t build_arena(uint32_t n, uint32_t stride, BbBuffers &bf, cudaStream_t on = nullptr) {
+        return carve_alloc(arena, async, on ? on : st, [&](BbArena &a) { bb_carve(a, n, tri_bytes(n, stride), bf); });
+    }
 };
 
-// ---- the scene built from a tree: one builder for ct_gpu_upload_scene and ct_gpu_update_triangles ------------------------------
+// ---- the scene built from a tree: one builder for ct_gpu_upload_scene and ct_gpu_update_scene ----------------------------------
 // A binary tree in the reference's layout on the device and what the scene arrays are made from with it.
 struct DeviceTree {
     const ct_bvh_node *nodes = nullptr;
@@ -315,6 +354,7 @@ struct DeviceTree {
     uint32_t stride = 72, n_nodes = 0, n_pairs = 0;
     ct_bvh_node root{};
     int depth = 0;
+    bool leaf_dfs_order = false;             // DeviceState::leaf_dfs_order: bvh_depth's verdict on a caller's tree, true for BuildBVH's
     DevWide *wide = nullptr;                 // the early-exit walks' wide tree, in scratch (collapse_wide)
     uint32_t n_wide = 0;
 };
@@ -336,6 +376,7 @@ int build_device_tree(Staging &stg, const BbBuffers &bf, uint32_t stride, uint32
     k_pid_leaves<<<blocks, kBbThreads, 0, stg.st>>>(bf.out, t.n_nodes, pid);
     CU(cudaGetLastError());
     t.nodes = bf.out; t.pid = pid; t.tri_index = bf.tri_index; t.tris = bf.raw; t.stride = stride;
+    t.leaf_dfs_order = true;                                                // BuildBVH's leaves come in DFS order (bvh.cpp:70-97)
     return CT_OK;
 }
 
@@ -426,17 +467,18 @@ int path_commit(DeviceState &s, PathPlan &pl, cudaStream_t st) {
     CU(cudaMemsetAsync(s.path_mem[PA_OCC], 0, pl.bytes[PA_OCC], st));
     CU(cudaStreamSynchronize(st));
     Params &p = s.p;
+    PathArrays &a = s.path;
     void *const *m = s.path_mem;
     p.hit0_t = static_cast<float *>(m[PA_HIT0_T]); p.hit0_pos = static_cast<uint32_t *>(m[PA_HIT0_POS]);
     p.stack_color = static_cast<uint32_t *>(m[PA_STACK_COLOR]); p.term_level = static_cast<uint8_t *>(m[PA_TERM_LEVEL]);
     p.stack_refl = static_cast<float *>(m[PA_STACK_REFL]);
-    s.occ_all = static_cast<uint32_t *>(m[PA_OCC]);
-    s.ovf_all = static_cast<OvfRay *>(m[PA_OVF]); s.ovf_huge_all = static_cast<uint32_t *>(m[PA_OVF_HUGE]);
-    s.hitb_t_all = static_cast<float *>(m[PA_HITB_T]); s.hitb_pos_all = static_cast<uint32_t *>(m[PA_HITB_POS]);
-    s.rays_all = static_cast<double *>(m[PA_RAYS]); s.path_slot_all = static_cast<uint32_t *>(m[PA_PATH_SLOT]);
-    s.parent_q_all = static_cast<uint32_t *>(m[PA_PARENT_Q]); s.far_all = static_cast<uint32_t *>(m[PA_FAR]);
-    p.occ = s.occ_all; p.occ_words = pl.occ_words;
-    p.ovf = s.ovf_all; p.ovf_huge = s.ovf_huge_all; p.ovf_cap = pl.ovf_cap;
+    a.occ_all = static_cast<uint32_t *>(m[PA_OCC]);
+    a.ovf_all = static_cast<OvfRay *>(m[PA_OVF]); a.ovf_huge_all = static_cast<uint32_t *>(m[PA_OVF_HUGE]);
+    a.hitb_t_all = static_cast<float *>(m[PA_HITB_T]); a.hitb_pos_all = static_cast<uint32_t *>(m[PA_HITB_POS]);
+    a.rays_all = static_cast<double *>(m[PA_RAYS]); a.path_slot_all = static_cast<uint32_t *>(m[PA_PATH_SLOT]);
+    a.parent_q_all = static_cast<uint32_t *>(m[PA_PARENT_Q]); a.far_all = static_cast<uint32_t *>(m[PA_FAR]);
+    p.occ = a.occ_all; p.occ_words = pl.occ_words;
+    p.ovf = a.ovf_all; p.ovf_huge = a.ovf_huge_all; p.ovf_cap = pl.ovf_cap;
     s.levels = pl.levels;
     return CT_OK;
 }
@@ -456,10 +498,9 @@ int build_lights(Staging &stg, cudaStream_t st, const ct_light *in, uint32_t n, 
 struct SceneArrays { unsigned char *hot; DevPair64 *pairs64; uint32_t *pair_parent, *tri_parent; DevTri *tris; };
 
 // The scene arrays from tree t (k_build_pairs, k_build_tris, the wide tree copied into the hot allocation at hot_layout's offsets)
-// and what the build reports about them.  materials: the scene's, by original id, already on the device.  The scratch is taken
-// before anything is written; the rest is enqueued on st, which is synchronised.
-int build_scene_arrays(Staging &stg, cudaStream_t st, const DeviceTree &t, const ct_material *materials, uint32_t n_tri, const SceneArrays &out,
-                       int n_sm, BuildReport *rep) {
+// and what the build reports about them.  The scratch is taken before anything is written; the rest is enqueued on st, which is
+// synchronised.
+int build_scene_arrays(Staging &stg, cudaStream_t st, const DeviceTree &t, uint32_t n_tri, const SceneArrays &out, int n_sm, BuildReport *rep) {
     uint32_t *seen = nullptr; BuildReport *drep = nullptr;
     const size_t seen_words = ((size_t)n_tri + 31u) / 32u;
     CU(stg.alloc(&drep, 1));
@@ -476,7 +517,7 @@ int build_scene_arrays(Staging &stg, cudaStream_t st, const DeviceTree &t, const
     CU(cudaMemsetAsync(out.tri_parent, 0xff, (size_t)n_tri * 4, st));
     const int build_blocks = n_sm * 8;
     k_build_pairs<<<build_blocks, 256, 0, st>>>(t.nodes, t.pid, t.n_nodes, dp32, out.pairs64, out.pair_parent, out.tri_parent, n_tri, drep);
-    k_build_tris<<<build_blocks, 256, 0, st>>>(t.tris, t.stride, t.tri_index, materials, n_tri, out.tris, dt32, seen, drep);
+    k_build_tris<<<build_blocks, 256, 0, st>>>(t.tris, t.stride, t.tri_index, n_tri, out.tris, dt32, seen, drep);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(rep, drep, sizeof *rep, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -507,6 +548,7 @@ void set_tree(DeviceState &s, const DeviceTree &t, const SceneArrays &out, const
     p.pair_parent = out.pair_parent; p.tri_parent = out.tri_parent;
     s.hot_base = out.hot; s.hot_bytes = hl.bytes;
     s.depth = t.depth;
+    s.leaf_dfs_order = t.leaf_dfs_order;
 }
 
 int launch_grid(const DeviceState &s, int blocks_per_sm) { return s.n_sm * blocks_per_sm; }
@@ -586,25 +628,19 @@ int trace_impl(DeviceState &s, int kind, uint32_t n, const double *org, const do
     uint32_t ovf_cap = 0;
     if (park) ovf_cap = std::min<uint32_t>(n, primary && park_cap ? std::min(park_cap, s.p.ovf_cap) : s.p.ovf_cap);
     // the scratch: scheduler and totals records, one occlusion word and one hit record per ray, the parking buffer and huge list --
-    // carved from one allocation (first pass: sizes only)
-    char *base = nullptr;
-    size_t used = 0;
-    auto take = [&](size_t bytes) { char *q = base ? base + used : nullptr; used += (bytes + 255u) & ~(size_t)255u; return q; };
+    // carved from one allocation
+    BbArena a;
     DevSched *sched = nullptr; DevTotals *tot = nullptr; uint32_t *occ = nullptr, *hpos = nullptr, *huge = nullptr; float *ht = nullptr;
     OvfRay *ovf = nullptr;
-    auto carve = [&]() {
-        used = 0;
-        sched = (DevSched *)take(sizeof(DevSched)); tot = (DevTotals *)take(sizeof(DevTotals));
-        occ = (uint32_t *)take(4ull * n); ht = (float *)take(4ull * n); hpos = (uint32_t *)take(4ull * n);
-        if (ovf_cap) { ovf = (OvfRay *)take(sizeof(OvfRay) * (size_t)ovf_cap); huge = (uint32_t *)take(4ull * ovf_cap); }
-    };
-    carve();
-    cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&base), used, st);
+    const cudaError_t e = carve_alloc(a, true, st, [&](BbArena &m) {
+        sched = m.take<DevSched>(1); tot = m.take<DevTotals>(1);
+        occ = m.take<uint32_t>(n); ht = m.take<float>(n); hpos = m.take<uint32_t>(n);
+        if (ovf_cap) { ovf = m.take<OvfRay>(ovf_cap); huge = m.take<uint32_t>(ovf_cap); }
+    });
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "cudaMallocAsync(%zu bytes): %s", used, cudaGetErrorString(e));
+        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "cudaMallocAsync(%zu bytes): %s", a.used, cudaGetErrorString(e));
     }
-    carve();
     Params v = s.p;
     v.sched = sched; v.tot = tot; v.occ = occ; v.occ_words = 1;
     v.hit0_t = v.hitb_t = ht; v.hit0_pos = v.hitb_pos = hpos;
@@ -632,7 +668,7 @@ int trace_impl(DeviceState &s, int kind, uint32_t n, const double *org, const do
         return cudaGetLastError();
     };
     const cudaError_t r = enqueue();
-    const cudaError_t f = cudaFreeAsync(base, st);
+    const cudaError_t f = cudaFreeAsync(a.base, st);
     if (r != cudaSuccess) return fail(CT_ERR_CUDA, "ray query: %s", cudaGetErrorString(r));
     if (f != cudaSuccess) return fail(CT_ERR_CUDA, "cudaFreeAsync: %s", cudaGetErrorString(f));
     return CT_OK;
@@ -667,15 +703,6 @@ int debug_query(int device, int kind, uint32_t n, const double *origins, const d
 #undef CUX
     return CT_OK;
 }
-
-// The per-depth path state the stages of a tile or of a shade query batch work on: [depth][cap] arrays as DeviceState describes
-// them, parking buffers [2 * depth + kind][ovf_cap].  A frame's are allocated at upload, a query's per call (shade_impl).
-struct PathArrays {
-    float *hitb_t_all; uint32_t *hitb_pos_all;
-    double *rays_all; uint32_t *path_slot_all;
-    uint32_t *occ_all, *parent_q_all, *far_all;
-    OvfRay *ovf_all; uint32_t *ovf_huge_all;
-};
 
 // The stages of one tile (render_impl) or of one batch of a shade query (shade_impl, QUERY: the query forms of k_primary, k_shadow,
 // k_shade and k_resolve).  pk: what every launch starts from, pk.max_depth the depth the recursion goes to (0 without a reflective
@@ -812,35 +839,29 @@ int shade_impl(DeviceState &s, uint32_t n, int max_depth, const double *org, con
     const size_t cap = (batch + kChunkMax - 1u) / kChunkMax * kChunkMax;
     const uint32_t ovf_cap = s.can_overflow ? std::min<uint32_t>(batch, s.p.ovf_cap) : 0u;
     const size_t words = s.p.occ_words;
-    char *base = nullptr;
-    size_t used = 0;
-    auto take = [&](size_t bytes) { char *q = base ? base + used : nullptr; used += (bytes + 255u) & ~(size_t)255u; return q; };
+    BbArena arena;
     Params pk = s.p;
     PathArrays a{};
-    auto carve = [&]() {                                            // (first pass: sizes only)
-        used = 0;
-        pk.sched = (DevSched *)take(sizeof(DevSched)); pk.tot = (DevTotals *)take(sizeof(DevTotals));
-        pk.hit0_t = (float *)take(4 * cap); pk.hit0_pos = (uint32_t *)take(4 * cap);
-        pk.stack_color = (uint32_t *)take(4 * cap * levels);
-        pk.term_level = (uint8_t *)take(cap);
-        pk.own_chunks = (uint32_t *)take(4 * ((cap >> kChunkLocalShift) + 1));
-        a.occ_all = (uint32_t *)take(4 * cap * words * levels);
-        if (ovf_cap) { a.ovf_all = (OvfRay *)take(sizeof(OvfRay) * ovf_cap * 2 * levels); a.ovf_huge_all = (uint32_t *)take(4ull * ovf_cap * 2 * levels); }
+    const cudaError_t e = carve_alloc(arena, true, st, [&](BbArena &m) {
+        pk.sched = m.take<DevSched>(1); pk.tot = m.take<DevTotals>(1);
+        pk.hit0_t = m.take<float>(cap); pk.hit0_pos = m.take<uint32_t>(cap);
+        pk.stack_color = m.take<uint32_t>(cap * levels);
+        pk.term_level = m.take<uint8_t>(cap);
+        pk.own_chunks = m.take<uint32_t>((cap >> kChunkLocalShift) + 1);
+        a.occ_all = m.take<uint32_t>(cap * words * levels);
+        if (ovf_cap) { a.ovf_all = m.take<OvfRay>((size_t)ovf_cap * 2 * levels); a.ovf_huge_all = m.take<uint32_t>((size_t)ovf_cap * 2 * levels); }
         if (levels > 1) {
-            a.hitb_t_all = (float *)take(4 * cap * levels); a.hitb_pos_all = (uint32_t *)take(4 * cap * levels);
-            pk.stack_refl = (float *)take(4 * cap * levels);
-            a.rays_all = (double *)take(48 * cap * (levels + 1)); a.path_slot_all = (uint32_t *)take(4 * cap * (levels + 1));
-            a.parent_q_all = (uint32_t *)take(4 * cap * (levels + 1));
-            a.far_all = (uint32_t *)take(4 * cap * levels);
+            a.hitb_t_all = m.take<float>(cap * levels); a.hitb_pos_all = m.take<uint32_t>(cap * levels);
+            pk.stack_refl = m.take<float>(cap * levels);
+            a.rays_all = m.take<double>(6 * cap * (levels + 1)); a.path_slot_all = m.take<uint32_t>(cap * (levels + 1));
+            a.parent_q_all = m.take<uint32_t>(cap * (levels + 1));
+            a.far_all = m.take<uint32_t>(cap * levels);
         }
-    };
-    carve();
-    cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&base), used, st);
+    });
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "cudaMallocAsync(%zu bytes): %s", used, cudaGetErrorString(e));
+        return fail(e == cudaErrorMemoryAllocation ? CT_ERR_OOM : CT_ERR_CUDA, "cudaMallocAsync(%zu bytes): %s", arena.used, cudaGetErrorString(e));
     }
-    carve();
     if (levels == 1) pk.stack_refl = nullptr;
     pk.max_depth = depth_max;
     pk.cap = (uint32_t)cap;
@@ -865,7 +886,7 @@ int shade_impl(DeviceState &s, uint32_t n, int max_depth, const double *org, con
         rc = enqueue_stages<true>(s, v, a, false, true, st, [](const char *, int) { return (int)CT_OK; }, launches);
     }
     if (r == cudaSuccess) r = cudaGetLastError();
-    const cudaError_t f = cudaFreeAsync(base, st);
+    const cudaError_t f = cudaFreeAsync(arena.base, st);
     if (rc != CT_OK) return rc;
     if (r != cudaSuccess) return fail(CT_ERR_CUDA, "shade query: %s", cudaGetErrorString(r));
     if (f != cudaSuccess) return fail(CT_ERR_CUDA, "cudaFreeAsync: %s", cudaGetErrorString(f));
@@ -879,6 +900,143 @@ int check_device_array(int device, const void *p, size_t align, const char *name
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return fail(CT_ERR_INVALID, "%s: not a CUDA pointer", name); }
     if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != device)
         return fail(CT_ERR_INVALID, "%s is not device memory of device %d", name, device);
+    return CT_OK;
+}
+
+// Puts a scene into s, loaded or freshly reset by free_device (every capacity 0: every allocation is new): the tree (NULL: keep the
+// loaded one), the materials of n triangles (NULL: keep them; n is then the loaded count) and n_lights lights (NULL: keep them; n_lights
+// is then the loaded count).  The new parts are in stg's scratch on the device, stg.st behind their copies.  The camera, the frame
+// settings and the upload-time options in s stay.  Everything new is computed into scratch and every allocation it needs is taken
+// first -- a refused or failed build changes nothing; then, after the device has finished the work in flight, it is written over the
+// live state, reusing the allocations where the new records fit, and the L2 window follows the hot records.
+int install_scene(DeviceState &s, int device, Staging &stg, const DeviceTree *tree, const ct_material *materials, uint32_t n,
+                  const ct_light *lights, uint32_t n_lights, Laps &laps) {
+    Params &p = s.p;
+    const bool new_tri = tree != nullptr, new_mat = materials != nullptr, new_lit = lights != nullptr;
+    // What the frames derive from the materials and lights: whether any material reflects (the path state's depth), the lights and
+    // the compacted shadow lights (the path state's occlusion words, the any-hit walk's leaf list)
+    bool any_reflective = s.any_reflective;
+    if (new_mat) {
+        uint32_t *flag = nullptr, h = 0;
+        CU(stg.alloc(&flag, 1));
+        CU(cudaMemsetAsync(flag, 0, sizeof *flag, stg.st));
+        k_any_reflective<<<std::max(1, std::min(s.n_sm * 8, (int)((n + 255u) / 256u))), 256, 0, stg.st>>>(materials, n, flag);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(&h, flag, sizeof h, cudaMemcpyDeviceToHost, stg.st));
+        CU(cudaStreamSynchronize(stg.st));
+        any_reflective = h != 0;
+    }
+    DevLight *lit_new = nullptr; DevShadowLight *slit_new = nullptr;
+    uint32_t n_slights = p.n_slights;
+    if (new_lit) {
+        CU(stg.alloc(&lit_new, n_lights)); CU(stg.alloc(&slit_new, n_lights));
+        TRY(build_lights(stg, stg.st, lights, n_lights, lit_new, slit_new, &n_slights));
+        laps("materials and lights (device)");
+    }
+
+    // The live allocations the new state needs, taken before anything is written: the tree's (hot allocation, pairs64, pair_parent),
+    // the per-triangle arrays when the new count is larger, the light arrays when they hold fewer records (at least one, also for no
+    // lights), the path state when its depth, occlusion words or parking grow.
+    const bool can_overflow = new_tri ? walks_can_park(p, tree->n_nodes, n) : s.can_overflow;
+    const uint32_t light_recs = std::max<uint32_t>(n_lights, 1);
+    const bool grow_tri = n > s.tri_cap, grow_lit = light_recs > s.light_cap;
+    HotLayout hl{};
+    uint32_t pairs = 0;
+    SceneArrays out{};
+    bool fresh_hot = false, fresh_pairs = false, fresh_parent = false;
+    ct_material *mat_fresh = nullptr; DevLight *dl_fresh = nullptr; DevShadowLight *dsl_fresh = nullptr;
+    PathPlan pl;
+    auto take = [&]() -> int {
+        if (new_tri) {
+            hl = hot_layout(tree->n_wide, tree->n_pairs, n);
+            pairs = std::max<uint32_t>(tree->n_pairs, 1);
+            out.hot = hl.bytes <= s.hot_cap ? static_cast<unsigned char *>(s.hot_base) : nullptr;
+            out.pairs64 = pairs <= s.pairs_cap ? const_cast<DevPair64 *>(p.pairs64) : nullptr;
+            out.pair_parent = !can_overflow ? nullptr : pairs <= s.pair_parent_cap ? s.pair_parent_mem : nullptr;
+            out.tri_parent = grow_tri ? nullptr : const_cast<uint32_t *>(p.tri_parent);
+            out.tris = grow_tri ? nullptr : const_cast<DevTri *>(p.tris);
+            fresh_hot = !out.hot; fresh_pairs = !out.pairs64; fresh_parent = can_overflow && !out.pair_parent;
+            if (fresh_hot) TRY(dev_alloc(s, &out.hot, hl.bytes));
+            if (fresh_pairs) TRY(dev_alloc(s, &out.pairs64, pairs));
+            if (fresh_parent) TRY(dev_alloc(s, &out.pair_parent, pairs));
+            if (grow_tri) { TRY(dev_alloc(s, &out.tris, n)); TRY(dev_alloc(s, &out.tri_parent, n)); }
+        }
+        if (grow_tri) TRY(dev_alloc(s, &mat_fresh, n));                    // (a larger count comes with new materials)
+        if (grow_lit) { TRY(dev_alloc(s, &dl_fresh, light_recs)); TRY(dev_alloc(s, &dsl_fresh, light_recs)); }
+        TRY(path_take(s, any_reflective ? p.max_depth + 1 : 1, occ_words_for(n_lights), can_overflow ? parking_cap(p) : 0u, pl));
+        return CT_OK;
+    };
+    auto give_back = [&]() {                                             // the new allocations of a call that fails
+        if (fresh_hot) dev_release(s, out.hot);
+        if (fresh_pairs) dev_release(s, out.pairs64);
+        if (fresh_parent) dev_release(s, out.pair_parent);
+        if (grow_tri && new_tri) { dev_release(s, out.tris); dev_release(s, out.tri_parent); }
+        dev_release(s, mat_fresh); dev_release(s, dl_fresh); dev_release(s, dsl_fresh);
+        path_give_back(s, pl);
+    };
+    int rc = take();
+    if (rc != CT_OK) { give_back(); return rc; }
+    laps("allocation");
+
+    // frames and queries in flight finish on the previous scene (the rule of a re-upload, whose cudaFree waits for the device)
+    {
+        const cudaError_t e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) { give_back(); CU(e); }
+    }
+    // Past this point only a CUDA failure, or a caller's leaf permutation that the build finds out of range or repeated (an upload's:
+    // a tree built on the device has neither), returns early.
+    BuildReport rep{};
+    if (new_tri) {
+        rc = build_scene_arrays(stg, stg.st, *tree, n, out, s.n_sm, &rep);
+        if (rc == CT_OK && rep.bad_pos != kNoPos) {
+            uint32_t bad = 0;
+            cudaMemcpy(&bad, tree->tri_index + rep.bad_pos, sizeof bad, cudaMemcpyDeviceToHost);
+            rc = fail(CT_ERR_INVALID, "tri_indexes[%u] = %u out of range", rep.bad_pos, bad);
+        } else if (rc == CT_OK && (rep.duplicate || rep.pos0 == kNoPos)) {
+            rc = fail(CT_ERR_INVALID, "tri_indexes is not a permutation of 0..n_triangles-1 (an index occurs twice)");
+        }
+        if (rc != CT_OK) { give_back(); return rc; }
+        laps("scene arrays built on the device");
+    }
+    ct_material *const mats = grow_tri ? mat_fresh : const_cast<ct_material *>(p.materials);
+    DevLight *const dl = grow_lit ? dl_fresh : const_cast<DevLight *>(p.lights);
+    DevShadowLight *const dsl = grow_lit ? dsl_fresh : const_cast<DevShadowLight *>(p.slights);
+    {
+        cudaError_t e = cudaSuccess;
+        if (new_mat) e = cudaMemcpyAsync(mats, materials, (size_t)n * sizeof(ct_material), cudaMemcpyDeviceToDevice, stg.st);
+        if (e == cudaSuccess && new_lit && n_lights) e = cudaMemcpyAsync(dl, lit_new, (size_t)n_lights * sizeof(DevLight), cudaMemcpyDeviceToDevice, stg.st);
+        if (e == cudaSuccess && new_lit && n_slights) e = cudaMemcpyAsync(dsl, slit_new, (size_t)n_slights * sizeof(DevShadowLight), cudaMemcpyDeviceToDevice, stg.st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(stg.st);
+        if (e != cudaSuccess) { give_back(); CU(e); }
+    }
+
+    // The new state in place of the old: the replaced allocations go back, the frames' parameters follow.
+    void *const old_hot = s.hot_base;
+    const size_t old_hot_bytes = s.hot_bytes;
+    if (new_tri) {
+        if (fresh_hot) { dev_release(s, s.hot_base); s.hot_cap = hl.bytes; }
+        if (fresh_pairs) { dev_release(s, const_cast<DevPair64 *>(p.pairs64)); s.pairs_cap = pairs; }
+        if (fresh_parent) { dev_release(s, s.pair_parent_mem); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
+        if (grow_tri) { dev_release(s, const_cast<DevTri *>(p.tris)); dev_release(s, const_cast<uint32_t *>(p.tri_parent)); }
+    }
+    if (grow_tri) { dev_release(s, const_cast<ct_material *>(p.materials)); s.tri_cap = n; }
+    if (grow_lit) { dev_release(s, const_cast<DevLight *>(p.lights)); dev_release(s, const_cast<DevShadowLight *>(p.slights)); s.light_cap = light_recs; }
+    p.materials = mats; p.lights = dl; p.slights = dsl;
+    p.n_tri = n; p.n_lights = n_lights; p.n_slights = n_slights;
+    p.any_leaves = any_leaves_for(s.any_leaves_option, n_slights);
+    s.any_reflective = any_reflective;
+    s.can_overflow = can_overflow;
+    TRY(path_commit(s, pl, stg.st));
+    if (new_tri) set_tree(s, *tree, out, rep);
+    laps("previous allocations freed");
+    if (s.hot_base != old_hot || s.hot_bytes != old_hot_bytes) {
+        // the window over the hot records, sized for the new ones, on every stream the frames run on
+        release_l2(s);
+        TRY(apply_l2_policy(s, device, s.own_stream));
+        if (s.stream != s.own_stream) TRY(apply_l2_policy(s, device, s.stream));
+        for (cudaStream_t a : s.aux) TRY(apply_l2_policy(s, device, a));
+        laps("L2 window applied");
+    }
     return CT_OK;
 }
 }  // namespace
@@ -913,61 +1071,60 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     if (d->max_depth < 0 || d->max_depth > 15) return fail(CT_ERR_LIMIT, "max_depth %d outside 0..15", d->max_depth);
     if ((d->flags & CT_FLAG_SUPERSAMPLING) && (d->flags & CT_FLAG_KEEP_HITS))
         return fail(CT_ERR_INVALID, "CT_FLAG_SUPERSAMPLING cannot be combined with CT_FLAG_KEEP_HITS (a pixel has 16 primary rays)");
-    bool ok = true, dfs_order = true;          // a tree BuildBVH makes has its leaves in DFS order (bvh.cpp:70-97)
+    DeviceTree t;
     std::vector<uint8_t> reachable;
-    int depth = 0;
     if (!build) {
-        depth = bvh_depth(d->nodes, d->n_nodes, d->n_triangles, &ok, &dfs_order, reachable);
+        bool ok = true;
+        t.depth = bvh_depth(d->nodes, d->n_nodes, d->n_triangles, &ok, &t.leaf_dfs_order, reachable);
         if (!ok) return fail(CT_ERR_INVALID, "BVH is malformed (child or triangle range out of bounds, overlapping leaves, a cycle or a shared child)");
-        if (depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", depth, kStackMax);
+        if (t.depth > kStackMax) return fail(CT_ERR_LIMIT, "BVH depth %d exceeds the device traversal stack (%d)", t.depth, kStackMax);
     }
     TRY(check_device(device));
     DEVICE_GUARD(device);
     std::lock_guard<std::mutex> lock(g_mutex);
     DeviceState &s = g_dev[device];
-    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
-    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
-    const double t_begin = now_ms();
-    double t_mark = t_begin;
-    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_upload_scene: %-28s %7.1f ms\n", what, t - t_mark); t_mark = t; } };
+    Laps laps{"ct_gpu_upload_scene"};
     int n_sm = 0;
     CU(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
 
-    // The binary tree, the leaf permutation and the triangles on the device.  With CT_FLAG_BUILD_BVH the tree is built here, into
-    // buffers of the upload's own, BEFORE the previous scene is released: a refused tree leaves that scene loaded.
-    const size_t tri_bytes = (size_t)(d->n_triangles - 1) * d->triangle_stride + 72;      // the last triangle may end at its third vertex
+    // The binary tree, the leaf permutation, the triangles, the materials and the lights on the device, in buffers of the upload's own
+    // (with CT_FLAG_BUILD_BVH the tree is built here), BEFORE the previous scene is released: a refused tree leaves that scene loaded.
+    const size_t raw_bytes = tri_bytes(d->n_triangles, d->triangle_stride);
     Staging stg;
     CU(cudaStreamCreateWithFlags(&stg.st, cudaStreamNonBlocking));
-    DeviceTree t;
     if (build) {
         BbBuffers bf;
-        bb_carve(stg.arena, d->n_triangles, tri_bytes, bf);
-        CU(cudaMalloc(&stg.arena.base, stg.arena.used));
-        stg.arena.used = 0;
-        bb_carve(stg.arena, d->n_triangles, tri_bytes, bf);
-        CU(cudaMemcpyAsync(bf.raw, d->triangles, tri_bytes, cudaMemcpyHostToDevice, stg.st));
+        CU(stg.build_arena(d->n_triangles, d->triangle_stride, bf));
+        CU(cudaMemcpyAsync(bf.raw, d->triangles, raw_bytes, cudaMemcpyHostToDevice, stg.st));
         TRY(build_device_tree(stg, bf, d->triangle_stride, d->n_triangles, n_sm, t));
-        lap("BVH built on the device");
+        laps("BVH built on the device");
     } else {
         t.root = d->nodes[0];
-        t.n_nodes = d->n_nodes; t.depth = depth; t.stride = d->triangle_stride;
+        t.n_nodes = d->n_nodes; t.stride = d->triangle_stride;
         // nodes: reference layout -> per-interior-node child pairs, built on the device from the raw arrays (k_build_pairs); the host
         // only numbers the interior nodes it validated
         std::vector<uint32_t> pid_of(d->n_nodes, kNoPos);
         for (uint32_t i = 0; i < d->n_nodes; i++)
             if (reachable[i]) pid_of[i] = d->nodes[i].triangle_count == 0 ? t.n_pairs++ : kLeafMark;      // unreachable slots get no record and write nothing
         ct_bvh_node *rn = nullptr; uint32_t *rp = nullptr, *ri = nullptr; unsigned char *rt = nullptr;
-        CU(stg.alloc(&rn, d->n_nodes)); CU(stg.alloc(&rp, d->n_nodes)); CU(stg.alloc(&ri, d->n_triangles)); CU(stg.alloc(&rt, tri_bytes));
+        CU(stg.alloc(&rn, d->n_nodes)); CU(stg.alloc(&rp, d->n_nodes)); CU(stg.alloc(&ri, d->n_triangles)); CU(stg.alloc(&rt, raw_bytes));
         CU(cudaMemcpyAsync(rn, d->nodes, (size_t)d->n_nodes * sizeof(ct_bvh_node), cudaMemcpyHostToDevice, stg.st));
         CU(cudaMemcpyAsync(rp, pid_of.data(), (size_t)d->n_nodes * 4, cudaMemcpyHostToDevice, stg.st));
         CU(cudaMemcpyAsync(ri, d->tri_indexes, (size_t)d->n_triangles * 4, cudaMemcpyHostToDevice, stg.st));
-        CU(cudaMemcpyAsync(rt, d->triangles, tri_bytes, cudaMemcpyHostToDevice, stg.st));
+        CU(cudaMemcpyAsync(rt, d->triangles, raw_bytes, cudaMemcpyHostToDevice, stg.st));
         t.nodes = rn; t.pid = rp; t.tri_index = ri; t.tris = rt;
-        lap("interior-node numbering (host)");
+        laps("interior-node numbering (host)");
     }
-    // the early-exit walks' wide tree, into scratch first: its size decides the layout of the hot allocation below
+    // the early-exit walks' wide tree, into scratch first: its size decides the layout of the hot allocation
     TRY(collapse_wide(stg, t, n_sm));
-    lap("wide tree (device)");
+    laps("wide tree (device)");
+    ct_material *mat_in = nullptr;
+    ct_light *lit_in = nullptr;
+    CU(stg.alloc(&mat_in, d->n_triangles));
+    CU(stg.alloc(&lit_in, d->n_lights));
+    CU(cudaMemcpyAsync(mat_in, d->materials, (size_t)d->n_triangles * sizeof(ct_material), cudaMemcpyHostToDevice, stg.st));
+    if (d->n_lights) CU(cudaMemcpyAsync(lit_in, d->lights, (size_t)d->n_lights * sizeof(ct_light), cudaMemcpyHostToDevice, stg.st));
+    laps("materials and lights copied");
 
     free_device(s);
     s.n_sm = n_sm;
@@ -985,48 +1142,9 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     s.p.warp_budget = g_warp_budget_option > 0 ? (uint32_t)std::min<long long>(g_warp_budget_option, 1ll << 30) : kWarpBudget;
     s.p.primary_budget = g_primary_budget_option < 0 ? 0u : g_primary_budget_option > 0 ? (uint32_t)std::min<long long>(g_primary_budget_option, 1ll << 30) : kDefaultPrimaryBudget;
     s.flags = d->flags;
-    s.leaf_dfs_order = dfs_order;
-
     s.any_leaves_option = g_any_leaves;
 
     Params &p = s.p;
-    p.n_tri = d->n_triangles; p.n_lights = d->n_lights;
-    s.can_overflow = walks_can_park(p, t.n_nodes, p.n_tri);
-
-    SceneArrays out{};
-    ct_material *dm = nullptr;
-    const uint32_t pairs = std::max<uint32_t>(t.n_pairs, 1);
-    s.hot_cap = hot_layout(t.n_wide, t.n_pairs, d->n_triangles).bytes;
-    TRY(dev_alloc(s, &out.hot, s.hot_cap));
-    TRY(dev_alloc(s, &out.pairs64, pairs)); s.pairs_cap = pairs;
-    TRY(dev_alloc(s, &out.tris, d->n_triangles)); TRY(dev_alloc(s, &dm, d->n_triangles));
-    TRY(dev_alloc(s, &out.tri_parent, d->n_triangles));
-    s.tri_cap = d->n_triangles;
-    if (s.can_overflow) { TRY(dev_alloc(s, &out.pair_parent, pairs)); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
-    BuildReport rep{};
-    {
-        const cudaError_t e = cudaMemcpyAsync(dm, d->materials, (size_t)d->n_triangles * sizeof(ct_material), cudaMemcpyHostToDevice, s.stream);
-        if (e != cudaSuccess) { free_device(s); CU(e); }
-        const int rc = build_scene_arrays(stg, s.stream, t, dm, d->n_triangles, out, s.n_sm, &rep);
-        if (rc != CT_OK) { free_device(s); return rc; }
-    }
-    if (rep.bad_pos != kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes[%u] = %u out of range", rep.bad_pos, build ? 0u : d->tri_indexes[rep.bad_pos]); }
-    if (rep.duplicate || rep.pos0 == kNoPos) { free_device(s); return fail(CT_ERR_INVALID, "tri_indexes is not a permutation of 0..n_triangles-1 (an index occurs twice)"); }
-    s.any_reflective = rep.any_reflective != 0;
-    set_tree(s, t, out, rep);
-    p.materials = dm;
-    lap("scene arrays built on the device");
-    // the lights: the caller's records to the device, converted there by the kernel ct_gpu_update_scene runs on new lights
-    DevLight *dl = nullptr; DevShadowLight *dsl = nullptr; ct_light *lights_in = nullptr;
-    s.light_cap = std::max<uint32_t>(d->n_lights, 1);
-    TRY(dev_alloc(s, &dl, s.light_cap));
-    TRY(dev_alloc(s, &dsl, s.light_cap));
-    CU(stg.alloc(&lights_in, d->n_lights));
-    if (d->n_lights) CU(cudaMemcpyAsync(lights_in, d->lights, (size_t)d->n_lights * sizeof(ct_light), cudaMemcpyHostToDevice, stg.st));
-    TRY(build_lights(stg, stg.st, lights_in, d->n_lights, dl, dsl, &p.n_slights));
-    p.any_leaves = any_leaves_for(s.any_leaves_option, p.n_slights);
-    p.slights = dsl; p.lights = dl;
-
     memcpy(p.cam, d->camera_position, sizeof p.cam);
     memcpy(p.rot, d->camera_rotation, sizeof p.rot);
     p.vp_w = d->viewport[0]; p.vp_h = d->viewport[1]; p.vp_d = d->viewport[2];
@@ -1048,11 +1166,12 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
         p.cap = (uint32_t)((slots + kChunkMax - 1u) / kChunkMax * kChunkMax);
     }
 
+    // the scene itself: on the reset state every allocation is new
     {
-        PathPlan pl;
-        TRY(path_take(s, s.any_reflective ? d->max_depth + 1 : 1, occ_words_for(d->n_lights), s.can_overflow ? parking_cap(p) : 0u, pl));
-        TRY(path_commit(s, pl, s.stream));
+        const int rc = install_scene(s, device, stg, &t, mat_in, d->n_triangles, lit_in, d->n_lights, laps);
+        if (rc != CT_OK) { free_device(s); return rc; }
     }
+    // what the frames own
     TRY(dev_alloc(s, &p.fb, (size_t)d->width * d->height, true));       // calloc'd like cobbletrace.cpp:57
     p.subsample = (d->flags & CT_FLAG_SUBSAMPLING) ? 1 : 0;
     p.supersample = (d->flags & CT_FLAG_SUPERSAMPLING) ? 1 : 0;
@@ -1067,10 +1186,8 @@ int ct_gpu_upload_scene(int device, const ct_scene_desc *d) {
     }
     TRY(dev_alloc(s, &p.sched, 1, true));
     TRY(dev_alloc(s, &p.tot, 1, true));
-    lap("path state allocation");
-    TRY(apply_l2_policy(s, device, s.stream));
-    for (cudaStream_t a : s.aux) TRY(apply_l2_policy(s, device, a));
-    if (timing) fprintf(stderr, "ct_gpu_upload_scene: L2 window %zu bytes, set-aside %zu bytes; total %.1f ms\n", s.l2_window, s.l2_set_aside, now_ms() - t_begin);
+    laps("frame allocation");
+    if (laps.on) fprintf(stderr, "ct_gpu_upload_scene: L2 window %zu bytes, set-aside %zu bytes; total %.2f ms\n", s.l2_window, s.l2_set_aside, Laps::now() - laps.begin);
     s.loaded = true;
     return CT_OK;
 }
@@ -1090,44 +1207,32 @@ int ct_gpu_build_bvh(int device, uint32_t n_triangles, const void *triangles, ui
     int n_sm = 0;
     cudaError_t e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
     if (e != cudaSuccess) return cu_fail(e, "cudaDeviceGetAttribute");
-    // a stream and buffers of its own: a scene uploaded on this device is not touched
-    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
-    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
-    double t_mark = now_ms();
-    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "ct_gpu_build_bvh: %-28s %7.2f ms\n", what, t - t_mark); t_mark = t; } };
-    cudaStream_t st = nullptr;
-    if ((e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking)) != cudaSuccess) return cu_fail(e, "cudaStreamCreate");
-    BbArena arena;
-    struct Release { cudaStream_t s; BbArena &a; ~Release() { cudaStreamSynchronize(s); cudaStreamDestroy(s); cudaFree(a.base); } } release{st, arena};
-    const size_t tri_bytes = (size_t)(n_triangles - 1) * triangle_stride + 72;      // the last triangle may end at its third vertex
+    Laps laps{"ct_gpu_build_bvh"};
+    Staging stg;                      // a stream and buffers of its own: a scene uploaded on this device is not touched
+    if ((e = cudaStreamCreateWithFlags(&stg.st, cudaStreamNonBlocking)) != cudaSuccess) return cu_fail(e, "cudaStreamCreate");
     BbBuffers bf;
-    bb_carve(arena, n_triangles, tri_bytes, bf);
-    if ((e = cudaMalloc(&arena.base, arena.used)) != cudaSuccess) { arena.base = nullptr; return cu_fail(e, "cudaMalloc"); }
-    arena.used = 0;
-    bb_carve(arena, n_triangles, tri_bytes, bf);
-    lap("allocation");
-    if ((e = cudaMemcpyAsync(bf.raw, triangles, tri_bytes, cudaMemcpyHostToDevice, st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
-    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
-    lap("triangles to the device");
+    if ((e = stg.build_arena(n_triangles, triangle_stride, bf)) != cudaSuccess) return cu_fail(e, "cudaMalloc");
+    laps("allocation");
+    if ((e = cudaMemcpyAsync(bf.raw, triangles, tri_bytes(n_triangles, triangle_stride), cudaMemcpyHostToDevice, stg.st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaStreamSynchronize(stg.st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
+    laps("triangles to the device");
     uint32_t n_nodes = 0;
     int depth = 0;
-    if ((e = bb_build(bf, triangle_stride, n_triangles, n_sm, st, &n_nodes, &depth)) != cudaSuccess) return cu_fail(e, "build");
-    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
-    if (timing) fprintf(stderr, "ct_gpu_build_bvh: %u nodes, %d levels\n", n_nodes, depth);
-    lap("tree built on the device");
+    if ((e = bb_build(bf, triangle_stride, n_triangles, n_sm, stg.st, &n_nodes, &depth)) != cudaSuccess) return cu_fail(e, "build");
+    if ((e = cudaStreamSynchronize(stg.st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
+    if (laps.on) fprintf(stderr, "ct_gpu_build_bvh: %u nodes, %d levels\n", n_nodes, depth);
+    laps("tree built on the device");
     if (n_nodes > (uint32_t)INT32_MAX) return fail(CT_ERR_LIMIT, "%u nodes do not fit the return value", n_nodes);
-    if ((e = cudaMemcpyAsync(nodes, bf.out, (size_t)n_nodes * sizeof(ct_bvh_node), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
-    if ((e = cudaMemcpyAsync(tri_indexes, bf.tri_index, (size_t)n_triangles * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
-    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
-    lap("tree to the host");
+    if ((e = cudaMemcpyAsync(nodes, bf.out, (size_t)n_nodes * sizeof(ct_bvh_node), cudaMemcpyDeviceToHost, stg.st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaMemcpyAsync(tri_indexes, bf.tri_index, (size_t)n_triangles * sizeof(uint32_t), cudaMemcpyDeviceToHost, stg.st)) != cudaSuccess) return cu_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaStreamSynchronize(stg.st)) != cudaSuccess) return cu_fail(e, "cudaStreamSynchronize");
+    laps("tree to the host");
     return (int)n_nodes;
 }
 
 // The scene ct_gpu_upload_scene with CT_FLAG_BUILD_BVH would load from the caller's new triangles, materials and / or lights and the
-// loaded scene's other parts, camera and frame, built by the upload's functions (ct_gpu_update_scene; ct_gpu_update_triangles is
-// what = CT_UPDATE_TRIANGLES).  Everything new is computed into scratch and every allocation it needs is taken first -- a refused or
-// failed build changes nothing; then, after the device has finished the work in flight, it is written over the live state, reusing the
-// allocations where the new records fit.  Everything else the device holds stays.
+// loaded scene's other parts, camera and frame (ct_gpu_update_scene; ct_gpu_update_triangles is what = CT_UPDATE_TRIANGLES): the
+// caller's arrays are checked and staged here, install_scene puts them in place.  Everything else the device holds stays.
 static int update_impl(int device, const ct_scene_update &u, const char *who) {
     if (u.what == 0 || (u.what & ~(uint32_t)(CT_UPDATE_TRIANGLES | CT_UPDATE_MATERIALS | CT_UPDATE_LIGHTS)))
         return fail(CT_ERR_INVALID, "what = %#x: a non-empty mask of CT_UPDATE_TRIANGLES, CT_UPDATE_MATERIALS, CT_UPDATE_LIGHTS", u.what);
@@ -1153,11 +1258,7 @@ static int update_impl(int device, const ct_scene_update &u, const char *who) {
     if (new_tri) TRY(check_device_array(device, u.triangles, 8, "triangles"));
     if (new_mat) TRY(check_device_array(device, u.materials, 4, "materials"));
     if (new_lit && u.n_lights) TRY(check_device_array(device, u.lights, 8, "lights"));
-    const bool timing = getenv("CT_GPU_TIMING") != nullptr;
-    auto now_ms = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
-    const double t_begin = now_ms();
-    double t_mark = t_begin;
-    auto lap = [&](const char *what) { if (timing) { double t = now_ms(); fprintf(stderr, "%s: %-28s %7.2f ms\n", who, what, t - t_mark); t_mark = t; } };
+    Laps laps{who};
     const cudaStream_t st = u.stream ? static_cast<cudaStream_t>(u.stream) : s.stream;
     const uint32_t n_lights = new_lit ? u.n_lights : p.n_lights;
 
@@ -1173,21 +1274,15 @@ static int update_impl(int device, const ct_scene_update &u, const char *who) {
         auto stage = [&]() -> cudaError_t {
             cudaError_t e = cudaSuccess;
             if (new_tri) {
-                const size_t tri_bytes = (size_t)(n - 1) * u.triangle_stride + 72;      // the last triangle may end at its third vertex
-                bb_carve(stg.arena, n, tri_bytes, bf);
-                if ((e = cudaMallocAsync(reinterpret_cast<void **>(&stg.arena.base), stg.arena.used, st)) != cudaSuccess) { stg.arena.base = nullptr; return e; }
-                stg.arena.used = 0;
-                bb_carve(stg.arena, n, tri_bytes, bf);
-                if ((e = cudaMemcpyAsync(bf.raw, u.triangles, tri_bytes, cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
+                if ((e = stg.build_arena(n, u.triangle_stride, bf, st)) != cudaSuccess) return e;
+                if ((e = cudaMemcpyAsync(bf.raw, u.triangles, tri_bytes(n, u.triangle_stride), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
             }
             if (new_mat) {
-                if ((e = cudaMallocAsync(reinterpret_cast<void **>(&mat_in), (size_t)n * sizeof(ct_material), st)) != cudaSuccess) return e;
-                stg.ptrs.push_back(mat_in);
+                if ((e = stg.alloc(&mat_in, n, st)) != cudaSuccess) return e;
                 if ((e = cudaMemcpyAsync(mat_in, u.materials, (size_t)n * sizeof(ct_material), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
             }
             if (new_lit) {
-                if ((e = cudaMallocAsync(reinterpret_cast<void **>(&lit_in), (size_t)std::max<uint32_t>(n_lights, 1) * sizeof(ct_light), st)) != cudaSuccess) return e;
-                stg.ptrs.push_back(lit_in);
+                if ((e = stg.alloc(&lit_in, n_lights, st)) != cudaSuccess) return e;
                 if (n_lights && (e = cudaMemcpyAsync(lit_in, u.lights, (size_t)n_lights * sizeof(ct_light), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
             }
             if ((e = cudaEventRecord(stg.ready, st)) != cudaSuccess) return e;
@@ -1199,129 +1294,13 @@ static int update_impl(int device, const ct_scene_update &u, const char *who) {
     DeviceTree t;
     if (new_tri) {
         TRY(build_device_tree(stg, bf, u.triangle_stride, n, s.n_sm, t));
-        lap("BVH built on the device");
+        laps("BVH built on the device");
         TRY(collapse_wide(stg, t, s.n_sm));
-        lap("wide tree (device)");
+        laps("wide tree (device)");
     }
-    // What the frames derive from the materials and lights: whether any material reflects (the path state's depth), the lights and
-    // the compacted shadow lights (the path state's occlusion words, the any-hit walk's leaf list)
-    bool any_reflective = s.any_reflective;
-    if (new_mat) {
-        uint32_t *flag = nullptr, h = 0;
-        CU(stg.alloc(&flag, 1));
-        CU(cudaMemsetAsync(flag, 0, sizeof *flag, stg.st));
-        k_any_reflective<<<std::max(1, std::min(s.n_sm * 8, (int)((n + 255u) / 256u))), 256, 0, stg.st>>>(mat_in, n, flag);
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(&h, flag, sizeof h, cudaMemcpyDeviceToHost, stg.st));
-        CU(cudaStreamSynchronize(stg.st));
-        any_reflective = h != 0;
-    }
-    DevLight *lit_new = nullptr; DevShadowLight *slit_new = nullptr;
-    uint32_t n_slights = p.n_slights;
-    if (new_lit) {
-        CU(stg.alloc(&lit_new, std::max<uint32_t>(n_lights, 1))); CU(stg.alloc(&slit_new, std::max<uint32_t>(n_lights, 1)));
-        TRY(build_lights(stg, stg.st, lit_in, n_lights, lit_new, slit_new, &n_slights));
-        lap("materials and lights (device)");
-    }
-
-    // The live allocations the new state needs, taken before anything is written: the tree's (hot allocation, pairs64, pair_parent),
-    // the per-triangle and light arrays when the new count is larger, the path state when its depth, occlusion words or parking grow.
-    const bool can_overflow = new_tri ? walks_can_park(p, t.n_nodes, n) : s.can_overflow;
-    const bool grow_tri = n > s.tri_cap, grow_lit = n_lights > s.light_cap;
-    HotLayout hl{};
-    uint32_t pairs = 0;
-    SceneArrays out{};
-    bool fresh_hot = false, fresh_pairs = false, fresh_parent = false;
-    ct_material *mat_fresh = nullptr; DevLight *dl_fresh = nullptr; DevShadowLight *dsl_fresh = nullptr;
-    PathPlan pl;
-    auto take = [&]() -> int {
-        if (new_tri) {
-            hl = hot_layout(t.n_wide, t.n_pairs, n);
-            pairs = std::max<uint32_t>(t.n_pairs, 1);
-            out.hot = hl.bytes <= s.hot_cap ? static_cast<unsigned char *>(s.hot_base) : nullptr;
-            out.pairs64 = pairs <= s.pairs_cap ? const_cast<DevPair64 *>(p.pairs64) : nullptr;
-            out.pair_parent = !can_overflow ? nullptr : pairs <= s.pair_parent_cap ? s.pair_parent_mem : nullptr;
-            out.tri_parent = grow_tri ? nullptr : const_cast<uint32_t *>(p.tri_parent);
-            out.tris = grow_tri ? nullptr : const_cast<DevTri *>(p.tris);
-            fresh_hot = !out.hot; fresh_pairs = !out.pairs64; fresh_parent = can_overflow && !out.pair_parent;
-            if (fresh_hot) TRY(dev_alloc(s, &out.hot, hl.bytes));
-            if (fresh_pairs) TRY(dev_alloc(s, &out.pairs64, pairs));
-            if (fresh_parent) TRY(dev_alloc(s, &out.pair_parent, pairs));
-            if (grow_tri) { TRY(dev_alloc(s, &out.tris, n)); TRY(dev_alloc(s, &out.tri_parent, n)); }
-        }
-        if (grow_tri) TRY(dev_alloc(s, &mat_fresh, n));                    // (a larger count comes with new materials)
-        if (grow_lit) { TRY(dev_alloc(s, &dl_fresh, n_lights)); TRY(dev_alloc(s, &dsl_fresh, n_lights)); }
-        TRY(path_take(s, any_reflective ? p.max_depth + 1 : 1, occ_words_for(n_lights), can_overflow ? parking_cap(p) : 0u, pl));
-        return CT_OK;
-    };
-    auto give_back = [&]() {                                             // the new allocations of a call that fails
-        if (fresh_hot) dev_release(s, out.hot);
-        if (fresh_pairs) dev_release(s, out.pairs64);
-        if (fresh_parent) dev_release(s, out.pair_parent);
-        if (grow_tri && new_tri) { dev_release(s, out.tris); dev_release(s, out.tri_parent); }
-        dev_release(s, mat_fresh); dev_release(s, dl_fresh); dev_release(s, dsl_fresh);
-        path_give_back(s, pl);
-    };
-    int rc = take();
-    if (rc != CT_OK) { give_back(); return rc; }
-    lap("allocation");
-
-    // frames and queries in flight finish on the previous scene (the rule of a re-upload, whose cudaFree waits for the device)
-    {
-        const cudaError_t e = cudaDeviceSynchronize();
-        if (e != cudaSuccess) { give_back(); CU(e); }
-    }
-    // Past this point only a CUDA failure returns early (nothing was written when build_scene_arrays cannot take its scratch).
-    BuildReport rep{};
-    if (new_tri) {
-        rc = build_scene_arrays(stg, stg.st, t, new_mat ? mat_in : p.materials, n, out, s.n_sm, &rep);
-        if (rc != CT_OK) { give_back(); return rc; }
-        lap("scene arrays built on the device");
-    }
-    ct_material *const mats = grow_tri ? mat_fresh : const_cast<ct_material *>(p.materials);
-    DevLight *const dl = grow_lit ? dl_fresh : const_cast<DevLight *>(p.lights);
-    DevShadowLight *const dsl = grow_lit ? dsl_fresh : const_cast<DevShadowLight *>(p.slights);
-    {
-        cudaError_t e = cudaSuccess;
-        if (new_mat) e = cudaMemcpyAsync(mats, mat_in, (size_t)n * sizeof(ct_material), cudaMemcpyDeviceToDevice, stg.st);
-        if (e == cudaSuccess && new_lit && n_lights) e = cudaMemcpyAsync(dl, lit_new, (size_t)n_lights * sizeof(DevLight), cudaMemcpyDeviceToDevice, stg.st);
-        if (e == cudaSuccess && new_lit && n_slights) e = cudaMemcpyAsync(dsl, slit_new, (size_t)n_slights * sizeof(DevShadowLight), cudaMemcpyDeviceToDevice, stg.st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(stg.st);
-        if (e != cudaSuccess) { give_back(); CU(e); }
-    }
-
-    // The new state in place of the old: the replaced allocations go back, the frames' parameters follow.
-    void *const old_hot = s.hot_base;
-    const size_t old_hot_bytes = s.hot_bytes;
-    if (new_tri) {
-        if (fresh_hot) { dev_release(s, s.hot_base); s.hot_cap = hl.bytes; }
-        if (fresh_pairs) { dev_release(s, const_cast<DevPair64 *>(p.pairs64)); s.pairs_cap = pairs; }
-        if (fresh_parent) { dev_release(s, s.pair_parent_mem); s.pair_parent_mem = out.pair_parent; s.pair_parent_cap = pairs; }
-        if (grow_tri) { dev_release(s, const_cast<DevTri *>(p.tris)); dev_release(s, const_cast<uint32_t *>(p.tri_parent)); }
-    }
-    if (grow_tri) { dev_release(s, const_cast<ct_material *>(p.materials)); s.tri_cap = n; }
-    if (grow_lit) { dev_release(s, const_cast<DevLight *>(p.lights)); dev_release(s, const_cast<DevShadowLight *>(p.slights)); s.light_cap = n_lights; }
-    p.materials = mats; p.lights = dl; p.slights = dsl;
-    p.n_tri = n; p.n_lights = n_lights; p.n_slights = n_slights;
-    p.any_leaves = any_leaves_for(s.any_leaves_option, n_slights);
-    s.any_reflective = any_reflective;
-    s.can_overflow = can_overflow;
-    TRY(path_commit(s, pl, stg.st));
-    if (new_tri) {
-        s.leaf_dfs_order = true;                                         // BuildBVH's leaves come in DFS order (bvh.cpp:70-97)
-        set_tree(s, t, out, rep);
-    }
-    lap("previous allocations freed");
-    if (s.hot_base != old_hot || s.hot_bytes != old_hot_bytes) {
-        // the window over the hot records, sized as an upload sizes it, on every stream the frames run on
-        release_l2(s);
-        TRY(apply_l2_policy(s, device, s.own_stream));
-        if (s.stream != s.own_stream) TRY(apply_l2_policy(s, device, s.stream));
-        for (cudaStream_t a : s.aux) TRY(apply_l2_policy(s, device, a));
-        lap("L2 window re-applied");
-    }
-    if (timing) fprintf(stderr, "%s: %u triangles, %u lights, %d levels, L2 window %zu bytes; total %.2f ms\n", who, n, n_lights, s.levels,
-                        s.l2_window, now_ms() - t_begin);
+    TRY(install_scene(s, device, stg, new_tri ? &t : nullptr, mat_in, n, lit_in, n_lights, laps));
+    if (laps.on) fprintf(stderr, "%s: %u triangles, %u lights, %d levels, L2 window %zu bytes; total %.2f ms\n", who, n, n_lights, s.levels,
+                         s.l2_window, Laps::now() - laps.begin);
     return CT_OK;
 }
 
@@ -1464,8 +1443,8 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
     }
     p.fb_out = shared ? s.share_fb : p.fb;
     Params pk = p; pk.max_depth = depth_max;   // with no reflective material the recursion never goes past depth 0 (:369)
-    pk.parent_q_all = s.parent_q_all; pk.hitb_t_all = s.hitb_t_all; pk.occ_all = s.occ_all;
-    pk.reuse_shadow = (g_shadow_reuse && s.parent_q_all) ? 1u : 0u;
+    pk.parent_q_all = s.path.parent_q_all; pk.hitb_t_all = s.path.hitb_t_all; pk.occ_all = s.path.occ_all;
+    pk.reuse_shadow = (g_shadow_reuse && s.path.parent_q_all) ? 1u : 0u;
     cudaStream_t st = s.stream;
     if (shared && !same_frame) {
         if (s.share_cursor == s.cursor_own) CU(cudaMemsetAsync(s.cursor_own + kCursorStride * ((s.shared_frames + 1ull) & 1ull), 0, sizeof(unsigned long long), st));
@@ -1484,9 +1463,7 @@ static int render_impl(int device, int y_start, int y_end, ct_ray_counters *coun
         CU(cudaEventRecord(s.stage_ev[s.n_stages], st));
         return CT_OK;
     };
-    const PathArrays arrays{s.hitb_t_all, s.hitb_pos_all, s.rays_all, s.path_slot_all, s.occ_all, s.parent_q_all, s.far_all,
-                            s.ovf_all, s.ovf_huge_all};
-    TRY(enqueue_stages<false>(s, pk, arrays, count, stages, st, mark, s.launches));
+    TRY(enqueue_stages<false>(s, pk, s.path, count, stages, st, mark, s.launches));
     CU(cudaEventRecord(s.ev1, st));
     CU(cudaEventRecord(s.tile_done[s.tiles_submitted % 8], st));
     s.tiles_submitted++;
